@@ -2,7 +2,21 @@
 """bench.py -- Bellman cell-updates/s of the MDP value-iteration hot path.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+                  [--dump-outputs DIR]
   torchrun ... bench.py --gpus N ...        (N > 1: one rank per GPU, NCCL)
+
+K is the number of timed steps of the headline and of e2e (the syn16k and
+QV-tree sections keep their own fixed counts, so that their checksums and
+medians stay comparable between runs).
+
+--dump-outputs DIR writes, after the timed steps, what they computed in their
+last step (inputs are seeded, so two builds can be compared file for file):
+mdp_cost / mdp_action (the whole grid, gathered to rank 0, at the cells listed
+in mdp_sample_index), mdp_residual, e2e_cost / e2e_action (rank 0's rows as
+the host received them in the last step of the e2e run that downloads J, same
+cells), qv_actions / qv_values (rank 0's queries of the last timed QV batch).
+With --impl reference, each step is then a whole main-arm step (100 sweeps)
+instead of a timing-sized sample, and mdp_sweeps holds the sweep count.
 
 Workload (BASELINE.json configs[2], SURVEY.md section 8d): synthetic 4096 x
 4096 grid per GPU, i.i.d. 20 % occupied (numpy PCG64 seed 12345), goal at the
@@ -37,6 +51,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 TILE = 4096
 SWEEPS_PER_STEP = 100
 ALGO_BYTES_PER_CELL_UPDATE = 10   # SURVEY.md section 8d
+DUMP_CELLS = 1 << 20              # --dump-outputs: cells sampled per grid (~24 MB written)
 METRIC = "bellman_cell_updates_per_sec"
 UNIT = "cell-updates/s"
 
@@ -114,6 +129,18 @@ def make_grid(n_tiles):
     return grid, goal
 
 
+def dump_sample(cells):
+    """The cells --dump-outputs keeps: a fixed, seeded sample, sorted."""
+    return np.sort(np.random.default_rng(0).choice(cells, min(cells, DUMP_CELLS),
+                                                   replace=False))
+
+
+def write_dump(directory, arrays):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 # --------------------------------------------------------------------------
 def host_cores():
     return len(os.sched_getaffinity(0))
@@ -172,12 +199,22 @@ def run_reference_arm(args):
     per = time.perf_counter() - t0
     total_steps = max(1, args.steps + args.warmup)
     sweeps_per_step = max(1, min(SWEEPS_PER_STEP, int(100.0 / total_steps / max(per, 1e-6))))
+    if args.dump_outputs:
+        # the dumped solution must not depend on a timing: whole main-arm steps
+        sweeps_per_step = SWEEPS_PER_STEP
     for _ in range(args.warmup):
         ora.sweeps(sweeps_per_step)
     t0 = time.perf_counter()
     for _ in range(args.steps):
         ora.sweeps(sweeps_per_step)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        sample = dump_sample(grid.size)
+        write_dump(args.dump_outputs, {
+            "mdp_sample_index": sample.astype(np.float64),
+            "mdp_cost": ora.cost.reshape(-1)[sample].astype(np.float32),
+            "mdp_action": ora.act.reshape(-1)[sample].astype(np.float32),
+            "mdp_sweeps": np.array([ora.n], np.float64)})
     value = grid.size * sweeps_per_step * args.steps / dt
     sample_txt = (f"each step = {sweeps_per_step} of the 100 sweeps of a main-arm step, on the "
                   f"whole {TILE}x{TILE} per-GPU grid with the main arm's goal {goal}; "
@@ -284,9 +321,10 @@ def syn16k_section(rank, world, barrier, steps=5):
             * ALGO_BYTES_PER_CELL_UPDATE / 1e9 / world}
 
 
-def qv_tree_section(rank, world, with_cpu):
+def qv_tree_section(rank, world, with_cpu, dump=None):
     """BASELINE.json configs[4]: batched QV-Tree Search, 1250 queries per GPU
-    (10 000 on 8 GPUs), sharded independently, no collective on the data path."""
+    (10 000 on 8 GPUs), sharded independently, no collective on the data path.
+    dump: dict that receives this rank's actions and values of the last batch."""
     import torch
     import torch.distributed as dist
     import cases
@@ -325,6 +363,9 @@ def qv_tree_section(rank, world, with_cpu):
             w1 = p.work_counters()
         dt = torch.tensor([sorted(times)[1]], dtype=torch.float64, device="cuda")
         p_live = p.live_cells()
+    if dump is not None:
+        dump["qv_actions"] = np.asarray(acts, np.float32)
+        dump["qv_values"] = np.asarray(vals, np.float32)
     if world > 1:
         dist.all_reduce(dt, op=dist.ReduceOp.MAX)
     dt = float(dt.item())
@@ -513,6 +554,19 @@ def run_main_arm(args):
         except Exception:
             pass
 
+    # what the timed steps computed: the whole J and action grid after the last
+    # step, sampled at fixed cells (the same cells for every run of a grid size)
+    dump = None
+    if args.dump_outputs:
+        dump = {}
+        cost, action = vi.gather()
+        sample = dump_sample(cells)
+        if rank == 0:
+            dump["mdp_sample_index"] = sample.astype(np.float64)
+            dump["mdp_cost"] = cost.reshape(-1)[sample].astype(np.float32)
+            dump["mdp_action"] = action.reshape(-1)[sample].astype(np.float32)
+            dump["mdp_residual"] = np.array([residual], np.float32)
+
     # e2e: public API, host buffers, copies inside the timed region
     p2p_used = vi.p2p
     vi.close()
@@ -559,7 +613,7 @@ def run_main_arm(args):
     e2e_step(0)
     mdp_handle.download_wait()
     first = (cost_host[0].clone(), act_host[0].clone())
-    e2e_steps = max(2, min(args.steps, 20))   # (the drain of the last download is inside the timed region)
+    e2e_steps = args.steps   # (the drain of the last download is inside the timed region)
 
     def e2e_run(with_cost):
         barrier()
@@ -572,7 +626,7 @@ def run_main_arm(args):
         if world > 1:
             dist.all_reduce(sec, op=dist.ReduceOp.MAX)
         # every step solved the same problem: all downloads must hold the same bits
-        for k in range(2):
+        for k in range(min(2, e2e_steps)):
             if not ((not with_cost or
                      torch.equal(cost_host[k].view(torch.int32), first[0].view(torch.int32)))
                     and torch.equal(act_host[k], first[1])):
@@ -580,6 +634,12 @@ def run_main_arm(args):
         return cells * SWEEPS_PER_STEP * e2e_steps / float(sec.item())
 
     e2e_val = e2e_run(True)
+    if dump is not None and rank == 0:
+        # this rank's rows as the host received them in the last step
+        own = sample[sample < n_own]
+        last = (e2e_steps - 1) % 2
+        dump["e2e_cost"] = cost_host[last].numpy()[own].astype(np.float32)
+        dump["e2e_action"] = act_host[last].numpy()[own].astype(np.float32)
     if trace is not None:
         print(f"rank {rank} e2e ms per phase [reset, enqueue sweeps, residual, download_wait, "
               f"download_begin]: {trace[1:]}", file=sys.stderr)
@@ -655,12 +715,15 @@ def run_main_arm(args):
     if rank == 0 and syn16k:
         line["syn16k"] = syn16k
     try:
-        qv = None if args.no_qv else qv_tree_section(rank, world, world == 1 and not args.no_cpu)
+        qv = None if args.no_qv else qv_tree_section(rank, world, world == 1 and not args.no_cpu,
+                                                       dump)
     except Exception as e:  # pragma: no cover
         qv = {"error": repr(e)}
     if rank == 0:
         if qv:
             line["qv_tree"] = qv
+        if dump is not None:
+            write_dump(args.dump_outputs, dump)
         args.emit(json.dumps(line))
     if world > 1:
         dist.barrier()
@@ -709,7 +772,13 @@ def main():
                          "staging it under the previous solve (A/B)")
     ap.add_argument("--no-ref-cuda", action="store_true",
                     help="skip the reference-kernels-on-this-GPU line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what they computed as DIR/<name>.npy "
+                         "(float32, J and action at a fixed sample of 2^20 cells, sample "
+                         "indices as float64), for comparing two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     with StdoutGuard() as out:
         args.emit = out.emit
         if args.impl == "reference":

@@ -30,10 +30,25 @@
   python tests/golden/make_golden.py tree [outdir]
       (GPU box)  The reference's own QV-tree host code (SearchTree, VNode,
       QNode, evaluateFibCpu, evaluatePbviCpu) -> tree_<case>.npz.
+
+  python tests/golden/make_golden.py live_cases [outdir]
+      Records of the cases that only the live reference tests used to run,
+      so that a checkout without oracle/_ref still compares against them:
+      ref_rand_512x384.npz (test_reference_pin_gpu random_512),
+      bench_ref_<h>x<w>.npz (test_mdp_gpu, the benchmarked sizes solved to
+      convergence: sweeps, residuals, CRC-32 of every J and action row),
+      kernels_ref_syn_23x31.npz (test_pomdp_gpu: model tables, Bayes updates,
+      FIB) and, where a GPU is present, pbvi_ref_map_5x5_g0.7_n25.npz
+      (test_pbvi_gpu).  They are computed without the reference: by the CPU
+      restatements (oracle/) and, for PBVI, by the library with its cuBLAS
+      checker.  With these library and oracle sources the live tests passed
+      against the reference on a B200 on exactly these inputs, asserting
+      bit-for-bit equality, so the records hold the reference's bits.
 """
 import ctypes
 import os
 import sys
+import zlib
 
 import numpy as np
 
@@ -231,8 +246,86 @@ def make_tree(outdir, only=None):
                        check=True)
 
 
+# the benchmarked grids of test_mdp_gpu: (rows, cols), goal; synthetic, 20 %, seed 12345
+BENCH_SIZES = [((4096, 4096), (2048, 2048)), ((1536, 16384), (8192, 700))]
+
+
+def crc_rows(a):
+    """CRC-32 of every row's bytes."""
+    a = np.ascontiguousarray(a)
+    return np.array([zlib.crc32(r.tobytes()) for r in a], np.uint32)
+
+
+def pomdp_live_case():
+    """Inputs of test_pomdp_gpu's live kernel pin: grid, goal, belief, actions,
+    observations, FIB sweep cap."""
+    grid, goal = cases.synthetic_map(23, 31, 0.3, seed=4)
+    b = (np.random.default_rng(0).random(grid.size, dtype=np.float32) ** 18
+         * 1e-30).astype(np.float32)
+    us = np.arange(9, dtype=np.uint8)
+    zs = (np.arange(9) * 7 % 16).astype(np.uint8)
+    return grid, goal, b, us, zs, 30
+
+
+def make_live_cases(outdir):
+    import oracle_py
+    import pomdp_oracle_py as po
+    os.makedirs(outdir, exist_ok=True)
+    grid, goal = cases.synthetic_map(512, 384, 0.2, seed=99)
+    J, A, n, res = oracle_py.value_iteration(grid, goal, cases.GAMMA, 1)
+    np.savez_compressed(os.path.join(outdir, "ref_rand_512x384.npz"), grid=grid,
+                        goal=np.array(goal), gamma=np.float32(cases.GAMMA), J=J, action=A,
+                        sweeps=np.int32(n), residuals=res)
+    print("rand_512x384 sweeps", n)
+    grid, goal, b, us, zs, cap = pomdp_live_case()
+    m = po.Model(grid, goal)
+    fib, n_fib = m.fib(cases.GAMMA, cap)
+    np.savez_compressed(os.path.join(outdir, "kernels_ref_syn_23x31.npz"),
+                        trans_prob=m.tp, meas_prob=m.mp, stage_reward=m.sr,
+                        bayes=np.stack([m.bayes(b, int(u), int(z))[0] for u, z in zip(us, zs)]),
+                        fib=np.ascontiguousarray(fib).reshape(-1), fib_sweeps=np.int32(n_fib))
+    print("syn_23x31 fib sweeps", n_fib)
+    for (h, w), goal in BENCH_SIZES:
+        grid, goal = cases.synthetic_map(h, w, 0.20, seed=12345, goal=goal)
+        J, A, n, res = oracle_py.value_iteration(grid, goal, cases.GAMMA)
+        np.savez_compressed(os.path.join(outdir, f"bench_ref_{h}x{w}.npz"),
+                            goal=np.array(goal), sweeps=np.int32(n), residuals=res,
+                            J_crc=crc_rows(J.view(np.uint32)), action_crc=crc_rows(A))
+        print(f"bench {h}x{w} sweeps", n, "residuals", res[-2:])
+    try:
+        import torch
+        gpu = torch.cuda.is_available()
+    except ImportError:
+        gpu = False
+    if gpu:
+        make_pbvi_5x5(outdir)
+
+
+def make_pbvi_5x5(outdir):
+    """pbvi_ref_*.npz layout of tools/ref_offline.py for map_5x5, goal (3, 2),
+    gamma 0.7, 25 beliefs, rand_seed 1: the library with its cuBLAS checker."""
+    os.environ["PP2D_PBVI_CUBLAS"] = "1"
+    sys.path.insert(0, ROOT)
+    from path_planning_2d_b200 import PomdpPathPlanning2d
+    grid, goal, gamma, n = cases.load_bundled("map_5x5"), (3, 2), 0.7, 25
+    free = 1.0 - grid.astype(np.float32).reshape(-1)
+    s = np.float32(0)
+    for v in free:                    # src/pomdp/path_planning_2d.cu:100-107
+        s = np.float32(s + v)
+    b0 = (free / s).astype(np.float32)
+    with PomdpPathPlanning2d(grid, goal, gamma) as p:
+        fib, fa, _ = p.fastInformedBound()
+        bs, al, ac = p.pointBasedValueIteration(b0, n, rand_seed=1)
+    np.savez_compressed(os.path.join(outdir, "pbvi_ref_map_5x5_g0.7_n25.npz"), grid=grid,
+                        goal=np.array(goal), gamma=np.float32(gamma), b0=b0, fib=fib,
+                        fib_actions=fa, belief_set=bs, pbvi=al, pbvi_actions=ac)
+    print("pbvi map_5x5", bs.shape)
+
+
 if __name__ == "__main__":
-    if len(sys.argv) >= 2 and sys.argv[1] == "pi":
+    if len(sys.argv) >= 2 and sys.argv[1] == "live_cases":
+        make_live_cases(sys.argv[2] if len(sys.argv) > 2 else HERE)
+    elif len(sys.argv) >= 2 and sys.argv[1] == "pi":
         make_pi(sys.argv[2] if len(sys.argv) > 2 else
                 os.path.join(ROOT, "gpurun_out", "golden_ref"))
     elif len(sys.argv) >= 2 and sys.argv[1] == "tree":

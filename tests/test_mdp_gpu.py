@@ -309,6 +309,27 @@ def test_benchmarked_sizes_to_convergence_vs_the_reference_kernels(shape, goal):
     assert n >= 300 and res[-1] <= 5.0 / (1.0 - np.float32(cases.GAMMA)) * 1e-3 < res[-2]
 
 
+@pytest.mark.parametrize("shape,goal", [((4096, 4096), (2048, 2048)),
+                                        ((1536, 16384), (8192, 700))])
+def test_benchmarked_sizes_to_convergence_vs_the_reference_record(shape, goal):
+    """The comparison above against its stored record (tests/golden/
+    bench_ref_<h>x<w>.npz): same number of sweeps, same residuals, and the
+    CRC-32 of every J row (bits) and action row."""
+    import sys
+    sys.path.insert(0, cases.GOLDEN)
+    import make_golden
+    h, w = shape
+    g = np.load(os.path.join(cases.GOLDEN, f"bench_ref_{h}x{w}.npz"))
+    grid, goal = cases.synthetic_map(h, w, 0.20, seed=12345, goal=goal)
+    assert tuple(int(v) for v in g["goal"]) == goal
+    with MdpPathPlanning2d(grid, goal, cases.GAMMA) as mdp:
+        sweeps, residuals = mdp.initialize()
+        assert sweeps == int(g["sweeps"])
+        assert np.array_equal(residuals, g["residuals"])
+        assert np.array_equal(make_golden.crc_rows(_bits(mdp.optimal_cost)), g["J_crc"])
+        assert np.array_equal(make_golden.crc_rows(mdp.optimal_action), g["action_crc"])
+
+
 def test_full_size_16384_row_shards_equal_the_unsharded_grid():
     """BASELINE.json configs[3] size (16384 x 16384, 2.7e8 cells) on one GPU:
     8 row shards of 2048 rows with ghost-row exchange after every launch must

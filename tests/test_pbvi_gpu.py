@@ -22,7 +22,9 @@ decision over its 167 iterations.  Therefore:
 tests/golden/pbvi_ref_*.npz are outputs of generateBeliefSet /
 backupAlphaVectors / fastInformedBound of the unmodified reference
 translation units (oracle/_ref/libpp2d_ref_pomdp_full.so) run on a B200 by
-tools/ref_offline.py, rand() seeded like a fresh process.  The bundled-map
+tools/ref_offline.py, rand() seeded like a fresh process; map_5x5 (the case of
+the live test below) is its record in the same layout, `make_golden.py
+live_cases`.  The bundled-map
 case (500 beliefs x 4000 cells, 167 backups; 165 s + 228 s in the reference)
 is stored as one CRC-32 per belief / alpha vector.  Bar: bit-exact."""
 import os
@@ -39,7 +41,7 @@ from path_planning_2d_b200 import PomdpPathPlanning2d
 pytestmark = pytest.mark.gpu
 bits = lambda a: np.ascontiguousarray(a, np.float32).view(np.uint32)
 SMALL = ["pbvi_ref_map_3x3_g0.5_n12", "pbvi_ref_map_10x10_g0.8_n40",
-         "pbvi_ref_map_10x10_g0.95_n60"]
+         "pbvi_ref_map_10x10_g0.95_n60", "pbvi_ref_map_5x5_g0.7_n25"]
 
 
 def crc_rows(rows):

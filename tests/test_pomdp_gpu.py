@@ -349,6 +349,27 @@ def test_reference_pomdp_kernels_vs_restatement():
     assert n == on and np.array_equal(bits(fib), bits(ofib.reshape(-1)))
 
 
+def test_pomdp_kernels_equal_the_reference_record():
+    """The case of the live pin above, against its stored record
+    (tests/golden/kernels_ref_syn_23x31.npz): the product's model tables,
+    unnormalised Bayes updates and capped FIB solve, bit for bit."""
+    import sys
+    sys.path.insert(0, cases.GOLDEN)
+    import make_golden
+    g = np.load(os.path.join(cases.GOLDEN, "kernels_ref_syn_23x31.npz"))
+    grid, goal, b, us, zs, cap = make_golden.pomdp_live_case()
+    with PomdpPathPlanning2d(grid, goal, cases.GAMMA) as p:
+        tp, mp, sr = p.model_tables()
+        assert np.array_equal(bits(tp).reshape(-1), bits(g["trans_prob"]))
+        assert np.array_equal(bits(mp).reshape(-1), bits(g["meas_prob"]))
+        assert np.array_equal(bits(sr).reshape(-1), bits(g["stage_reward"]))
+        out = p.bayes_update(np.stack([b] * len(us)), us, zs)
+        assert np.array_equal(bits(out), bits(g["bayes"]))
+        fib, _, n = p.fastInformedBound(cap)
+    assert n == int(g["fib_sweeps"])
+    assert np.array_equal(bits(fib).reshape(-1), bits(g["fib"]))
+
+
 @pytest.mark.parametrize("name,goal", [("map_10x10", (8, 7)), ("sparse_map_100x40", (95, 34))])
 def test_fib_solver_bit_exact(name, goal):
     """"next" row 1: the FIB offline solver, same sweeps and bits as the

@@ -100,6 +100,25 @@ def test_oracle_matches_reference_kernels(path):
             assert z == g["obs"][a, k], (a, k)
 
 
+def test_oracle_matches_reference_record_of_the_live_kernel_case():
+    """tests/golden/kernels_ref_syn_23x31.npz: the case of test_pomdp_gpu's
+    live pin against the reference kernels -- tables, Bayes updates, FIB."""
+    import sys
+    sys.path.insert(0, cases.GOLDEN)
+    import make_golden
+    g = np.load(os.path.join(cases.GOLDEN, "kernels_ref_syn_23x31.npz"))
+    grid, goal, b, us, zs, cap = make_golden.pomdp_live_case()
+    m = po.Model(grid, goal)
+    bits = lambda a: np.ascontiguousarray(a, np.float32).view(np.uint32).reshape(-1)
+    assert np.array_equal(bits(m.tp), bits(g["trans_prob"]))
+    assert np.array_equal(bits(m.mp), bits(g["meas_prob"]))
+    assert np.array_equal(bits(m.sr), bits(g["stage_reward"]))
+    for i, (u, z) in enumerate(zip(us, zs)):
+        assert np.array_equal(bits(m.bayes(b, int(u), int(z))[0]), bits(g["bayes"][i])), i
+    fib, n = m.fib(cases.GAMMA, cap)
+    assert n == int(g["fib_sweeps"]) and np.array_equal(bits(fib), bits(g["fib"]))
+
+
 def test_tree_runs_and_is_deterministic():
     import pomdp_fixtures as pf
     grid = cases.load_bundled("map_10x10")

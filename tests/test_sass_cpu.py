@@ -25,11 +25,15 @@ def mangled(t, cw, policy, p2p, lin):
 
 @pytest.fixture(scope="module")
 def sass():
-    if shutil.which("cuobjdump") is None:
-        pytest.skip("cuobjdump not on PATH")
+    from path_planning_2d_b200 import build
+    # the toolkit that built the library also has cuobjdump, on PATH or not
+    cuobjdump = (shutil.which("cuobjdump")
+                 or os.path.join(os.path.dirname(build.NVCC), "cuobjdump"))
+    if not os.path.exists(cuobjdump):
+        pytest.skip("cuobjdump not found")
     out = {}
     for key in FUSED:
-        txt = subprocess.run(["cuobjdump", "-sass", "-fun", mangled(*key), LIB],
+        txt = subprocess.run([cuobjdump, "-sass", "-fun", mangled(*key), LIB],
                              capture_output=True, text=True).stdout
         ins = re.findall(r"^\s+/\*[0-9a-f]{4,}\*/\s+(.*?);", txt, flags=re.M)
         assert len(ins) > 500, f"kernel {key} not found in {LIB}"
