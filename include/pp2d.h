@@ -233,6 +233,17 @@ int pp2d_mdp_waypoints(pp2d_mdp* h, uint32_t start_x, uint32_t start_y,
 uint32_t pp2d_mdp_sweep_count(const pp2d_mdp* h);
 
 /*
+ * Work of the fused two-sweep row-block launches so far (cumulative, counted
+ * on the device; summed over the devices of a multi-GPU handle):
+ * out[0] = units run, out[1] = units launched.  A unit whose 3x3 unit
+ * neighbourhood did not change in the previous launch is skipped: its output
+ * is already in the buffer the launch writes (DESIGN.md section 4).
+ * PP2D_MDP_SKIP=0 at handle creation turns skipping off (then out[0] ==
+ * out[1]).  Measurement only, no reference counterpart.
+ */
+int pp2d_mdp_work_counters(pp2d_mdp* h, uint64_t out[2]);
+
+/*
  * Ghost-row exchange for shards.  depth = 2 rows.  After any
  * pp2d_mdp_sweeps call the caller copies `bytes` bytes
  *   from this rank's send_top  to the upper neighbour's recv_bottom,

@@ -14,6 +14,7 @@
 // CUDA failures keep the reference's print-and-exit behaviour
 // (helper_cuda.h:984-999) through PP2D_CHECK.
 #pragma once
+#include <array>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -160,6 +161,13 @@ class MdpPathPlanning2d : public PathPlanning2dBase {
     PP2D_CHECK(pp2d_mdp_waypoints(mdp_, sx, sy, cells.data(), (uint32_t)cells.size(), &n));
     cells.resize(n);
     return cells;
+  }
+
+  // Units run / launched by the fused sweeps so far (pp2d_mdp_work_counters).
+  std::array<uint64_t, 2> workCounters() {
+    std::array<uint64_t, 2> c{};
+    PP2D_CHECK(pp2d_mdp_work_counters(mdp_, c.data()));
+    return c;
   }
 
   std::vector<float> optimal_cost;

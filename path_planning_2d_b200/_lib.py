@@ -57,6 +57,7 @@ SIGNATURES = {
     "pp2d_mdp_waypoints": (_i, [_vp, _u32, _u32, _vp, _u32,
                                 ctypes.POINTER(_u32)]),
     "pp2d_mdp_sweep_count": (_u32, [_vp]),
+    "pp2d_mdp_work_counters": (_i, [_vp, _vp]),
     "pp2d_mdp_halo": (_i, [_vp, ctypes.POINTER(Halo)]),
     "pp2d_mdp_ipc_export": (_i, [_vp, _vp]),
     "pp2d_mdp_ipc_connect": (_i, [_vp, _vp, _vp]),

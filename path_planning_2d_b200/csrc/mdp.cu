@@ -183,6 +183,18 @@ struct pp2d_mdp {
   // reset; occupied cells then follow J_n = (gamma*J_{n-1}) + 2
   bool pi_mode = false;
   std::vector<float> trapped_pi;
+  // skipping of units whose two-sweep input is unchanged (PP2D_MDP_SKIP,
+  // DESIGN.md section 4): three rotating unit masks of the fused row-block
+  // launches.  need_valid: the mask the next such launch reads was written by
+  // the launch right before it, on the same geometry; otherwise it runs every
+  // unit.
+  bool skip = true;
+  uint32_t* need[3] = {nullptr, nullptr, nullptr};
+  int need_words = 0, need_rot = 0;
+  int need_units = 0, need_rows_per_unit = 0;
+  bool need_valid = false;
+  unsigned long long* work = nullptr;   // [0] units run, [1] units launched
+  uint32_t* need_alloc = nullptr;
   int device = 0;                  // CUDA device the buffers live on
   bool owns_stream = false;
   // launch geometry cache (the occupancy query and the count of boundary units
@@ -458,6 +470,41 @@ static int launch_sweep(pp2d_mdp* h) {
   lc.lin_len = p.lin_len;
   lc.rows_per_unit = p.rows_per_unit;
   lc.n_units = p.n_units;
+  // Unit skipping: fused row-block launches only (not the strip-major runs,
+  // not the peer-to-peer kernels); units of at least 2 rows, so that the 2-row
+  // dependency cone of a unit lies inside its 3x3 unit neighbourhood.
+  bool book = false;
+  if constexpr (T == 2 && CW == 2 && !P2P) {
+    p.work = h->work;
+    book = h->skip && p.lin_len == 0 && p.rows_per_unit >= 2;
+  }
+  if (book) {
+    const int words = (p.n_units + 31) / 32;
+    if (p.n_units != h->need_units || p.rows_per_unit != h->need_rows_per_unit) {
+      if (words > h->need_words) {
+        cudaFree(h->need_alloc);
+        h->need_alloc = nullptr;
+        h->need_words = 0;
+        PP2D_CUDA(cudaMalloc(&h->need_alloc, 3 * (size_t)words * sizeof(uint32_t)));
+        h->need_words = words;
+      }
+      // (stream-ordered: a previous launch may still read the old masks)
+      PP2D_CUDA(cudaMemsetAsync(h->need_alloc, 0, 3 * (size_t)h->need_words * sizeof(uint32_t),
+                                h->stream));
+      for (int i = 0; i < 3; ++i) h->need[i] = h->need_alloc + (size_t)i * h->need_words;
+      h->need_units = p.n_units;
+      h->need_rows_per_unit = p.rows_per_unit;
+      h->need_rot = 0;
+      h->need_valid = false;
+    }
+    p.need_in = h->need[h->need_rot];
+    p.need_out = h->need[(h->need_rot + 1) % 3];
+    p.need_clear = h->need[(h->need_rot + 2) % 3];
+    // The arg-min launch runs every unit: the action grid is always complete.
+    p.all_live = (POLICY || !h->need_valid) ? 1 : 0;
+    // ghost rows of a shard with neighbours change under the row blocks next to them
+    p.edge_live = (h->sharded && (h->row_begin > 0 || h->row_begin + h->H < h->Htot)) ? 1 : 0;
+  }
   const int warps_per_cta = kWarpsPerCta;
   const int grid = (p.n_units + warps_per_cta - 1) / warps_per_cta;
   // Fused launches follow each other back to back: with programmatic dependent
@@ -485,6 +532,9 @@ static int launch_sweep(pp2d_mdp* h) {
   PP2D_CUDA(cudaGetLastError());
   h->cur ^= 1;
   h->n_sweeps += T;
+  // Any other launch changes J without change bits: the next one runs all.
+  if (book) h->need_rot = (h->need_rot + 1) % 3;
+  h->need_valid = book;
   return PP2D_OK;
 }
 
@@ -562,6 +612,7 @@ static int upload_map(pp2d_mdp* h, const uint8_t* map) {
   h->n_sweeps = h->n_chk = h->action_sweep = 0;
   h->action_host_valid = false;
   h->pi_mode = false;
+  h->need_valid = false;
   return PP2D_OK;
 }
 
@@ -615,6 +666,7 @@ static int create_impl(uint32_t height, uint32_t width, const uint8_t* map,
   h->fused_policy = env_int("PP2D_MDP_FUSED_POLICY", 1) != 0;
   h->linear_units = env_int("PP2D_MDP_LINEAR_UNITS", -1);
   h->pdl = env_int("PP2D_MDP_PDL", 1) != 0;
+  h->skip = env_int("PP2D_MDP_SKIP", 1) != 0;
   h->rows_per_unit = env_int("PP2D_MDP_ROWS_PER_UNIT", 0);
   h->prefetch_rows = env_int("PP2D_MDP_PREFETCH_ROWS", 6);
   h->waves = env_int("PP2D_MDP_WAVES", 1);
@@ -645,6 +697,8 @@ static int create_impl(uint32_t height, uint32_t width, const uint8_t* map,
     PP2D_CUDA(cudaMalloc(&h->resid, sizeof(uint32_t)));
     PP2D_CUDA(cudaMalloc(&h->flags, kFlagWords * sizeof(unsigned int)));
     PP2D_CUDA(cudaMemset(h->flags, 0, kFlagWords * sizeof(unsigned int)));
+    PP2D_CUDA(cudaMalloc(&h->work, 2 * sizeof(unsigned long long)));
+    PP2D_CUDA(cudaMemset(h->work, 0, 2 * sizeof(unsigned long long)));
     PP2D_CUDA(cudaMallocHost(&h->resid_host, sizeof(uint32_t)));
     std::vector<float4> lut;
     build_lut(gamma, lut);
@@ -991,6 +1045,8 @@ void pp2d_mdp_destroy(pp2d_mdp* h) {
   cudaFree(h->resid);
   for (void* q : h->ipc_opened) if (q) cudaIpcCloseMemHandle(q);
   cudaFree(h->flags);
+  cudaFree(h->work);
+  cudaFree(h->need_alloc);
   if (h->resid_host) cudaFreeHost(h->resid_host);
   delete h;
 }
@@ -1060,6 +1116,28 @@ int pp2d_mdp_sweeps(pp2d_mdp* h, uint32_t n) {
 }
 
 uint32_t pp2d_mdp_sweep_count(const pp2d_mdp* h) { return h ? h->n_sweeps : 0; }
+
+int pp2d_mdp_work_counters(pp2d_mdp* h, uint64_t out[2]) {
+  if (!h || !out) return fail(PP2D_ERR_INVALID, "NULL argument");
+  out[0] = out[1] = 0;
+  if (!h->parts.empty()) {
+    DeviceGuard guard;
+    for (pp2d_mdp* part : h->parts) {
+      uint64_t c[2];
+      PP2D_TRY_MDP(multi_set_device(part));
+      PP2D_TRY_MDP(pp2d_mdp_work_counters(part, c));
+      out[0] += c[0];
+      out[1] += c[1];
+    }
+    return PP2D_OK;
+  }
+  unsigned long long c[2] = {0, 0};
+  PP2D_CUDA(cudaMemcpyAsync(c, h->work, sizeof(c), cudaMemcpyDeviceToHost, h->stream));
+  PP2D_CUDA(cudaStreamSynchronize(h->stream));
+  out[0] = c[0];
+  out[1] = c[1];
+  return PP2D_OK;
+}
 
 int pp2d_mdp_residual_device(pp2d_mdp* h, void** dev_float_out) {
   if (!h) return fail(PP2D_ERR_INVALID, "handle is NULL");
@@ -1146,6 +1224,7 @@ int pp2d_mdp_policy_iteration(pp2d_mdp* h, uint32_t* evaluation_sweeps, double* 
     return fail(PP2D_ERR_STATE, "pp2d_mdp_policy_iteration starts from J = 0, action = 0: "
                                 "call pp2d_mdp_reset first");
   h->pi_mode = true;
+  h->need_valid = false;
   const size_t owned = (size_t)h->H * h->W;
   PolicyParams p;
   p.code = h->code; p.action = h->action;

@@ -148,7 +148,23 @@ struct SweepParams {
   // neighbours (see publish_flags), -1: the last boundary unit to finish its
   // edge rows does it itself.
   int publisher_unit;
+  // --- skipping of unchanged units (fused row-block kernels, DESIGN.md 4) ---
+  // need_out == NULL: every unit runs on its own warp, no bookkeeping.
+  // Otherwise bit u of need_in says unit u must run; a unit whose output
+  // differs from its input sets the bits of its 3x3 unit neighbourhood in
+  // need_out (the mask of the next launch), and need_clear (the mask of the
+  // launch after that) is cleared.
+  const uint32_t* need_in;
+  uint32_t* need_out;
+  uint32_t* need_clear;
+  unsigned long long* work;  // [0] += units run, [1] += units of the launch (may be NULL)
+  int all_live;              // need_in is not read: every unit runs
+  int edge_live;             // the row blocks next to the ghost rows of a shard always run
 };
+
+// Shortest row segment a live unit is split into when few units are live:
+// every segment pays 2 priming steps of the T = 2 march.
+constexpr int kMinSegRows = 8;
 
 // Flag block of a shard (uint32 each, cudaMalloc'ed, IPC-shared).
 constexpr int kFlagFromUp = 0;     // written by the up neighbour: its launch #
@@ -462,6 +478,10 @@ struct Sweeper {
   using G = StripGeom<T, CW>;
   // bulk-copy ring: the fused row-block kernel only (one march per warp)
   static constexpr bool kTma = PP2D_TMA && T == 2 && CW == 2 && !P2P && !LIN;
+  // the instantiations that can skip units: they OR the bit difference between
+  // J^2 and J^0 of every produced cell into `diff`
+  static constexpr bool kSkip = T == 2 && CW == 2 && !P2P && !LIN;
+  uint32_t diff = 0;
   uint32_t ring_base = 0;    // kTma: shared address of this warp's ring (slot 0)
   int lane_id = 0;
   float A[3][CW + 2];        // J^0 rows y-1, y, y+1 (rotating)
@@ -584,6 +604,13 @@ struct Sweeper {
                                  act2[j]);
         }
         if (valid) store_own<CW>(pout, v2);
+        if constexpr (kSkip) {
+          // J^0 of row y-1 is still in the window: one LOP3 per cell
+#pragma unroll
+          for (int j = 0; j < CW; ++j)
+            asm("lop3.b32 %0, %1, %2, %0, 0xBE;"      // (a ^ b) | diff
+                : "+r"(diff) : "r"(__float_as_uint(v2[j])), "r"(__float_as_uint(A[a0][j + 1])));
+        }
         if constexpr (POLICY) {
           // (single predicated stores: no divergent region inside the marching loop)
 #pragma unroll
@@ -913,6 +940,85 @@ __device__ __forceinline__ void publish_flags(const SweepParams& p, int lane) {
   }
 }
 
+// Bits of word i of a unit mask that stand for the units [lo, hi).
+__device__ __forceinline__ uint32_t unit_range_bits(int i, int lo, int hi) {
+  const int a = min(max(lo - 32 * i, 0), 32), b = min(max(hi - 32 * i, 0), 32);
+  const uint32_t m = b - a >= 32 ? 0xffffffffu : (1u << max(b - a, 0)) - 1u;
+  return m << (a & 31);
+}
+
+// Word i of the units this launch must run.
+__device__ __forceinline__ uint32_t need_word(const SweepParams& p, int i, int n_words) {
+  if (i >= n_words) return 0u;
+  uint32_t m = p.need_in[i];
+  if (p.edge_live) {
+    // every row block with a row whose 2-row cone reaches a ghost row: rows
+    // 0, 1 (block 0, blocks have >= 2 rows) and rows H-2, H-1 (the last block,
+    // and the one before it when the last block has 1 row)
+    const int rb_bot = max(0, (p.y_end - p.y_begin - 2) / p.rows_per_unit);
+    m |= unit_range_bits(i, 0, p.n_strips) |
+         unit_range_bits(i, rb_bot * p.n_strips, p.n_units);
+  }
+  return m;
+}
+
+// Work of warp w of a fused row-block launch: unit `unit`, rows [y0, y1).
+// Without bookkeeping (need_out == NULL) warp w runs unit w, as it always
+// did.  Otherwise the n_live units that must run share the launch's warps:
+// s = max(1, warps / n_live) warps per live unit, warp w takes live unit w / s
+// and row segment w % s of it (segments of at least kMinSegRows rows).  Every
+// lane computes the same values (lane-0 shuffles and ballots): the march that
+// follows stays warp-uniform.  Returns false when the warp has nothing to do.
+__device__ __forceinline__ bool unit_plan(const SweepParams& p, int w, int lane, int& unit,
+                                          int& y0, int& y1) {
+  const bool book = p.need_out != nullptr;
+  const int n_words = (p.n_units + 31) >> 5;
+  const int per = (n_words + 31) >> 5;          // mask words per lane
+  int n_live = p.n_units, cnt = 0, incl = 0;
+  if (book && !p.all_live) {
+#pragma unroll 1
+    for (int i = 0; i < per; ++i) cnt += __popc(need_word(p, lane * per + i, n_words));
+    incl = cnt;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int t = __shfl_up_sync(0xffffffffu, incl, o);
+      incl += lane >= o ? t : 0;
+    }
+    n_live = __shfl_sync(0xffffffffu, incl, 31);
+  }
+  if (p.work != nullptr && w == 0 && lane == 0) {
+    atomicAdd(p.work, (unsigned long long)n_live);
+    atomicAdd(p.work + 1, (unsigned long long)p.n_units);
+  }
+  const int s = book ? max(1, (int)(gridDim.x * kWarpsPerCta) / max(n_live, 1)) : 1;
+  const int li = w / s;
+  if (li >= n_live) return false;
+  if (book && !p.all_live) {
+    // the lane whose words hold live unit number li finds its index
+    int r = li - (incl - cnt), u = -1;
+#pragma unroll 1
+    for (int i = 0; i < per; ++i) {
+      const uint32_t m = need_word(p, lane * per + i, n_words);
+      const int c = __popc(m);
+      if (u < 0 && r >= 0 && r < c) u = (lane * per + i) * 32 + (int)__fns(m, 0u, r + 1);
+      r -= c;
+    }
+    const uint32_t owner = __ballot_sync(0xffffffffu, u >= 0);
+    unit = __shfl_sync(0xffffffffu, u, __ffs(owner) - 1);
+  } else {
+    unit = li;
+  }
+  const int rb = unit / p.n_strips;
+  const int uy0 = p.y_begin + rb * p.rows_per_unit;
+  const int rows = min(uy0 + p.rows_per_unit, p.y_end) - uy0;
+  const int nseg = min(s, max(1, rows / kMinSegRows));
+  const int seg = w - li * s;
+  if (seg >= nseg) return false;
+  y0 = uy0 + seg * rows / nseg;
+  y1 = uy0 + (seg + 1) * rows / nseg;
+  return true;
+}
+
 // Dynamic shared memory of a launch (PP2D_LUT6 builds; the 8 KB table keeps
 // its static buffer so that the default build's code is untouched).
 template <int T, int CW>
@@ -969,13 +1075,24 @@ mdp_sweep_kernel(const SweepParams p) {
   const int warp = (int)(threadIdx.x >> 5);
 #endif
   const int unit = blockIdx.x * (blockDim.x >> 5) + warp;
+  using Sw = Sweeper<T, CW, POLICY, P2P, LIN>;
   if constexpr (P2P) {
     if (unit == p.publisher_unit) {
       publish_flags(p, lane);
       return;
     }
   }
-  if (unit >= p.n_units) return;
+  int run_unit = unit, y0 = 0, y1 = 0;
+  if constexpr (Sw::kSkip) {
+    // The mask the launch after next reads: the previous launch read it and
+    // has completed (griddepcontrol.wait above).  (Reductions, not stores.)
+    if (p.need_out != nullptr && blockIdx.x == 0)
+      for (int i = threadIdx.x; i < (p.n_units + 31) >> 5; i += blockDim.x)
+        atomicAnd(p.need_clear + i, 0u);
+    if (!unit_plan(p, unit, lane, run_unit, y0, y1)) return;
+  } else {
+    if (unit >= p.n_units) return;
+  }
   // Produced by a volatile asm after the barrier: the table loads (plain asm,
   // free to be scheduled) depend on it and so cannot move above the barrier.
   uint32_t lane_base;
@@ -983,8 +1100,23 @@ mdp_sweep_kernel(const SweepParams p) {
                : "=r"(lane_base) : "r"(lut_addr), "r"((lane & 7) << 4) : "memory");
   const uint32_t ring_warp =
       lut_addr + kLutFloat4 * 16 + warp * G::kRingBytesPerWarp;
-  Sweeper<T, CW, POLICY, P2P, LIN> s(p, lane_base, ring_warp);
-  s.run(unit, lane);
+  Sw s(p, lane_base, ring_warp);
+  if constexpr (Sw::kSkip) {
+    const int k = run_unit % p.n_strips;
+    s.run_segment(k, y0, y1, lane);
+    // Output of the segment differs from its input somewhere: the 3x3 unit
+    // neighbourhood must run in the next launch (lanes 0..8, one unit each).
+    const bool changed = __any_sync(0xffffffffu, s.valid && s.diff != 0u);
+    if (p.need_out != nullptr && changed && lane < 9) {
+      const int rb = run_unit / p.n_strips + lane / 3 - 1, kk = k + lane % 3 - 1;
+      if (rb >= 0 && rb < p.n_units / p.n_strips && kk >= 0 && kk < p.n_strips) {
+        const int v = rb * p.n_strips + kk;
+        atomicOr(p.need_out + (v >> 5), 1u << (v & 31));
+      }
+    }
+  } else {
+    s.run(unit, lane);
+  }
 }
 
 // ---------------------------------------------------------------------------

@@ -191,6 +191,13 @@ class MdpPathPlanning2d:
     def sweep_count(self):
         return self._lib.pp2d_mdp_sweep_count(self._h)
 
+    def work_counters(self):
+        """(units run, units launched) of the fused two-sweep launches so far
+        (pp2d_mdp_work_counters)."""
+        out = np.zeros(2, dtype=np.uint64)
+        _lib.check(self._lib.pp2d_mdp_work_counters(self._h, out.ctypes.data))
+        return int(out[0]), int(out[1])
+
     # -- online -----------------------------------------------------------
     def beliefCallback(self, belief):
         """Action at the belief mode (path_planning_2d.cu:168-189)."""

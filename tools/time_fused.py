@@ -1,5 +1,7 @@
 """GPU box: time the fused 2-sweep kernel of the library in PP2D_LIB (4096^2 syn grid)
-and print a checksum of J after 100 sweeps.  usage: PP2D_LIB=... python tools/time_fused.py [size]"""
+and print a checksum of J after 100 sweeps.  usage: PP2D_LIB=... python tools/time_fused.py [size]
+The timed sweeps (100-600) are where unit skipping starts: run with
+PP2D_MDP_SKIP=0 to time the dense kernel."""
 import os
 import sys
 import zlib
