@@ -133,6 +133,34 @@ int pp2d_mdp_reset(pp2d_mdp* h, const uint8_t* map, uint32_t goal_x,
  */
 int pp2d_mdp_stage_map(pp2d_mdp* h, const uint8_t* map);
 
+/*
+ * Re-plan on a changed map (same height/width/rows) and/or goal from the
+ * current solution instead of from J = 0.  Same checks and error codes as
+ * pp2d_mdp_reset; on an error the handle is unchanged.  Afterwards:
+ *   - J' = what pp2d_mdp_download returned just before the call, except that
+ *     every cell occupied in the new map gets trapped(n) (the value every
+ *     occupied cell has after n sweeps, n = pp2d_mdp_sweep_count) and the new
+ *     goal gets 0.  Everything else keeps its value, including newly freed
+ *     cells (they keep the trapped(n) they were reported with) and the old goal
+ *     (it stays 0).
+ *   - the model (codes) is that of the new map and goal;
+ *   - pp2d_mdp_sweep_count is unchanged and keeps counting;
+ *   - the next pp2d_mdp_residual measures the change since this call;
+ *   - the action grid is left as it was: it belongs to the old map until the
+ *     next sweep that writes actions, which rewrites all of it.
+ * So "update, then k sweeps" equals k of the reference's sweeps on the new
+ * map started from J', and pp2d_mdp_solve after it runs the reference's
+ * stopping rule from J'.  Only the units the change reaches are recomputed by
+ * the following fused sweeps while the rest of the grid stays at its fixed
+ * point (DESIGN.md section 4).  A map staged with pp2d_mdp_stage_map is used
+ * when the same pointer is passed (the call then does not block the host);
+ * otherwise the call returns once the map has been copied.  Works on every
+ * handle kind (a shard applies the rule to its own and its ghost rows).
+ * After pp2d_mdp_policy_iteration: PP2D_ERR_STATE.
+ */
+int pp2d_mdp_update_map(pp2d_mdp* h, const uint8_t* map, uint32_t goal_x,
+                        uint32_t goal_y);
+
 
 /* Replaces freeDeviceMemory (src/mdp/path_planning_2d_cuda.cu:66-74). */
 void pp2d_mdp_destroy(pp2d_mdp* h);

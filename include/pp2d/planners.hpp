@@ -200,6 +200,30 @@ class MdpPathPlanning2d : public PathPlanning2dBase {
     return true;
   }
 
+  // Not in the reference (one map per process): re-plan on a changed map of
+  // the same size and/or a new goal from the current solution
+  // (pp2d_mdp_update_map), then valueIteration() from there and the download,
+  // as initialize() does.  total_iterations and residuals carry on.  Returns
+  // false and changes nothing when the goal is occupied or out of the map.
+ public:
+  bool updateMap(const std::vector<uint8_t>& map, int32_t goal_x, int32_t goal_y) {
+    if (map.size() != (size_t)map_width * map_height) return false;
+    const int rc = pp2d_mdp_update_map(mdp_, map.data(), (uint32_t)goal_x, (uint32_t)goal_y);
+    if (rc == PP2D_ERR_GOAL_OCCUPIED || rc == PP2D_ERR_INVALID) {
+      std::fprintf(stderr, "The assigned goal (%d %d) is at a occupied cell...\n", goal_x,
+                   goal_y);
+      return false;
+    }
+    PP2D_CHECK(rc);
+    grid_map = map;
+    goal[0] = goal_x;
+    goal[1] = goal_y;
+    valueIteration();
+    PP2D_CHECK(pp2d_mdp_download(mdp_, optimal_cost.data(), optimal_action.data()));
+    return true;
+  }
+
+ private:
   // src/mdp/path_planning_2d.cu:207-269 (imshow windows dropped)
   void valueIteration() {
     float cost_inf_norm = 0.0f;

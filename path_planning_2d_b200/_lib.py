@@ -40,6 +40,7 @@ SIGNATURES = {
     "pp2d_mdp_device_count": (_i, [_vp, ctypes.POINTER(_i)]),
     "pp2d_mdp_reset": (_i, [_vp, _vp, _u32, _u32]),
     "pp2d_mdp_stage_map": (_i, [_vp, _vp]),
+    "pp2d_mdp_update_map": (_i, [_vp, _vp, _u32, _u32]),
     "pp2d_mdp_destroy": (None, [_vp]),
     "pp2d_mdp_set_stream": (_i, [_vp, _vp]),
     "pp2d_mdp_set_async": (_i, [_vp, _i]),

@@ -616,6 +616,54 @@ static int upload_map(pp2d_mdp* h, const uint8_t* map) {
   return PP2D_OK;
 }
 
+// New map and goal (h->gx, h->gy already set) on a handle that keeps its J:
+// codes rebuilt, J' and Jchk written by mdp_update_map_kernel, the sweep count
+// kept.  The new rows always arrive through the staging buffer: a map that
+// was not staged with pp2d_mdp_stage_map is staged here and waited for.
+static int update_map(pp2d_mdp* h, const uint8_t* map) {
+  const bool staged = h->staged_map != nullptr && h->staged_map == map;
+  if (!staged) PP2D_TRY_MDP(pp2d_mdp_stage_map(h, map));
+  h->staged_map = nullptr;
+  PP2D_CUDA(cudaStreamWaitEvent(h->stream, h->ev_staged, 0));
+  const int occ_row0 = (int)h->row_begin - 3 < 0 ? 0 : (int)h->row_begin - 3;
+  const int row_end = (int)(h->row_begin + h->H);
+  const int occ_row1 = row_end + 3 > (int)h->Htot ? (int)h->Htot : row_end + 3;
+  UpdateParams up;
+  CodeParams& cp = up.c;
+  cp.occ = h->occ_next; cp.code = h->code; cp.W = (int)h->W; cp.Htot = (int)h->Htot;
+  cp.pitch = h->pitch; cp.rows_phys = (int)h->H + 2 * kPadRows;
+  cp.row_begin = (int)h->row_begin; cp.occ_row0 = occ_row0; cp.occ_rows = occ_row1 - occ_row0;
+  cp.gx = (int)h->gx; cp.gy = (int)h->gy;
+  up.j = h->j[h->cur];
+  up.jchk = h->jchk;
+  up.trapped = trapped_cost(h, h->n_sweeps);
+  up.H = (int)h->H;
+  // Seed the mask of the next fused row-block launch.  Without a valid mask
+  // that launch runs every unit anyway.
+  up.need = nullptr;
+  up.n_strips = ((int)h->W + StripGeom<2, 2>::S - 1) / StripGeom<2, 2>::S;
+  up.rows_per_unit = up.n_rb = 1;
+  if (h->need_valid) {
+    up.need = h->need[h->need_rot];
+    up.rows_per_unit = h->need_rows_per_unit;
+    up.n_rb = h->need_units / up.n_strips;
+  }
+  dim3 grid((h->pitch / 4 + kCodeThreads - 1) / kCodeThreads,
+            (cp.rows_phys + kCodeRows - 1) / kCodeRows);
+  mdp_update_map_kernel<<<grid, kCodeThreads, 0, h->stream>>>(up);
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  PP2D_CUDA(cudaGetLastError());
+  PP2D_CUDA(cudaEventRecord(h->ev_code_built, h->stream));
+  // (the caller may free `map` on return: wait for the copy)
+  if (!staged) PP2D_CUDA(cudaStreamSynchronize(h->stream));
+  std::swap(h->occ, h->occ_next);
+  h->has_occupied =
+      memchr(map + (size_t)h->row_begin * h->W, 1, (size_t)h->H * h->W) != nullptr;
+  h->n_chk = h->n_sweeps;
+  h->chk_is_zero = false;
+  return PP2D_OK;
+}
+
 static int create_impl(uint32_t height, uint32_t width, const uint8_t* map,
                        uint32_t gx, uint32_t gy, float gamma,
                        uint32_t row_begin, uint32_t row_end, bool sharded,
@@ -849,6 +897,26 @@ static int multi_reset(pp2d_mdp* m, const uint8_t* map, uint32_t gx, uint32_t gy
   return PP2D_OK;
 }
 
+// Each part applies the update rule to its owned and ghost rows from its own
+// occupancy rows; the rule is local, so the ghost rows stay equal to what the
+// neighbour writes into its owned rows.
+static int multi_update_map(pp2d_mdp* m, const uint8_t* map, uint32_t gx, uint32_t gy) {
+  DeviceGuard guard;
+  PP2D_TRY_MDP(multi_sync(m));               // no device may still write a neighbour's rows
+  for (pp2d_mdp* part : m->parts) {
+    PP2D_TRY_MDP(multi_set_device(part));
+    part->gx = gx;
+    part->gy = gy;
+    int rc = update_map(part, map);
+    if (rc != PP2D_OK) return rc;
+  }
+  m->gx = gx;
+  m->gy = gy;
+  m->n_chk = m->n_sweeps;
+  m->fused_pending = false;
+  return PP2D_OK;
+}
+
 static void multi_destroy(pp2d_mdp* m) {
   DeviceGuard guard;
   for (size_t i = 0; i < m->parts.size(); ++i) {
@@ -975,8 +1043,9 @@ int pp2d_mdp_device_count(const pp2d_mdp* h, int* peer_to_peer) {
   return h->parts.empty() ? 1 : (int)h->parts.size();
 }
 
-int pp2d_mdp_reset(pp2d_mdp* h, const uint8_t* map, uint32_t goal_x,
-                   uint32_t goal_y) {
+// Arguments of a new map and goal on an existing handle (reset, update).
+static int check_map_goal(const pp2d_mdp* h, const uint8_t* map, uint32_t goal_x,
+                          uint32_t goal_y) {
   if (!h || !map) return fail(PP2D_ERR_INVALID, "NULL argument");
   if (goal_x >= h->W || goal_y >= h->Htot)
     return fail(PP2D_ERR_INVALID, "goal (%u %u) outside the %ux%u map", goal_x,
@@ -985,10 +1054,27 @@ int pp2d_mdp_reset(pp2d_mdp* h, const uint8_t* map, uint32_t goal_x,
     return fail(PP2D_ERR_GOAL_OCCUPIED,
                 "The assigned goal (%u %u) is at a occupied cell...", goal_x,
                 goal_y);
+  return PP2D_OK;
+}
+
+int pp2d_mdp_reset(pp2d_mdp* h, const uint8_t* map, uint32_t goal_x,
+                   uint32_t goal_y) {
+  PP2D_TRY_MDP(check_map_goal(h, map, goal_x, goal_y));
   if (!h->parts.empty()) return multi_reset(h, map, goal_x, goal_y);
   h->gx = goal_x;
   h->gy = goal_y;
   return upload_map(h, map);
+}
+
+int pp2d_mdp_update_map(pp2d_mdp* h, const uint8_t* map, uint32_t goal_x, uint32_t goal_y) {
+  PP2D_TRY_MDP(check_map_goal(h, map, goal_x, goal_y));
+  if (h->pi_mode)
+    return fail(PP2D_ERR_STATE, "pp2d_mdp_update_map continues value iteration: the handle "
+                                "ran policy iteration, call pp2d_mdp_reset first");
+  if (!h->parts.empty()) return multi_update_map(h, map, goal_x, goal_y);
+  h->gx = goal_x;
+  h->gy = goal_y;
+  return update_map(h, map);
 }
 
 int pp2d_mdp_stage_map(pp2d_mdp* h, const uint8_t* map) {

@@ -1168,6 +1168,30 @@ __device__ __forceinline__ uint32_t occ_mask6(const CodeParams& p, int x0, int g
 constexpr int kCodeRows = 16;
 constexpr int kCodeThreads = 128;
 
+// Codes of the 4 cells x0 .. x0+3 of global row gy from the occupancy masks
+// m0, m1, m2 of rows gy-1, gy, gy+1 (occ_mask6).  Used by the code kernel and
+// the map-update kernel, so that both build the same bits.
+__device__ __forceinline__ void cell_codes4(const CodeParams& p, int x0, int gy, uint32_t m0,
+                                            uint32_t m1, uint32_t m2, uint32_t (&code)[4]) {
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const int x = x0 + j;
+    uint32_t cd = kCodeOccBit;   // padding
+    if (x >= 0 && x < p.W && gy >= 0 && gy < p.Htot) {
+      // slots: 0 1 2 / 3 4 5 / 6 7 8 ; ring: s0 s1 s2 s5 s8 s7 s6 s3 s0 s1
+      const uint32_t t = m0 >> j, c = m1 >> j, b = m2 >> j;
+      const uint32_t s0 = t & 1u, s1 = (t >> 1) & 1u, s2 = (t >> 2) & 1u, s3 = c & 1u,
+                     s4 = (c >> 1) & 1u, s5 = (c >> 2) & 1u, s6 = b & 1u,
+                     s7 = (b >> 1) & 1u, s8 = (b >> 2) & 1u;
+      cd = s0 | (s1 << 1) | (s2 << 2) | (s5 << 3) | (s8 << 4) | (s7 << 5) |
+           (s6 << 6) | (s3 << 7) | (s0 << 8) | (s1 << 9);
+      if (s4) cd |= kCodeOccBit;
+      else if (!(x == p.gx && gy == p.gy)) cd |= kCodeLiveBit;
+    }
+    code[j] = cd;
+  }
+}
+
 template <bool FAST>
 __device__ __forceinline__ void code_march(const CodeParams& p, int c0, int r0) {
   const int x0 = c0 - kPadLeft;
@@ -1177,23 +1201,7 @@ __device__ __forceinline__ void code_march(const CodeParams& p, int c0, int r0) 
   for (int r = r0; r < r1; ++r, ++gy) {
     const uint32_t m2 = occ_mask6<FAST>(p, x0, gy + 1);
     uint32_t code[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int x = x0 + j;
-      uint32_t cd = kCodeOccBit;   // padding
-      if (x >= 0 && x < p.W && gy >= 0 && gy < p.Htot) {
-        // slots: 0 1 2 / 3 4 5 / 6 7 8 ; ring: s0 s1 s2 s5 s8 s7 s6 s3 s0 s1
-        const uint32_t t = m0 >> j, c = m1 >> j, b = m2 >> j;
-        const uint32_t s0 = t & 1u, s1 = (t >> 1) & 1u, s2 = (t >> 2) & 1u, s3 = c & 1u,
-                       s4 = (c >> 1) & 1u, s5 = (c >> 2) & 1u, s6 = b & 1u,
-                       s7 = (b >> 1) & 1u, s8 = (b >> 2) & 1u;
-        cd = s0 | (s1 << 1) | (s2 << 2) | (s5 << 3) | (s8 << 4) | (s7 << 5) |
-             (s6 << 6) | (s3 << 7) | (s0 << 8) | (s1 << 9);
-        if (s4) cd |= kCodeOccBit;
-        else if (!(x == p.gx && gy == p.gy)) cd |= kCodeLiveBit;
-      }
-      code[j] = cd;
-    }
+    cell_codes4(p, x0, gy, m0, m1, m2, code);
     // pitch is a multiple of 32 and c0 of 4: the 4 codes are 8-byte aligned
     *reinterpret_cast<uint2*>(p.code + (size_t)r * p.pitch + c0) =
         make_uint2(code[0] | (code[1] << 16), code[2] | (code[3] << 16));
@@ -1212,6 +1220,116 @@ __global__ void __launch_bounds__(kCodeThreads) mdp_code_kernel(const CodeParams
                     (reinterpret_cast<uintptr_t>(p.occ) & 3u) == 0;
   if (fast) code_march<true>(p, c0, r0);
   else code_march<false>(p, c0, r0);
+}
+
+// ---------------------------------------------------------------------------
+// New map on a solved handle (pp2d_mdp_update_map, DESIGN.md section 4): the
+// codes of the new map and goal, and J' in place of J_n:
+//   newly occupied cell -> stored 0 (occupied cells are stored as 0);
+//   newly freed cell    -> trapped(n), the value it was reported with;
+//   the new goal        -> 0;
+// every other cell keeps its value.  Jchk <- J' on the owned rows (the next
+// residual measures the change since the update).  A cell whose code or
+// stored J changed is dirty; every dirty unit of the fused row-block launch
+// geometry sets the bits of its 3x3 unit neighbourhood in `need`, the mask the
+// next fused launch reads.
+struct UpdateParams {
+  CodeParams c;          // occupancy of the new map, code plane, new goal
+  float* j;              // current J plane (ghost rows included)
+  float* jchk;           // residual snapshot
+  float trapped;         // J_n of an occupied cell, n = sweep count
+  uint32_t* need;        // NULL: no seeding (the next fused launch runs every unit)
+  int n_strips, rows_per_unit, n_rb;   // unit = row_block * n_strips + strip
+  int H;                 // owned rows
+};
+
+__device__ __forceinline__ void mark_unit_neighbourhood(const UpdateParams& p, int rb, int k) {
+#pragma unroll 1
+  for (int i = 0; i < 9; ++i) {
+    const int r = rb + i / 3 - 1, kk = k + i % 3 - 1;
+    if (r >= 0 && r < p.n_rb && kk >= 0 && kk < p.n_strips) {
+      const int v = r * p.n_strips + kk;
+      atomicOr(p.need + (v >> 5), 1u << (v & 31));
+    }
+  }
+}
+
+// Same thread shape as mdp_code_kernel (4 cells per thread, kCodeRows rows
+// marched with the occupancy masks in registers), but every lane of a warp
+// runs the whole march: the dirty units are aggregated per warp.
+__global__ void __launch_bounds__(kCodeThreads) mdp_update_map_kernel(const UpdateParams p) {
+  const CodeParams& cp = p.c;
+  const int lane = threadIdx.x & 31;
+  const int c0 = 4 * (blockIdx.x * kCodeThreads + threadIdx.x);
+  const int r0 = blockIdx.y * kCodeRows;
+  if (r0 >= cp.rows_phys) return;                 // uniform over the block
+  const bool active = c0 < cp.pitch;
+  const int x0 = c0 - kPadLeft;
+  const bool fast = (cp.W & 3) == 0 && (x0 & 3) == 0 && x0 >= 0 && x0 + 3 < cp.W &&
+                    (reinterpret_cast<uintptr_t>(cp.occ) & 3u) == 0;
+  auto mask = [&](int gy) {
+    return fast ? occ_mask6<true>(cp, x0, gy) : occ_mask6<false>(cp, x0, gy);
+  };
+  // strip of cell x0 (or of x = 0); the 4 cells lie in it or in the next one
+  constexpr int kStrip = StripGeom<2, 2>::S;
+  const int k_lo = max(x0, 0) / kStrip;
+  const int r1 = min(r0 + kCodeRows, cp.rows_phys);
+  int gy = cp.row_begin + r0 - kPadRows;
+  uint32_t m0 = mask(gy - 1), m1 = mask(gy);
+  for (int r = r0; r < r1; ++r, ++gy) {
+    const uint32_t m2 = mask(gy + 1);
+    uint32_t code[4];
+    cell_codes4(cp, x0, gy, m0, m1, m2, code);
+    m0 = m1;
+    m1 = m2;
+    bool dirty_lo = false, dirty_hi = false;
+    if (active) {
+      const size_t q = (size_t)r * cp.pitch + c0;
+      const uint2 oc2 = *reinterpret_cast<const uint2*>(cp.code + q);
+      const uint32_t old[4] = {oc2.x & 0xFFFFu, oc2.x >> 16, oc2.y & 0xFFFFu, oc2.y >> 16};
+      const float4 jv = *reinterpret_cast<const float4*>(p.j + q);
+      const float jo[4] = {jv.x, jv.y, jv.z, jv.w};
+      float jn[4];
+      bool code_changed = false, j_changed = false;
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const bool occ_new = code[i] & kCodeOccBit, occ_old = old[i] & kCodeOccBit;
+        jn[i] = jo[i];
+        if (occ_new && !occ_old) jn[i] = 0.0f;
+        if (!occ_new && occ_old) jn[i] = p.trapped;
+        if (!(code[i] & (kCodeOccBit | kCodeLiveBit))) jn[i] = 0.0f;   // the goal
+        const bool cc = code[i] != old[i];
+        const bool jc = __float_as_uint(jn[i]) != __float_as_uint(jo[i]);
+        code_changed |= cc;
+        j_changed |= jc;
+        if (cc || jc) {
+          if ((x0 + i) / kStrip == k_lo || x0 + i < 0) dirty_lo = true;
+          else dirty_hi = true;
+        }
+      }
+      if (code_changed)
+        *reinterpret_cast<uint2*>(cp.code + q) =
+            make_uint2(code[0] | (code[1] << 16), code[2] | (code[3] << 16));
+      const float4 jw = make_float4(jn[0], jn[1], jn[2], jn[3]);
+      if (j_changed) *reinterpret_cast<float4*>(p.j + q) = jw;
+      if (r >= kPadRows && r < kPadRows + p.H) *reinterpret_cast<float4*>(p.jchk + q) = jw;
+    }
+    if (p.need != nullptr && __any_sync(0xffffffffu, dirty_lo || dirty_hi)) {
+      // ghost rows belong to the row block next to them
+      const int y = min(max(r - kPadRows, 0), p.H - 1);
+      const int rb = min(y / p.rows_per_unit, p.n_rb - 1);
+#pragma unroll
+      for (int side = 0; side < 2; ++side) {
+        const bool d = side ? dirty_hi : dirty_lo;
+        const uint32_t m = __ballot_sync(0xffffffffu, d);
+        if (d) {
+          const int k = k_lo + side;
+          const uint32_t peers = __match_any_sync(m, k);
+          if (__ffs(peers) - 1 == lane) mark_unit_neighbourhood(p, rb, k);
+        }
+      }
+    }
+  }
 }
 
 // ---------------------------------------------------------------------------

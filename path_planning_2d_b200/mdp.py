@@ -99,6 +99,27 @@ class MdpPathPlanning2d:
         _lib.check(self._lib.pp2d_mdp_reset(self._h, self._map.ctypes.data,
                                             self.goal[0], self.goal[1]))
 
+    def update_map(self, grid_map=None, goal=None):
+        """New map (same shape) and/or goal, keeping the current solution as
+        the start of the next sweeps (pp2d_mdp_update_map): occupied cells of
+        the new map take the trapped cost of the current sweep count, the new
+        goal 0, every other cell keeps its J; the sweep count carries on and
+        the next residual measures the change since this call.  Pass an array
+        given to stage_map() to use the staged rows."""
+        new_map, new_goal = self._map, self.goal
+        if grid_map is not None:
+            new_map = grid_map
+            if not (isinstance(grid_map, np.ndarray) and grid_map.dtype == np.uint8
+                    and grid_map.flags.c_contiguous):
+                new_map = np.ascontiguousarray(grid_map, dtype=np.uint8)
+            if new_map.shape != (self.map_height, self.map_width):
+                raise ValueError("update_map() needs a map of the same shape")
+        if goal is not None:
+            new_goal = (int(goal[0]), int(goal[1]))
+        _lib.check(self._lib.pp2d_mdp_update_map(self._h, new_map.ctypes.data,
+                                                 new_goal[0], new_goal[1]))
+        self._map, self.goal = new_map, new_goal
+
     def stage_map(self, grid_map):
         """Start uploading the map of the next reset() while the current solve
         runs (pp2d_mdp_stage_map); pass the SAME array to reset() afterwards.
