@@ -317,6 +317,82 @@ int pp2d_mdp_p2p_status(pp2d_mdp* h, int* timed_out);
 int pp2d_mdp_residual_device(pp2d_mdp* h, void** dev_float_out);
 
 /* ------------------------------------------------------------------------
+ * MDP batches: many goals or maps of one size solved together
+ * ------------------------------------------------------------------------ */
+typedef struct pp2d_mdp_batch pp2d_mdp_batch;
+
+/*
+ * `count` independent value-iteration instances of one height x width size on
+ * the current device: a fleet with one goal per robot, cost-to-go fields for
+ * every docking station of a map, a sweep over maps.  No counterpart in the
+ * reference (one goal per process).  The instances are stacked into one tall
+ * grid with an occupied separator row between neighbours (DESIGN.md section
+ * 4, "Batches"), so every instance computes bit for bit what pp2d_mdp_create on its map
+ * and goal computes, while all of them share the launches.
+ * maps: `count` maps of height*width bytes, `map_stride` bytes apart;
+ * map_stride == 0: one map shared by all instances (only goals differ).
+ * goals_xy: uint32_t[count][2], (x, y) per instance.  The checks of
+ * pp2d_mdp_create apply per instance; an occupied goal gives
+ * PP2D_ERR_GOAL_OCCUPIED with the instance index in the message.
+ * PP2D_ERR_INVALID for count == 0, map_stride below height*width, or a
+ * stacked grid (count*(height+1)-1 rows) too large for int row and element
+ * indices.  J = 0, actions = 0, sweep count 0.  Not sharded, one device.
+ */
+int pp2d_mdp_batch_create(uint32_t height, uint32_t width, uint32_t count, const uint8_t* maps,
+                          size_t map_stride, const uint32_t* goals_xy, float gamma,
+                          pp2d_mdp_batch** out);
+/* New maps and goals (same size and count) on the same allocations, as
+ * pp2d_mdp_reset; map_stride may differ from the one given at creation (a
+ * shared map may become one map per instance and back).  On an error the
+ * handle is unchanged. */
+int pp2d_mdp_batch_reset(pp2d_mdp_batch* h, const uint8_t* maps, size_t map_stride,
+                         const uint32_t* goals_xy);
+void pp2d_mdp_batch_destroy(pp2d_mdp_batch* h);
+/* As pp2d_mdp_set_stream; calls still synchronise before they return. */
+int pp2d_mdp_batch_set_stream(pp2d_mdp_batch* h, void* stream);
+
+/* n sweeps of every instance, as pp2d_mdp_sweeps (the action grids come
+ * from the last one).  PP2D_ERR_STATE after pp2d_mdp_batch_solve until
+ * pp2d_mdp_batch_reset. */
+int pp2d_mdp_batch_sweeps(pp2d_mdp_batch* h, uint32_t n);
+/* out[count]: per instance, what pp2d_mdp_residual returns for it: the
+ * inf-norm of the change since the previous call, with the occupied-cell
+ * floor when its own map has an occupied cell.  PP2D_ERR_STATE after
+ * pp2d_mdp_batch_solve. */
+int pp2d_mdp_batch_residual(pp2d_mdp_batch* h, float* out);
+/*
+ * pp2d_mdp_solve per instance: batches of 100 sweeps, instance k stops after
+ * its first batch whose residual is <= 5/(1-gamma)*1e-3.  sweeps_out[count]
+ * (optional) and residuals (optional, [count][max_residuals], entries past an
+ * instance's last batch are not written) are exactly what pp2d_mdp_solve
+ * returns for each instance alone.  Returns once every instance has stopped;
+ * each then holds its J and actions at its own stopping point.  A stopped
+ * instance is frozen: its results are kept aside and its rows stop costing
+ * work in the launches that the others still need.  Afterwards sweeps,
+ * residual and solve return PP2D_ERR_STATE until pp2d_mdp_batch_reset.
+ */
+int pp2d_mdp_batch_solve(pp2d_mdp_batch* h, uint32_t* sweeps_out, double* residuals,
+                         uint32_t max_residuals);
+/* Results of instances [first, first+n): cost [n][height][width] floats
+ * (occupied cells filled in as by pp2d_mdp_download), action
+ * [n][height][width] bytes; either may be NULL. */
+int pp2d_mdp_batch_download(pp2d_mdp_batch* h, uint32_t first, uint32_t n, float* cost,
+                            uint8_t* action);
+/* pp2d_mdp_plan_batch where belief i ([n][height*width] floats) reads the
+ * action grid of instance instance[i]. */
+int pp2d_mdp_batch_plan(pp2d_mdp_batch* h, const uint32_t* instance, const float* beliefs,
+                        uint32_t n, uint8_t* actions);
+/* pp2d_mdp_waypoints on instance k. */
+int pp2d_mdp_batch_waypoints(pp2d_mdp_batch* h, uint32_t k, uint32_t start_x,
+                             uint32_t start_y, uint32_t* cells, uint32_t max_len,
+                             uint32_t* n_out);
+/* out[count]: sweeps applied to each instance (a frozen instance keeps the
+ * count it stopped at). */
+int pp2d_mdp_batch_sweep_counts(const pp2d_mdp_batch* h, uint32_t* out);
+/* As pp2d_mdp_work_counters, over the launches of the whole batch. */
+int pp2d_mdp_batch_work_counters(pp2d_mdp_batch* h, uint64_t out[2]);
+
+/* ------------------------------------------------------------------------
  * POMDP model, belief propagation, bounds and QV-Tree Search
  * (SURVEY.md rows B1-B10)
  * ------------------------------------------------------------------------ */

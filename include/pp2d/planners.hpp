@@ -14,6 +14,7 @@
 // CUDA failures keep the reference's print-and-exit behaviour
 // (helper_cuda.h:984-999) through PP2D_CHECK.
 #pragma once
+#include <algorithm>
 #include <array>
 #include <cstdint>
 #include <cstdio>
@@ -256,6 +257,70 @@ class MdpPathPlanning2d : public PathPlanning2dBase {
   pp2d_mdp* mdp_ = nullptr;
   int32_t num_gpus = 1;
   std::vector<int> gpu_devices;
+};
+
+// Not in the reference (one goal per process): many goals or maps of one size
+// solved together on one GPU (pp2d_mdp_batch_*), e.g. one goal per robot of a
+// fleet.  maps: height*width bytes shared by every goal, or one map per goal
+// back to back; goals: one (x, y) per instance.  Instance k's results equal
+// those of MdpPathPlanning2d on its map and goal bit for bit.
+class MdpBatchPathPlanning2d {
+ public:
+  MdpBatchPathPlanning2d(uint32_t height, uint32_t width, const std::vector<uint8_t>& maps,
+                         const std::vector<std::array<uint32_t, 2>>& goals, float gamma)
+      : height_(height), width_(width), count_((uint32_t)goals.size()) {
+    const size_t hw = (size_t)height * width;
+    if (maps.size() != hw && maps.size() != hw * goals.size()) {
+      std::fprintf(stderr, "MdpBatchPathPlanning2d: one shared map or one map per goal\n");
+      std::exit(EXIT_FAILURE);
+    }
+    PP2D_CHECK(pp2d_mdp_batch_create(height, width, count_, maps.data(),
+                                     maps.size() == hw ? 0 : hw, goals.data()->data(), gamma,
+                                     &batch_));
+  }
+  MdpBatchPathPlanning2d(const MdpBatchPathPlanning2d&) = delete;
+  MdpBatchPathPlanning2d& operator=(const MdpBatchPathPlanning2d&) = delete;
+  ~MdpBatchPathPlanning2d() { pp2d_mdp_batch_destroy(batch_); }
+
+  // valueIteration() of every instance (src/mdp/path_planning_2d.cu:207-269);
+  // sweeps[k] and residuals[k] are instance k's.
+  void valueIteration() {
+    const uint32_t cap = 64;
+    std::vector<double> res((size_t)count_ * cap);
+    sweeps.assign(count_, 0);
+    PP2D_CHECK(pp2d_mdp_batch_solve(batch_, sweeps.data(), res.data(), cap));
+    residuals.assign(count_, {});
+    for (uint32_t k = 0; k < count_; ++k)
+      residuals[k].assign(res.begin() + (size_t)k * cap,
+                          res.begin() + (size_t)k * cap + std::min(cap, sweeps[k] / 100));
+  }
+
+  std::vector<float> optimalCost(uint32_t k) const {
+    std::vector<float> c((size_t)height_ * width_);
+    PP2D_CHECK(pp2d_mdp_batch_download(batch_, k, 1, c.data(), nullptr));
+    return c;
+  }
+  std::vector<uint8_t> optimalAction(uint32_t k) const {
+    std::vector<uint8_t> a((size_t)height_ * width_);
+    PP2D_CHECK(pp2d_mdp_batch_download(batch_, k, 1, nullptr, a.data()));
+    return a;
+  }
+  std::vector<uint32_t> waypoints(uint32_t k, uint32_t sx, uint32_t sy) const {
+    std::vector<uint32_t> cells((size_t)height_ * width_);
+    uint32_t n = 0;
+    PP2D_CHECK(pp2d_mdp_batch_waypoints(batch_, k, sx, sy, cells.data(), (uint32_t)cells.size(),
+                                        &n));
+    cells.resize(n);
+    return cells;
+  }
+
+  uint32_t count() const { return count_; }
+  std::vector<uint32_t> sweeps;
+  std::vector<std::vector<double>> residuals;
+
+ private:
+  uint32_t height_, width_, count_;
+  pp2d_mdp_batch* batch_ = nullptr;
 };
 
 // ---------------------------------------------------------------------------

@@ -63,6 +63,20 @@ SIGNATURES = {
     "pp2d_mdp_ipc_export": (_i, [_vp, _vp]),
     "pp2d_mdp_ipc_connect": (_i, [_vp, _vp, _vp]),
     "pp2d_mdp_p2p_status": (_i, [_vp, ctypes.POINTER(_i)]),
+    "pp2d_mdp_batch_create": (_i, [_u32, _u32, _u32, _vp, ctypes.c_size_t, _vp,
+                                   ctypes.c_float, ctypes.POINTER(_vp)]),
+    "pp2d_mdp_batch_reset": (_i, [_vp, _vp, ctypes.c_size_t, _vp]),
+    "pp2d_mdp_batch_destroy": (None, [_vp]),
+    "pp2d_mdp_batch_set_stream": (_i, [_vp, _vp]),
+    "pp2d_mdp_batch_sweeps": (_i, [_vp, _u32]),
+    "pp2d_mdp_batch_residual": (_i, [_vp, _vp]),
+    "pp2d_mdp_batch_solve": (_i, [_vp, _vp, _vp, _u32]),
+    "pp2d_mdp_batch_download": (_i, [_vp, _u32, _u32, _vp, _vp]),
+    "pp2d_mdp_batch_plan": (_i, [_vp, _vp, _vp, _u32, _vp]),
+    "pp2d_mdp_batch_waypoints": (_i, [_vp, _u32, _u32, _u32, _vp, _u32,
+                                      ctypes.POINTER(_u32)]),
+    "pp2d_mdp_batch_sweep_counts": (_i, [_vp, _vp]),
+    "pp2d_mdp_batch_work_counters": (_i, [_vp, _vp]),
     "pp2d_pomdp_create": (_i, [_u32, _u32, _vp, _u32, _u32, ctypes.c_float,
                                ctypes.POINTER(_vp)]),
     "pp2d_pomdp_destroy": (None, [_vp]),

@@ -664,6 +664,9 @@ static int update_map(pp2d_mdp* h, const uint8_t* map) {
   return PP2D_OK;
 }
 
+static int make_handle(uint32_t height, uint32_t width, float gamma, uint32_t row_begin,
+                       uint32_t row_end, bool sharded, size_t occ_bytes, pp2d_mdp** out);
+
 static int create_impl(uint32_t height, uint32_t width, const uint8_t* map,
                        uint32_t gx, uint32_t gy, float gamma,
                        uint32_t row_begin, uint32_t row_end, bool sharded,
@@ -684,6 +687,23 @@ static int create_impl(uint32_t height, uint32_t width, const uint8_t* map,
   if (map[(size_t)gy * width + gx] > 0)   // path_planning_2d.cu:84-88
     return fail(PP2D_ERR_GOAL_OCCUPIED,
                 "The assigned goal (%u %u) is at a occupied cell...", gx, gy);
+  const int occ_rows = (int)((row_end + 3 > height ? height : row_end + 3) -
+                             ((int)row_begin - 3 < 0 ? 0 : row_begin - 3));
+  pp2d_mdp* h = nullptr;
+  PP2D_TRY_MDP(make_handle(height, width, gamma, row_begin, row_end, sharded,
+                           (size_t)occ_rows * width, &h));
+  h->gx = gx; h->gy = gy;
+  const int rc = upload_map(h, map);
+  if (rc != PP2D_OK) { pp2d_mdp_destroy(h); return rc; }
+  *out = h;
+  return PP2D_OK;
+}
+
+// Device buffers, table and tuning knobs of a handle that owns rows
+// [row_begin, row_end) of a height x width grid, with occ_bytes of occupancy
+// storage; the map itself is uploaded by the caller.
+static int make_handle(uint32_t height, uint32_t width, float gamma, uint32_t row_begin,
+                       uint32_t row_end, bool sharded, size_t occ_bytes, pp2d_mdp** out) {
   int dev_count = 0;
   PP2D_CUDA(cudaGetDeviceCount(&dev_count));
   if (dev_count == 0) return fail(PP2D_ERR_CUDA, "no CUDA device");
@@ -698,7 +718,7 @@ static int create_impl(uint32_t height, uint32_t width, const uint8_t* map,
   pp2d_mdp* h = new (std::nothrow) pp2d_mdp;
   if (!h) return fail(PP2D_ERR_INVALID, "out of host memory");
   h->Htot = height; h->W = width; h->row_begin = row_begin;
-  h->H = row_end - row_begin; h->gx = gx; h->gy = gy; h->gamma = gamma;
+  h->H = row_end - row_begin; h->gamma = gamma;
   h->sharded = sharded;
   h->device = dev;
   h->sm_count = prop.multiProcessorCount;
@@ -731,8 +751,6 @@ static int create_impl(uint32_t height, uint32_t width, const uint8_t* map,
   if (h->prefetch_rows < kPrefetch) h->prefetch_rows = kPrefetch;
   if (h->prefetch_rows > kSlackRows) h->prefetch_rows = kSlackRows;
 
-  const int occ_rows = (int)((row_end + 3 > height ? height : row_end + 3) -
-                             ((int)row_begin - 3 < 0 ? 0 : row_begin - 3));
   const size_t owned = (size_t)h->H * width;
   int rc = [&]() -> int {
     PP2D_CUDA(cudaMalloc(&h->j[0], h->plane * sizeof(float)));
@@ -740,7 +758,7 @@ static int create_impl(uint32_t height, uint32_t width, const uint8_t* map,
     PP2D_CUDA(cudaMalloc(&h->jchk, h->plane * sizeof(float)));
     PP2D_CUDA(cudaMalloc(&h->code, h->plane * sizeof(uint16_t)));
     PP2D_CUDA(cudaMalloc(&h->action, owned));
-    PP2D_CUDA(cudaMalloc(&h->occ, (size_t)occ_rows * width));
+    PP2D_CUDA(cudaMalloc(&h->occ, occ_bytes));
     PP2D_CUDA(cudaMalloc(&h->lut, kLutFloat4 / 8 * sizeof(float4)));
     PP2D_CUDA(cudaMalloc(&h->resid, sizeof(uint32_t)));
     PP2D_CUDA(cudaMalloc(&h->flags, kFlagWords * sizeof(unsigned int)));
@@ -752,7 +770,7 @@ static int create_impl(uint32_t height, uint32_t width, const uint8_t* map,
     build_lut(gamma, lut);
     PP2D_CUDA(cudaMemcpy(h->lut, lut.data(), kLutFloat4 / 8 * sizeof(float4),
                          cudaMemcpyHostToDevice));
-    return upload_map(h, map);
+    return PP2D_OK;
   }();
   if (rc != PP2D_OK) { pp2d_mdp_destroy(h); return rc; }
   *out = h;
@@ -1504,6 +1522,23 @@ int pp2d_mdp_plan(pp2d_mdp* h, const float* belief, uint8_t* action) {
   return pp2d_mdp_plan_batch(h, belief, 1, action);
 }
 
+// Greedy rollout of a dense H x W action grid from (sx, sy): follow
+// (u%3-1, u/3-1) until action 4 (stay), the map border or max_len cells;
+// returns the number of cells written.
+static uint32_t rollout(const uint8_t* action, uint32_t W, uint32_t H, uint32_t sx, uint32_t sy,
+                        uint32_t* cells, uint32_t max_len) {
+  uint32_t n = 0;
+  int64_t x = sx, y = sy;
+  while (n < max_len && x >= 0 && x < (int64_t)W && y >= 0 && y < (int64_t)H) {
+    cells[n++] = (uint32_t)(y * W + x);
+    const uint8_t u = action[(size_t)y * W + x];
+    if (u == 4) break;
+    x += (int)(u % 3) - 1;   // path_planning_2d_cuda.cu:83-88
+    y += (int)(u / 3) - 1;
+  }
+  return n;
+}
+
 int pp2d_mdp_waypoints(pp2d_mdp* h, uint32_t sx, uint32_t sy, uint32_t* cells,
                        uint32_t max_len, uint32_t* n_out) {
   if (!h || !cells || !n_out) return fail(PP2D_ERR_INVALID, "NULL argument");
@@ -1517,17 +1552,7 @@ int pp2d_mdp_waypoints(pp2d_mdp* h, uint32_t sx, uint32_t sy, uint32_t* cells,
     if (rc != PP2D_OK) return rc;
     h->action_host_valid = true;
   }
-  uint32_t n = 0;
-  int64_t x = sx, y = sy;
-  while (n < max_len && x >= 0 && x < (int64_t)h->W && y >= 0 &&
-         y < (int64_t)h->H) {
-    cells[n++] = (uint32_t)(y * h->W + x);
-    const uint8_t u = h->action_host[(size_t)y * h->W + x];
-    if (u == 4) break;
-    x += (int)(u % 3) - 1;   // path_planning_2d_cuda.cu:83-88
-    y += (int)(u / 3) - 1;
-  }
-  *n_out = n;
+  *n_out = rollout(h->action_host.data(), h->W, h->H, sx, sy, cells, max_len);
   return PP2D_OK;
 }
 
@@ -1624,6 +1649,401 @@ int pp2d_mdp_halo(pp2d_mdp* h, pp2d_halo* out) {
   out->bytes = kPadRows * row * sizeof(float);
   h->halo_budget = kPadRows;     // the caller is about to refresh the ghost rows
   return PP2D_OK;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------
+// Batches of equal-size instances (pp2d_mdp_batch_*, DESIGN.md section 4): the
+// instances are stacked into one tall grid with an occupied separator row
+// between neighbours, and an ordinary handle (`grid`) runs its fused sweeps
+// unchanged.  The batch adds the per-instance codes, residuals, stopping and
+// results around it.
+struct pp2d_mdp_batch {
+  pp2d_mdp* grid = nullptr;        // the tall grid; grid->occ holds the maps
+  uint32_t H = 0, W = 0, count = 0;
+  size_t map_stride = 0;           // device: H*W, or 0 for one shared map
+  uint32_t* goals = nullptr;       // device [count][2]
+  uint8_t* has_occ_dev = nullptr;  // device [count]
+  std::vector<uint8_t> has_occ;    // instance k's own map has an occupied cell
+  uint8_t* frozen_dev = nullptr;   // device [count]
+  std::vector<uint8_t> frozen;     // instance k met the stopping rule in solve
+  std::vector<uint32_t> stop_sweeps;   // sweep count of a frozen instance
+  uint32_t* list = nullptr;        // device [count]: instances of the next kernel
+  uint32_t* resid = nullptr;       // device [count] float bits
+  std::vector<uint32_t> resid_host;
+  float* res_cost = nullptr;       // device [count][H][W]: snapshots and downloads
+  uint8_t* res_action = nullptr;   // device [count][H][W]
+  bool solved = false;             // pp2d_mdp_batch_solve has run since the reset
+};
+
+namespace pp2d {
+
+// Arguments of a batch (create and reset).  The size check comes first: it
+// reads neither the maps nor the goals.
+static int batch_check(uint32_t height, uint32_t width, uint32_t count, const uint8_t* maps,
+                       size_t map_stride, const uint32_t* goals) {
+  if (!maps || !goals) return fail(PP2D_ERR_INVALID, "NULL argument");
+  if (height == 0 || width == 0) return fail(PP2D_ERR_INVALID, "empty map");
+  if (count == 0) return fail(PP2D_ERR_INVALID, "a batch needs at least one instance");
+  const uint64_t hw = (uint64_t)height * width;
+  if (map_stride != 0 && map_stride < hw)
+    return fail(PP2D_ERR_INVALID, "map_stride %zu is below height*width = %llu", map_stride,
+                (unsigned long long)hw);
+  // the kernels index rows, units and plane elements of the tall grid with int
+  const uint64_t rows = (uint64_t)count * (height + 1ull) - 1;
+  const uint64_t pitch = (kPadLeft + (uint64_t)width + 128 + 31) / 32 * 32;
+  const uint64_t plane = (rows + 2 * kPadRows + kSlackRows) * pitch;
+  if (rows > (uint64_t)INT32_MAX || plane > (uint64_t)INT32_MAX)
+    return fail(PP2D_ERR_INVALID, "%u instances of %ux%u stack to a grid of %llu rows x %llu "
+                                  "columns: too large for one batch", count, width, height,
+                (unsigned long long)rows, (unsigned long long)pitch);
+  for (uint32_t k = 0; k < count; ++k) {
+    const uint32_t gx = goals[2 * (size_t)k], gy = goals[2 * (size_t)k + 1];
+    if (gx >= width || gy >= height)
+      return fail(PP2D_ERR_INVALID, "instance %u: goal (%u %u) outside the %ux%u map", k, gx, gy,
+                  width, height);
+    if (maps[k * map_stride + (size_t)gy * width + gx] > 0)
+      return fail(PP2D_ERR_GOAL_OCCUPIED,
+                  "instance %u: The assigned goal (%u %u) is at a occupied cell...", k, gx, gy);
+  }
+  return PP2D_OK;
+}
+
+// Maps, goals and codes of a checked batch; J = 0, actions = 0, sweep count 0.
+static int batch_upload(pp2d_mdp_batch* b, const uint8_t* maps, size_t map_stride,
+                        const uint32_t* goals) {
+  pp2d_mdp* g = b->grid;
+  const size_t hw = (size_t)b->H * b->W;
+  PP2D_CUDA(cudaMemsetAsync(g->j[0], 0, g->plane * sizeof(float), g->stream));
+  PP2D_CUDA(cudaMemsetAsync(g->j[1], 0, g->plane * sizeof(float), g->stream));
+  PP2D_CUDA(cudaMemsetAsync(g->jchk, 0, g->plane * sizeof(float), g->stream));
+  PP2D_CUDA(cudaMemsetAsync(g->action, 0, (size_t)g->H * g->W, g->stream));
+  // the maps go back to back on the device (one copy of a shared map)
+  if (map_stride == 0 || map_stride == hw)
+    PP2D_CUDA(cudaMemcpyAsync(g->occ, maps, (map_stride ? b->count : 1) * hw,
+                              cudaMemcpyHostToDevice, g->stream));
+  else
+    PP2D_CUDA(cudaMemcpy2DAsync(g->occ, hw, maps, map_stride, hw, b->count,
+                                cudaMemcpyHostToDevice, g->stream));
+  b->map_stride = map_stride ? hw : 0;
+  PP2D_CUDA(cudaMemcpyAsync(b->goals, goals, 2 * sizeof(uint32_t) * b->count,
+                            cudaMemcpyHostToDevice, g->stream));
+  for (uint32_t k = 0; k < b->count; ++k)
+    b->has_occ[k] = (map_stride == 0 && k > 0)
+                        ? b->has_occ[0]
+                        : memchr(maps + k * map_stride, 1, hw) != nullptr;
+  PP2D_CUDA(cudaMemcpyAsync(b->has_occ_dev, b->has_occ.data(), b->count, cudaMemcpyHostToDevice,
+                            g->stream));
+  std::fill(b->frozen.begin(), b->frozen.end(), 0);
+  std::fill(b->stop_sweeps.begin(), b->stop_sweeps.end(), 0);
+  PP2D_CUDA(cudaMemsetAsync(b->frozen_dev, 0, b->count, g->stream));
+  BatchCodeParams cp;
+  cp.maps = g->occ; cp.map_stride = b->map_stride; cp.goals = b->goals; cp.code = g->code;
+  cp.W = (int)b->W; cp.H = (int)b->H; cp.count = (int)b->count; cp.pitch = g->pitch;
+  cp.rows_phys = (int)g->H + 2 * kPadRows;
+  const int row_groups = (cp.rows_phys + kCodeRows - 1) / kCodeRows;
+  dim3 grid((g->pitch / 4 + kCodeThreads - 1) / kCodeThreads, std::min(row_groups, 65535));
+  mdp_batch_code_kernel<<<grid, kCodeThreads, 0, g->stream>>>(cp);
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  PP2D_CUDA(cudaGetLastError());
+  // (the caller may free the maps on return)
+  PP2D_CUDA(cudaStreamSynchronize(g->stream));
+  g->cur = 0;
+  g->n_sweeps = g->n_chk = g->action_sweep = 0;
+  g->action_host_valid = false;
+  g->pi_mode = false;
+  g->need_valid = false;
+  b->solved = false;
+  return PP2D_OK;
+}
+
+static int upload_list(pp2d_mdp_batch* b, const std::vector<uint32_t>& list) {
+  PP2D_CUDA(cudaMemcpyAsync(b->list, list.data(), list.size() * sizeof(uint32_t),
+                            cudaMemcpyHostToDevice, b->grid->stream));
+  return PP2D_OK;
+}
+
+// Residuals of the instances in `list` into b->resid_host (one launch, one
+// round trip).
+static int batch_residual(pp2d_mdp_batch* b, const std::vector<uint32_t>& list) {
+  pp2d_mdp* g = b->grid;
+  PP2D_TRY_MDP(upload_list(b, list));
+  PP2D_CUDA(cudaMemsetAsync(b->resid, 0, b->count * sizeof(uint32_t), g->stream));
+  const float floor_val = fabsf(trapped_cost(g, g->n_sweeps) - trapped_cost(g, g->n_chk));
+  uint32_t floor_bits;
+  memcpy(&floor_bits, &floor_val, sizeof(floor_bits));
+  const size_t n4 = (size_t)b->H * g->pitch / 4;
+  const size_t fill = std::max<size_t>(1, (size_t)g->sm_count * 8 / list.size());
+  const int blocks_per = (int)std::min((n4 + 255) / 256, fill);
+  mdp_batch_residual_kernel<<<(unsigned)(list.size() * blocks_per), 256, 0, g->stream>>>(
+      g->j[g->cur], g->jchk, b->list, blocks_per, (int)b->H, g->pitch, floor_bits,
+      b->has_occ_dev, b->resid);
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  PP2D_CUDA(cudaGetLastError());
+  g->n_chk = g->n_sweeps;
+  PP2D_CUDA(cudaMemcpyAsync(b->resid_host.data(), b->resid, b->count * sizeof(uint32_t),
+                            cudaMemcpyDeviceToHost, g->stream));
+  PP2D_CUDA(cudaStreamSynchronize(g->stream));
+  return PP2D_OK;
+}
+
+// Snapshot of the instances in `list` into their result slots; FREEZE: they
+// just stopped (b->frozen already says so) and leave the live grid.
+template <bool FREEZE>
+static int batch_snapshot(pp2d_mdp_batch* b, const std::vector<uint32_t>& list) {
+  pp2d_mdp* g = b->grid;
+  PP2D_TRY_MDP(upload_list(b, list));
+  BatchFreezeParams p;
+  memset(&p, 0, sizeof(p));
+  p.j[0] = g->j[0]; p.j[1] = g->j[1]; p.cur = g->cur;
+  p.code = g->code; p.action = g->action;
+  p.res_cost = b->res_cost; p.res_action = b->res_action;
+  p.list = b->list; p.n_list = (int)list.size();
+  p.W = (int)b->W; p.H = (int)b->H; p.pitch = g->pitch;
+  p.trapped = trapped_cost(g, g->n_sweeps);
+  p.need = nullptr;
+  if (FREEZE) {
+    PP2D_CUDA(cudaMemcpyAsync(b->frozen_dev, b->frozen.data(), b->count,
+                              cudaMemcpyHostToDevice, g->stream));
+    p.frozen = b->frozen_dev;
+    p.count = (int)b->count;
+    p.Htot = (int)g->H;
+    p.n_strips = ((int)b->W + StripGeom<2, 2>::S - 1) / StripGeom<2, 2>::S;
+    // the mask the next fused row-block launch reads (seeded by the arg-min
+    // launch that ended the batch); without one that launch runs every unit
+    if (g->need_valid) {
+      p.need = g->need[g->need_rot];
+      p.rows_per_unit = g->need_rows_per_unit;
+      p.n_rb = g->need_units / p.n_strips;
+    }
+  }
+  const size_t work = std::max<size_t>((size_t)list.size() * b->H * b->W, (size_t)p.n_rb);
+  const int grid = (int)std::min<size_t>((work + 255) / 256, (size_t)g->sm_count * 16);
+  mdp_batch_freeze_kernel<FREEZE><<<std::max(grid, 1), 256, 0, g->stream>>>(p);
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  PP2D_CUDA(cudaGetLastError());
+  return PP2D_OK;
+}
+
+}  // namespace pp2d
+
+extern "C" {
+
+int pp2d_mdp_batch_create(uint32_t height, uint32_t width, uint32_t count, const uint8_t* maps,
+                          size_t map_stride, const uint32_t* goals_xy, float gamma,
+                          pp2d_mdp_batch** out) {
+  if (!out) return fail(PP2D_ERR_INVALID, "out is NULL");
+  *out = nullptr;
+  PP2D_TRY_MDP(batch_check(height, width, count, maps, map_stride, goals_xy));
+  const uint32_t rows = count * (height + 1) - 1;
+  const size_t hw = (size_t)height * width;
+  pp2d_mdp* g = nullptr;
+  // room for one map per instance whatever this call passes: a later reset
+  // may switch from a shared map to per-instance maps
+  PP2D_TRY_MDP(make_handle(rows, width, gamma, 0, rows, false, (size_t)count * hw, &g));
+  pp2d_mdp_batch* b = new (std::nothrow) pp2d_mdp_batch;
+  if (!b) { pp2d_mdp_destroy(g); return fail(PP2D_ERR_INVALID, "out of host memory"); }
+  b->grid = g;
+  b->H = height; b->W = width; b->count = count;
+  b->has_occ.assign(count, 0);
+  b->frozen.assign(count, 0);
+  b->stop_sweeps.assign(count, 0);
+  b->resid_host.assign(count, 0);
+  int rc = [&]() -> int {
+    PP2D_CUDA(cudaMalloc(&b->goals, 2 * sizeof(uint32_t) * count));
+    PP2D_CUDA(cudaMalloc(&b->has_occ_dev, count));
+    PP2D_CUDA(cudaMalloc(&b->frozen_dev, count));
+    PP2D_CUDA(cudaMalloc(&b->list, count * sizeof(uint32_t)));
+    PP2D_CUDA(cudaMalloc(&b->resid, count * sizeof(uint32_t)));
+    PP2D_CUDA(cudaMalloc(&b->res_cost, count * hw * sizeof(float)));
+    PP2D_CUDA(cudaMalloc(&b->res_action, count * hw));
+    return batch_upload(b, maps, map_stride, goals_xy);
+  }();
+  if (rc != PP2D_OK) { pp2d_mdp_batch_destroy(b); return rc; }
+  *out = b;
+  return PP2D_OK;
+}
+
+int pp2d_mdp_batch_reset(pp2d_mdp_batch* h, const uint8_t* maps, size_t map_stride,
+                         const uint32_t* goals_xy) {
+  if (!h) return fail(PP2D_ERR_INVALID, "handle is NULL");
+  PP2D_TRY_MDP(batch_check(h->H, h->W, h->count, maps, map_stride, goals_xy));
+  return batch_upload(h, maps, map_stride, goals_xy);
+}
+
+void pp2d_mdp_batch_destroy(pp2d_mdp_batch* h) {
+  if (!h) return;
+  if (h->grid) cudaStreamSynchronize(h->grid->stream);
+  cudaFree(h->goals); cudaFree(h->has_occ_dev); cudaFree(h->frozen_dev); cudaFree(h->list);
+  cudaFree(h->resid); cudaFree(h->res_cost); cudaFree(h->res_action);
+  pp2d_mdp_destroy(h->grid);
+  delete h;
+}
+
+int pp2d_mdp_batch_set_stream(pp2d_mdp_batch* h, void* stream) {
+  if (!h) return fail(PP2D_ERR_INVALID, "handle is NULL");
+  return pp2d_mdp_set_stream(h->grid, stream);
+}
+
+int pp2d_mdp_batch_sweeps(pp2d_mdp_batch* h, uint32_t n) {
+  if (!h) return fail(PP2D_ERR_INVALID, "handle is NULL");
+  if (h->solved)
+    return fail(PP2D_ERR_STATE, "the batch was solved (its instances stopped at their own "
+                                "sweep counts): call pp2d_mdp_batch_reset first");
+  return pp2d_mdp_sweeps(h->grid, n);
+}
+
+int pp2d_mdp_batch_residual(pp2d_mdp_batch* h, float* out) {
+  if (!h || !out) return fail(PP2D_ERR_INVALID, "NULL argument");
+  if (h->solved)
+    return fail(PP2D_ERR_STATE, "the batch was solved: call pp2d_mdp_batch_reset first");
+  std::vector<uint32_t> all(h->count);
+  for (uint32_t k = 0; k < h->count; ++k) all[k] = k;
+  PP2D_TRY_MDP(batch_residual(h, all));
+  memcpy(out, h->resid_host.data(), h->count * sizeof(float));
+  return PP2D_OK;
+}
+
+int pp2d_mdp_batch_solve(pp2d_mdp_batch* h, uint32_t* sweeps_out, double* residuals,
+                         uint32_t max_residuals) {
+  if (!h) return fail(PP2D_ERR_INVALID, "handle is NULL");
+  if (h->solved)
+    return fail(PP2D_ERR_STATE, "the batch was solved: call pp2d_mdp_batch_reset first");
+  // pp2d_mdp_solve per instance (path_planning_2d.cu:219-263), all instances
+  // in the same launches; an instance leaves after its first batch of 100
+  // sweeps whose residual meets the rule.
+  pp2d_mdp* g = h->grid;
+  const double max_optimal_cost = 5.0 / (1.0 - g->gamma);
+  std::vector<uint32_t> active(h->count), still, stopped;
+  for (uint32_t k = 0; k < h->count; ++k) active[k] = k;
+  uint32_t batch = 0, total = 0;
+  while (!active.empty()) {
+    PP2D_TRY_MDP(pp2d_mdp_sweeps(g, 100));
+    total += 100;
+    PP2D_TRY_MDP(batch_residual(h, active));
+    still.clear();
+    stopped.clear();
+    for (uint32_t k : active) {
+      float r;
+      memcpy(&r, &h->resid_host[k], sizeof(float));
+      const double cost_inf_norm = r;
+      if (residuals && batch < max_residuals)
+        residuals[(size_t)k * max_residuals + batch] = cost_inf_norm;
+      if (cost_inf_norm > max_optimal_cost * 1e-3) {
+        still.push_back(k);
+      } else {
+        stopped.push_back(k);
+        h->frozen[k] = 1;
+        h->stop_sweeps[k] = g->n_sweeps;
+        if (sweeps_out) sweeps_out[k] = total;
+      }
+    }
+    if (!stopped.empty()) PP2D_TRY_MDP(batch_snapshot<true>(h, stopped));
+    active.swap(still);
+    ++batch;
+  }
+  h->solved = true;
+  PP2D_CUDA(cudaStreamSynchronize(g->stream));
+  return PP2D_OK;
+}
+
+int pp2d_mdp_batch_download(pp2d_mdp_batch* h, uint32_t first, uint32_t n, float* cost,
+                            uint8_t* action) {
+  if (!h) return fail(PP2D_ERR_INVALID, "handle is NULL");
+  if (first >= h->count || n > h->count - first)
+    return fail(PP2D_ERR_INVALID, "instances [%u, %llu) outside the batch of %u", first,
+                (unsigned long long)first + n, h->count);
+  if (n == 0 || (!cost && !action)) return PP2D_OK;
+  pp2d_mdp* g = h->grid;
+  // instances still in the live grid are exported into their result slots;
+  // the slots of frozen instances hold their snapshots
+  std::vector<uint32_t> live;
+  for (uint32_t k = first; k < first + n; ++k)
+    if (!h->frozen[k]) live.push_back(k);
+  if (!live.empty()) PP2D_TRY_MDP(batch_snapshot<false>(h, live));
+  const size_t hw = (size_t)h->H * h->W;
+  if (cost)
+    PP2D_CUDA(cudaMemcpyAsync(cost, h->res_cost + first * hw, n * hw * sizeof(float),
+                              cudaMemcpyDeviceToHost, g->stream));
+  if (action)
+    PP2D_CUDA(cudaMemcpyAsync(action, h->res_action + first * hw, n * hw,
+                              cudaMemcpyDeviceToHost, g->stream));
+  PP2D_CUDA(cudaStreamSynchronize(g->stream));
+  return PP2D_OK;
+}
+
+int pp2d_mdp_batch_plan(pp2d_mdp_batch* h, const uint32_t* instance, const float* beliefs,
+                        uint32_t n, uint8_t* actions) {
+  if (!h || !instance || !beliefs || !actions) return fail(PP2D_ERR_INVALID, "NULL argument");
+  for (uint32_t i = 0; i < n; ++i)
+    if (instance[i] >= h->count)
+      return fail(PP2D_ERR_INVALID, "belief %u names instance %u of a batch of %u", i,
+                  instance[i], h->count);
+  if (n == 0) return PP2D_OK;
+  pp2d_mdp* g = h->grid;
+  const size_t hw = (size_t)h->H * h->W;
+  // action grid of each belief's instance: its snapshot once frozen, else its
+  // rows of the live grid (H*W bytes either way)
+  std::vector<const uint8_t*> bases(n);
+  for (uint32_t i = 0; i < n; ++i) {
+    const uint32_t k = instance[i];
+    bases[i] = h->frozen[k] ? h->res_action + k * hw
+                            : g->action + (size_t)k * (h->H + 1) * h->W;
+  }
+  float* d_b = nullptr;
+  const uint8_t** d_base = nullptr;
+  uint8_t* d_a = nullptr;
+  int rc = [&]() -> int {
+    PP2D_CUDA(cudaMalloc(&d_b, hw * n * sizeof(float)));
+    PP2D_CUDA(cudaMalloc(&d_base, n * sizeof(uint8_t*)));
+    PP2D_CUDA(cudaMalloc(&d_a, n));
+    PP2D_CUDA(cudaMemcpyAsync(d_b, beliefs, hw * n * sizeof(float), cudaMemcpyHostToDevice,
+                              g->stream));
+    PP2D_CUDA(cudaMemcpyAsync(d_base, bases.data(), n * sizeof(uint8_t*),
+                              cudaMemcpyHostToDevice, g->stream));
+    mdp_batch_plan_kernel<<<n, 256, 0, g->stream>>>(d_b, hw, d_base, d_a);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    PP2D_CUDA(cudaGetLastError());
+    PP2D_CUDA(cudaMemcpyAsync(actions, d_a, n, cudaMemcpyDeviceToHost, g->stream));
+    PP2D_CUDA(cudaStreamSynchronize(g->stream));
+    return PP2D_OK;
+  }();
+  cudaFree(d_b);
+  cudaFree(d_base);
+  cudaFree(d_a);
+  return rc;
+}
+
+int pp2d_mdp_batch_waypoints(pp2d_mdp_batch* h, uint32_t k, uint32_t sx, uint32_t sy,
+                             uint32_t* cells, uint32_t max_len, uint32_t* n_out) {
+  if (!h || !cells || !n_out) return fail(PP2D_ERR_INVALID, "NULL argument");
+  if (k >= h->count)
+    return fail(PP2D_ERR_INVALID, "instance %u outside the batch of %u", k, h->count);
+  if (sx >= h->W || sy >= h->H)
+    return fail(PP2D_ERR_INVALID, "start (%u %u) outside the map", sx, sy);
+  // instance k's action grid: its snapshot once frozen, else its rows of the
+  // live grid (H*W bytes either way, as in pp2d_mdp_batch_plan)
+  const size_t hw = (size_t)h->H * h->W;
+  const uint8_t* src = h->frozen[k] ? h->res_action + k * hw
+                                    : h->grid->action + (size_t)k * (h->H + 1) * h->W;
+  std::vector<uint8_t> a(hw);
+  PP2D_CUDA(cudaMemcpyAsync(a.data(), src, hw, cudaMemcpyDeviceToHost, h->grid->stream));
+  PP2D_CUDA(cudaStreamSynchronize(h->grid->stream));
+  *n_out = rollout(a.data(), h->W, h->H, sx, sy, cells, max_len);
+  return PP2D_OK;
+}
+
+int pp2d_mdp_batch_sweep_counts(const pp2d_mdp_batch* h, uint32_t* out) {
+  if (!h || !out) return fail(PP2D_ERR_INVALID, "NULL argument");
+  for (uint32_t k = 0; k < h->count; ++k)
+    out[k] = h->frozen[k] ? h->stop_sweeps[k] : h->grid->n_sweeps;
+  return PP2D_OK;
+}
+
+int pp2d_mdp_batch_work_counters(pp2d_mdp_batch* h, uint64_t out[2]) {
+  if (!h || !out) return fail(PP2D_ERR_INVALID, "NULL argument");
+  return pp2d_mdp_work_counters(h->grid, out);
 }
 
 }  // extern "C"

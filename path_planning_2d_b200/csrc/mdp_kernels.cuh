@@ -1505,13 +1505,9 @@ __global__ void mdp_export_kernel(const float* __restrict__ j,
 }
 
 // MdpPathPlanning2d::beliefCallback (path_planning_2d.cu:168-189): index of
-// the first strict maximum of the belief starting from (0.0f, index 0), then
-// the action stored there.  One CTA per belief.
-__global__ void __launch_bounds__(256)
-mdp_plan_kernel(const float* __restrict__ beliefs, size_t n,
-                const uint8_t* __restrict__ action, uint8_t* __restrict__ out,
-                unsigned long long* __restrict__ out_index) {
-  const float* b = beliefs + (size_t)blockIdx.x * n;
+// the first strict maximum of the belief b[0 .. n) starting from (0.0f,
+// index 0), valid in thread 0 of a 256-thread CTA.
+__device__ __forceinline__ unsigned long long belief_mode(const float* __restrict__ b, size_t n) {
   float bm = 0.0f;
   unsigned long long bi = 0;
   for (size_t i = threadIdx.x; i < n; i += blockDim.x) {
@@ -1529,16 +1525,211 @@ mdp_plan_kernel(const float* __restrict__ beliefs, size_t n,
   __shared__ unsigned long long si[8];
   if ((threadIdx.x & 31) == 0) { sv[threadIdx.x >> 5] = bm; si[threadIdx.x >> 5] = bi; }
   __syncthreads();
-  if (threadIdx.x == 0) {
+  if (threadIdx.x == 0)
     for (int i = 1; i < 8; ++i)
       if (sv[i] > bm || (sv[i] == bm && si[i] < bi)) { bm = sv[i]; bi = si[i]; }
-    // all beliefs <= 0: the reference keeps index 0.
-    const unsigned long long mode = bm > 0.0f ? bi : 0;
+  // all beliefs <= 0: the reference keeps index 0.
+  return bm > 0.0f ? bi : 0;
+}
+
+// The action at the belief mode.  One CTA per belief.
+__global__ void __launch_bounds__(256)
+mdp_plan_kernel(const float* __restrict__ beliefs, size_t n,
+                const uint8_t* __restrict__ action, uint8_t* __restrict__ out,
+                unsigned long long* __restrict__ out_index) {
+  const unsigned long long mode = belief_mode(beliefs + (size_t)blockIdx.x * n, n);
+  if (threadIdx.x == 0) {
     // (a multi-GPU handle keeps the action grid spread over its devices: the
     // cell index goes back and the host looks the action up)
     if (action != nullptr) out[blockIdx.x] = action[mode];
     else out_index[blockIdx.x] = mode;
   }
+}
+
+// ---------------------------------------------------------------------------
+// Batches of equal-size instances (pp2d_mdp_batch_*, DESIGN.md section 4).
+// Instance k owns rows [k*(H+1), k*(H+1)+H) of one tall grid of
+// count*(H+1)-1 rows; the row between two instances is an occupied separator
+// whose J stays +0, so the fused sweep kernel runs the tall grid unchanged.
+struct BatchCodeParams {
+  const uint8_t* maps;   // count maps of H*W bytes back to back, or one shared map
+  size_t map_stride;     // H*W, or 0 for the shared map
+  const uint32_t* goals; // [count][2]: (x, y) of each instance
+  uint16_t* code;        // code plane of the tall grid
+  int W, H, count, pitch, rows_phys;
+};
+
+// CodeParams of the instance that owns tall row gy, and gy's row ly in it.
+// Rows above the first instance belong to instance 0 and rows below the last
+// one to the last instance; like a separator (ly == H) they lie outside the
+// instance's rows [0, H) and so read as out of map = occupied.
+__device__ __forceinline__ CodeParams batch_row(const BatchCodeParams& p, int gy, int& ly) {
+  const int k = min(gy < 0 ? 0 : gy / (p.H + 1), p.count - 1);
+  ly = gy - k * (p.H + 1);
+  CodeParams c;
+  c.occ = p.maps + (size_t)k * p.map_stride;
+  c.code = p.code;
+  c.W = p.W;
+  c.Htot = p.H;
+  c.pitch = p.pitch;
+  c.rows_phys = p.rows_phys;
+  c.row_begin = 0;
+  c.occ_row0 = 0;
+  c.occ_rows = p.H;
+  c.gx = (int)__ldg(p.goals + 2 * k);
+  c.gy = (int)__ldg(p.goals + 2 * k + 1);
+  return c;
+}
+
+// code_march on the tall grid: every row is built from the map and goal of
+// its own instance with the single-grid occ_mask6 / cell_codes4.
+template <bool FAST>
+__device__ __forceinline__ void batch_code_march(const BatchCodeParams& p, int c0, int r0) {
+  const int x0 = c0 - kPadLeft;
+  const int r1 = min(r0 + kCodeRows, p.rows_phys);
+  auto mask = [&](int gy) {
+    int ly;
+    const CodeParams c = batch_row(p, gy, ly);
+    return occ_mask6<FAST>(c, x0, ly);
+  };
+  int gy = r0 - kPadRows;
+  uint32_t m0 = mask(gy - 1), m1 = mask(gy);
+  for (int r = r0; r < r1; ++r, ++gy) {
+    const uint32_t m2 = mask(gy + 1);
+    int ly;
+    const CodeParams c = batch_row(p, gy, ly);
+    uint32_t code[4];
+    cell_codes4(c, x0, ly, m0, m1, m2, code);
+    *reinterpret_cast<uint2*>(p.code + (size_t)r * p.pitch + c0) =
+        make_uint2(code[0] | (code[1] << 16), code[2] | (code[3] << 16));
+    m0 = m1;
+    m1 = m2;
+  }
+}
+
+// grid: (ceil(pitch / 4 / kCodeThreads), any); blocks stride over the
+// kCodeRows row groups.
+__global__ void __launch_bounds__(kCodeThreads) mdp_batch_code_kernel(const BatchCodeParams p) {
+  const int c0 = 4 * (blockIdx.x * kCodeThreads + threadIdx.x);
+  if (c0 >= p.pitch) return;
+  const int x0 = c0 - kPadLeft;
+  // instance bases are H*W apart: 4-aligned whenever W is
+  const bool fast = (p.W & 3) == 0 && (x0 & 3) == 0 && x0 >= 0 && x0 + 3 < p.W &&
+                    (reinterpret_cast<uintptr_t>(p.maps) & 3u) == 0;
+  for (int r0 = blockIdx.y * kCodeRows; r0 < p.rows_phys; r0 += gridDim.y * kCodeRows) {
+    if (fast) batch_code_march<true>(p, c0, r0);
+    else batch_code_march<false>(p, c0, r0);
+  }
+}
+
+// Per-instance max |J - Jchk| over the rows of the instances in `list` (the
+// separators are not read), then Jchk = J there: mdp_residual_kernel
+// segmented by instance.  blocks_per CTAs serve one instance: block b takes
+// instance list[b / blocks_per].  The floor (the change of the occupied
+// cells' closed form) counts for the instances whose map has an occupied cell.
+__global__ void __launch_bounds__(256)
+mdp_batch_residual_kernel(const float* __restrict__ j, float* __restrict__ chk,
+                          const uint32_t* __restrict__ list, int blocks_per, int H, int pitch,
+                          uint32_t floor_bits, const uint8_t* __restrict__ has_occ,
+                          uint32_t* result) {
+  const uint32_t k = list[blockIdx.x / blocks_per];
+  const int part = (int)(blockIdx.x % blocks_per);
+  const size_t off = ((size_t)k * (H + 1) + kPadRows) * pitch;
+  const float4* __restrict__ a4 = reinterpret_cast<const float4*>(j + off);
+  float4* __restrict__ b4 = reinterpret_cast<float4*>(chk + off);
+  const size_t n4 = (size_t)H * pitch / 4;
+  float m = has_occ[k] ? __uint_as_float(floor_bits) : 0.0f;
+  for (size_t i = (size_t)part * blockDim.x + threadIdx.x; i < n4;
+       i += (size_t)blocks_per * blockDim.x) {
+    const float4 a = a4[i];
+    const float4 b = b4[i];
+    m = fmaxf(m, fmaxf(fmaxf(fabsf(a.x - b.x), fabsf(a.y - b.y)),
+                       fmaxf(fabsf(a.z - b.z), fabsf(a.w - b.w))));
+    b4[i] = a;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  __shared__ float wm[8];
+  if ((threadIdx.x & 31) == 0) wm[threadIdx.x >> 5] = m;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int i = 1; i < 8; ++i) m = fmaxf(m, wm[i]);
+    atomicMax(result + k, __float_as_uint(m));
+  }
+}
+
+struct BatchFreezeParams {
+  float* j[2];             // both J planes of the tall grid; j[cur] holds J_n
+  int cur;
+  uint16_t* code;
+  const uint8_t* action;   // dense action grid of the tall grid
+  float* res_cost;         // [count][H][W]
+  uint8_t* res_action;     // [count][H][W]
+  const uint32_t* list;    // instances to snapshot
+  int n_list;
+  int W, H, pitch;
+  float trapped;           // J_n of an occupied cell
+  // FREEZE, mask part: NULL = no valid mask to clear
+  uint32_t* need;          // the mask the next fused row-block launch reads
+  const uint8_t* frozen;   // [count]: 1 = instance stopped
+  int count, Htot, n_strips, rows_per_unit, n_rb;
+};
+
+// Snapshot of the instances in `list` into their result slots: J with the
+// occupied cells at `trapped`, and the action grid (the dense export of
+// mdp_export_kernel, one slot per instance).  FREEZE (instances that just met
+// the stopping rule):
+//   (a) after the snapshot their rows of the tall grid become occupied rows:
+//       code = padding, J = 0 in both planes.  Their live values are never
+//       read again, and a unit made of such rows and separators computes
+//       +0 from +0, so it never marks its neighbours when it runs;
+//   (b) the bits of every unit whose rows all lie in stopped instances and
+//       separators are cleared in `need`.
+// One thread per cell, then one thread per row block (grid-stride loops).
+template <bool FREEZE>
+__global__ void __launch_bounds__(256) mdp_batch_freeze_kernel(const BatchFreezeParams p) {
+  const size_t hw = (size_t)p.H * p.W;
+  const size_t cells = hw * (size_t)p.n_list;
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  const size_t t0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  for (size_t t = t0; t < cells; t += stride) {
+    const uint32_t k = p.list[t / hw];
+    const size_t c = t % hw;
+    const int y = (int)(c / p.W), x = (int)(c - (size_t)y * p.W);
+    const size_t ty = (size_t)k * (p.H + 1) + y;     // row in the tall grid
+    const size_t q = (ty + kPadRows) * p.pitch + x + kPadLeft;
+    const size_t dst = (size_t)k * hw + c;
+    p.res_cost[dst] = (p.code[q] & kCodeOccBit) ? p.trapped : p.j[p.cur][q];
+    p.res_action[dst] = p.action[ty * p.W + x];
+    if (FREEZE) {
+      p.code[q] = (uint16_t)kCodeOccBit;
+      p.j[0][q] = 0.0f;
+      p.j[1][q] = 0.0f;
+    }
+  }
+  if (!FREEZE || p.need == nullptr) return;
+  for (size_t rb = t0; rb < (size_t)p.n_rb; rb += stride) {
+    const int y0 = (int)rb * p.rows_per_unit;
+    const int y1 = min(y0 + p.rows_per_unit, p.Htot);
+    // instances with a row in [y0, y1): a separator row belongs to none
+    int k0 = y0 / (p.H + 1), k1 = (y1 - 1) / (p.H + 1);
+    if (y0 - k0 * (p.H + 1) == p.H) ++k0;
+    if ((y1 - 1) - k1 * (p.H + 1) == p.H) --k1;
+    bool all_frozen = true;
+    for (int k = k0; k <= k1 && all_frozen; ++k) all_frozen = p.frozen[k] != 0;
+    if (!all_frozen) continue;
+    const int u0 = (int)rb * p.n_strips;
+    for (int w = u0 >> 5; w <= (u0 + p.n_strips - 1) >> 5; ++w)
+      atomicAnd(p.need + w, ~unit_range_bits(w, u0, u0 + p.n_strips));
+  }
+}
+
+// mdp_plan_kernel with an action grid per belief (H*W bytes at bases[i]).
+__global__ void __launch_bounds__(256)
+mdp_batch_plan_kernel(const float* __restrict__ beliefs, size_t n,
+                      const uint8_t* const* __restrict__ bases, uint8_t* __restrict__ out) {
+  const unsigned long long mode = belief_mode(beliefs + (size_t)blockIdx.x * n, n);
+  if (threadIdx.x == 0) out[blockIdx.x] = bases[blockIdx.x][mode];
 }
 
 }  // namespace pp2d

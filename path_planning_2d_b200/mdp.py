@@ -264,3 +264,141 @@ class MdpPathPlanning2d:
         h = _lib.Halo()
         _lib.check(self._lib.pp2d_mdp_halo(self._h, ctypes.byref(h)))
         return h
+
+
+class MdpBatchPathPlanning2d:
+    """Many value-iteration instances of one size solved together on one GPU
+    (pp2d_mdp_batch_*): one goal per robot on a shared map, or one map per
+    instance.  Every instance computes bit for bit what MdpPathPlanning2d
+    computes on its map and goal.
+
+    grid_maps: (H, W) shared by all instances, or (K, H, W); goals: K (x, y)
+    pairs."""
+
+    def __init__(self, grid_maps, goals, discount_factor):
+        self.discount_factor = np.float32(discount_factor)
+        self._lib = _lib.load()
+        self._h = ctypes.c_void_p()
+        maps, stride, goals = self._arguments(grid_maps, goals)
+        self.count = goals.shape[0]
+        self.map_height, self.map_width = maps.shape[-2:]
+        _lib.check(self._lib.pp2d_mdp_batch_create(
+            self.map_height, self.map_width, self.count, maps.ctypes.data, stride,
+            goals.ctypes.data, float(self.discount_factor), ctypes.byref(self._h)))
+
+    def _arguments(self, grid_maps, goals, shape=None):
+        maps = np.ascontiguousarray(grid_maps, dtype=np.uint8)
+        goals = np.ascontiguousarray(goals, dtype=np.uint32).reshape(-1, 2)
+        if maps.ndim not in (2, 3):
+            raise ValueError("grid_maps must be (H, W) or (K, H, W)")
+        if maps.ndim == 3 and maps.shape[0] != goals.shape[0]:
+            raise ValueError("one map per goal, or one shared (H, W) map")
+        if shape is not None and (maps.shape[-2:] != shape or goals.shape[0] != self.count):
+            raise ValueError("reset() needs maps of the same shape and the same count")
+        stride = 0 if maps.ndim == 2 else maps.shape[1] * maps.shape[2]
+        return maps, stride, goals
+
+    # -- lifetime ---------------------------------------------------------
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h.value:
+            self._lib.pp2d_mdp_batch_destroy(self._h)
+            self._h = ctypes.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def reset(self, grid_maps, goals):
+        """New maps and goals (same shape and count) on the same buffers."""
+        maps, stride, goals = self._arguments(grid_maps, goals,
+                                              (self.map_height, self.map_width))
+        _lib.check(self._lib.pp2d_mdp_batch_reset(self._h, maps.ctypes.data, stride,
+                                                  goals.ctypes.data))
+
+    # -- solver -----------------------------------------------------------
+    def set_stream(self, cuda_stream_ptr):
+        _lib.check(self._lib.pp2d_mdp_batch_set_stream(self._h, cuda_stream_ptr))
+
+    def sweeps(self, n):
+        """n sweeps of every instance."""
+        _lib.check(self._lib.pp2d_mdp_batch_sweeps(self._h, n))
+
+    def residual(self):
+        """Per-instance inf-norm of the change since the previous call."""
+        out = np.zeros(self.count, dtype=np.float32)
+        _lib.check(self._lib.pp2d_mdp_batch_residual(self._h, out.ctypes.data))
+        return out
+
+    def valueIteration(self, max_batches=64):
+        """The reference's stopping rule per instance; returns (sweeps[K],
+        [inf-norm per batch] for each instance)."""
+        n = np.zeros(self.count, dtype=np.uint32)
+        res = np.zeros((self.count, max_batches), dtype=np.float64)
+        _lib.check(self._lib.pp2d_mdp_batch_solve(self._h, n.ctypes.data, res.ctypes.data,
+                                                  max_batches))
+        return n, [res[k, :min(max_batches, int(n[k]) // 100)].copy()
+                   for k in range(self.count)]
+
+    def sweep_counts(self):
+        out = np.zeros(self.count, dtype=np.uint32)
+        _lib.check(self._lib.pp2d_mdp_batch_sweep_counts(self._h, out.ctypes.data))
+        return out
+
+    def work_counters(self):
+        """(units run, units launched) of the fused two-sweep launches so far."""
+        out = np.zeros(2, dtype=np.uint64)
+        _lib.check(self._lib.pp2d_mdp_batch_work_counters(self._h, out.ctypes.data))
+        return int(out[0]), int(out[1])
+
+    def download(self, instances=None):
+        """(cost[K, H, W], action[K, H, W]) of the instances range(first, stop)
+        given as a range or slice (default: all)."""
+        if instances is None:
+            first, stop = 0, self.count
+        elif isinstance(instances, (range, slice)):
+            first, stop, step = instances.start or 0, instances.stop, instances.step or 1
+            if stop is None:
+                stop = self.count
+            if step != 1:
+                raise ValueError("download() takes a contiguous range of instances")
+        else:
+            first = int(instances)
+            stop = first + 1
+        n = max(stop - first, 0)
+        c = np.empty((n, self.map_height, self.map_width), dtype=np.float32)
+        a = np.empty((n, self.map_height, self.map_width), dtype=np.uint8)
+        _lib.check(self._lib.pp2d_mdp_batch_download(self._h, first, n, c.ctypes.data,
+                                                     a.ctypes.data))
+        return c, a
+
+    # -- online -----------------------------------------------------------
+    def plan_batch(self, instances, beliefs):
+        """Action at the mode of beliefs[i] on the action grid of instances[i]."""
+        idx = np.ascontiguousarray(instances, dtype=np.uint32).reshape(-1)
+        b = np.ascontiguousarray(beliefs, dtype=np.float32).reshape(
+            idx.size, self.map_height * self.map_width) if idx.size else None
+        if idx.size == 0:
+            return np.empty(0, dtype=np.uint8)
+        if b.shape[1] != self.map_height * self.map_width:
+            raise ValueError("belief size != height*width")
+        out = np.empty(idx.size, dtype=np.uint8)
+        _lib.check(self._lib.pp2d_mdp_batch_plan(self._h, idx.ctypes.data, b.ctypes.data,
+                                                 idx.size, out.ctypes.data))
+        return out
+
+    def waypoints(self, k, start, max_len=None):
+        max_len = max_len or self.map_height * self.map_width
+        cells = np.empty(max_len, dtype=np.uint32)
+        n = ctypes.c_uint32()
+        _lib.check(self._lib.pp2d_mdp_batch_waypoints(
+            self._h, int(k), int(start[0]), int(start[1]), cells.ctypes.data, max_len,
+            ctypes.byref(n)))
+        return cells[:n.value].copy()
