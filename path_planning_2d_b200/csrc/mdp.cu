@@ -101,18 +101,8 @@ static void build_lut(float gamma, std::vector<float4>& lut) {
     // reference kernel: FMUL then FFMA).
     return make_float4(g[u0], gamma * p4[u0], g[u1], gamma * p4[u1]);
   };
-#if PP2D_LUT6
-  // table (q, half): pair 2q + half, indexed by the 6 ring bits 4q .. 4q+5 of
-  // which the pair reads bits 2*half .. 2*half+3
-  for (int q = 0; q < 2; ++q)
-    for (int half = 0; half < 2; ++half)
-      for (int f6 = 0; f6 < 64; ++f6) {
-        lut[(q * 2 + half) * 64 + f6] = pair_row(2 * q + half, (f6 >> (2 * half)) & 15);
-      }
-#else
   for (int p = 0; p < 4; ++p)
     for (int f = 0; f < 16; ++f) lut[p * 16 + f] = pair_row(p, f);
-#endif
 }
 
 }  // namespace pp2d
@@ -167,17 +157,14 @@ struct pp2d_mdp {
   uint32_t up_H = 0;
   void* ipc_opened[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
   unsigned int p2p_iter = 0, p2p_expect_top = 0, p2p_expect_bot = 0;
-  int p2p_debug = 0, p2p_edge_rows = 16;
+  int p2p_debug = 0;
   int p2p_edge_short = 20;         // rows the boundary row blocks are shorter (hand-shake cost)
-  bool p2p_publisher = true;       // a warp without rows publishes the flags (PP2D_P2P_PUBLISHER)
   unsigned int p2p_spin_limit = 1u << 24;   // polls (32-256 ns apart) before kFlagError
   // ghost-row contract of a shard without peer-to-peer rows: sweeps that may
   // still run before the caller has to refresh the ghost rows (pp2d_mdp_halo)
   int halo_budget = kPadRows;
-  // tuning knobs (environment overridable, see mdp_config)
-  int cw2 = 2, cw1 = 4, rows_per_unit = 0, prefetch_rows = 6, waves = 1;
-  bool fused_policy = true;   // arg-min sweep as the second half of a fused pair
-  bool pdl = true;            // programmatic dependent launch of the sweep kernels
+  // tuning knobs (environment overridable, read in make_handle)
+  int cw2 = 2, cw1 = 4, rows_per_unit = 0;
   int linear_units = -1;      // -1 = choose per launch, 0 = row blocks, 1 = strip-major runs
   // policy iteration (pp2d_mdp_policy_iteration): evaluation sweeps since the
   // reset; occupied cells then follow J_n = (gamma*J_{n-1}) + 2
@@ -245,6 +232,14 @@ static float occupied_cost(pp2d_mdp* h, uint32_t n) {
   return h->pi_mode ? trapped_cost_pi(h, n) : trapped_cost(h, n);
 }
 
+// CW == 1 kernels: rows ahead of the marching row touched with prefetch.global.L1
+// (the slack rows below the plane bound how far ahead that may reach).
+constexpr int kL1PrefetchRows = 6;
+static_assert(kL1PrefetchRows >= kPrefetch && kL1PrefetchRows <= kSlackRows, "prefetch rows");
+// P2P kernels: rows of a boundary unit marched before it publishes its flag.
+constexpr int kP2pEdgeRows = 16;
+static_assert(kP2pEdgeRows >= kPadRows, "edge rows");
+
 template <int T, int CW, bool POLICY, bool P2P = false>
 static int launch_sweep(pp2d_mdp* h) {
   // strip-major runs exist for the fused kernels at CW = 2 (the ones that
@@ -273,30 +268,20 @@ static int launch_sweep(pp2d_mdp* h) {
   p.lin_len = 0;
   pp2d_mdp::LaunchCache& lc =
       h->launch_cache[T - 1][CW == 1 ? 0 : (CW == 2 ? 1 : 2)][POLICY ? 1 : 0][P2P ? 1 : 0];
-  if (!lc.valid && sweep_smem_bytes<T, CW>() > 0) {
-    PP2D_CUDA(cudaFuncSetAttribute(mdp_sweep_kernel<T, CW, POLICY, P2P, false>,
-                                   cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   (int)sweep_smem_bytes<T, CW>()));
-    if (kHasLin)
-      PP2D_CUDA(cudaFuncSetAttribute(mdp_sweep_kernel<T, CW, POLICY, P2P, kHasLin>,
-                                     cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)sweep_smem_bytes<T, CW>()));
-  }
   if (lc.valid && lc.y_rows == rows) {
     p.lin_len = lc.lin_len;
     p.rows_per_unit = lc.rows_per_unit;
     p.n_units = lc.n_units;
     p.unit_lo = lc.d_unit_lo;
   } else if (rpu <= 0) {
-    // Launch sized to exactly `waves` full waves of resident CTAs (one unit
-    // per warp); the units are equal runs of the strip-major row sequence.
+    // Launch sized to exactly one full wave of resident CTAs (one unit per
+    // warp); the units are equal runs of the strip-major row sequence.
     int ctas_per_sm = 0;
     PP2D_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(
-        &ctas_per_sm, mdp_sweep_kernel<T, CW, POLICY, P2P>, kWarpsPerCta * 32,
-        sweep_smem_bytes<T, CW>()));
+        &ctas_per_sm, mdp_sweep_kernel<T, CW, POLICY, P2P>, kWarpsPerCta * 32, 0));
     if (ctas_per_sm < 1) ctas_per_sm = 1;
     lc.ctas_per_sm = ctas_per_sm;
-    const long long slots = (long long)h->sm_count * ctas_per_sm * kWarpsPerCta * h->waves;
+    const long long slots = (long long)h->sm_count * ctas_per_sm * kWarpsPerCta;
     // (a) whole row blocks per strip: floor(slots / strips) blocks, no restart;
     long long rb = slots / p.n_strips;
     if (rb < 1) rb = 1;
@@ -347,7 +332,7 @@ static int launch_sweep(pp2d_mdp* h) {
         return (long long)lo_out.size() - 1;
       };
       // (one slot stays free for the warp that publishes the flags)
-      const long long avail = slots - (h->p2p_publisher ? 1 : 0);
+      const long long avail = slots - 1;
       double lo_t = (double)total / (double)slots, hi_t = 4.0 * lo_t + 4.0 * (c_edge + c_seg) + 16.0;
       for (int it = 0; it < 24; ++it) {
         const double mid = 0.5 * (lo_t + hi_t);
@@ -374,7 +359,7 @@ static int launch_sweep(pp2d_mdp* h) {
     const int n_rb = (rows + rpu - 1) / rpu;
     p.n_units = p.n_strips * n_rb;
   }
-  p.prefetch_rows = h->prefetch_rows;
+  p.prefetch_rows = kL1PrefetchRows;
   p.gamma = h->gamma * 1.0f;
   p.ga = h->gamma * 0.7f;
   p.gb = h->gamma * 0.1f;
@@ -457,14 +442,14 @@ static int launch_sweep(pp2d_mdp* h) {
     p.expect_top = h->p2p_expect_top;
     p.expect_bot = h->p2p_expect_bot;
     p.p2p_debug = (unsigned int)h->p2p_debug;
-    p.edge_rows = h->p2p_edge_rows;
+    p.edge_rows = kP2pEdgeRows;
     p.spin_limit = h->p2p_spin_limit;
   }
   // P2P: a warp slot of the launch that has no rows publishes the flags (the
   // marching warps then never execute a system fence); without a free slot in
   // the last CTA the last boundary unit does it, as before.
   p.publisher_unit = -1;
-  if (P2P && h->p2p_publisher && p.n_units % kWarpsPerCta != 0) p.publisher_unit = p.n_units;
+  if (P2P && p.n_units % kWarpsPerCta != 0) p.publisher_unit = p.n_units;
   lc.valid = true;
   lc.y_rows = rows;
   lc.lin_len = p.lin_len;
@@ -513,13 +498,12 @@ static int launch_sweep(pp2d_mdp* h) {
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = dim3(grid);
   cfg.blockDim = dim3(warps_per_cta * 32);
-  cfg.dynamicSmemBytes = sweep_smem_bytes<T, CW>();
   cfg.stream = h->stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = h->pdl ? 1 : 0;
+  cfg.numAttrs = 1;
   if constexpr (kHasLin) {
     if (p.lin_len > 0)
       PP2D_CUDA(cudaLaunchKernelEx(&cfg, mdp_sweep_kernel<T, CW, POLICY, P2P, true>, p));
@@ -727,29 +711,15 @@ static int make_handle(uint32_t height, uint32_t width, float gamma, uint32_t ro
   h->trapped.push_back(0.0f);
   h->cw2 = env_int("PP2D_MDP_CW2", 2);
   h->cw1 = env_int("PP2D_MDP_CW1", 4);
-  if (PP2D_TMA) {            // 10 pad columns: the 16-byte per-lane vectors of CW = 4 are misaligned
-    if (h->cw2 == 4) h->cw2 = 2;
-    if (h->cw1 == 4) h->cw1 = 2;
-  }
-  h->fused_policy = env_int("PP2D_MDP_FUSED_POLICY", 1) != 0;
   h->linear_units = env_int("PP2D_MDP_LINEAR_UNITS", -1);
-  h->pdl = env_int("PP2D_MDP_PDL", 1) != 0;
   h->skip = env_int("PP2D_MDP_SKIP", 1) != 0;
   h->rows_per_unit = env_int("PP2D_MDP_ROWS_PER_UNIT", 0);
-  h->prefetch_rows = env_int("PP2D_MDP_PREFETCH_ROWS", 6);
-  h->waves = env_int("PP2D_MDP_WAVES", 1);
   h->p2p_debug = env_int("PP2D_P2P_DEBUG", 0);
-  h->p2p_edge_rows = env_int("PP2D_P2P_EDGE_ROWS", 16);
   {
     const int lim = env_int("PP2D_P2P_SPIN_LIMIT", 1 << 24);
     h->p2p_spin_limit = lim > 0 ? (unsigned int)lim : 1u;
   }
-  if (h->p2p_edge_rows < kPadRows) h->p2p_edge_rows = kPadRows;
   h->p2p_edge_short = env_int("PP2D_P2P_EDGE_SHORT", 20);
-  h->p2p_publisher = env_int("PP2D_P2P_PUBLISHER", 1) != 0;
-  if (h->waves < 1) h->waves = 1;
-  if (h->prefetch_rows < kPrefetch) h->prefetch_rows = kPrefetch;
-  if (h->prefetch_rows > kSlackRows) h->prefetch_rows = kSlackRows;
 
   const size_t owned = (size_t)h->H * width;
   int rc = [&]() -> int {
@@ -857,7 +827,7 @@ static int multi_sweeps(pp2d_mdp* m, uint32_t n, int want_action) {
     const uint32_t k = left >= 2 ? 2 : 1;
     const bool last = left == k;
     const int wa = want_action && last;
-    const bool fused = m->multi_p2p && k == 2 && (!wa || m->parts[0]->fused_policy);
+    const bool fused = m->multi_p2p && k == 2;
     if (!fused && m->multi_p2p && m->fused_pending) PP2D_TRY_MDP(multi_barrier(m));
     for (pp2d_mdp* part : m->parts) {
       PP2D_TRY_MDP(multi_set_device(part));
@@ -1181,10 +1151,10 @@ int pp2d_mdp_sweeps_ex(pp2d_mdp* h, uint32_t n, int want_action) {
                                 "need a pp2d_mdp_reset first");
   // Ghost rows are good for kPadRows sweeps.  Fused peer-to-peer launches
   // refresh the neighbours' ghost rows themselves; everything else (shards
-  // without peer mappings, single sweeps, PP2D_MDP_FUSED_POLICY=0) consumes
-  // the budget until the caller exchanges rows through pp2d_mdp_halo.
+  // without peer mappings, single sweeps) consumes the budget until the caller
+  // exchanges rows through pp2d_mdp_halo.
   const bool has_neighbour = h->sharded && (h->row_begin > 0 || h->row_begin + h->H < h->Htot);
-  const bool p2p_fused = h->p2p && n == 2 && (!want_action || h->fused_policy);
+  const bool p2p_fused = h->p2p && n == 2;
   if (has_neighbour && !p2p_fused) {
     if ((int)n > h->halo_budget)
       return fail(PP2D_ERR_STATE,
@@ -1196,7 +1166,7 @@ int pp2d_mdp_sweeps_ex(pp2d_mdp* h, uint32_t n, int want_action) {
   // last sweep is the arg-min variant, which leaves exactly what the
   // reference holds after n launches of cudaOneStepValueIteration.
   // With n >= 2 the arg-min sweep is the second half of a fused pair.
-  const bool fused_tail = want_action && n >= 2 && h->fused_policy;
+  const bool fused_tail = want_action && n >= 2;
   uint32_t plain = want_action ? n - (fused_tail ? 2 : 1) : n;
   int rc;
   while (plain >= 2) {

@@ -48,63 +48,15 @@ namespace pp2d {
 constexpr int kPadRows = 2;   // ghost rows above and below the owned rows
 constexpr int kSlackRows = 8; // extra rows at the bottom: prefetch may overrun
 constexpr int kPrefetch = 2;  // CW == 1 path: rows held in registers ahead of use
-#ifndef PP2D_KRING
-#define PP2D_KRING 3
-#endif
-constexpr int kRing = PP2D_KRING;  // CW >= 2 path: cp.async ring slots per lane (1, 2, 3 or 6)
-// PP2D_TMA = 1 (experiment, A/B-timed in profiles/): the row ring of the fused
-// CW = 2 kernel is filled by bulk async copies (cp.async.bulk, the TMA engine)
-// issued by one lane per warp and completed on a per-slot mbarrier, instead of
-// per-lane cp.async.  A bulk copy needs 16-byte aligned addresses: with 10 pad
-// columns a warp's 64-float row segment (strip k starts at column 60 k - 2)
-// is aligned; the CW = 4 kernels (16-byte per-lane vectors) then are not, so
-// such a build only runs CW <= 2.
-#ifndef PP2D_TMA
-#define PP2D_TMA 0
-#endif
-constexpr int kPadLeft = PP2D_TMA ? 10 : 8;   // zero columns left of x = 0
-// Table layouts (build-time choice, both give the same bits):
-//   PP2D_LUT6 = 0: 4 tables (one per action pair) x 16 rows (4 ring bits) x 8
-//     lane replicas of one float4 = 8 KB; a cell needs 4 row addresses.
-//   PP2D_LUT6 = 1: two ring-adjacent action pairs share 6 ring bits, so ONE row
-//     address serves both: 2 super-pairs x 2 halves x 64 rows x 8 replicas =
-//     32 KB, 2 row addresses per cell (each SHF + LOP3) instead of 4.
-#ifndef PP2D_LUT6
-#define PP2D_LUT6 0
-#endif
-// PP2D_UWARP = 1: the warp index is read through a shuffle from lane 0, which
-// tells the compiler it is warp-uniform (unit, row counts and loop exits then
-// are, too: no divergence guard in front of the shuffles of the marching loop).
-#ifndef PP2D_UWARP
-#define PP2D_UWARP 1
-#endif
-#if PP2D_LUT6
-constexpr int kLutFloat4 = 2 * 2 * 64 * 8;
-constexpr int kLutAlign = 8192;         // row bits 7..12 + replica bits 4..6 are OR-ed in
-#else
-constexpr int kLutFloat4 = 4 * 16 * 8;  // 4 action pairs x 16 rows x 8 copies
+constexpr int kRing = 3;      // CW >= 2 path: cp.async ring slots per lane (divides the 6-step unroll)
+constexpr int kPadLeft = 8;   // zero columns left of x = 0
+// Table: 4 tables (one per action pair) x 16 rows (4 ring bits) x 8 lane
+// replicas of one float4 = 8 KB; a cell needs 4 row addresses.
+constexpr int kLutFloat4 = 4 * 16 * 8;
 constexpr int kLutAlign = 2048;
-#endif
-// Tuning knobs (tools/sweep_variants.py builds alternates): how the minimum
-// over the 9 actions is taken, warps per CTA and resident CTAs per SM of the
-// fused kernel.
-#ifndef PP2D_MINV
-#define PP2D_MINV 0
-#endif
-// PP2D_ARGMIN_EQ = 1: the arg-min variant takes the minimum with FMNMX3 and
-// finds its first index by equality (see backup()); 0: compare-and-keep chain.
-// (236 against 245 instructions per marching step of the fused arg-min kernel,
-// but the P2P strip-major instantiation then spills two registers: off.)
-#ifndef PP2D_ARGMIN_EQ
-#define PP2D_ARGMIN_EQ 0
-#endif
-#ifndef PP2D_WARPS
-#define PP2D_WARPS 8
-#endif
-#ifndef PP2D_MINCTAS
-#define PP2D_MINCTAS 2
-#endif
-constexpr int kWarpsPerCta = PP2D_WARPS;
+// Fused kernel: 8 warps per CTA, 2 resident CTAs per SM (the other occupancies
+// that were timed are in DESIGN.md section 4).
+constexpr int kWarpsPerCta = 8;
 
 // Code bits.
 constexpr uint32_t kCodeRingMask = 0x3FFu;   // bits 0..9
@@ -216,28 +168,11 @@ __device__ __forceinline__ float backup(float j0, float j1, float j2, float j3,
   float c7 = fmaf(gb, j8, fmaf(ga, j7, fmaf(gb, j6, fmaf(t[2].y, j4, t[2].x))));
   float c8 = fmaf(ga, j8, fmaf(gb, j7, fmaf(gb, j5, fmaf(t[1].w, j4, t[1].z))));
   if (POLICY) {
-#if PP2D_ARGMIN_EQ
-    // path_planning_2d_cuda.cu:244-258 keeps the first strict minimum, u
-    // ascending = the lowest u whose cost equals the minimum.  The minimum is
-    // taken as in the value-only kernel (costs are finite and >= +0: no NaN or
-    // -0 for FMNMX to choose differently), then one compare + select per
-    // action in DESCENDING order, so that the lowest index is written last: 4
-    // FMNMX3 + 8 FSETP + 8 SEL with one live predicate, instead of a chain of
-    // 8 x (FSETP, FSEL, SEL) that keeps 8 predicates alive.
-    const float best = min3(min3(c0, c1, c2), min3(c3, c4, c5), min3(c6, c7, c8));
-    uint32_t a = 8;
-    a = (c7 == best) ? 7u : a;
-    a = (c6 == best) ? 6u : a;
-    a = (c5 == best) ? 5u : a;
-    a = (c4 == best) ? 4u : a;
-    a = (c3 == best) ? 3u : a;
-    a = (c2 == best) ? 2u : a;
-    a = (c1 == best) ? 1u : a;
-    a = (c0 == best) ? 0u : a;
-    act = a;
-    return best;
-#else
     // path_planning_2d_cuda.cu:244-258: first strict minimum, u ascending.
+    // (A compare-and-keep chain: the equality form -- FMNMX3 minimum, then the
+    // lowest index whose cost equals it -- took 236 against 245 instructions
+    // per marching step of the fused arg-min kernel, but the P2P strip-major
+    // instantiation spilled two registers with it.)
     float best = c0;
     uint32_t a = 0;
     if (c1 < best) { best = c1; a = 1; }
@@ -250,22 +185,8 @@ __device__ __forceinline__ float backup(float j0, float j1, float j2, float j3,
     if (c8 < best) { best = c8; a = 8; }
     act = a;
     return best;
-#endif
   } else {
-#if PP2D_MINV == 1
-    return fminf(fminf(fminf(c0, c1), fminf(c2, c3)),
-                 fminf(fminf(fminf(c4, c5), fminf(c6, c7)), c8));
-#elif PP2D_MINV == 2
-    // Costs are finite and >= +0, so their order as floats is their order as
-    // unsigned integers: the 3-input integer minimum (VIMNMX3) gives the same
-    // bits as FMNMX3.
-    const uint32_t m0 = __vimin3_u32(__float_as_uint(c0), __float_as_uint(c1), __float_as_uint(c2));
-    const uint32_t m1 = __vimin3_u32(__float_as_uint(c3), __float_as_uint(c4), __float_as_uint(c5));
-    const uint32_t m2 = __vimin3_u32(__float_as_uint(c6), __float_as_uint(c7), __float_as_uint(c8));
-    return __uint_as_float(__vimin3_u32(m0, m1, m2));
-#else
     return min3(min3(c0, c1, c2), min3(c3, c4, c5), min3(c6, c7, c8));
-#endif
   }
 }
 
@@ -362,23 +283,10 @@ __device__ __forceinline__ float4 lut_row(uint32_t lane_base, uint32_t word) {
 template <bool HI>
 __device__ __forceinline__ void lut_fetch(uint32_t lane_base, uint32_t word,
                                           float4 (&t)[4], float& g4) {
-#if PP2D_LUT6
-  // super-pair 0: ring bits 0..5 (pairs 0 and 1), super-pair 1: ring bits 4..9
-  // (pairs 2 and 3); row offset = 6 bits << 7, the two halves 8 KB apart
-  const uint32_t s0 = HI ? (word >> 9) : (word << 7);
-  const uint32_t a0 = (s0 & 0x1F80u) | lane_base;
-  t[0] = lds128<0>(a0);
-  t[1] = lds128<8192>(a0);
-  const uint32_t s1 = HI ? (word >> 13) : (word << 3);
-  const uint32_t a1 = (s1 & 0x1F80u) | lane_base;
-  t[2] = lds128<16384>(a1);
-  t[3] = lds128<24576>(a1);
-#else
   t[0] = lut_row<HI, 0>(lane_base, word);
   t[1] = lut_row<HI, 1>(lane_base, word);
   t[2] = lut_row<HI, 2>(lane_base, word);
   t[3] = lut_row<HI, 3>(lane_base, word);
-#endif
   // live bit (14 of the code) -> 2.0f (0x40000000); goal, occupied cells and
   // padding -> 0.0f, which makes "stay" cost exactly 0 there (their J is 0).
   g4 = __uint_as_float((HI ? word : (word << 16)) & 0x40000000u);
@@ -415,59 +323,15 @@ __device__ __forceinline__ void lds_codes(uint32_t saddr,
   }
 }
 
-// ---- bulk-copy (TMA) staging helpers (PP2D_TMA builds) -----------------------
-// (lane 0 only, predicated: no divergent branch)
-__device__ __forceinline__ void mbar_init_lane0(int lane, uint32_t bar, uint32_t count) {
-  asm volatile(
-      "{\n"
-      ".reg .pred P0;\n"
-      "setp.eq.s32 P0, %0, 0;\n"
-      "@P0 mbarrier.init.shared::cta.b64 [%1], %2;\n"
-      "}\n" :: "r"(lane), "r"(bar), "r"(count) : "memory");
-}
-// Spin until the phase with the given parity of the barrier has completed.
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred P1;\n"
-      "LAB_WAIT:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n"
-      "@P1 bra DONE;\n"
-      "bra LAB_WAIT;\n"
-      "DONE:\n"
-      "}\n" :: "r"(bar), "r"(parity) : "memory");
-}
-// Lane 0 (predicated, no branch: the warp stays converged for the compiler):
-// expect JB + CB bytes on the barrier and start the two bulk copies.
-template <int JB, int CB>
-__device__ __forceinline__ void tma_fill(int lane, uint32_t bar, uint32_t dst_j, const void* src_j,
-                                         uint32_t dst_c, const void* src_c) {
-  asm volatile(
-      "{\n"
-      ".reg .pred P0;\n"
-      "setp.eq.s32 P0, %0, 0;\n"
-      "@P0 mbarrier.arrive.expect_tx.shared::cta.b64 _, [%1], %6;\n"
-      "@P0 cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%2], [%3], %7, [%1];\n"
-      "@P0 cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%4], [%5], %8, [%1];\n"
-      "}\n"
-      :: "r"(lane), "r"(bar), "r"(dst_j), "l"(src_j), "r"(dst_c), "l"(src_c), "n"(JB + CB),
-         "n"(JB), "n"(CB)
-      : "memory");
-}
-
 template <int T, int CW>
 struct StripGeom {
   static constexpr int HL = (T + CW - 1) / CW;          // halo lanes per side
   static constexpr int S = (32 - 2 * HL) * CW;          // valid columns/strip
   static constexpr int XOFF = -HL * CW;                 // x of lane 0, cell 0
   // cp.async ring: per warp and slot, 32 lanes x (CW floats + CW codes).
-  // (TMA builds: 16 more bytes of codes per slot -- the code segment is copied
-  // from the 16-byte boundary below it -- and kRing mbarriers per warp.)
-  static constexpr int kSlotBytes = 32 * CW * 6 + (PP2D_TMA ? 16 : 0);
+  static constexpr int kSlotBytes = 32 * CW * 6;
   static constexpr int kCodeOff = 32 * CW * 4;
-  static constexpr int kBarOff = kRing * kSlotBytes;
-  static constexpr int kRingBytesPerWarp =
-      (CW >= 2) ? kRing * kSlotBytes + (PP2D_TMA ? 32 : 0) : 0;
+  static constexpr int kRingBytesPerWarp = (CW >= 2) ? kRing * kSlotBytes : 0;
 };
 
 // LIN: units are runs of the strip-major row sequence (see run()); a separate
@@ -476,14 +340,10 @@ struct StripGeom {
 template <int T, int CW, bool POLICY, bool P2P = false, bool LIN = false>
 struct Sweeper {
   using G = StripGeom<T, CW>;
-  // bulk-copy ring: the fused row-block kernel only (one march per warp)
-  static constexpr bool kTma = PP2D_TMA && T == 2 && CW == 2 && !P2P && !LIN;
   // the instantiations that can skip units: they OR the bit difference between
   // J^2 and J^0 of every produced cell into `diff`
   static constexpr bool kSkip = T == 2 && CW == 2 && !P2P && !LIN;
   uint32_t diff = 0;
-  uint32_t ring_base = 0;    // kTma: shared address of this warp's ring (slot 0)
-  int lane_id = 0;
   float A[3][CW + 2];        // J^0 rows y-1, y, y+1 (rotating)
   float B[3][CW + 2];        // J^1 rows y-2, y-1, y (T == 2)
   float4 L[2][CW][4];        // LUT rows of row y (cur) and y-1 (prev)
@@ -517,17 +377,7 @@ struct Sweeper {
     constexpr int a0 = I % 3, a1 = (I + 1) % 3, a2 = (I + 2) % 3;
     constexpr int lc = I % 2, lp = (I + 1) % 2;
     uint32_t cc[(CW + 1) / 2];
-    if constexpr (kTma) {
-      constexpr int slot = I % kRing;
-      // use number (step / kRing) of this slot: its parity is a compile-time
-      // constant because the unrolled period (6) is a multiple of 2 * kRing
-      static_assert(6 % (2 * kRing) == 0 || kRing == 3, "ring depth vs unroll");
-      mbar_wait(ring_base + G::kBarOff + 8 * slot, (I / kRing) & 1);
-      float own[CW];
-      lds_row<CW, slot * G::kSlotBytes>(ring_j, own);
-      lds_codes<CW, slot * G::kSlotBytes + G::kCodeOff>(ring_c, cc);
-      fill_row<CW>(own, A[a2]);
-    } else if constexpr (CW >= 2) {
+    if constexpr (CW >= 2) {
       constexpr int slot = I % kRing;
       // The oldest of the kRing groups in flight (row y+1, codes of row y)
       // has landed in this lane's slot.
@@ -538,10 +388,11 @@ struct Sweeper {
       fill_row<CW>(own, A[a2]);
       // Refill the slot with row y+1+kRing / codes of row y+kRing (the planes
       // have kSlackRows spare rows, so the last steps may run past the end).
-      // (Issued here, right after the slot was read: refilling at the END of the
-      // step saves the three predicated-off LDS ptxas puts in front of the
-      // LDGSTS pair -- 193 instead of 195 instructions per step -- but runs
-      // slower, 64.8 vs 63.4 us per launch: the copy has one step less to land.)
+      // (Issued here, right after the slot was read.  Refilling at the END of
+      // the step was tried: it saved the three predicated-off LDS ptxas puts in
+      // front of the LDGSTS pair -- 193 instead of 195 instructions per step --
+      // but ran slower, 64.8 vs 63.4 us per launch: the copy had one step less
+      // to land.)
       cp_async<CW * 4>(ring_j + slot * G::kSlotBytes, pin);
       cp_async<CW * 2>(ring_c + slot * G::kSlotBytes + G::kCodeOff, pcode);
       cp_async_commit();
@@ -554,10 +405,8 @@ struct Sweeper {
       asm volatile("prefetch.global.L1 [%0];" :: "l"(pin + l1_ahead));
       asm volatile("prefetch.global.L1 [%0];" :: "l"(pcode + l1_ahead));
     }
-    if constexpr (!kTma) {
-      pin += p.pitch;
-      pcode += p.pitch;
-    }
+    pin += p.pitch;
+    pcode += p.pitch;
     // Table rows of row y.
 #pragma unroll
     for (int j = 0; j < CW; ++j) {
@@ -642,17 +491,6 @@ struct Sweeper {
         for (int j = 0; j < (CW + 1) / 2; ++j) cprev[j] = cc[j];
       }
     }
-    if constexpr (kTma) {
-      // Refill the slot read at the top of this step (its values have been
-      // consumed by the arithmetic above) with row y+1+kRing / codes of row
-      // y+kRing; pcode points at the 16-byte boundary below the code segment.
-      constexpr int slot = I % kRing;
-      tma_fill<32 * CW * 4, 32 * CW * 2 + 16>(
-          lane_id, ring_base + G::kBarOff + 8 * slot, ring_base + slot * G::kSlotBytes, pin,
-          ring_base + slot * G::kSlotBytes + G::kCodeOff, pcode);
-      pin += p.pitch;
-      pcode += p.pitch;
-    }
   }
 
   // March over rows [y0, y1) of this lane's columns.  PEER: rows 0,1 / H-2,H-1
@@ -674,27 +512,7 @@ struct Sweeper {
     }
     pin = jin + 2 * pitch;                                  // row ys+1
     pcode = p.code + col + (size_t)(ys + kPadRows) * pitch; // row ys
-    const int total_steps = steps;
-    if constexpr (kTma) {
-      // lane 0's pointers are the warp's row segment; codes are fetched from
-      // the 16-byte boundary below it and read back at that offset
-      const uint32_t coff =
-          __shfl_sync(0xffffffffu, (uint32_t)(reinterpret_cast<uintptr_t>(pcode) & 15u), 0);
-      pcode = reinterpret_cast<const uint16_t*>(reinterpret_cast<const char*>(pcode) - coff);
-      ring_c += coff;
-#pragma unroll
-      for (int d = 0; d < kRing; ++d) mbar_init_lane0(lane_id, ring_base + G::kBarOff + 8 * d, 1);
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-      __syncwarp();
-#pragma unroll
-      for (int d = 0; d < kRing; ++d) {
-        tma_fill<32 * CW * 4, 32 * CW * 2 + 16>(
-            lane_id, ring_base + G::kBarOff + 8 * d, ring_base + d * G::kSlotBytes, pin,
-            ring_base + d * G::kSlotBytes + G::kCodeOff, pcode);
-        pin += pitch;
-        pcode += pitch;
-      }
-    } else if constexpr (CW >= 2) {
+    if constexpr (CW >= 2) {
 #pragma unroll
       for (int d = 0; d < kRing; ++d) {
         cp_async<CW * 4>(ring_j + d * G::kSlotBytes, pin);
@@ -738,15 +556,7 @@ struct Sweeper {
       }
     }
     // Do not leave the slot ring with copies in flight.
-    if constexpr (kTma) {
-      // slot d was filled once by the priming and once by every step j with
-      // j % kRing == d; wait for its last fill (use number fills - 1)
-#pragma unroll
-      for (int d = 0; d < kRing; ++d) {
-        const int fills = 1 + (total_steps > d ? (total_steps - d + kRing - 1) / kRing : 0);
-        mbar_wait(ring_base + G::kBarOff + 8 * d, (uint32_t)(fills - 1) & 1u);
-      }
-    } else if constexpr (CW >= 2) cp_async_wait<0>();
+    if constexpr (CW >= 2) cp_async_wait<0>();
   }
 
   // A unit is a run of `lin_len` rows of the strip-major sequence (strip 0 rows
@@ -802,8 +612,6 @@ struct Sweeper {
     if constexpr (!LIN) {
       l1_ahead = (size_t)(p.prefetch_rows - kPrefetch) * (size_t)p.pitch;
       if constexpr (CW >= 2) {
-        ring_base = ring_j;
-        lane_id = lane;
         ring_j += lane * (CW * 4);
         ring_c += lane * (CW * 2);
       }
@@ -1019,24 +827,9 @@ __device__ __forceinline__ bool unit_plan(const SweepParams& p, int w, int lane,
   return true;
 }
 
-// Dynamic shared memory of a launch (PP2D_LUT6 builds; the 8 KB table keeps
-// its static buffer so that the default build's code is untouched).
-template <int T, int CW>
-constexpr size_t sweep_smem_bytes() {
-#if PP2D_LUT6
-  return (size_t)kLutFloat4 * 16 + kLutAlign + (size_t)kWarpsPerCta * StripGeom<T, CW>::kRingBytesPerWarp;
-#else
-  return 0;
-#endif
-}
-
 // One warp per (column strip, row block) unit; kWarpsPerCta warps per CTA.
 template <int T, int CW, bool POLICY, bool P2P = false, bool LIN = false>
-#ifdef PP2D_MAXNREG
-__global__ void __maxnreg__(PP2D_MAXNREG)
-#else
-__global__ void __launch_bounds__(kWarpsPerCta * 32, (T == 2 && CW == 2) ? PP2D_MINCTAS : 1)
-#endif
+__global__ void __launch_bounds__(kWarpsPerCta * 32, (T == 2 && CW == 2) ? 2 : 1)
 mdp_sweep_kernel(const SweepParams p) {
   // The table must start on a 2 KB boundary of the shared window so that the
   // row offset (bits 7..10) and the lane replica (bits 4..6) can be OR-ed
@@ -1050,12 +843,8 @@ mdp_sweep_kernel(const SweepParams p) {
   // has completed and its writes are visible.  Both are no-ops for a launch
   // without the attribute.
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#if PP2D_LUT6
-  extern __shared__ __align__(16) unsigned char lut_raw[];   // sweep_smem_bytes<T, CW>()
-#else
   __shared__ __align__(16) unsigned char
       lut_raw[kLutFloat4 * 16 + kLutAlign + kWarps * G::kRingBytesPerWarp];
-#endif
   const uint32_t raw_addr = (uint32_t)__cvta_generic_to_shared(lut_raw);
   const uint32_t lut_addr = (raw_addr + (uint32_t)(kLutAlign - 1)) & ~(uint32_t)(kLutAlign - 1);
   float4* lut_s = reinterpret_cast<float4*>(lut_raw + (lut_addr - raw_addr));
@@ -1069,11 +858,10 @@ mdp_sweep_kernel(const SweepParams p) {
   __syncthreads();
   asm volatile("griddepcontrol.wait;" ::: "memory");
   const int lane = threadIdx.x & 31;
-#if PP2D_UWARP
+  // The warp index is read through a shuffle from lane 0, which tells the
+  // compiler it is warp-uniform (unit, row counts and loop exits then are, too:
+  // no divergence guard in front of the shuffles of the marching loop).
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
-#else
-  const int warp = (int)(threadIdx.x >> 5);
-#endif
   const int unit = blockIdx.x * (blockDim.x >> 5) + warp;
   using Sw = Sweeper<T, CW, POLICY, P2P, LIN>;
   if constexpr (P2P) {

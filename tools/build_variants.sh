@@ -1,6 +1,6 @@
 #!/bin/bash
 # Alternate builds of libpp2d.so for tuning experiments: name=flags ...
-# usage: bash tools/build_variants.sh "minv2=-DPP2D_MINV=2" "w4c5=-DPP2D_WARPS=4 -DPP2D_MINCTAS=5"
+# usage: bash tools/build_variants.sh "cs16=-DPP2D_CS_BATCH=16" "evm128=-DPP2D_EVM=128"
 cd "$(dirname "$0")/.."
 mkdir -p build/variants
 for spec in "$@"; do

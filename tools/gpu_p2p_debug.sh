@@ -8,5 +8,3 @@ PP2D_P2P=0 run nccl
 PP2D_P2P_DEBUG=7 run p2p_nothing
 PP2D_P2P_DEBUG=5 run p2p_stores_only
 PP2D_P2P_DEBUG=0 run p2p_full
-PP2D_P2P_DEBUG=0 PP2D_P2P_EDGE_ROWS=8 run p2p_full_edge8
-PP2D_P2P_DEBUG=0 PP2D_P2P_EDGE_ROWS=32 run p2p_full_edge32

@@ -6,7 +6,7 @@ Geometry of the fused row-block launch: strips of 60 useful columns, the row
 blocks that fill the warp slots of one wave (mdp.cu launch_sweep).  The slots
 are SMs x resident CTAs per SM x 8 warps: 148 x 2 x 8 on a B200, where the
 library reads the CTA count from cudaOccupancyMaxActiveBlocksPerMultiprocessor.
-A build or a setting that changes it (other register counts, PP2D_MDP_WAVES,
+A build or a setting that changes it (other register counts,
 PP2D_MDP_ROWS_PER_UNIT) launches another geometry: pass --sms /
 --ctas-per-sm / --rows-per-unit to match it, or the prediction is off.
 

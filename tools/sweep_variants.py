@@ -18,10 +18,9 @@ size = int(sys.argv[1]) if len(sys.argv) > 1 else 4096
 grid, goal = cases.synthetic_map(size, size, 0.20, seed=12345)
 rows = []
 quick = len(sys.argv) > 2
-combos = [(2, 0, 1), (2, 0, 2), (2, 64, 1), (2, 128, 1)]
-for cw2, rpu, pf in combos:
+combos = [(2, 0), (2, 64), (2, 128)]
+for cw2, rpu in combos:
     os.environ["PP2D_MDP_CW2"] = str(cw2)
-    os.environ["PP2D_MDP_WAVES"] = str(pf)
     os.environ["PP2D_MDP_ROWS_PER_UNIT"] = str(rpu)
     with MdpPathPlanning2d(grid, goal, cases.GAMMA) as m:
         m.set_stream(torch.cuda.current_stream().cuda_stream, asynchronous=True)
@@ -37,7 +36,7 @@ for cw2, rpu, pf in combos:
             best = min(best, e0.elapsed_time(e1))
         rate = size * size * 100 / (best * 1e-3)
         rows.append((cw2, rpu, best / 50, rate))
-        print(f"T=2 cw={cw2} rows_per_unit={rpu:4d} waves={pf}  {best/50*1e3:8.1f} us/launch  "
+        print(f"T=2 cw={cw2} rows_per_unit={rpu:4d}  {best/50*1e3:8.1f} us/launch  "
               f"{rate/1e9:8.1f} Gcell/s  {rate*10/6537.6e9:.3f} of HBM roofline", flush=True)
 for cw1 in ([] if quick else [1, 2, 4]):
     os.environ["PP2D_MDP_CW1"] = str(cw1)
