@@ -370,9 +370,32 @@ int pp2d_mdp_batch_residual(pp2d_mdp_batch* h, float* out);
  * instance is frozen: its results are kept aside and its rows stop costing
  * work in the launches that the others still need.  Afterwards sweeps,
  * residual and solve return PP2D_ERR_STATE until pp2d_mdp_batch_reset.
+ * After pp2d_mdp_batch_update, solve runs the instances that are active
+ * (never frozen, or re-activated by the update); sweeps_out[k] and residual
+ * row k are written for those only, and solve returns PP2D_ERR_STATE when
+ * none is active.  sweeps and residual return PP2D_ERR_STATE while any
+ * instance is frozen.
  */
 int pp2d_mdp_batch_solve(pp2d_mdp_batch* h, uint32_t* sweeps_out, double* residuals,
                          uint32_t max_residuals);
+/*
+ * pp2d_mdp_update_map on the instances instances[0 .. n) (distinct indices):
+ * instance instances[i] gets the map at maps + i*map_stride (map_stride == 0:
+ * one map for all n) and the goal (goals_xy[2i], goals_xy[2i+1]), and keeps
+ * its solution.  With n_k its sweep count (pp2d_mdp_batch_sweep_counts), J'
+ * is its download just before the call with every occupied cell of the new
+ * map at trapped(n_k) and the new goal at 0.  n_k carries on, the next
+ * residual of the instance measures the change since the update, and its
+ * action grid (plan, way-points) stays as it was until its next sweep.  An
+ * instance frozen by a solve becomes active again from its result.  Instances
+ * not listed are left bit for bit as they were; frozen ones stay frozen.
+ * PP2D_ERR_INVALID for NULL pointers, an index >= count or listed twice, a
+ * non-zero map_stride below height*width or a goal outside the map;
+ * PP2D_ERR_GOAL_OCCUPIED for an occupied goal (messages name the instance).
+ * On an error the handle is unchanged; n == 0 does nothing.
+ */
+int pp2d_mdp_batch_update(pp2d_mdp_batch* h, const uint32_t* instances, uint32_t n,
+                          const uint8_t* maps, size_t map_stride, const uint32_t* goals_xy);
 /* Results of instances [first, first+n): cost [n][height][width] floats
  * (occupied cells filled in as by pp2d_mdp_download), action
  * [n][height][width] bytes; either may be NULL. */

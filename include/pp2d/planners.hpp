@@ -295,6 +295,31 @@ class MdpBatchPathPlanning2d {
                           res.begin() + (size_t)k * cap + std::min(cap, sweeps[k] / 100));
   }
 
+  // Re-plan the listed instances on new maps and goals from their current
+  // solutions (pp2d_mdp_batch_update), then valueIteration() of the instances
+  // that are active; sweeps[k] and residuals[k] of the others are 0 and empty.
+  // maps: one height*width map shared by the listed instances, or one per
+  // instance back to back.  Returns false and changes nothing on a bad
+  // argument or an occupied goal.
+  bool updateMap(const std::vector<uint32_t>& instances, const std::vector<uint8_t>& maps,
+                 const std::vector<std::array<uint32_t, 2>>& goals) {
+    const size_t hw = (size_t)height_ * width_;
+    if (goals.size() != instances.size() ||
+        (maps.size() != hw && maps.size() != hw * instances.size()))
+      return false;
+    if (instances.empty()) return true;
+    const int rc = pp2d_mdp_batch_update(batch_, instances.data(), (uint32_t)instances.size(),
+                                         maps.data(), maps.size() == hw ? 0 : hw,
+                                         goals.data()->data());
+    if (rc == PP2D_ERR_GOAL_OCCUPIED || rc == PP2D_ERR_INVALID) {
+      std::fprintf(stderr, "%s\n", pp2d_last_error());
+      return false;
+    }
+    PP2D_CHECK(rc);
+    valueIteration();
+    return true;
+  }
+
   std::vector<float> optimalCost(uint32_t k) const {
     std::vector<float> c((size_t)height_ * width_);
     PP2D_CHECK(pp2d_mdp_batch_download(batch_, k, 1, c.data(), nullptr));

@@ -71,6 +71,7 @@ SIGNATURES = {
     "pp2d_mdp_batch_sweeps": (_i, [_vp, _u32]),
     "pp2d_mdp_batch_residual": (_i, [_vp, _vp]),
     "pp2d_mdp_batch_solve": (_i, [_vp, _vp, _vp, _u32]),
+    "pp2d_mdp_batch_update": (_i, [_vp, _vp, _u32, _vp, ctypes.c_size_t, _vp]),
     "pp2d_mdp_batch_download": (_i, [_vp, _u32, _u32, _vp, _vp]),
     "pp2d_mdp_batch_plan": (_i, [_vp, _vp, _vp, _u32, _vp]),
     "pp2d_mdp_batch_waypoints": (_i, [_vp, _u32, _u32, _u32, _vp, _u32,

@@ -1634,17 +1634,24 @@ struct pp2d_mdp_batch {
   uint32_t H = 0, W = 0, count = 0;
   size_t map_stride = 0;           // device: H*W, or 0 for one shared map
   uint32_t* goals = nullptr;       // device [count][2]
-  uint8_t* has_occ_dev = nullptr;  // device [count]
+  std::vector<uint32_t> goals_host;
   std::vector<uint8_t> has_occ;    // instance k's own map has an occupied cell
   uint8_t* frozen_dev = nullptr;   // device [count]
   std::vector<uint8_t> frozen;     // instance k met the stopping rule in solve
+  uint32_t n_frozen = 0;
   std::vector<uint32_t> stop_sweeps;   // sweep count of a frozen instance
-  uint32_t* list = nullptr;        // device [count]: instances of the next kernel
+  // Sweep count and check point of a live instance minus the grid's
+  // n_sweeps and n_chk (mod 2^32): 0 until an update re-activates an instance
+  // that stopped at another count, or gives one a new check point.
+  std::vector<uint32_t> sweep_off, chk_off;
+  // device [3][count]: instances of the next kernel, then up to two arrays of
+  // one 32-bit value per listed instance (upload_list)
+  uint32_t* list = nullptr;
+  std::vector<uint32_t> list_host;
   uint32_t* resid = nullptr;       // device [count] float bits
   std::vector<uint32_t> resid_host;
   float* res_cost = nullptr;       // device [count][H][W]: snapshots and downloads
   uint8_t* res_action = nullptr;   // device [count][H][W]
-  bool solved = false;             // pp2d_mdp_batch_solve has run since the reset
 };
 
 namespace pp2d {
@@ -1697,16 +1704,18 @@ static int batch_upload(pp2d_mdp_batch* b, const uint8_t* maps, size_t map_strid
     PP2D_CUDA(cudaMemcpy2DAsync(g->occ, hw, maps, map_stride, hw, b->count,
                                 cudaMemcpyHostToDevice, g->stream));
   b->map_stride = map_stride ? hw : 0;
+  b->goals_host.assign(goals, goals + 2 * (size_t)b->count);
   PP2D_CUDA(cudaMemcpyAsync(b->goals, goals, 2 * sizeof(uint32_t) * b->count,
                             cudaMemcpyHostToDevice, g->stream));
   for (uint32_t k = 0; k < b->count; ++k)
     b->has_occ[k] = (map_stride == 0 && k > 0)
                         ? b->has_occ[0]
                         : memchr(maps + k * map_stride, 1, hw) != nullptr;
-  PP2D_CUDA(cudaMemcpyAsync(b->has_occ_dev, b->has_occ.data(), b->count, cudaMemcpyHostToDevice,
-                            g->stream));
   std::fill(b->frozen.begin(), b->frozen.end(), 0);
+  b->n_frozen = 0;
   std::fill(b->stop_sweeps.begin(), b->stop_sweeps.end(), 0);
+  std::fill(b->sweep_off.begin(), b->sweep_off.end(), 0);
+  std::fill(b->chk_off.begin(), b->chk_off.end(), 0);
   PP2D_CUDA(cudaMemsetAsync(b->frozen_dev, 0, b->count, g->stream));
   BatchCodeParams cp;
   cp.maps = g->occ; cp.map_stride = b->map_stride; cp.goals = b->goals; cp.code = g->code;
@@ -1724,12 +1733,33 @@ static int batch_upload(pp2d_mdp_batch* b, const uint8_t* maps, size_t map_strid
   g->action_host_valid = false;
   g->pi_mode = false;
   g->need_valid = false;
-  b->solved = false;
   return PP2D_OK;
 }
 
-static int upload_list(pp2d_mdp_batch* b, const std::vector<uint32_t>& list) {
-  PP2D_CUDA(cudaMemcpyAsync(b->list, list.data(), list.size() * sizeof(uint32_t),
+// Sweep count and check point of instance k.
+static uint32_t batch_sweeps_of(const pp2d_mdp_batch* b, uint32_t k) {
+  return b->frozen[k] ? b->stop_sweeps[k] : b->grid->n_sweeps + b->sweep_off[k];
+}
+static uint32_t batch_chk_of(const pp2d_mdp_batch* b, uint32_t k) {
+  return b->grid->n_chk + b->chk_off[k];
+}
+static uint32_t word_of(float v) {
+  uint32_t w;
+  memcpy(&w, &v, sizeof(w));
+  return w;
+}
+
+// Host side of b->list: the n instances of the next kernel, then `arrays`
+// arrays of one 32-bit value per listed instance (array a at (a + 1) * n,
+// filled by the caller), all sent by one upload_list.
+static uint32_t* stage_list(pp2d_mdp_batch* b, const std::vector<uint32_t>& list, int arrays) {
+  const size_t n = list.size();
+  b->list_host.resize((size_t)(arrays + 1) * n);
+  std::copy(list.begin(), list.end(), b->list_host.begin());
+  return b->list_host.data();
+}
+static int upload_list(pp2d_mdp_batch* b) {
+  PP2D_CUDA(cudaMemcpyAsync(b->list, b->list_host.data(), b->list_host.size() * sizeof(uint32_t),
                             cudaMemcpyHostToDevice, b->grid->stream));
   return PP2D_OK;
 }
@@ -1738,20 +1768,26 @@ static int upload_list(pp2d_mdp_batch* b, const std::vector<uint32_t>& list) {
 // round trip).
 static int batch_residual(pp2d_mdp_batch* b, const std::vector<uint32_t>& list) {
   pp2d_mdp* g = b->grid;
-  PP2D_TRY_MDP(upload_list(b, list));
+  const size_t n = list.size();
+  uint32_t* words = stage_list(b, list, 1);
+  for (size_t i = 0; i < n; ++i) {
+    const uint32_t k = list[i];
+    words[n + i] = word_of(b->has_occ[k] ? fabsf(trapped_cost(g, batch_sweeps_of(b, k)) -
+                                                 trapped_cost(g, batch_chk_of(b, k)))
+                                         : 0.0f);
+  }
+  PP2D_TRY_MDP(upload_list(b));
   PP2D_CUDA(cudaMemsetAsync(b->resid, 0, b->count * sizeof(uint32_t), g->stream));
-  const float floor_val = fabsf(trapped_cost(g, g->n_sweeps) - trapped_cost(g, g->n_chk));
-  uint32_t floor_bits;
-  memcpy(&floor_bits, &floor_val, sizeof(floor_bits));
   const size_t n4 = (size_t)b->H * g->pitch / 4;
-  const size_t fill = std::max<size_t>(1, (size_t)g->sm_count * 8 / list.size());
+  const size_t fill = std::max<size_t>(1, (size_t)g->sm_count * 8 / n);
   const int blocks_per = (int)std::min((n4 + 255) / 256, fill);
-  mdp_batch_residual_kernel<<<(unsigned)(list.size() * blocks_per), 256, 0, g->stream>>>(
-      g->j[g->cur], g->jchk, b->list, blocks_per, (int)b->H, g->pitch, floor_bits,
-      b->has_occ_dev, b->resid);
+  mdp_batch_residual_kernel<<<(unsigned)(n * blocks_per), 256, 0, g->stream>>>(
+      g->j[g->cur], g->jchk, b->list, reinterpret_cast<const float*>(b->list + n), blocks_per,
+      (int)b->H, g->pitch, b->resid);
   g_launches.fetch_add(1, std::memory_order_relaxed);
   PP2D_CUDA(cudaGetLastError());
   g->n_chk = g->n_sweeps;
+  for (uint32_t k : list) b->chk_off[k] = b->sweep_off[k];
   PP2D_CUDA(cudaMemcpyAsync(b->resid_host.data(), b->resid, b->count * sizeof(uint32_t),
                             cudaMemcpyDeviceToHost, g->stream));
   PP2D_CUDA(cudaStreamSynchronize(g->stream));
@@ -1763,15 +1799,19 @@ static int batch_residual(pp2d_mdp_batch* b, const std::vector<uint32_t>& list) 
 template <bool FREEZE>
 static int batch_snapshot(pp2d_mdp_batch* b, const std::vector<uint32_t>& list) {
   pp2d_mdp* g = b->grid;
-  PP2D_TRY_MDP(upload_list(b, list));
+  const size_t n = list.size();
+  uint32_t* words = stage_list(b, list, 1);
+  for (size_t i = 0; i < n; ++i)
+    words[n + i] = word_of(trapped_cost(g, batch_sweeps_of(b, list[i])));
+  PP2D_TRY_MDP(upload_list(b));
   BatchFreezeParams p;
   memset(&p, 0, sizeof(p));
   p.j[0] = g->j[0]; p.j[1] = g->j[1]; p.cur = g->cur;
   p.code = g->code; p.action = g->action;
   p.res_cost = b->res_cost; p.res_action = b->res_action;
-  p.list = b->list; p.n_list = (int)list.size();
+  p.list = b->list; p.n_list = (int)n;
+  p.trapped = reinterpret_cast<const float*>(b->list + n);
   p.W = (int)b->W; p.H = (int)b->H; p.pitch = g->pitch;
-  p.trapped = trapped_cost(g, g->n_sweeps);
   p.need = nullptr;
   if (FREEZE) {
     PP2D_CUDA(cudaMemcpyAsync(b->frozen_dev, b->frozen.data(), b->count,
@@ -1819,12 +1859,13 @@ int pp2d_mdp_batch_create(uint32_t height, uint32_t width, uint32_t count, const
   b->has_occ.assign(count, 0);
   b->frozen.assign(count, 0);
   b->stop_sweeps.assign(count, 0);
+  b->sweep_off.assign(count, 0);
+  b->chk_off.assign(count, 0);
   b->resid_host.assign(count, 0);
   int rc = [&]() -> int {
     PP2D_CUDA(cudaMalloc(&b->goals, 2 * sizeof(uint32_t) * count));
-    PP2D_CUDA(cudaMalloc(&b->has_occ_dev, count));
     PP2D_CUDA(cudaMalloc(&b->frozen_dev, count));
-    PP2D_CUDA(cudaMalloc(&b->list, count * sizeof(uint32_t)));
+    PP2D_CUDA(cudaMalloc(&b->list, 3 * (size_t)count * sizeof(uint32_t)));
     PP2D_CUDA(cudaMalloc(&b->resid, count * sizeof(uint32_t)));
     PP2D_CUDA(cudaMalloc(&b->res_cost, count * hw * sizeof(float)));
     PP2D_CUDA(cudaMalloc(&b->res_action, count * hw));
@@ -1845,7 +1886,7 @@ int pp2d_mdp_batch_reset(pp2d_mdp_batch* h, const uint8_t* maps, size_t map_stri
 void pp2d_mdp_batch_destroy(pp2d_mdp_batch* h) {
   if (!h) return;
   if (h->grid) cudaStreamSynchronize(h->grid->stream);
-  cudaFree(h->goals); cudaFree(h->has_occ_dev); cudaFree(h->frozen_dev); cudaFree(h->list);
+  cudaFree(h->goals); cudaFree(h->frozen_dev); cudaFree(h->list);
   cudaFree(h->resid); cudaFree(h->res_cost); cudaFree(h->res_action);
   pp2d_mdp_destroy(h->grid);
   delete h;
@@ -1858,7 +1899,7 @@ int pp2d_mdp_batch_set_stream(pp2d_mdp_batch* h, void* stream) {
 
 int pp2d_mdp_batch_sweeps(pp2d_mdp_batch* h, uint32_t n) {
   if (!h) return fail(PP2D_ERR_INVALID, "handle is NULL");
-  if (h->solved)
+  if (h->n_frozen)
     return fail(PP2D_ERR_STATE, "the batch was solved (its instances stopped at their own "
                                 "sweep counts): call pp2d_mdp_batch_reset first");
   return pp2d_mdp_sweeps(h->grid, n);
@@ -1866,7 +1907,7 @@ int pp2d_mdp_batch_sweeps(pp2d_mdp_batch* h, uint32_t n) {
 
 int pp2d_mdp_batch_residual(pp2d_mdp_batch* h, float* out) {
   if (!h || !out) return fail(PP2D_ERR_INVALID, "NULL argument");
-  if (h->solved)
+  if (h->n_frozen)
     return fail(PP2D_ERR_STATE, "the batch was solved: call pp2d_mdp_batch_reset first");
   std::vector<uint32_t> all(h->count);
   for (uint32_t k = 0; k < h->count; ++k) all[k] = k;
@@ -1878,15 +1919,17 @@ int pp2d_mdp_batch_residual(pp2d_mdp_batch* h, float* out) {
 int pp2d_mdp_batch_solve(pp2d_mdp_batch* h, uint32_t* sweeps_out, double* residuals,
                          uint32_t max_residuals) {
   if (!h) return fail(PP2D_ERR_INVALID, "handle is NULL");
-  if (h->solved)
-    return fail(PP2D_ERR_STATE, "the batch was solved: call pp2d_mdp_batch_reset first");
-  // pp2d_mdp_solve per instance (path_planning_2d.cu:219-263), all instances
-  // in the same launches; an instance leaves after its first batch of 100
-  // sweeps whose residual meets the rule.
+  if (h->n_frozen == h->count)
+    return fail(PP2D_ERR_STATE, "the batch was solved: call pp2d_mdp_batch_reset or "
+                                "pp2d_mdp_batch_update first");
+  // pp2d_mdp_solve per instance (path_planning_2d.cu:219-263), all active
+  // instances in the same launches; an instance leaves after its first batch
+  // of 100 sweeps whose residual meets the rule.
   pp2d_mdp* g = h->grid;
   const double max_optimal_cost = 5.0 / (1.0 - g->gamma);
-  std::vector<uint32_t> active(h->count), still, stopped;
-  for (uint32_t k = 0; k < h->count; ++k) active[k] = k;
+  std::vector<uint32_t> active, still, stopped;
+  for (uint32_t k = 0; k < h->count; ++k)
+    if (!h->frozen[k]) active.push_back(k);
   uint32_t batch = 0, total = 0;
   while (!active.empty()) {
     PP2D_TRY_MDP(pp2d_mdp_sweeps(g, 100));
@@ -1904,8 +1947,9 @@ int pp2d_mdp_batch_solve(pp2d_mdp_batch* h, uint32_t* sweeps_out, double* residu
         still.push_back(k);
       } else {
         stopped.push_back(k);
+        h->stop_sweeps[k] = batch_sweeps_of(h, k);
         h->frozen[k] = 1;
-        h->stop_sweeps[k] = g->n_sweeps;
+        ++h->n_frozen;
         if (sweeps_out) sweeps_out[k] = total;
       }
     }
@@ -1913,8 +1957,105 @@ int pp2d_mdp_batch_solve(pp2d_mdp_batch* h, uint32_t* sweeps_out, double* residu
     active.swap(still);
     ++batch;
   }
-  h->solved = true;
   PP2D_CUDA(cudaStreamSynchronize(g->stream));
+  return PP2D_OK;
+}
+
+int pp2d_mdp_batch_update(pp2d_mdp_batch* h, const uint32_t* instances, uint32_t n,
+                          const uint8_t* maps, size_t map_stride, const uint32_t* goals_xy) {
+  if (!h || !instances || !maps || !goals_xy) return fail(PP2D_ERR_INVALID, "NULL argument");
+  const size_t hw = (size_t)h->H * h->W;
+  if (map_stride != 0 && map_stride < hw)
+    return fail(PP2D_ERR_INVALID, "map_stride %zu is below height*width = %zu", map_stride, hw);
+  std::vector<uint8_t> listed(h->count, 0);
+  for (uint32_t i = 0; i < n; ++i) {
+    const uint32_t k = instances[i];
+    if (k >= h->count)
+      return fail(PP2D_ERR_INVALID, "entry %u names instance %u of a batch of %u", i, k, h->count);
+    if (listed[k]) return fail(PP2D_ERR_INVALID, "instance %u is listed twice", k);
+    listed[k] = 1;
+  }
+  for (uint32_t i = 0; i < n; ++i) {
+    const uint32_t k = instances[i];
+    const uint32_t gx = goals_xy[2 * (size_t)i], gy = goals_xy[2 * (size_t)i + 1];
+    if (gx >= h->W || gy >= h->H)
+      return fail(PP2D_ERR_INVALID, "instance %u: goal (%u %u) outside the %ux%u map", k, gx, gy,
+                  h->W, h->H);
+    if (maps[i * map_stride + (size_t)gy * h->W + gx] > 0)
+      return fail(PP2D_ERR_GOAL_OCCUPIED,
+                  "instance %u: The assigned goal (%u %u) is at a occupied cell...", k, gx, gy);
+  }
+  if (n == 0) return PP2D_OK;
+  pp2d_mdp* g = h->grid;
+  // Per listed instance: its trapped(n_k) and whether a solve froze it.
+  const std::vector<uint32_t> list(instances, instances + n);
+  uint32_t* words = stage_list(h, list, 2);
+  for (uint32_t i = 0; i < n; ++i) {
+    const uint32_t k = list[i];
+    words[n + i] = word_of(trapped_cost(g, batch_sweeps_of(h, k)));
+    words[2 * n + i] = h->frozen[k];
+  }
+  PP2D_TRY_MDP(upload_list(h));
+  // The device maps are read only while codes are built: the new maps go to
+  // the front of g->occ in list order (one copy of a map shared by the list),
+  // and no instance reads its map again before the next reset or update.
+  if (map_stride == 0 || map_stride == hw)
+    PP2D_CUDA(cudaMemcpyAsync(g->occ, maps, (map_stride ? n : 1) * hw, cudaMemcpyHostToDevice,
+                              g->stream));
+  else
+    PP2D_CUDA(cudaMemcpy2DAsync(g->occ, hw, maps, map_stride, hw, n, cudaMemcpyHostToDevice,
+                                g->stream));
+  for (uint32_t i = 0; i < n; ++i) {
+    h->goals_host[2 * (size_t)list[i]] = goals_xy[2 * (size_t)i];
+    h->goals_host[2 * (size_t)list[i] + 1] = goals_xy[2 * (size_t)i + 1];
+  }
+  PP2D_CUDA(cudaMemcpyAsync(h->goals, h->goals_host.data(), 2 * sizeof(uint32_t) * h->count,
+                            cudaMemcpyHostToDevice, g->stream));
+  BatchUpdateParams p;
+  memset(&p, 0, sizeof(p));
+  p.c.goals = h->goals; p.c.code = g->code;
+  p.c.W = (int)h->W; p.c.H = (int)h->H; p.c.count = (int)h->count; p.c.pitch = g->pitch;
+  p.c.rows_phys = (int)g->H + 2 * kPadRows;
+  p.maps = g->occ;
+  p.map_stride = map_stride ? hw : 0;
+  p.list = h->list;
+  p.trapped = reinterpret_cast<const float*>(h->list + n);
+  p.thaw = h->list + 2 * (size_t)n;
+  p.n_list = (int)n;
+  p.groups = ((int)h->H + kCodeRows - 1) / kCodeRows;
+  p.j = g->j[g->cur];
+  p.jchk = g->jchk;
+  p.action = g->action;
+  p.res_cost = h->res_cost;
+  p.res_action = h->res_action;
+  // Seed the mask of the next fused row-block launch, as update_map does.
+  p.need = nullptr;
+  p.n_strips = ((int)h->W + StripGeom<2, 2>::S - 1) / StripGeom<2, 2>::S;
+  p.rows_per_unit = p.n_rb = 1;
+  if (g->need_valid) {
+    p.need = g->need[g->need_rot];
+    p.rows_per_unit = g->need_rows_per_unit;
+    p.n_rb = g->need_units / p.n_strips;
+  }
+  const size_t groups = (size_t)n * p.groups;
+  dim3 grid((g->pitch / 4 + kCodeThreads - 1) / kCodeThreads,
+            (unsigned)std::min<size_t>(groups, 65535));
+  mdp_batch_update_kernel<<<grid, kCodeThreads, 0, g->stream>>>(p);
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  PP2D_CUDA(cudaGetLastError());
+  // (the caller may free the maps on return)
+  PP2D_CUDA(cudaStreamSynchronize(g->stream));
+  for (uint32_t i = 0; i < n; ++i) {
+    const uint32_t k = list[i];
+    const uint32_t nk = batch_sweeps_of(h, k);
+    if (h->frozen[k]) {
+      h->frozen[k] = 0;
+      --h->n_frozen;
+    }
+    h->sweep_off[k] = nk - g->n_sweeps;
+    h->chk_off[k] = nk - g->n_chk;        // the next residual measures the change from J'
+    h->has_occ[k] = memchr(maps + i * map_stride, 1, hw) != nullptr;
+  }
   return PP2D_OK;
 }
 
@@ -2007,7 +2148,7 @@ int pp2d_mdp_batch_waypoints(pp2d_mdp_batch* h, uint32_t k, uint32_t sx, uint32_
 int pp2d_mdp_batch_sweep_counts(const pp2d_mdp_batch* h, uint32_t* out) {
   if (!h || !out) return fail(PP2D_ERR_INVALID, "NULL argument");
   for (uint32_t k = 0; k < h->count; ++k)
-    out[k] = h->frozen[k] ? h->stop_sweeps[k] : h->grid->n_sweeps;
+    out[k] = batch_sweeps_of(h, k);
   return PP2D_OK;
 }
 

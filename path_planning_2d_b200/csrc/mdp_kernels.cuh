@@ -1031,7 +1031,9 @@ struct UpdateParams {
   int H;                 // owned rows
 };
 
-__device__ __forceinline__ void mark_unit_neighbourhood(const UpdateParams& p, int rb, int k) {
+// P: UpdateParams or BatchUpdateParams (need, n_rb, n_strips)
+template <class P>
+__device__ __forceinline__ void mark_unit_neighbourhood(const P& p, int rb, int k) {
 #pragma unroll 1
   for (int i = 0; i < 9; ++i) {
     const int r = rb + i / 3 - 1, kk = k + i % 3 - 1;
@@ -1413,20 +1415,21 @@ __global__ void __launch_bounds__(kCodeThreads) mdp_batch_code_kernel(const Batc
 // Per-instance max |J - Jchk| over the rows of the instances in `list` (the
 // separators are not read), then Jchk = J there: mdp_residual_kernel
 // segmented by instance.  blocks_per CTAs serve one instance: block b takes
-// instance list[b / blocks_per].  The floor (the change of the occupied
-// cells' closed form) counts for the instances whose map has an occupied cell.
+// instance list[b / blocks_per].  floor[i] is list[i]'s floor: the change of
+// the occupied cells' closed form between its own check point and sweep
+// count, or 0 when its map has no occupied cell.
 __global__ void __launch_bounds__(256)
 mdp_batch_residual_kernel(const float* __restrict__ j, float* __restrict__ chk,
-                          const uint32_t* __restrict__ list, int blocks_per, int H, int pitch,
-                          uint32_t floor_bits, const uint8_t* __restrict__ has_occ,
-                          uint32_t* result) {
-  const uint32_t k = list[blockIdx.x / blocks_per];
+                          const uint32_t* __restrict__ list, const float* __restrict__ floor,
+                          int blocks_per, int H, int pitch, uint32_t* result) {
+  const uint32_t i = blockIdx.x / blocks_per;
+  const uint32_t k = list[i];
   const int part = (int)(blockIdx.x % blocks_per);
   const size_t off = ((size_t)k * (H + 1) + kPadRows) * pitch;
   const float4* __restrict__ a4 = reinterpret_cast<const float4*>(j + off);
   float4* __restrict__ b4 = reinterpret_cast<float4*>(chk + off);
   const size_t n4 = (size_t)H * pitch / 4;
-  float m = has_occ[k] ? __uint_as_float(floor_bits) : 0.0f;
+  float m = floor[i];
   for (size_t i = (size_t)part * blockDim.x + threadIdx.x; i < n4;
        i += (size_t)blocks_per * blockDim.x) {
     const float4 a = a4[i];
@@ -1454,9 +1457,9 @@ struct BatchFreezeParams {
   float* res_cost;         // [count][H][W]
   uint8_t* res_action;     // [count][H][W]
   const uint32_t* list;    // instances to snapshot
+  const float* trapped;    // [n_list]: J of an occupied cell at list[i]'s sweep count
   int n_list;
   int W, H, pitch;
-  float trapped;           // J_n of an occupied cell
   // FREEZE, mask part: NULL = no valid mask to clear
   uint32_t* need;          // the mask the next fused row-block launch reads
   const uint8_t* frozen;   // [count]: 1 = instance stopped
@@ -1481,13 +1484,14 @@ __global__ void __launch_bounds__(256) mdp_batch_freeze_kernel(const BatchFreeze
   const size_t stride = (size_t)gridDim.x * blockDim.x;
   const size_t t0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   for (size_t t = t0; t < cells; t += stride) {
-    const uint32_t k = p.list[t / hw];
+    const size_t i = t / hw;
+    const uint32_t k = p.list[i];
     const size_t c = t % hw;
     const int y = (int)(c / p.W), x = (int)(c - (size_t)y * p.W);
     const size_t ty = (size_t)k * (p.H + 1) + y;     // row in the tall grid
     const size_t q = (ty + kPadRows) * p.pitch + x + kPadLeft;
     const size_t dst = (size_t)k * hw + c;
-    p.res_cost[dst] = (p.code[q] & kCodeOccBit) ? p.trapped : p.j[p.cur][q];
+    p.res_cost[dst] = (p.code[q] & kCodeOccBit) ? p.trapped[i] : p.j[p.cur][q];
     p.res_action[dst] = p.action[ty * p.W + x];
     if (FREEZE) {
       p.code[q] = (uint16_t)kCodeOccBit;
@@ -1509,6 +1513,124 @@ __global__ void __launch_bounds__(256) mdp_batch_freeze_kernel(const BatchFreeze
     const int u0 = (int)rb * p.n_strips;
     for (int w = u0 >> 5; w <= (u0 + p.n_strips - 1) >> 5; ++w)
       atomicAnd(p.need + w, ~unit_range_bits(w, u0, u0 + p.n_strips));
+  }
+}
+
+// New maps and goals for the instances in `list` (pp2d_mdp_batch_update,
+// DESIGN.md section 4): mdp_update_map_kernel on their rows of the tall grid
+// only, with each instance's own trapped(n_k).  An instance that a solve froze
+// (thaw[i] != 0) has padding codes and J = +0 in its rows: its J comes from
+// its result slot, where the occupied cells already hold trapped(n_k), and
+// its action rows are restored from the slot, so that plan and way-points
+// return what they returned before the update.
+struct BatchUpdateParams {
+  BatchCodeParams c;       // goals (the new ones), code plane and sizes; maps unused
+  const uint8_t* maps;     // the new map of list[i] at maps + i * map_stride (0: one map)
+  size_t map_stride;
+  const uint32_t* list;    // [n_list] instances
+  const float* trapped;    // [n_list] J of an occupied cell at list[i]'s sweep count
+  const uint32_t* thaw;    // [n_list] 1: list[i] is frozen
+  int n_list, groups;      // groups: kCodeRows row groups per instance
+  float* j;                // j[cur]
+  float* jchk;
+  uint8_t* action;         // dense action grid of the tall grid
+  const float* res_cost;   // [count][H][W]
+  const uint8_t* res_action;
+  uint32_t* need;          // NULL: no seeding (the next fused launch runs every unit)
+  int n_strips, rows_per_unit, n_rb;
+};
+
+// grid: (ceil(pitch / 4 / kCodeThreads), any); blocks stride over the row
+// groups of the listed instances.  Thread shape and dirty-unit seeding as in
+// mdp_update_map_kernel.
+__global__ void __launch_bounds__(kCodeThreads) mdp_batch_update_kernel(const BatchUpdateParams p) {
+  const int lane = threadIdx.x & 31;
+  const int c0 = 4 * (blockIdx.x * kCodeThreads + threadIdx.x);
+  const bool active = c0 < p.c.pitch;
+  const int x0 = c0 - kPadLeft;
+  const int W = p.c.W, H = p.c.H;
+  const size_t hw = (size_t)H * W;
+  // the maps are H*W bytes apart: 4-aligned whenever W is
+  const bool fast = (W & 3) == 0 && (x0 & 3) == 0 && x0 >= 0 && x0 + 3 < W &&
+                    (reinterpret_cast<uintptr_t>(p.maps) & 3u) == 0;
+  constexpr int kStrip = StripGeom<2, 2>::S;
+  const int k_lo = max(x0, 0) / kStrip;
+  for (int g = blockIdx.y; g < p.n_list * p.groups; g += gridDim.y) {   // uniform over the block
+    const int i = g / p.groups;
+    const int ly0 = (g - i * p.groups) * kCodeRows;
+    const int ly1 = min(ly0 + kCodeRows, H);
+    const uint32_t k = __ldg(p.list + i);
+    const float trapped = __ldg(p.trapped + i);
+    const bool thaw = __ldg(p.thaw + i) != 0;
+    // batch_row over a one-map view: every row of instance k reads map i
+    BatchCodeParams bp = p.c;
+    bp.maps = p.maps + (size_t)i * p.map_stride;
+    bp.map_stride = 0;
+    auto mask = [&](int gy) {
+      int ly;
+      const CodeParams c = batch_row(bp, gy, ly);
+      return fast ? occ_mask6<true>(c, x0, ly) : occ_mask6<false>(c, x0, ly);
+    };
+    int ty = (int)k * (H + 1) + ly0;              // row of the tall grid
+    uint32_t m0 = mask(ty - 1), m1 = mask(ty);
+    for (int ly = ly0; ly < ly1; ++ly, ++ty) {
+      const uint32_t m2 = mask(ty + 1);
+      int cy;
+      const CodeParams c = batch_row(bp, ty, cy);
+      uint32_t code[4];
+      cell_codes4(c, x0, cy, m0, m1, m2, code);
+      m0 = m1;
+      m1 = m2;
+      bool dirty_lo = false, dirty_hi = false;
+      if (active) {
+        const size_t q = (size_t)(ty + kPadRows) * p.c.pitch + c0;
+        const size_t slot = (size_t)k * hw + (size_t)ly * W;   // row ly of k's result slot
+        const uint2 oc2 = *reinterpret_cast<const uint2*>(p.c.code + q);
+        const uint32_t old[4] = {oc2.x & 0xFFFFu, oc2.x >> 16, oc2.y & 0xFFFFu, oc2.y >> 16};
+        const float4 jv = *reinterpret_cast<const float4*>(p.j + q);
+        const float jo[4] = {jv.x, jv.y, jv.z, jv.w};
+        float jn[4];
+        bool code_changed = false, j_changed = false;
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+          const bool occ_new = code[e] & kCodeOccBit, occ_old = old[e] & kCodeOccBit;
+          jn[e] = jo[e];
+          if (occ_new && !occ_old) jn[e] = 0.0f;
+          // (a frozen row's codes are all padding: every free cell takes its slot value)
+          if (!occ_new && occ_old) jn[e] = thaw ? __ldg(p.res_cost + slot + x0 + e) : trapped;
+          if (!(code[e] & (kCodeOccBit | kCodeLiveBit))) jn[e] = 0.0f;   // the goal
+          const bool cc = code[e] != old[e];
+          const bool jc = __float_as_uint(jn[e]) != __float_as_uint(jo[e]);
+          code_changed |= cc;
+          j_changed |= jc;
+          if (cc || jc) {
+            if ((x0 + e) / kStrip == k_lo || x0 + e < 0) dirty_lo = true;
+            else dirty_hi = true;
+          }
+          if (thaw && x0 + e >= 0 && x0 + e < W)
+            p.action[(size_t)ty * W + x0 + e] = __ldg(p.res_action + slot + x0 + e);
+        }
+        if (code_changed)
+          *reinterpret_cast<uint2*>(p.c.code + q) =
+              make_uint2(code[0] | (code[1] << 16), code[2] | (code[3] << 16));
+        const float4 jw = make_float4(jn[0], jn[1], jn[2], jn[3]);
+        if (j_changed) *reinterpret_cast<float4*>(p.j + q) = jw;
+        *reinterpret_cast<float4*>(p.jchk + q) = jw;
+      }
+      if (p.need != nullptr && __any_sync(0xffffffffu, dirty_lo || dirty_hi)) {
+        const int rb = min(ty / p.rows_per_unit, p.n_rb - 1);
+#pragma unroll
+        for (int side = 0; side < 2; ++side) {
+          const bool d = side ? dirty_hi : dirty_lo;
+          const uint32_t m = __ballot_sync(0xffffffffu, d);
+          if (d) {
+            const int kk = k_lo + side;
+            const uint32_t peers = __match_any_sync(m, kk);
+            if (__ffs(peers) - 1 == lane) mark_unit_neighbourhood(p, rb, kk);
+          }
+        }
+      }
+    }
   }
 }
 

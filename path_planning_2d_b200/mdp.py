@@ -347,6 +347,22 @@ class MdpBatchPathPlanning2d:
         return n, [res[k, :min(max_batches, int(n[k]) // 100)].copy()
                    for k in range(self.count)]
 
+    def update_map(self, instances, grid_maps, goals):
+        """New maps and goals for the listed instances, each continuing from
+        its current solution as MdpPathPlanning2d.update_map does; an instance
+        that valueIteration() stopped becomes active again.  grid_maps: (H, W)
+        shared by the listed instances, or (n, H, W); goals: n (x, y) pairs."""
+        idx = np.ascontiguousarray(instances, dtype=np.uint32).reshape(-1)
+        maps = np.ascontiguousarray(grid_maps, dtype=np.uint8)
+        goals = np.ascontiguousarray(goals, dtype=np.uint32).reshape(-1, 2)
+        if maps.ndim not in (2, 3) or maps.shape[-2:] != (self.map_height, self.map_width):
+            raise ValueError("grid_maps must be (H, W) or (n, H, W) of the batch's map size")
+        if goals.shape[0] != idx.size or (maps.ndim == 3 and maps.shape[0] != idx.size):
+            raise ValueError("one goal per listed instance, and one map each or one shared map")
+        stride = 0 if maps.ndim == 2 else self.map_height * self.map_width
+        _lib.check(self._lib.pp2d_mdp_batch_update(self._h, idx.ctypes.data, idx.size,
+                                                   maps.ctypes.data, stride, goals.ctypes.data))
+
     def sweep_counts(self):
         out = np.zeros(self.count, dtype=np.uint32)
         _lib.check(self._lib.pp2d_mdp_batch_sweep_counts(self._h, out.ctypes.data))
