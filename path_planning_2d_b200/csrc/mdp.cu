@@ -232,6 +232,70 @@ static float occupied_cost(pp2d_mdp* h, uint32_t n) {
   return h->pi_mode ? trapped_cost_pi(h, n) : trapped_cost(h, n);
 }
 
+// The reference's stopping rule (path_planning_2d.cu:219-263): sweeping goes
+// on while the residual exceeds 1e-3 of the largest optimal cost.
+static bool keeps_sweeping(double residual, float gamma) {
+  const double max_optimal_cost = 5.0 / (1.0 - gamma);
+  return residual > max_optimal_cost * 1e-3;
+}
+
+// The goal of a width x height map must lie inside it, on a free cell
+// (path_planning_2d.cu:84-88).  instance >= 0: the batch instance the
+// messages name.
+static int check_goal(const uint8_t* map, uint32_t width, uint32_t height, uint32_t gx,
+                      uint32_t gy, int64_t instance = -1) {
+  char who[32] = "";
+  if (instance >= 0) snprintf(who, sizeof(who), "instance %u: ", (uint32_t)instance);
+  if (gx >= width || gy >= height)
+    return fail(PP2D_ERR_INVALID, "%sgoal (%u %u) outside the %ux%u map", who, gx, gy, width,
+                height);
+  if (map[(size_t)gy * width + gx] > 0)
+    return fail(PP2D_ERR_GOAL_OCCUPIED, "%sThe assigned goal (%u %u) is at a occupied cell...",
+                who, gx, gy);
+  return PP2D_OK;
+}
+
+// Occupancy rows [row0, row0 + rows) that a handle owning rows [row_begin,
+// row_end) of a grid of `height` rows keeps on the device: the codes of its
+// owned and ghost rows read up to 3 rows beyond them.
+struct OccWindow {
+  int row0, rows;
+};
+static OccWindow occ_window(uint32_t row_begin, uint32_t row_end, uint32_t height) {
+  const int row0 = (int)row_begin - 3 < 0 ? 0 : (int)row_begin - 3;
+  const int row1 = (int)row_end + 3 > (int)height ? (int)height : (int)row_end + 3;
+  return {row0, row1 - row0};
+}
+
+// CodeParams of h's code plane built from the occupancy rows at `occ`, and the
+// grid of a code or update kernel launch over it.
+static CodeParams code_params(const pp2d_mdp* h, const uint8_t* occ) {
+  const OccWindow ow = occ_window(h->row_begin, h->row_begin + h->H, h->Htot);
+  CodeParams cp;
+  cp.occ = occ; cp.code = h->code; cp.W = (int)h->W; cp.Htot = (int)h->Htot;
+  cp.pitch = h->pitch; cp.rows_phys = (int)h->H + 2 * kPadRows;
+  cp.row_begin = (int)h->row_begin; cp.occ_row0 = ow.row0; cp.occ_rows = ow.rows;
+  cp.gx = (int)h->gx; cp.gy = (int)h->gy;
+  return cp;
+}
+static dim3 code_grid(const CodeParams& cp) {
+  return dim3((cp.pitch / 4 + kCodeThreads - 1) / kCodeThreads,
+              (cp.rows_phys + kCodeRows - 1) / kCodeRows);
+}
+
+// The unit mask of h's next fused row-block launch, for a kernel that seeds or
+// clears it.  Without a valid mask that launch runs every unit anyway, and
+// `need` is NULL.
+static UnitMask next_unit_mask(const pp2d_mdp* h) {
+  UnitMask m = {nullptr, ((int)h->W + kUnitStrip - 1) / kUnitStrip, 1, 1};
+  if (h->need_valid) {
+    m.need = h->need[h->need_rot];
+    m.rows_per_unit = h->need_rows_per_unit;
+    m.n_rb = h->need_units / m.n_strips;
+  }
+  return m;
+}
+
 // CW == 1 kernels: rows ahead of the marching row touched with prefetch.global.L1
 // (the slack rows below the plane bound how far ahead that may reach).
 constexpr int kL1PrefetchRows = 6;
@@ -552,10 +616,6 @@ static int env_int(const char* name, int dflt) {
 // path_planning_2d.cu:94-106).
 static int upload_map(pp2d_mdp* h, const uint8_t* map) {
   const size_t owned = (size_t)h->H * h->W;
-  const int occ_row0 = (int)h->row_begin - 3 < 0 ? 0 : (int)h->row_begin - 3;
-  const int row_end = (int)(h->row_begin + h->H);
-  const int occ_row1 = row_end + 3 > (int)h->Htot ? (int)h->Htot : row_end + 3;
-  const int occ_rows = occ_row1 - occ_row0;
   PP2D_CUDA(cudaMemsetAsync(h->j[0], 0, h->plane * sizeof(float), h->stream));
   PP2D_CUDA(cudaMemsetAsync(h->j[1], 0, h->plane * sizeof(float), h->stream));
   h->chk_is_zero = true;          // Jchk = J_0 = 0: the first residual does not read it
@@ -572,18 +632,12 @@ static int upload_map(pp2d_mdp* h, const uint8_t* map) {
     PP2D_CUDA(cudaStreamWaitEvent(h->stream, h->ev_staged, 0));
     std::swap(h->occ, h->occ_next);
   } else {
-    PP2D_CUDA(cudaMemcpyAsync(h->occ, map + (size_t)occ_row0 * h->W,
-                              (size_t)occ_rows * h->W, cudaMemcpyHostToDevice,
-                              h->stream));
+    const OccWindow ow = occ_window(h->row_begin, h->row_begin + h->H, h->Htot);
+    PP2D_CUDA(cudaMemcpyAsync(h->occ, map + (size_t)ow.row0 * h->W, (size_t)ow.rows * h->W,
+                              cudaMemcpyHostToDevice, h->stream));
   }
-  CodeParams cp;
-  cp.occ = h->occ; cp.code = h->code; cp.W = (int)h->W; cp.Htot = (int)h->Htot;
-  cp.pitch = h->pitch; cp.rows_phys = (int)h->H + 2 * kPadRows;
-  cp.row_begin = (int)h->row_begin; cp.occ_row0 = occ_row0; cp.occ_rows = occ_rows;
-  cp.gx = (int)h->gx; cp.gy = (int)h->gy;
-  dim3 grid((h->pitch / 4 + kCodeThreads - 1) / kCodeThreads,
-            (cp.rows_phys + kCodeRows - 1) / kCodeRows);
-  mdp_code_kernel<<<grid, kCodeThreads, 0, h->stream>>>(cp);
+  const CodeParams cp = code_params(h, h->occ);
+  mdp_code_kernel<<<code_grid(cp), kCodeThreads, 0, h->stream>>>(cp);
   g_launches.fetch_add(1, std::memory_order_relaxed);
   PP2D_CUDA(cudaGetLastError());
   if (h->ev_code_built) PP2D_CUDA(cudaEventRecord(h->ev_code_built, h->stream));
@@ -609,32 +663,14 @@ static int update_map(pp2d_mdp* h, const uint8_t* map) {
   if (!staged) PP2D_TRY_MDP(pp2d_mdp_stage_map(h, map));
   h->staged_map = nullptr;
   PP2D_CUDA(cudaStreamWaitEvent(h->stream, h->ev_staged, 0));
-  const int occ_row0 = (int)h->row_begin - 3 < 0 ? 0 : (int)h->row_begin - 3;
-  const int row_end = (int)(h->row_begin + h->H);
-  const int occ_row1 = row_end + 3 > (int)h->Htot ? (int)h->Htot : row_end + 3;
   UpdateParams up;
-  CodeParams& cp = up.c;
-  cp.occ = h->occ_next; cp.code = h->code; cp.W = (int)h->W; cp.Htot = (int)h->Htot;
-  cp.pitch = h->pitch; cp.rows_phys = (int)h->H + 2 * kPadRows;
-  cp.row_begin = (int)h->row_begin; cp.occ_row0 = occ_row0; cp.occ_rows = occ_row1 - occ_row0;
-  cp.gx = (int)h->gx; cp.gy = (int)h->gy;
+  up.c = code_params(h, h->occ_next);
   up.j = h->j[h->cur];
   up.jchk = h->jchk;
   up.trapped = trapped_cost(h, h->n_sweeps);
+  up.mask = next_unit_mask(h);
   up.H = (int)h->H;
-  // Seed the mask of the next fused row-block launch.  Without a valid mask
-  // that launch runs every unit anyway.
-  up.need = nullptr;
-  up.n_strips = ((int)h->W + StripGeom<2, 2>::S - 1) / StripGeom<2, 2>::S;
-  up.rows_per_unit = up.n_rb = 1;
-  if (h->need_valid) {
-    up.need = h->need[h->need_rot];
-    up.rows_per_unit = h->need_rows_per_unit;
-    up.n_rb = h->need_units / up.n_strips;
-  }
-  dim3 grid((h->pitch / 4 + kCodeThreads - 1) / kCodeThreads,
-            (cp.rows_phys + kCodeRows - 1) / kCodeRows);
-  mdp_update_map_kernel<<<grid, kCodeThreads, 0, h->stream>>>(up);
+  mdp_update_map_kernel<<<code_grid(up.c), kCodeThreads, 0, h->stream>>>(up);
   g_launches.fetch_add(1, std::memory_order_relaxed);
   PP2D_CUDA(cudaGetLastError());
   PP2D_CUDA(cudaEventRecord(h->ev_code_built, h->stream));
@@ -668,14 +704,10 @@ static int create_impl(uint32_t height, uint32_t width, const uint8_t* map,
     return fail(PP2D_ERR_INVALID, "a shard needs at least %d rows", kPadRows);
   if ((uint64_t)height * width >= (1ull << 40))
     return fail(PP2D_ERR_INVALID, "map too large");
-  if (map[(size_t)gy * width + gx] > 0)   // path_planning_2d.cu:84-88
-    return fail(PP2D_ERR_GOAL_OCCUPIED,
-                "The assigned goal (%u %u) is at a occupied cell...", gx, gy);
-  const int occ_rows = (int)((row_end + 3 > height ? height : row_end + 3) -
-                             ((int)row_begin - 3 < 0 ? 0 : row_begin - 3));
+  PP2D_TRY_MDP(check_goal(map, width, height, gx, gy));
   pp2d_mdp* h = nullptr;
   PP2D_TRY_MDP(make_handle(height, width, gamma, row_begin, row_end, sharded,
-                           (size_t)occ_rows * width, &h));
+                           (size_t)occ_window(row_begin, row_end, height).rows * width, &h));
   h->gx = gx; h->gy = gy;
   const int rc = upload_map(h, map);
   if (rc != PP2D_OK) { pp2d_mdp_destroy(h); return rc; }
@@ -1035,14 +1067,7 @@ int pp2d_mdp_device_count(const pp2d_mdp* h, int* peer_to_peer) {
 static int check_map_goal(const pp2d_mdp* h, const uint8_t* map, uint32_t goal_x,
                           uint32_t goal_y) {
   if (!h || !map) return fail(PP2D_ERR_INVALID, "NULL argument");
-  if (goal_x >= h->W || goal_y >= h->Htot)
-    return fail(PP2D_ERR_INVALID, "goal (%u %u) outside the %ux%u map", goal_x,
-                goal_y, h->W, h->Htot);
-  if (map[(size_t)goal_y * h->W + goal_x] > 0)
-    return fail(PP2D_ERR_GOAL_OCCUPIED,
-                "The assigned goal (%u %u) is at a occupied cell...", goal_x,
-                goal_y);
-  return PP2D_OK;
+  return check_goal(map, h->W, h->Htot, goal_x, goal_y);
 }
 
 int pp2d_mdp_reset(pp2d_mdp* h, const uint8_t* map, uint32_t goal_x,
@@ -1075,10 +1100,8 @@ int pp2d_mdp_stage_map(pp2d_mdp* h, const uint8_t* map) {
     }
     return PP2D_OK;
   }
-  const int occ_row0 = (int)h->row_begin - 3 < 0 ? 0 : (int)h->row_begin - 3;
-  const int row_end = (int)(h->row_begin + h->H);
-  const int occ_row1 = row_end + 3 > (int)h->Htot ? (int)h->Htot : row_end + 3;
-  const size_t bytes = (size_t)(occ_row1 - occ_row0) * h->W;
+  const OccWindow ow = occ_window(h->row_begin, h->row_begin + h->H, h->Htot);
+  const size_t bytes = (size_t)ow.rows * h->W;
   if (!h->upload_stream) {
     PP2D_CUDA(cudaStreamCreateWithFlags(&h->upload_stream, cudaStreamNonBlocking));
     PP2D_CUDA(cudaEventCreateWithFlags(&h->ev_staged, cudaEventDisableTiming));
@@ -1089,7 +1112,7 @@ int pp2d_mdp_stage_map(pp2d_mdp* h, const uint8_t* map) {
     // (on the solve stream) must have read it before it is overwritten
     PP2D_CUDA(cudaStreamWaitEvent(h->upload_stream, h->ev_code_built, 0));
   }
-  PP2D_CUDA(cudaMemcpyAsync(h->occ_next, map + (size_t)occ_row0 * h->W, bytes,
+  PP2D_CUDA(cudaMemcpyAsync(h->occ_next, map + (size_t)ow.row0 * h->W, bytes,
                             cudaMemcpyHostToDevice, h->upload_stream));
   PP2D_CUDA(cudaEventRecord(h->ev_staged, h->upload_stream));
   h->staged_map = map;
@@ -1272,7 +1295,6 @@ int pp2d_mdp_solve(pp2d_mdp* h, uint32_t* sweeps_out, double* residuals,
     return fail(PP2D_ERR_STATE, "pp2d_mdp_solve needs an unsharded handle");
   // path_planning_2d.cu:219-263.
   double cost_inf_norm = 0.0;
-  const double max_optimal_cost = 5.0 / (1.0 - h->gamma);
   uint32_t batch = 0, total = 0;
   do {
     int rc = pp2d_mdp_sweeps(h, 100);
@@ -1284,7 +1306,7 @@ int pp2d_mdp_solve(pp2d_mdp* h, uint32_t* sweeps_out, double* residuals,
     cost_inf_norm = r;
     if (residuals && batch < max_residuals) residuals[batch] = cost_inf_norm;
     ++batch;
-  } while (cost_inf_norm > max_optimal_cost * 1e-3);
+  } while (keeps_sweeping(cost_inf_norm, h->gamma));
   if (sweeps_out) *sweeps_out = total;
   return PP2D_OK;
 }
@@ -1306,7 +1328,6 @@ int pp2d_mdp_policy_iteration(pp2d_mdp* h, uint32_t* evaluation_sweeps, double* 
   dim3 grid((h->W + 255) / 256, h->H);
   std::vector<uint8_t> a_prev(owned, 0), a_curr(owned);
   // path_planning_2d.cu:271-357
-  const double max_optimal_cost = 5.0 / (1.0 - h->gamma);
   double cost_inf_norm = 0.0;
   uint32_t round = 0;
   do {
@@ -1342,7 +1363,7 @@ int pp2d_mdp_policy_iteration(pp2d_mdp* h, uint32_t* evaluation_sweeps, double* 
     if (residuals && round < capacity) residuals[round] = cost_inf_norm;
     ++round;
     if (max_rounds > 0 && round >= max_rounds) break;
-  } while (cost_inf_norm > max_optimal_cost * 1e-3);
+  } while (keeps_sweeping(cost_inf_norm, h->gamma));
   if (evaluation_sweeps) *evaluation_sweeps = h->n_sweeps;
   return sync_if_needed(h);
 }
@@ -1675,15 +1696,22 @@ static int batch_check(uint32_t height, uint32_t width, uint32_t count, const ui
     return fail(PP2D_ERR_INVALID, "%u instances of %ux%u stack to a grid of %llu rows x %llu "
                                   "columns: too large for one batch", count, width, height,
                 (unsigned long long)rows, (unsigned long long)pitch);
-  for (uint32_t k = 0; k < count; ++k) {
-    const uint32_t gx = goals[2 * (size_t)k], gy = goals[2 * (size_t)k + 1];
-    if (gx >= width || gy >= height)
-      return fail(PP2D_ERR_INVALID, "instance %u: goal (%u %u) outside the %ux%u map", k, gx, gy,
-                  width, height);
-    if (maps[k * map_stride + (size_t)gy * width + gx] > 0)
-      return fail(PP2D_ERR_GOAL_OCCUPIED,
-                  "instance %u: The assigned goal (%u %u) is at a occupied cell...", k, gx, gy);
-  }
+  for (uint32_t k = 0; k < count; ++k)
+    PP2D_TRY_MDP(check_goal(maps + k * map_stride, width, height, goals[2 * (size_t)k],
+                            goals[2 * (size_t)k + 1], k));
+  return PP2D_OK;
+}
+
+// Maps i = 0 .. n-1 at maps + i * map_stride (map_stride 0: one map) to the
+// front of g->occ, back to back; a shared map is copied once.
+static int upload_maps(pp2d_mdp* g, const uint8_t* maps, size_t map_stride, size_t hw,
+                       uint32_t n) {
+  if (map_stride == 0 || map_stride == hw)
+    PP2D_CUDA(cudaMemcpyAsync(g->occ, maps, (map_stride ? n : 1) * hw, cudaMemcpyHostToDevice,
+                              g->stream));
+  else
+    PP2D_CUDA(cudaMemcpy2DAsync(g->occ, hw, maps, map_stride, hw, n, cudaMemcpyHostToDevice,
+                                g->stream));
   return PP2D_OK;
 }
 
@@ -1696,13 +1724,7 @@ static int batch_upload(pp2d_mdp_batch* b, const uint8_t* maps, size_t map_strid
   PP2D_CUDA(cudaMemsetAsync(g->j[1], 0, g->plane * sizeof(float), g->stream));
   PP2D_CUDA(cudaMemsetAsync(g->jchk, 0, g->plane * sizeof(float), g->stream));
   PP2D_CUDA(cudaMemsetAsync(g->action, 0, (size_t)g->H * g->W, g->stream));
-  // the maps go back to back on the device (one copy of a shared map)
-  if (map_stride == 0 || map_stride == hw)
-    PP2D_CUDA(cudaMemcpyAsync(g->occ, maps, (map_stride ? b->count : 1) * hw,
-                              cudaMemcpyHostToDevice, g->stream));
-  else
-    PP2D_CUDA(cudaMemcpy2DAsync(g->occ, hw, maps, map_stride, hw, b->count,
-                                cudaMemcpyHostToDevice, g->stream));
+  PP2D_TRY_MDP(upload_maps(g, maps, map_stride, hw, b->count));
   b->map_stride = map_stride ? hw : 0;
   b->goals_host.assign(goals, goals + 2 * (size_t)b->count);
   PP2D_CUDA(cudaMemcpyAsync(b->goals, goals, 2 * sizeof(uint32_t) * b->count,
@@ -1742,6 +1764,12 @@ static uint32_t batch_sweeps_of(const pp2d_mdp_batch* b, uint32_t k) {
 }
 static uint32_t batch_chk_of(const pp2d_mdp_batch* b, uint32_t k) {
   return b->grid->n_chk + b->chk_off[k];
+}
+// Instance k's action grid (H*W bytes): its snapshot once frozen, else its
+// rows of the live grid.
+static const uint8_t* batch_actions_of(const pp2d_mdp_batch* b, uint32_t k) {
+  return b->frozen[k] ? b->res_action + k * (size_t)b->H * b->W
+                      : b->grid->action + (size_t)k * (b->H + 1) * b->W;
 }
 static uint32_t word_of(float v) {
   uint32_t w;
@@ -1812,23 +1840,16 @@ static int batch_snapshot(pp2d_mdp_batch* b, const std::vector<uint32_t>& list) 
   p.list = b->list; p.n_list = (int)n;
   p.trapped = reinterpret_cast<const float*>(b->list + n);
   p.W = (int)b->W; p.H = (int)b->H; p.pitch = g->pitch;
-  p.need = nullptr;
   if (FREEZE) {
     PP2D_CUDA(cudaMemcpyAsync(b->frozen_dev, b->frozen.data(), b->count,
                               cudaMemcpyHostToDevice, g->stream));
     p.frozen = b->frozen_dev;
     p.count = (int)b->count;
     p.Htot = (int)g->H;
-    p.n_strips = ((int)b->W + StripGeom<2, 2>::S - 1) / StripGeom<2, 2>::S;
-    // the mask the next fused row-block launch reads (seeded by the arg-min
-    // launch that ended the batch); without one that launch runs every unit
-    if (g->need_valid) {
-      p.need = g->need[g->need_rot];
-      p.rows_per_unit = g->need_rows_per_unit;
-      p.n_rb = g->need_units / p.n_strips;
-    }
+    // (seeded by the arg-min launch that ended the batch)
+    p.mask = next_unit_mask(g);
   }
-  const size_t work = std::max<size_t>((size_t)list.size() * b->H * b->W, (size_t)p.n_rb);
+  const size_t work = std::max<size_t>((size_t)list.size() * b->H * b->W, (size_t)p.mask.n_rb);
   const int grid = (int)std::min<size_t>((work + 255) / 256, (size_t)g->sm_count * 16);
   mdp_batch_freeze_kernel<FREEZE><<<std::max(grid, 1), 256, 0, g->stream>>>(p);
   g_launches.fetch_add(1, std::memory_order_relaxed);
@@ -1926,7 +1947,6 @@ int pp2d_mdp_batch_solve(pp2d_mdp_batch* h, uint32_t* sweeps_out, double* residu
   // instances in the same launches; an instance leaves after its first batch
   // of 100 sweeps whose residual meets the rule.
   pp2d_mdp* g = h->grid;
-  const double max_optimal_cost = 5.0 / (1.0 - g->gamma);
   std::vector<uint32_t> active, still, stopped;
   for (uint32_t k = 0; k < h->count; ++k)
     if (!h->frozen[k]) active.push_back(k);
@@ -1943,7 +1963,7 @@ int pp2d_mdp_batch_solve(pp2d_mdp_batch* h, uint32_t* sweeps_out, double* residu
       const double cost_inf_norm = r;
       if (residuals && batch < max_residuals)
         residuals[(size_t)k * max_residuals + batch] = cost_inf_norm;
-      if (cost_inf_norm > max_optimal_cost * 1e-3) {
+      if (keeps_sweeping(cost_inf_norm, g->gamma)) {
         still.push_back(k);
       } else {
         stopped.push_back(k);
@@ -1975,16 +1995,9 @@ int pp2d_mdp_batch_update(pp2d_mdp_batch* h, const uint32_t* instances, uint32_t
     if (listed[k]) return fail(PP2D_ERR_INVALID, "instance %u is listed twice", k);
     listed[k] = 1;
   }
-  for (uint32_t i = 0; i < n; ++i) {
-    const uint32_t k = instances[i];
-    const uint32_t gx = goals_xy[2 * (size_t)i], gy = goals_xy[2 * (size_t)i + 1];
-    if (gx >= h->W || gy >= h->H)
-      return fail(PP2D_ERR_INVALID, "instance %u: goal (%u %u) outside the %ux%u map", k, gx, gy,
-                  h->W, h->H);
-    if (maps[i * map_stride + (size_t)gy * h->W + gx] > 0)
-      return fail(PP2D_ERR_GOAL_OCCUPIED,
-                  "instance %u: The assigned goal (%u %u) is at a occupied cell...", k, gx, gy);
-  }
+  for (uint32_t i = 0; i < n; ++i)
+    PP2D_TRY_MDP(check_goal(maps + i * map_stride, h->W, h->H, goals_xy[2 * (size_t)i],
+                            goals_xy[2 * (size_t)i + 1], instances[i]));
   if (n == 0) return PP2D_OK;
   pp2d_mdp* g = h->grid;
   // Per listed instance: its trapped(n_k) and whether a solve froze it.
@@ -1997,14 +2010,9 @@ int pp2d_mdp_batch_update(pp2d_mdp_batch* h, const uint32_t* instances, uint32_t
   }
   PP2D_TRY_MDP(upload_list(h));
   // The device maps are read only while codes are built: the new maps go to
-  // the front of g->occ in list order (one copy of a map shared by the list),
-  // and no instance reads its map again before the next reset or update.
-  if (map_stride == 0 || map_stride == hw)
-    PP2D_CUDA(cudaMemcpyAsync(g->occ, maps, (map_stride ? n : 1) * hw, cudaMemcpyHostToDevice,
-                              g->stream));
-  else
-    PP2D_CUDA(cudaMemcpy2DAsync(g->occ, hw, maps, map_stride, hw, n, cudaMemcpyHostToDevice,
-                                g->stream));
+  // the front of g->occ in list order, and no instance reads its map again
+  // before the next reset or update.
+  PP2D_TRY_MDP(upload_maps(g, maps, map_stride, hw, n));
   for (uint32_t i = 0; i < n; ++i) {
     h->goals_host[2 * (size_t)list[i]] = goals_xy[2 * (size_t)i];
     h->goals_host[2 * (size_t)list[i] + 1] = goals_xy[2 * (size_t)i + 1];
@@ -2028,15 +2036,7 @@ int pp2d_mdp_batch_update(pp2d_mdp_batch* h, const uint32_t* instances, uint32_t
   p.action = g->action;
   p.res_cost = h->res_cost;
   p.res_action = h->res_action;
-  // Seed the mask of the next fused row-block launch, as update_map does.
-  p.need = nullptr;
-  p.n_strips = ((int)h->W + StripGeom<2, 2>::S - 1) / StripGeom<2, 2>::S;
-  p.rows_per_unit = p.n_rb = 1;
-  if (g->need_valid) {
-    p.need = g->need[g->need_rot];
-    p.rows_per_unit = g->need_rows_per_unit;
-    p.n_rb = g->need_units / p.n_strips;
-  }
+  p.mask = next_unit_mask(g);
   const size_t groups = (size_t)n * p.groups;
   dim3 grid((g->pitch / 4 + kCodeThreads - 1) / kCodeThreads,
             (unsigned)std::min<size_t>(groups, 65535));
@@ -2094,14 +2094,8 @@ int pp2d_mdp_batch_plan(pp2d_mdp_batch* h, const uint32_t* instance, const float
   if (n == 0) return PP2D_OK;
   pp2d_mdp* g = h->grid;
   const size_t hw = (size_t)h->H * h->W;
-  // action grid of each belief's instance: its snapshot once frozen, else its
-  // rows of the live grid (H*W bytes either way)
   std::vector<const uint8_t*> bases(n);
-  for (uint32_t i = 0; i < n; ++i) {
-    const uint32_t k = instance[i];
-    bases[i] = h->frozen[k] ? h->res_action + k * hw
-                            : g->action + (size_t)k * (h->H + 1) * h->W;
-  }
+  for (uint32_t i = 0; i < n; ++i) bases[i] = batch_actions_of(h, instance[i]);
   float* d_b = nullptr;
   const uint8_t** d_base = nullptr;
   uint8_t* d_a = nullptr;
@@ -2133,13 +2127,9 @@ int pp2d_mdp_batch_waypoints(pp2d_mdp_batch* h, uint32_t k, uint32_t sx, uint32_
     return fail(PP2D_ERR_INVALID, "instance %u outside the batch of %u", k, h->count);
   if (sx >= h->W || sy >= h->H)
     return fail(PP2D_ERR_INVALID, "start (%u %u) outside the map", sx, sy);
-  // instance k's action grid: its snapshot once frozen, else its rows of the
-  // live grid (H*W bytes either way, as in pp2d_mdp_batch_plan)
   const size_t hw = (size_t)h->H * h->W;
-  const uint8_t* src = h->frozen[k] ? h->res_action + k * hw
-                                    : h->grid->action + (size_t)k * (h->H + 1) * h->W;
   std::vector<uint8_t> a(hw);
-  PP2D_CUDA(cudaMemcpyAsync(a.data(), src, hw, cudaMemcpyDeviceToHost, h->grid->stream));
+  PP2D_CUDA(cudaMemcpyAsync(a.data(), batch_actions_of(h, k), hw, cudaMemcpyDeviceToHost, h->grid->stream));
   PP2D_CUDA(cudaStreamSynchronize(h->grid->stream));
   *n_out = rollout(a.data(), h->W, h->H, sx, sy, cells, max_len);
   return PP2D_OK;

@@ -980,16 +980,27 @@ __device__ __forceinline__ void cell_codes4(const CodeParams& p, int x0, int gy,
   }
 }
 
-template <bool FAST>
-__device__ __forceinline__ void code_march(const CodeParams& p, int c0, int r0) {
+// The CodeParams grid row gy is built from, and its row ly in them: the row
+// itself on a single grid (batch_row below on the tall grid of a batch).
+__device__ __forceinline__ const CodeParams& row_of(const CodeParams& p, int gy, int& ly) {
+  ly = gy;
+  return p;
+}
+__device__ __forceinline__ int first_row(const CodeParams& p) { return p.row_begin; }
+
+// P: CodeParams or BatchCodeParams (code, pitch, rows_phys, row_of, first_row)
+template <bool FAST, class P>
+__device__ __forceinline__ void code_march(const P& p, int c0, int r0) {
   const int x0 = c0 - kPadLeft;
   const int r1 = min(r0 + kCodeRows, p.rows_phys);
-  int gy = p.row_begin + r0 - kPadRows;
-  uint32_t m0 = occ_mask6<FAST>(p, x0, gy - 1), m1 = occ_mask6<FAST>(p, x0, gy);
+  int gy = first_row(p) + r0 - kPadRows;
+  int ly;
+  uint32_t m0 = occ_mask6<FAST>(row_of(p, gy - 1, ly), x0, ly);
+  uint32_t m1 = occ_mask6<FAST>(row_of(p, gy, ly), x0, ly);
   for (int r = r0; r < r1; ++r, ++gy) {
-    const uint32_t m2 = occ_mask6<FAST>(p, x0, gy + 1);
+    const uint32_t m2 = occ_mask6<FAST>(row_of(p, gy + 1, ly), x0, ly);
     uint32_t code[4];
-    cell_codes4(p, x0, gy, m0, m1, m2, code);
+    cell_codes4(row_of(p, gy, ly), x0, ly, m0, m1, m2, code);
     // pitch is a multiple of 32 and c0 of 4: the 4 codes are 8-byte aligned
     *reinterpret_cast<uint2*>(p.code + (size_t)r * p.pitch + c0) =
         make_uint2(code[0] | (code[1] << 16), code[2] | (code[3] << 16));
@@ -1021,27 +1032,94 @@ __global__ void __launch_bounds__(kCodeThreads) mdp_code_kernel(const CodeParams
 // stored J changed is dirty; every dirty unit of the fused row-block launch
 // geometry sets the bits of its 3x3 unit neighbourhood in `need`, the mask the
 // next fused launch reads.
+
+// The unit mask of the next fused row-block launch; unit = row_block *
+// n_strips + strip.  need == NULL: no valid mask (that launch runs every unit).
+struct UnitMask {
+  uint32_t* need;
+  int n_strips, rows_per_unit, n_rb;
+};
+
 struct UpdateParams {
   CodeParams c;          // occupancy of the new map, code plane, new goal
   float* j;              // current J plane (ghost rows included)
   float* jchk;           // residual snapshot
   float trapped;         // J_n of an occupied cell, n = sweep count
-  uint32_t* need;        // NULL: no seeding (the next fused launch runs every unit)
-  int n_strips, rows_per_unit, n_rb;   // unit = row_block * n_strips + strip
+  UnitMask mask;         // seeded with the dirty units
   int H;                 // owned rows
 };
 
-// P: UpdateParams or BatchUpdateParams (need, n_rb, n_strips)
-template <class P>
-__device__ __forceinline__ void mark_unit_neighbourhood(const P& p, int rb, int k) {
+__device__ __forceinline__ void mark_unit_neighbourhood(const UnitMask& m, int rb, int k) {
 #pragma unroll 1
   for (int i = 0; i < 9; ++i) {
     const int r = rb + i / 3 - 1, kk = k + i % 3 - 1;
-    if (r >= 0 && r < p.n_rb && kk >= 0 && kk < p.n_strips) {
-      const int v = r * p.n_strips + kk;
-      atomicOr(p.need + (v >> 5), 1u << (v & 31));
+    if (r >= 0 && r < m.n_rb && kk >= 0 && kk < m.n_strips) {
+      const int v = r * m.n_strips + kk;
+      atomicOr(m.need + (v >> 5), 1u << (v & 31));
     }
   }
+}
+
+// Strip width of the fused row-block launches: a 4-cell group from column x0
+// lies in strip k_lo = max(x0, 0) / kUnitStrip or in the next one.
+constexpr int kUnitStrip = StripGeom<2, 2>::S;
+
+// Warp-wide: the units of row block rb that hold a dirty cell of this row
+// (dirty_lo: strip k_lo, dirty_hi: strip k_lo + 1) mark their 3x3 unit
+// neighbourhoods in m.need, one lane per unit.  All 32 lanes call it.
+__device__ __forceinline__ void seed_dirty_units(const UnitMask& m, int rb, int k_lo,
+                                                 bool dirty_lo, bool dirty_hi, int lane) {
+#pragma unroll
+  for (int side = 0; side < 2; ++side) {
+    const bool d = side ? dirty_hi : dirty_lo;
+    const uint32_t b = __ballot_sync(0xffffffffu, d);
+    if (d) {
+      const int k = k_lo + side;
+      const uint32_t peers = __match_any_sync(b, k);
+      if (__ffs(peers) - 1 == lane) mark_unit_neighbourhood(m, rb, k);
+    }
+  }
+}
+
+// The update rule on the 4 cells of plane index q (columns x0 .. x0+3), given
+// their new codes: reads the old codes and J, writes the codes and J that
+// changed, and J' into jchk unless it is NULL.  A newly freed cell takes
+// `trapped`, or its entry of the result-slot row `slot` (indexed by column)
+// when slot is not NULL.  Returns whether a cell of strip k_lo (or left of the
+// map) and of strip k_lo + 1 is dirty.
+__device__ __forceinline__ void replan_cells4(uint16_t* code_plane, float* j, float* jchk,
+                                              size_t q, int x0, int k_lo,
+                                              const uint32_t (&code)[4], float trapped,
+                                              const float* slot, bool& dirty_lo, bool& dirty_hi) {
+  const uint2 oc2 = *reinterpret_cast<const uint2*>(code_plane + q);
+  const uint32_t old[4] = {oc2.x & 0xFFFFu, oc2.x >> 16, oc2.y & 0xFFFFu, oc2.y >> 16};
+  const float4 jv = *reinterpret_cast<const float4*>(j + q);
+  const float jo[4] = {jv.x, jv.y, jv.z, jv.w};
+  float jn[4];
+  bool code_changed = false, j_changed = false;
+  dirty_lo = dirty_hi = false;
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const bool occ_new = code[i] & kCodeOccBit, occ_old = old[i] & kCodeOccBit;
+    jn[i] = jo[i];
+    if (occ_new && !occ_old) jn[i] = 0.0f;
+    if (!occ_new && occ_old) jn[i] = slot ? __ldg(slot + x0 + i) : trapped;
+    if (!(code[i] & (kCodeOccBit | kCodeLiveBit))) jn[i] = 0.0f;   // the goal
+    const bool cc = code[i] != old[i];
+    const bool jc = __float_as_uint(jn[i]) != __float_as_uint(jo[i]);
+    code_changed |= cc;
+    j_changed |= jc;
+    if (cc || jc) {
+      if ((x0 + i) / kUnitStrip == k_lo || x0 + i < 0) dirty_lo = true;
+      else dirty_hi = true;
+    }
+  }
+  if (code_changed)
+    *reinterpret_cast<uint2*>(code_plane + q) =
+        make_uint2(code[0] | (code[1] << 16), code[2] | (code[3] << 16));
+  const float4 jw = make_float4(jn[0], jn[1], jn[2], jn[3]);
+  if (j_changed) *reinterpret_cast<float4*>(j + q) = jw;
+  if (jchk != nullptr) *reinterpret_cast<float4*>(jchk + q) = jw;
 }
 
 // Same thread shape as mdp_code_kernel (4 cells per thread, kCodeRows rows
@@ -1060,9 +1138,7 @@ __global__ void __launch_bounds__(kCodeThreads) mdp_update_map_kernel(const Upda
   auto mask = [&](int gy) {
     return fast ? occ_mask6<true>(cp, x0, gy) : occ_mask6<false>(cp, x0, gy);
   };
-  // strip of cell x0 (or of x = 0); the 4 cells lie in it or in the next one
-  constexpr int kStrip = StripGeom<2, 2>::S;
-  const int k_lo = max(x0, 0) / kStrip;
+  const int k_lo = max(x0, 0) / kUnitStrip;
   const int r1 = min(r0 + kCodeRows, cp.rows_phys);
   int gy = cp.row_begin + r0 - kPadRows;
   uint32_t m0 = mask(gy - 1), m1 = mask(gy);
@@ -1074,58 +1150,36 @@ __global__ void __launch_bounds__(kCodeThreads) mdp_update_map_kernel(const Upda
     m1 = m2;
     bool dirty_lo = false, dirty_hi = false;
     if (active) {
-      const size_t q = (size_t)r * cp.pitch + c0;
-      const uint2 oc2 = *reinterpret_cast<const uint2*>(cp.code + q);
-      const uint32_t old[4] = {oc2.x & 0xFFFFu, oc2.x >> 16, oc2.y & 0xFFFFu, oc2.y >> 16};
-      const float4 jv = *reinterpret_cast<const float4*>(p.j + q);
-      const float jo[4] = {jv.x, jv.y, jv.z, jv.w};
-      float jn[4];
-      bool code_changed = false, j_changed = false;
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const bool occ_new = code[i] & kCodeOccBit, occ_old = old[i] & kCodeOccBit;
-        jn[i] = jo[i];
-        if (occ_new && !occ_old) jn[i] = 0.0f;
-        if (!occ_new && occ_old) jn[i] = p.trapped;
-        if (!(code[i] & (kCodeOccBit | kCodeLiveBit))) jn[i] = 0.0f;   // the goal
-        const bool cc = code[i] != old[i];
-        const bool jc = __float_as_uint(jn[i]) != __float_as_uint(jo[i]);
-        code_changed |= cc;
-        j_changed |= jc;
-        if (cc || jc) {
-          if ((x0 + i) / kStrip == k_lo || x0 + i < 0) dirty_lo = true;
-          else dirty_hi = true;
-        }
-      }
-      if (code_changed)
-        *reinterpret_cast<uint2*>(cp.code + q) =
-            make_uint2(code[0] | (code[1] << 16), code[2] | (code[3] << 16));
-      const float4 jw = make_float4(jn[0], jn[1], jn[2], jn[3]);
-      if (j_changed) *reinterpret_cast<float4*>(p.j + q) = jw;
-      if (r >= kPadRows && r < kPadRows + p.H) *reinterpret_cast<float4*>(p.jchk + q) = jw;
+      const bool owned = r >= kPadRows && r < kPadRows + p.H;
+      replan_cells4(cp.code, p.j, owned ? p.jchk : nullptr, (size_t)r * cp.pitch + c0, x0, k_lo,
+                    code, p.trapped, nullptr, dirty_lo, dirty_hi);
     }
-    if (p.need != nullptr && __any_sync(0xffffffffu, dirty_lo || dirty_hi)) {
+    if (p.mask.need != nullptr && __any_sync(0xffffffffu, dirty_lo || dirty_hi)) {
       // ghost rows belong to the row block next to them
       const int y = min(max(r - kPadRows, 0), p.H - 1);
-      const int rb = min(y / p.rows_per_unit, p.n_rb - 1);
-#pragma unroll
-      for (int side = 0; side < 2; ++side) {
-        const bool d = side ? dirty_hi : dirty_lo;
-        const uint32_t m = __ballot_sync(0xffffffffu, d);
-        if (d) {
-          const int k = k_lo + side;
-          const uint32_t peers = __match_any_sync(m, k);
-          if (__ffs(peers) - 1 == lane) mark_unit_neighbourhood(p, rb, k);
-        }
-      }
+      seed_dirty_units(p.mask, min(y / p.mask.rows_per_unit, p.mask.n_rb - 1), k_lo, dirty_lo,
+                       dirty_hi, lane);
     }
   }
 }
 
 // ---------------------------------------------------------------------------
+// Maximum of m over a CTA of 256 threads into *result, as float bits:
+// atomicMax on uint is order preserving for non-negative floats.
+__device__ __forceinline__ void block_max_to(float m, uint32_t* result) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  __shared__ float wm[8];
+  if ((threadIdx.x & 31) == 0) wm[threadIdx.x >> 5] = m;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int i = 1; i < 8; ++i) m = fmaxf(m, wm[i]);
+    atomicMax(result, __float_as_uint(m));
+  }
+}
+
 // max |J - Jchk| over the owned rows, then Jchk = J
-// (path_planning_2d.cu:243-251).  result: float bits, atomicMax on uint is
-// order preserving for non-negative floats.
+// (path_planning_2d.cu:243-251), into *result (block_max_to).
 // CHK_ZERO: first check after a reset -- Jchk is J_0 = 0 by definition and is
 // not read (the reset then does not have to zero it).
 template <bool CHK_ZERO>
@@ -1145,15 +1199,7 @@ mdp_residual_kernel(const float4* __restrict__ j, float4* __restrict__ chk,
                        fmaxf(fabsf(a.z - b.z), fabsf(a.w - b.w))));
     chk[i] = a;
   }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
-  __shared__ float wm[8];
-  if ((threadIdx.x & 31) == 0) wm[threadIdx.x >> 5] = m;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    for (int i = 1; i < 8; ++i) m = fmaxf(m, wm[i]);
-    atomicMax(result, __float_as_uint(m));
-  }
+  block_max_to(m, result);
 }
 
 // ---------------------------------------------------------------------------
@@ -1372,30 +1418,11 @@ __device__ __forceinline__ CodeParams batch_row(const BatchCodeParams& p, int gy
 }
 
 // code_march on the tall grid: every row is built from the map and goal of
-// its own instance with the single-grid occ_mask6 / cell_codes4.
-template <bool FAST>
-__device__ __forceinline__ void batch_code_march(const BatchCodeParams& p, int c0, int r0) {
-  const int x0 = c0 - kPadLeft;
-  const int r1 = min(r0 + kCodeRows, p.rows_phys);
-  auto mask = [&](int gy) {
-    int ly;
-    const CodeParams c = batch_row(p, gy, ly);
-    return occ_mask6<FAST>(c, x0, ly);
-  };
-  int gy = r0 - kPadRows;
-  uint32_t m0 = mask(gy - 1), m1 = mask(gy);
-  for (int r = r0; r < r1; ++r, ++gy) {
-    const uint32_t m2 = mask(gy + 1);
-    int ly;
-    const CodeParams c = batch_row(p, gy, ly);
-    uint32_t code[4];
-    cell_codes4(c, x0, ly, m0, m1, m2, code);
-    *reinterpret_cast<uint2*>(p.code + (size_t)r * p.pitch + c0) =
-        make_uint2(code[0] | (code[1] << 16), code[2] | (code[3] << 16));
-    m0 = m1;
-    m1 = m2;
-  }
+// its own instance.
+__device__ __forceinline__ CodeParams row_of(const BatchCodeParams& p, int gy, int& ly) {
+  return batch_row(p, gy, ly);
 }
+__device__ __forceinline__ int first_row(const BatchCodeParams&) { return 0; }
 
 // grid: (ceil(pitch / 4 / kCodeThreads), any); blocks stride over the
 // kCodeRows row groups.
@@ -1407,8 +1434,8 @@ __global__ void __launch_bounds__(kCodeThreads) mdp_batch_code_kernel(const Batc
   const bool fast = (p.W & 3) == 0 && (x0 & 3) == 0 && x0 >= 0 && x0 + 3 < p.W &&
                     (reinterpret_cast<uintptr_t>(p.maps) & 3u) == 0;
   for (int r0 = blockIdx.y * kCodeRows; r0 < p.rows_phys; r0 += gridDim.y * kCodeRows) {
-    if (fast) batch_code_march<true>(p, c0, r0);
-    else batch_code_march<false>(p, c0, r0);
+    if (fast) code_march<true>(p, c0, r0);
+    else code_march<false>(p, c0, r0);
   }
 }
 
@@ -1438,15 +1465,7 @@ mdp_batch_residual_kernel(const float* __restrict__ j, float* __restrict__ chk,
                        fmaxf(fabsf(a.z - b.z), fabsf(a.w - b.w))));
     b4[i] = a;
   }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
-  __shared__ float wm[8];
-  if ((threadIdx.x & 31) == 0) wm[threadIdx.x >> 5] = m;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    for (int i = 1; i < 8; ++i) m = fmaxf(m, wm[i]);
-    atomicMax(result + k, __float_as_uint(m));
-  }
+  block_max_to(m, result + k);
 }
 
 struct BatchFreezeParams {
@@ -1460,10 +1479,9 @@ struct BatchFreezeParams {
   const float* trapped;    // [n_list]: J of an occupied cell at list[i]'s sweep count
   int n_list;
   int W, H, pitch;
-  // FREEZE, mask part: NULL = no valid mask to clear
-  uint32_t* need;          // the mask the next fused row-block launch reads
+  UnitMask mask;           // FREEZE: the mask to clear
   const uint8_t* frozen;   // [count]: 1 = instance stopped
-  int count, Htot, n_strips, rows_per_unit, n_rb;
+  int count, Htot;
 };
 
 // Snapshot of the instances in `list` into their result slots: J with the
@@ -1475,7 +1493,7 @@ struct BatchFreezeParams {
 //       read again, and a unit made of such rows and separators computes
 //       +0 from +0, so it never marks its neighbours when it runs;
 //   (b) the bits of every unit whose rows all lie in stopped instances and
-//       separators are cleared in `need`.
+//       separators are cleared in mask.need.
 // One thread per cell, then one thread per row block (grid-stride loops).
 template <bool FREEZE>
 __global__ void __launch_bounds__(256) mdp_batch_freeze_kernel(const BatchFreezeParams p) {
@@ -1499,10 +1517,11 @@ __global__ void __launch_bounds__(256) mdp_batch_freeze_kernel(const BatchFreeze
       p.j[1][q] = 0.0f;
     }
   }
-  if (!FREEZE || p.need == nullptr) return;
-  for (size_t rb = t0; rb < (size_t)p.n_rb; rb += stride) {
-    const int y0 = (int)rb * p.rows_per_unit;
-    const int y1 = min(y0 + p.rows_per_unit, p.Htot);
+  const UnitMask& m = p.mask;
+  if (!FREEZE || m.need == nullptr) return;
+  for (size_t rb = t0; rb < (size_t)m.n_rb; rb += stride) {
+    const int y0 = (int)rb * m.rows_per_unit;
+    const int y1 = min(y0 + m.rows_per_unit, p.Htot);
     // instances with a row in [y0, y1): a separator row belongs to none
     int k0 = y0 / (p.H + 1), k1 = (y1 - 1) / (p.H + 1);
     if (y0 - k0 * (p.H + 1) == p.H) ++k0;
@@ -1510,9 +1529,9 @@ __global__ void __launch_bounds__(256) mdp_batch_freeze_kernel(const BatchFreeze
     bool all_frozen = true;
     for (int k = k0; k <= k1 && all_frozen; ++k) all_frozen = p.frozen[k] != 0;
     if (!all_frozen) continue;
-    const int u0 = (int)rb * p.n_strips;
-    for (int w = u0 >> 5; w <= (u0 + p.n_strips - 1) >> 5; ++w)
-      atomicAnd(p.need + w, ~unit_range_bits(w, u0, u0 + p.n_strips));
+    const int u0 = (int)rb * m.n_strips;
+    for (int w = u0 >> 5; w <= (u0 + m.n_strips - 1) >> 5; ++w)
+      atomicAnd(m.need + w, ~unit_range_bits(w, u0, u0 + m.n_strips));
   }
 }
 
@@ -1536,8 +1555,7 @@ struct BatchUpdateParams {
   uint8_t* action;         // dense action grid of the tall grid
   const float* res_cost;   // [count][H][W]
   const uint8_t* res_action;
-  uint32_t* need;          // NULL: no seeding (the next fused launch runs every unit)
-  int n_strips, rows_per_unit, n_rb;
+  UnitMask mask;           // seeded with the dirty units
 };
 
 // grid: (ceil(pitch / 4 / kCodeThreads), any); blocks stride over the row
@@ -1553,8 +1571,7 @@ __global__ void __launch_bounds__(kCodeThreads) mdp_batch_update_kernel(const Ba
   // the maps are H*W bytes apart: 4-aligned whenever W is
   const bool fast = (W & 3) == 0 && (x0 & 3) == 0 && x0 >= 0 && x0 + 3 < W &&
                     (reinterpret_cast<uintptr_t>(p.maps) & 3u) == 0;
-  constexpr int kStrip = StripGeom<2, 2>::S;
-  const int k_lo = max(x0, 0) / kStrip;
+  const int k_lo = max(x0, 0) / kUnitStrip;
   for (int g = blockIdx.y; g < p.n_list * p.groups; g += gridDim.y) {   // uniform over the block
     const int i = g / p.groups;
     const int ly0 = (g - i * p.groups) * kCodeRows;
@@ -1583,53 +1600,21 @@ __global__ void __launch_bounds__(kCodeThreads) mdp_batch_update_kernel(const Ba
       m1 = m2;
       bool dirty_lo = false, dirty_hi = false;
       if (active) {
-        const size_t q = (size_t)(ty + kPadRows) * p.c.pitch + c0;
-        const size_t slot = (size_t)k * hw + (size_t)ly * W;   // row ly of k's result slot
-        const uint2 oc2 = *reinterpret_cast<const uint2*>(p.c.code + q);
-        const uint32_t old[4] = {oc2.x & 0xFFFFu, oc2.x >> 16, oc2.y & 0xFFFFu, oc2.y >> 16};
-        const float4 jv = *reinterpret_cast<const float4*>(p.j + q);
-        const float jo[4] = {jv.x, jv.y, jv.z, jv.w};
-        float jn[4];
-        bool code_changed = false, j_changed = false;
+        // row ly of k's result slot; a frozen row's codes are all padding:
+        // every free cell takes its slot value
+        const size_t slot = (size_t)k * hw + (size_t)ly * W;
+        replan_cells4(p.c.code, p.j, p.jchk, (size_t)(ty + kPadRows) * p.c.pitch + c0, x0, k_lo,
+                      code, trapped, thaw ? p.res_cost + slot : nullptr, dirty_lo, dirty_hi);
+        if (thaw) {
 #pragma unroll
-        for (int e = 0; e < 4; ++e) {
-          const bool occ_new = code[e] & kCodeOccBit, occ_old = old[e] & kCodeOccBit;
-          jn[e] = jo[e];
-          if (occ_new && !occ_old) jn[e] = 0.0f;
-          // (a frozen row's codes are all padding: every free cell takes its slot value)
-          if (!occ_new && occ_old) jn[e] = thaw ? __ldg(p.res_cost + slot + x0 + e) : trapped;
-          if (!(code[e] & (kCodeOccBit | kCodeLiveBit))) jn[e] = 0.0f;   // the goal
-          const bool cc = code[e] != old[e];
-          const bool jc = __float_as_uint(jn[e]) != __float_as_uint(jo[e]);
-          code_changed |= cc;
-          j_changed |= jc;
-          if (cc || jc) {
-            if ((x0 + e) / kStrip == k_lo || x0 + e < 0) dirty_lo = true;
-            else dirty_hi = true;
-          }
-          if (thaw && x0 + e >= 0 && x0 + e < W)
-            p.action[(size_t)ty * W + x0 + e] = __ldg(p.res_action + slot + x0 + e);
-        }
-        if (code_changed)
-          *reinterpret_cast<uint2*>(p.c.code + q) =
-              make_uint2(code[0] | (code[1] << 16), code[2] | (code[3] << 16));
-        const float4 jw = make_float4(jn[0], jn[1], jn[2], jn[3]);
-        if (j_changed) *reinterpret_cast<float4*>(p.j + q) = jw;
-        *reinterpret_cast<float4*>(p.jchk + q) = jw;
-      }
-      if (p.need != nullptr && __any_sync(0xffffffffu, dirty_lo || dirty_hi)) {
-        const int rb = min(ty / p.rows_per_unit, p.n_rb - 1);
-#pragma unroll
-        for (int side = 0; side < 2; ++side) {
-          const bool d = side ? dirty_hi : dirty_lo;
-          const uint32_t m = __ballot_sync(0xffffffffu, d);
-          if (d) {
-            const int kk = k_lo + side;
-            const uint32_t peers = __match_any_sync(m, kk);
-            if (__ffs(peers) - 1 == lane) mark_unit_neighbourhood(p, rb, kk);
-          }
+          for (int e = 0; e < 4; ++e)
+            if (x0 + e >= 0 && x0 + e < W)
+              p.action[(size_t)ty * W + x0 + e] = __ldg(p.res_action + slot + x0 + e);
         }
       }
+      if (p.mask.need != nullptr && __any_sync(0xffffffffu, dirty_lo || dirty_hi))
+        seed_dirty_units(p.mask, min(ty / p.mask.rows_per_unit, p.mask.n_rb - 1), k_lo, dirty_lo,
+                         dirty_hi, lane);
     }
   }
 }
