@@ -602,6 +602,51 @@ int pp2d_sim_update_belief_measurement(pp2d_sim* s, float* beliefs, uint32_t n,
 int pp2d_sim_step(pp2d_sim* s, float* beliefs, uint32_t n, const uint8_t* actions,
                   const uint8_t* measurements);
 
+/* ------------------------------------------------------------------------
+ * Closed-loop episodes: planner + simulator in one device loop (DESIGN.md
+ * section 7, "Closed-loop rollouts")
+ * ------------------------------------------------------------------------
+ * Episode i (global id e = first_episode + i) starts at cell starts_xy[2i],
+ * starts_xy[2i+1] (free in the simulator's map) with belief beliefs[i] ([n][HW];
+ * NULL: a point mass of 1.0f at the start).  Each step t: stop when the true
+ * cell is the planner's goal (reached = 1) or t == max_steps (reached = 0);
+ * u = the planner's action at the belief mode; move by the simulator's motion
+ * model (blocked or out-of-map targets: stay, collisions += 1); read the four
+ * cell sensors {up, left, right, down} of the simulator's map, each flipped
+ * with probability 0.02; filter the belief as pp2d_sim_step.  Random numbers:
+ * Philox4x32-10, key (seed & 0xffffffff, seed >> 32), step t of episode e uses
+ * the blocks of counters (t, e_lo, e_hi, 0) and (t, e_lo, e_hi, 1); a word w
+ * is the uniform (w >> 8) * 2^-24.  Results depend only on (maps, planner,
+ * start, belief, seed, e), not on the other episodes of the call.
+ *
+ * Every output pointer may be NULL; entries past an episode's last step are
+ * not written.  PP2D_ERR_INVALID (messages name the episode) for NULL handles
+ * or starts_xy, a world / planner size mismatch, a start outside the map or
+ * occupied in the simulator's map, an instance index >= count;
+ * PP2D_ERR_STATE for a shard or multi-GPU planner.  All checks come before any
+ * device work; n == 0 does nothing. */
+typedef struct pp2d_rollout {   /* every pointer may be NULL */
+  uint32_t* steps;          /* [n] steps taken */
+  uint8_t*  reached;        /* [n] 1: stopped on the goal */
+  uint32_t* collisions;     /* [n] moves into a blocked or out-of-map cell */
+  uint32_t* final_cell;     /* [n] y*W+x */
+  float*    final_belief;   /* [n][HW] */
+  uint32_t* cells;          /* [n][max_steps+1], start included */
+  uint8_t*  actions;        /* [n][max_steps] */
+  uint8_t*  measurements;   /* [n][max_steps], bit j = sensor j */
+} pp2d_rollout;
+/* Every episode follows the single-GPU handle `planner` (its goal, its action
+ * grid as pp2d_mdp_plan reads it). */
+int pp2d_sim_rollout_mdp(pp2d_sim* s, pp2d_mdp* planner, uint32_t n, const uint32_t* starts_xy,
+                         const float* beliefs, uint32_t max_steps, uint64_t seed,
+                         uint64_t first_episode, pp2d_rollout* out);
+/* Episode i follows batch instance instances[i] (its goal, and its action
+ * grid as pp2d_mdp_batch_plan reads it: the snapshot of a frozen instance). */
+int pp2d_sim_rollout_mdp_batch(pp2d_sim* s, pp2d_mdp_batch* planner, const uint32_t* instances,
+                               uint32_t n, const uint32_t* starts_xy, const float* beliefs,
+                               uint32_t max_steps, uint64_t seed, uint64_t first_episode,
+                               pp2d_rollout* out);
+
 #ifdef __cplusplus
 }
 #endif

@@ -26,6 +26,13 @@ class Halo(ctypes.Structure):
                 ("recv_bottom", _vp), ("bytes", ctypes.c_size_t)]
 
 
+class Rollout(ctypes.Structure):
+    """pp2d_rollout: output arrays of pp2d_sim_rollout_mdp*, each may be NULL."""
+    _fields_ = [("steps", _vp), ("reached", _vp), ("collisions", _vp), ("final_cell", _vp),
+                ("final_belief", _vp), ("cells", _vp), ("actions", _vp),
+                ("measurements", _vp)]
+
+
 # name -> (restype, argtypes); every symbol declared in include/pp2d.h.
 SIGNATURES = {
     "pp2d_last_error": (ctypes.c_char_p, []),
@@ -101,6 +108,10 @@ SIGNATURES = {
     "pp2d_sim_update_belief_action": (_i, [_vp, _vp, _u32, _vp]),
     "pp2d_sim_update_belief_measurement": (_i, [_vp, _vp, _u32, _vp]),
     "pp2d_sim_step": (_i, [_vp, _vp, _u32, _vp, _vp]),
+    "pp2d_sim_rollout_mdp": (_i, [_vp, _vp, _u32, _vp, _vp, _u32, ctypes.c_uint64,
+                                  ctypes.c_uint64, ctypes.POINTER(Rollout)]),
+    "pp2d_sim_rollout_mdp_batch": (_i, [_vp, _vp, _vp, _u32, _vp, _vp, _u32, ctypes.c_uint64,
+                                        ctypes.c_uint64, ctypes.POINTER(Rollout)]),
     "pp2d_tree_create": (_i, [_vp, _vp, ctypes.POINTER(_vp)]),
     "pp2d_tree_destroy": (None, [_vp]),
     "pp2d_tree_expand": (_i, [_vp]),

@@ -14,7 +14,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libpp2d.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 
-SOURCES = ["mdp.cu", "pomdp.cu", "pbvi.cu", "sim.cu"]
+SOURCES = ["mdp.cu", "pomdp.cu", "pbvi.cu", "sim.cu", "rollout.cu"]
 FLAGS = [
     "-std=c++17", "-O3", "-lineinfo",
     "-gencode", "arch=compute_100a,code=sm_100a",

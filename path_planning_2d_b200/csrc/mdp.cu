@@ -20,6 +20,7 @@
 #include <new>
 #include <vector>
 
+#include "handles.h"
 #include "mdp_kernels.cuh"
 
 namespace pp2d {
@@ -1855,6 +1856,26 @@ static int batch_snapshot(pp2d_mdp_batch* b, const std::vector<uint32_t>& list) 
   g_launches.fetch_add(1, std::memory_order_relaxed);
   PP2D_CUDA(cudaGetLastError());
   return PP2D_OK;
+}
+
+// Accessors of handles.h (the closed-loop rollouts of rollout.cu).
+PlannerView mdp_view(const pp2d_mdp* h) {
+  PlannerView v;
+  v.H = h->H; v.W = h->W;
+  v.sharded = h->sharded || !h->parts.empty();
+  v.action = h->action;
+  v.gx = h->gx; v.gy = h->gy;
+  v.stream = h->stream;
+  return v;
+}
+uint32_t mdp_batch_count(const pp2d_mdp_batch* b) { return b->count; }
+PlannerView mdp_batch_view(const pp2d_mdp_batch* b, uint32_t k) {
+  PlannerView v;
+  v.H = b->H; v.W = b->W;
+  v.action = batch_actions_of(b, k);
+  v.gx = b->goals_host[2 * (size_t)k]; v.gy = b->goals_host[2 * (size_t)k + 1];
+  v.stream = b->grid->stream;
+  return v;
 }
 
 }  // namespace pp2d

@@ -41,6 +41,7 @@
 #include <stdint.h>
 
 #include "async_copy.cuh"
+#include "belief.cuh"
 #include "fp_exact.cuh"
 
 namespace pp2d {
@@ -1338,34 +1339,6 @@ __global__ void mdp_export_kernel(const float* __restrict__ j,
   } else {
     out[(size_t)y * W + x] = (code[q] & kCodeOccBit) ? occupied_cost : j[q];
   }
-}
-
-// MdpPathPlanning2d::beliefCallback (path_planning_2d.cu:168-189): index of
-// the first strict maximum of the belief b[0 .. n) starting from (0.0f,
-// index 0), valid in thread 0 of a 256-thread CTA.
-__device__ __forceinline__ unsigned long long belief_mode(const float* __restrict__ b, size_t n) {
-  float bm = 0.0f;
-  unsigned long long bi = 0;
-  for (size_t i = threadIdx.x; i < n; i += blockDim.x) {
-    float v = b[i];
-    if (v > bm) { bm = v; bi = i; }   // ascending i per thread: first max kept
-  }
-  // (value, index) reduction: larger value wins, ties -> smaller index.
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    float ov = __shfl_xor_sync(0xffffffffu, bm, o);
-    unsigned long long oi = __shfl_xor_sync(0xffffffffu, bi, o);
-    if (ov > bm || (ov == bm && oi < bi)) { bm = ov; bi = oi; }
-  }
-  __shared__ float sv[8];
-  __shared__ unsigned long long si[8];
-  if ((threadIdx.x & 31) == 0) { sv[threadIdx.x >> 5] = bm; si[threadIdx.x >> 5] = bi; }
-  __syncthreads();
-  if (threadIdx.x == 0)
-    for (int i = 1; i < 8; ++i)
-      if (sv[i] > bm || (sv[i] == bm && si[i] < bi)) { bm = sv[i]; bi = si[i]; }
-  // all beliefs <= 0: the reference keeps index 0.
-  return bm > 0.0f ? bi : 0;
 }
 
 // The action at the belief mode.  One CTA per belief.

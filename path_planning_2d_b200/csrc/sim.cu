@@ -23,6 +23,8 @@
 #include <new>
 #include <vector>
 
+#include "belief.cuh"
+#include "handles.h"
 #include "pomdp_host.h"
 
 struct pp2d_sim {
@@ -30,25 +32,13 @@ struct pp2d_sim {
   uint8_t* d_map = nullptr;
   float *d_a = nullptr, *d_b = nullptr, *d_sum = nullptr;
   uint8_t* d_args = nullptr;
+  std::vector<uint8_t> map_host;      // checks of the rollouts' starts
   size_t cap = 0;                     // beliefs the buffers hold
   cudaStream_t stream = nullptr;
 };
 
 namespace {
 using namespace pp2d;
-
-// naive probability of slot i under action u (sim:459-495)
-__device__ __forceinline__ float naive_prob(int u, int i) {
-  if (u == 4) return i == 4 ? 1.0f : 0.0f;
-  if (i == u) return 0.7f;
-  if (i == 4) return 0.1f;
-  // the two side slots of each action
-  const int s0 = (u == 0) ? 1 : (u == 1) ? 0 : (u == 2) ? 1 : (u == 3) ? 0 :
-                 (u == 5) ? 2 : (u == 6) ? 3 : (u == 7) ? 6 : 5;
-  const int s1 = (u == 0) ? 3 : (u == 1) ? 2 : (u == 2) ? 5 : (u == 3) ? 6 :
-                 (u == 5) ? 8 : (u == 6) ? 7 : (u == 7) ? 8 : 7;
-  return (i == s0 || i == s1) ? 0.1f : 0.0f;
-}
 
 // updateBelief(u) without the normalisation: out[b][p] for every cell p.
 __global__ void __launch_bounds__(256)
@@ -198,6 +188,16 @@ int run(pp2d_sim* s, float* beliefs, uint32_t n, const uint8_t* actions, const u
 }
 }  // namespace
 
+namespace pp2d {
+SimView sim_view(const pp2d_sim* s) {
+  SimView v;
+  v.H = (uint32_t)s->H; v.W = (uint32_t)s->W;
+  v.map_host = s->map_host.data();
+  v.map = s->d_map;
+  return v;
+}
+}  // namespace pp2d
+
 extern "C" {
 
 int pp2d_sim_create(uint32_t height, uint32_t width, const uint8_t* map, pp2d_sim** out) {
@@ -221,6 +221,7 @@ int pp2d_sim_create(uint32_t height, uint32_t width, const uint8_t* map, pp2d_si
   int rc = [&]() -> int {
     PP2D_CUDA(cudaMalloc(&s->d_map, (size_t)s->HW));
     PP2D_CUDA(cudaMemcpy(s->d_map, map, (size_t)s->HW, cudaMemcpyHostToDevice));
+    s->map_host.assign(map, map + s->HW);
     return PP2D_OK;
   }();
   if (rc != PP2D_OK) { pp2d_sim_destroy(s); return rc; }

@@ -1,14 +1,22 @@
 """Host-side mirror of the belief filter of the reference's DummySimulator
 (/root/reference/dummy_simulator/src/dummy_simulator.cpp:671-773) over the C
 ABI.  The reference keeps ONE belief and updates it on the CPU once per
-control message; here any number of independent beliefs (Monte-Carlo runs of
-a planner, many simulated robots) are filtered in one call on the GPU, each
-with its own action / measurement, with the reference's bits."""
+control message; here any number of independent beliefs (many simulated
+robots) are filtered in one call on the GPU, each with its own action /
+measurement, with the reference's bits.
+
+rollout() runs the whole closed loop of the reference's planner + simulator
+pair on the GPU for many episodes at once (Monte-Carlo runs of an MDP
+planner): plan at the belief mode, move, sense, filter, until the goal or a
+step limit, with motion and sensor noise drawn from a counter-based Philox
+generator so that every episode is reproducible on its own (DESIGN.md
+section 7, "Closed-loop rollouts")."""
 import ctypes
 
 import numpy as np
 
 from . import _lib
+from .mdp import MdpBatchPathPlanning2d, MdpPathPlanning2d
 
 
 class DummySimulator:
@@ -63,3 +71,50 @@ class DummySimulator:
             raise ValueError("give an action, a measurement, or both")
         _lib.check(rc)
         return b
+
+    def rollout(self, planner, starts, max_steps, seed, beliefs=None, instances=None,
+                first_episode=0, record=False):
+        """Closed-loop episodes of `planner` (MdpPathPlanning2d, or
+        MdpBatchPathPlanning2d with `instances`: the instance each episode
+        follows) in this simulator's map, from starts [n][2] = (x, y), with
+        beliefs [n][H*W] (default: a point mass at each start).  Episode i
+        draws its noise as episode first_episode + i of `seed`.  Returns a dict
+        of steps, reached, collisions and final_cell (y*W+x) per episode; with
+        record=True also final_belief [n][H*W], cells [n][max_steps+1] (the
+        start first), actions and measurements [n][max_steps] (bit j = sensor
+        j of up, left, right, down).  Entries past an episode's last step are
+        0."""
+        st = np.ascontiguousarray(starts, dtype=np.uint32).reshape(-1, 2)
+        n = st.shape[0]
+        hw = self.map_height * self.map_width
+        b = None
+        if beliefs is not None:
+            b = np.ascontiguousarray(beliefs, dtype=np.float32).reshape(n, hw)
+        res = {"steps": np.zeros(n, np.uint32), "reached": np.zeros(n, np.uint8),
+               "collisions": np.zeros(n, np.uint32), "final_cell": np.zeros(n, np.uint32)}
+        if record:
+            res["final_belief"] = np.zeros((n, hw), np.float32)
+            res["cells"] = np.zeros((n, max_steps + 1), np.uint32)
+            res["actions"] = np.zeros((n, max_steps), np.uint8)
+            res["measurements"] = np.zeros((n, max_steps), np.uint8)
+        out = _lib.Rollout(**{k: v.ctypes.data for k, v in res.items()})
+        bp = b.ctypes.data if b is not None else None
+        if isinstance(planner, MdpBatchPathPlanning2d):
+            if instances is None:
+                raise ValueError("a batch planner needs `instances`, one per episode")
+            idx = np.ascontiguousarray(instances, dtype=np.uint32).reshape(-1)
+            if idx.size != n:
+                raise ValueError("one instance per episode")
+            rc = self._lib.pp2d_sim_rollout_mdp_batch(self._h, planner._h, idx.ctypes.data, n,
+                                                      st.ctypes.data, bp, max_steps, seed,
+                                                      first_episode, ctypes.byref(out))
+        elif isinstance(planner, MdpPathPlanning2d):
+            if instances is not None:
+                raise ValueError("`instances` is for a batch planner")
+            rc = self._lib.pp2d_sim_rollout_mdp(self._h, planner._h, n, st.ctypes.data, bp,
+                                                max_steps, seed, first_episode,
+                                                ctypes.byref(out))
+        else:
+            raise TypeError("planner must be an MdpPathPlanning2d or MdpBatchPathPlanning2d")
+        _lib.check(rc)
+        return res
