@@ -487,7 +487,8 @@ int pp2d_pomdp_generate_belief_set(pp2d_pomdp* h, const float* initial_belief,
                                    uint32_t n, uint32_t rand_seed, float* belief_set);
 /* backupAlphaVectors (pbvi:344-641) from alpha = 0: `iterations` point-based
  * backups of all n alpha vectors (0 = the reference's count,
- * ceil(log(1e-3/5)/log(gamma)), pbvi:427-431).  alphas [n][HW], actions [n]. */
+ * ceil(log(1e-3/5)/log(gamma)), pbvi:427-431; defined only for 0 < gamma < 1,
+ * PP2D_ERR_INVALID otherwise).  alphas [n][HW], actions [n]. */
 int pp2d_pomdp_backup_alphas(pp2d_pomdp* h, const float* belief_set, uint32_t n,
                              uint32_t iterations, float* alphas, uint8_t* actions);
 /* pointBasedValueIteration (pbvi:643-676): both steps without the round trip

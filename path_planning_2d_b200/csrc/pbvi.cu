@@ -27,14 +27,18 @@
 //     with a DEFINED summation order (one sequential FMA chain over the cells
 //     per output).  Its result R only feeds an arg-max -- which Gamma_ao vector
 //     each belief picks --; the alpha vectors are gathered from Gamma_ao, not
-//     computed from R.  The contract is therefore: identical alpha vectors
-//     whenever no arg-max is decided by the last bits of two near-equal R
-//     entries (cuBLAS's blocking order is unspecified, so the reference itself
-//     is only defined up to that).  On every fixture of the reference's own
-//     solver, including the 500-belief bundled-map case, the alpha vectors are
-//     bit-identical (tests/test_pbvi_gpu.py).  PP2D_PBVI_CUBLAS=1 switches to
-//     the library call (bound at run time with dlopen) as a checker for tests;
-//     nothing else in the library depends on cuBLAS.
+//     computed from R.  cuBLAS's blocking order is unspecified, so the
+//     reference itself is only defined up to arg-max decisions between R
+//     entries that agree to the last bits: against it the product path gives
+//     identical alpha vectors wherever no such near-tie occurs, and otherwise
+//     a lower-bound set of the same quality (tests/test_pbvi_gpu.py).  With
+//     the order defined, the product path is bit-identical on ANY input to
+//     the CPU oracle of this arithmetic (tests/pbvi_oracle.c,
+//     tests/test_pbvi_kernel_gpu.py).  PP2D_PBVI_CUBLAS=1 switches to the
+//     library call (bound at run time with dlopen) as a checker for tests: it
+//     reproduces the reference's alpha vectors bit for bit on every fixture,
+//     including the 500-belief bundled-map case.  Nothing else in the library
+//     depends on cuBLAS.
 #include <algorithm>
 #include <cfloat>
 #include <cmath>
@@ -515,7 +519,10 @@ int expand_belief_set(pp2d_pomdp* h, const float* b0, uint32_t max_size, uint32_
   return rc;
 }
 
-// max_backup_iterations of pbvi:427-431 (float arithmetic, as written there)
+// max_backup_iterations of pbvi:427-431 (float arithmetic, as written there).
+// Defined only for 0 < gamma < 1: gamma = 1 gives -inf, gamma > 1 a negative
+// count and gamma <= 0 or NaN a NaN, none of which converts to uint32_t.
+bool reference_iterations_defined(float gamma) { return gamma > 0.0f && gamma < 1.0f; }
 uint32_t reference_backup_iterations(float gamma) {
   return (uint32_t)ceilf(logf(1.0e-3f / 5.0f) / logf(gamma));
 }
@@ -620,7 +627,12 @@ int pp2d_pomdp_backup_alphas(pp2d_pomdp* h, const float* belief_set, uint32_t n,
                              uint32_t iterations, float* alphas, uint8_t* actions) {
   if (!h || !belief_set || !alphas || n == 0)
     return fail(PP2D_ERR_INVALID, "NULL argument or empty set");
-  if (iterations == 0) iterations = reference_backup_iterations(h->gamma);
+  if (iterations == 0) {
+    if (!reference_iterations_defined(h->gamma))
+      return fail(PP2D_ERR_INVALID, "iterations = 0 takes the reference's count, which needs "
+                  "0 < gamma < 1 (gamma = %g); pass a count", (double)h->gamma);
+    iterations = reference_backup_iterations(h->gamma);
+  }
   const size_t bytes = (size_t)n * h->HW * sizeof(float);
   float *d_B = nullptr, *d_al = nullptr;
   uint8_t* d_ac = nullptr;
@@ -650,7 +662,12 @@ int pp2d_pomdp_solve_pbvi(pp2d_pomdp* h, const float* initial_belief, uint32_t n
                           float* alphas, uint8_t* actions) {
   if (!h || !initial_belief || !alphas || n == 0)
     return fail(PP2D_ERR_INVALID, "NULL argument or empty set");
-  if (iterations == 0) iterations = reference_backup_iterations(h->gamma);
+  if (iterations == 0) {
+    if (!reference_iterations_defined(h->gamma))
+      return fail(PP2D_ERR_INVALID, "iterations = 0 takes the reference's count, which needs "
+                  "0 < gamma < 1 (gamma = %g); pass a count", (double)h->gamma);
+    iterations = reference_backup_iterations(h->gamma);
+  }
   const size_t bytes = (size_t)n * h->HW * sizeof(float);
   std::vector<int> set;
   float *d_B = nullptr, *d_al = nullptr;
