@@ -472,7 +472,10 @@ int pp2d_pomdp_set_alphas(pp2d_pomdp* h, const float* fib_alphas,
 /*
  * fastInformedBound (fast_informed_bound_cuda.cu:97-276): value iteration on
  * the 9 FIB alpha vectors, 10 sweeps per convergence check, stop when the
- * inf-norm of the change is <= 0.01 (or after max_sweeps > 0).  alphas:
+ * inf-norm of the change is <= 0.01 (or after max_sweeps > 0; a cap is
+ * rounded up to whole 10-sweep checks).  max_sweeps = 0 needs |gamma| < 1:
+ * for a NaN gamma or |gamma| >= 1 that rule is not reached in useful time, and
+ * the call returns PP2D_ERR_INVALID before any device work.  alphas:
  * f32[HW][9] (host), actions: u8[9] = identity (may be NULL).  The result is
  * what pp2d_pomdp_set_alphas takes as fib_alphas.
  */
@@ -534,7 +537,10 @@ int pp2d_pomdp_bayes_update(pp2d_pomdp* h, const float* beliefs_in, uint32_t n,
  * (fast_informed_bound_cuda.cu:278-297,
  * point_based_value_iteration_cuda.cu:678-699): upper = max_a <b, fib_a>,
  * lower = max_i <b, pbvi_i> and the action attached to the maximiser, same
- * summation order and roundings as the reference.  Outputs may be NULL.
+ * summation order and roundings as the reference.  The maximiser is the one
+ * std::max_element picks, also with non-finite alphas or beliefs: index 0 if
+ * its value is NaN, else the first maximum of the values that are not NaN
+ * (ties, +0 and -0 included, go to the smaller index).  Outputs may be NULL.
  */
 int pp2d_pomdp_evaluate(pp2d_pomdp* h, const float* beliefs, uint32_t n,
                         float* upper, uint8_t* upper_action, float* lower,

@@ -966,6 +966,13 @@ int pp2d_pomdp_set_alphas(pp2d_pomdp* h, const float* fib_alphas,
 int pp2d_pomdp_solve_fib(pp2d_pomdp* h, float* alphas, uint8_t* actions,
                          uint32_t* sweeps_out, uint32_t max_sweeps) {
   if (!h || !alphas) return fail(PP2D_ERR_INVALID, "NULL argument");
+  // The stopping rule is reached in useful time only for a contraction: with
+  // |gamma| >= 1 the change per sweep stays around the rewards (or the values
+  // reach -inf, whose NaN differences the inf-norm drops).
+  if (max_sweeps == 0 && !(fabsf(h->gamma) < 1.0f))
+    return fail(PP2D_ERR_INVALID,
+                "pp2d_pomdp_solve_fib: without a sweep cap the stopping rule needs |gamma| < 1 "
+                "(gamma = %g); pass max_sweeps", (double)h->gamma);
   const size_t n = (size_t)h->HW * 9;
   float *a1 = nullptr, *a2 = nullptr, *prev = nullptr;
   unsigned int* d_res = nullptr;

@@ -417,12 +417,16 @@ __global__ void pomdp_uniforms_kernel(int n, float* out) {
   out[2 * idx + 1] = curand_uniform(&st);
 }
 
-// tree:331-337 (state sample by inverse CDF: first prefix >= draw; the prefix
-// is non-decreasing, so a binary search finds the same element) followed by
+// tree:331-337 (state sample by inverse CDF: first prefix >= draw) followed by
 // tree:94-147 cudaForwardSampling.  One thread per (expanded node i, action
 // a, sample k); draws[(i*9+a)*S + k] are the host rand() values already
 // divided by RAND_MAX+1.  A draw beyond the last prefix sum is clamped to the
 // last cell (the reference indexes one past the belief there).
+// The binary search finds the same element as the linear search for every
+// belief whose entries are >= 0, +inf or NaN (a class the Bayes update keeps):
+// the prefix is non-decreasing up to its first NaN and NaN from there on, so
+// "prefix >= draw or NaN" is monotone, and a search that stops on a NaN
+// found no prefix >= draw before it.
 __global__ void __launch_bounds__(128)
 pomdp_sample_kernel(int H, int W, int n, int S,
                     const float* __restrict__ trans_prob,
@@ -436,12 +440,13 @@ pomdp_sample_kernel(int H, int W, int n, int S,
   const int k = t % S, a = (t / S) % 9, i = t / (9 * S);
   const int HW = H * W;
   const float r = draws[t];
-  int lo = 0, hi = HW;                       // first s with prefix[s] >= r
+  const float* pre = prefix + (size_t)i * HW;
+  int lo = 0, hi = HW;                       // first s with !(prefix[s] < r)
   while (lo < hi) {
     const int mid = (lo + hi) >> 1;
-    if (prefix[(size_t)i * HW + mid] >= r) hi = mid; else lo = mid + 1;
+    if (!(pre[mid] < r)) hi = mid; else lo = mid + 1;
   }
-  int s1 = lo < HW ? lo : HW - 1;
+  const int s1 = lo < HW && pre[lo] >= r ? lo : HW - 1;
   float cum = 0.0f;
   const float r2 = uniforms[2 * k];
   int s2 = 0;
@@ -817,31 +822,43 @@ pomdp_expand_kernel(int HW, int K, const int* __restrict__ kidx,
 // pbvi:696-698), as std::max_element does.  Packed per belief:
 //   out[i*4 + 0] upper, [1] lower, [2] = fib index | pbvi index << 8 (as int
 //   bits).
+// max_element's rule `if (v[best] < v[a]) best = a` with NaN values: a NaN at
+// index 0 is never replaced (NaN < x is false), so index 0 wins; otherwise a
+// NaN is never taken (x < NaN is false) and the result is the first maximum
+// of the other values.  +0 and -0 compare equal: the first of them wins.
 __global__ void __launch_bounds__(128)
 pomdp_bounds_kernel(int n, int ncol, int n_pbvi, const float* __restrict__ vals,
                     float* __restrict__ out) {
   // one warp per belief: lane-local first maximum over a strided subset of the
   // columns, then (value, index) reduction where ties keep the smaller index
-  // -- the element std::max_element returns.
+  // -- the element std::max_element returns.  A NaN enters a lane's candidate
+  // only at index 0, and a NaN candidate (index 0) beats every other one.
   const int i = blockIdx.x * 4 + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (i >= n) return;
   const float* v = vals + (size_t)i * ncol;
   float bu = 0.0f, bl = 0.0f;
   int iu = -1, il = -1;
-  if (lane < 9) { bu = v[lane]; iu = lane; }
+  if (lane < 9) {
+    bu = v[lane];
+    if (lane == 0 || bu == bu) iu = lane;
+  }
   for (int j = lane; j < n_pbvi; j += 32) {
     const float x = v[9 + j];
-    if (il < 0 || bl < x) { bl = x; il = j; }
+    if (il < 0 ? (j == 0 || x == x) : bl < x) { bl = x; il = j; }
   }
 #pragma unroll
   for (int off = 16; off > 0; off >>= 1) {
     const float ou = __shfl_xor_sync(0xffffffffu, bu, off);
     const int oiu = __shfl_xor_sync(0xffffffffu, iu, off);
-    if (oiu >= 0 && (iu < 0 || bu < ou || (bu == ou && oiu < iu))) { bu = ou; iu = oiu; }
+    if (oiu >= 0 && (iu < 0 || bu < ou || (bu == ou && oiu < iu) || ou != ou)) {
+      bu = ou; iu = oiu;
+    }
     const float ol = __shfl_xor_sync(0xffffffffu, bl, off);
     const int oil = __shfl_xor_sync(0xffffffffu, il, off);
-    if (oil >= 0 && (il < 0 || bl < ol || (bl == ol && oil < il))) { bl = ol; il = oil; }
+    if (oil >= 0 && (il < 0 || bl < ol || (bl == ol && oil < il) || ol != ol)) {
+      bl = ol; il = oil;
+    }
   }
   if (lane == 0) {
     float* o = out + (size_t)i * 4;
