@@ -565,7 +565,10 @@ uint32_t pp2d_tree_depth(const pp2d_tree* t);             /* getDepth() */
 int pp2d_tree_best_action(const pp2d_tree* t, uint8_t* action, float* value);
 int pp2d_tree_update(pp2d_tree* t, uint8_t action, uint8_t observation);
 int pp2d_tree_root_bounds(const pp2d_tree* t, float* upper, float* lower);
-/* beliefCallback's loop + getOptimalAction on an existing tree. */
+/* beliefCallback's loop + getOptimalAction on an existing tree.  Its
+ * iteration counter is a uint8_t as in the reference, so max_iter > 255 runs
+ * until the depth limit or a tree without a node to expand
+ * (pp2d_pomdp_plan_batch and pp2d_tree_batch_plan clamp max_iter to 255). */
 int pp2d_tree_plan(pp2d_tree* t, uint32_t max_depth, uint32_t max_iter,
                    uint8_t* action, float* value);
 /* SearchTree::print (search_tree_cuda.cu:288-309, 452-473, 628-633) into a
@@ -575,6 +578,42 @@ int pp2d_tree_plan(pp2d_tree* t, uint32_t max_depth, uint32_t max_iter,
  * id of vnode_to_expand (-1 = nullptr).  Writes at most cap_nodes nodes,
  * returns the number of nodes in the tree (negative on error). */
 int64_t pp2d_tree_dump(const pp2d_tree* t, float* out, uint64_t cap_nodes);
+
+/*
+ * Persistent tree batches: n SearchTrees on one planner handle that live
+ * across belief callbacks (one per robot of a fleet) and are updated and
+ * planned together.  Tree k behaves bit for bit like a pp2d_tree created from
+ * beliefs[k] and fed the same calls: its own rand() stream, seeded like a
+ * fresh process at creation and kept through updates, its own expansion count.
+ * The trees' beliefs stay resident in the handle's belief pool until the
+ * batch is destroyed (pp2d_pomdp_set_model_tables refuses meanwhile).
+ *
+ * create: pp2d_tree_create for every belief ([n][HW], host), one upload and
+ * one bounds launch for all roots.
+ * update: pp2d_tree_update(actions[i], observations[i]) on tree trees[i]; the
+ * new roots that need a Bayes update share one set of launches.  Every listed
+ * tree is checked before any changes: NULL pointers, an index >= n, an index
+ * listed twice, an action >= 9 or an observation >= 16 give PP2D_ERR_INVALID,
+ * an unexpanded root PP2D_ERR_STATE (messages name the tree).  Unlisted trees
+ * are untouched.
+ * plan: pp2d_tree_plan on every listed tree, the trees' expansion rounds
+ * batched as in pp2d_pomdp_plan_batch (max_iter clamped to 255).  actions,
+ * values (may be NULL) and stats (may be NULL; [n][4] = {V nodes, Q nodes,
+ * root depth, expansions since creation}) are indexed like `trees`.  Results
+ * do not depend on which other trees a call lists or on their order.
+ * dump: pp2d_tree_dump of tree k (negative for a bad k).
+ */
+typedef struct pp2d_tree_batch pp2d_tree_batch;
+int pp2d_tree_batch_create(pp2d_pomdp* h, const float* beliefs, uint32_t n,
+                           pp2d_tree_batch** out);
+void pp2d_tree_batch_destroy(pp2d_tree_batch* b);
+int pp2d_tree_batch_update(pp2d_tree_batch* b, const uint32_t* trees, uint32_t n,
+                           const uint8_t* actions, const uint8_t* observations);
+int pp2d_tree_batch_plan(pp2d_tree_batch* b, const uint32_t* trees, uint32_t n,
+                         uint32_t max_depth, uint32_t max_iter, uint8_t* actions, float* values,
+                         uint32_t* stats);
+int64_t pp2d_tree_batch_dump(const pp2d_tree_batch* b, uint32_t k, float* out,
+                             uint64_t cap_nodes);
 
 /* ------------------------------------------------------------------------
  * dummy_simulator's Bayes filter (SURVEY.md section 8f row 4b)
@@ -653,6 +692,21 @@ int pp2d_sim_rollout_mdp_batch(pp2d_sim* s, pp2d_mdp_batch* planner, const uint3
                                uint32_t n, const uint32_t* starts_xy, const float* beliefs,
                                uint32_t max_steps, uint64_t seed, uint64_t first_episode,
                                pp2d_rollout* out);
+/* Every episode follows the QV-tree planner `planner` (its goal; its alpha
+ * vectors must be set, PP2D_ERR_STATE otherwise) as PomdpPathPlanning2d's
+ * beliefCallback does (DESIGN.md section 7d): episode i keeps one search tree,
+ * created from beliefs[i] (NULL: the point mass at its start); step t plans it
+ * (pp2d_tree_plan with max_depth, max_iter), u = the best action, the world
+ * moves and senses as above, and the tree is updated with (u, z), z = the
+ * measurement byte.  The simulator's filter is not run: final_belief is the
+ * tree's root belief after the last update (the start belief if no step was
+ * taken).  max_depth == 0 or max_iter == 0 give PP2D_ERR_INVALID (a step must
+ * leave an expanded root to update).  Each step plans only the episodes still
+ * running, together, through one tree batch; the world steps on the host. */
+int pp2d_sim_rollout_pomdp(pp2d_sim* s, pp2d_pomdp* planner, uint32_t n, const uint32_t* starts_xy,
+                           const float* beliefs, uint32_t max_steps, uint32_t max_depth,
+                           uint32_t max_iter, uint64_t seed, uint64_t first_episode,
+                           pp2d_rollout* out);
 
 #ifdef __cplusplus
 }

@@ -364,6 +364,42 @@ class SearchTree {                     // search_tree.h:130-165
   pp2d_tree* t_ = nullptr;
 };
 
+// Not in the reference (one tree per process): many SearchTrees on one
+// planner handle that live across belief callbacks, e.g. one per robot of a
+// fleet, updated and planned together (pp2d_tree_batch_*).  Tree k behaves bit
+// for bit like SearchTree(h, beliefs + k * HW) fed the same calls.
+class SearchTreeBatch {
+ public:
+  SearchTreeBatch(pp2d_pomdp* h, const float* beliefs, uint32_t n) {
+    PP2D_CHECK(pp2d_tree_batch_create(h, beliefs, n, &b_));
+  }
+  SearchTreeBatch(const SearchTreeBatch&) = delete;
+  SearchTreeBatch& operator=(const SearchTreeBatch&) = delete;
+  ~SearchTreeBatch() { pp2d_tree_batch_destroy(b_); }
+  // update(actions[i], observations[i]) of tree trees[i]
+  void update(const std::vector<uint32_t>& trees, const std::vector<uint8_t>& actions,
+              const std::vector<uint8_t>& observations) {
+    if (actions.size() != trees.size() || observations.size() != trees.size()) {
+      std::fprintf(stderr, "SearchTreeBatch::update: one action and observation per tree\n");
+      std::exit(EXIT_FAILURE);
+    }
+    PP2D_CHECK(pp2d_tree_batch_update(b_, trees.data(), (uint32_t)trees.size(), actions.data(),
+                                      observations.data()));
+  }
+  // beliefCallback's loop + getOptimalAction of every listed tree
+  std::vector<uint8_t> plan(const std::vector<uint32_t>& trees, uint32_t max_depth,
+                            uint32_t max_iter, std::vector<float>* values = nullptr) {
+    std::vector<uint8_t> a(trees.size());
+    if (values) values->resize(trees.size());
+    PP2D_CHECK(pp2d_tree_batch_plan(b_, trees.data(), (uint32_t)trees.size(), max_depth, max_iter,
+                                    a.data(), values ? values->data() : nullptr, nullptr));
+    return a;
+  }
+
+ private:
+  pp2d_tree_batch* b_ = nullptr;
+};
+
 class PomdpPathPlanning2d : public PathPlanning2dBase {
  public:
   explicit PomdpPathPlanning2d(const Params& n) : PathPlanning2dBase(n) {}

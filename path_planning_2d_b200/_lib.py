@@ -27,7 +27,7 @@ class Halo(ctypes.Structure):
 
 
 class Rollout(ctypes.Structure):
-    """pp2d_rollout: output arrays of pp2d_sim_rollout_mdp*, each may be NULL."""
+    """pp2d_rollout: output arrays of pp2d_sim_rollout_*, each may be NULL."""
     _fields_ = [("steps", _vp), ("reached", _vp), ("collisions", _vp), ("final_cell", _vp),
                 ("final_belief", _vp), ("cells", _vp), ("actions", _vp),
                 ("measurements", _vp)]
@@ -121,6 +121,13 @@ SIGNATURES = {
     "pp2d_tree_root_bounds": (_i, [_vp, _vp, _vp]),
     "pp2d_tree_plan": (_i, [_vp, _u32, _u32, _vp, _vp]),
     "pp2d_tree_dump": (ctypes.c_int64, [_vp, _vp, ctypes.c_uint64]),
+    "pp2d_tree_batch_create": (_i, [_vp, _vp, _u32, ctypes.POINTER(_vp)]),
+    "pp2d_tree_batch_destroy": (None, [_vp]),
+    "pp2d_tree_batch_update": (_i, [_vp, _vp, _u32, _vp, _vp]),
+    "pp2d_tree_batch_plan": (_i, [_vp, _vp, _u32, _u32, _u32, _vp, _vp, _vp]),
+    "pp2d_tree_batch_dump": (ctypes.c_int64, [_vp, _u32, _vp, ctypes.c_uint64]),
+    "pp2d_sim_rollout_pomdp": (_i, [_vp, _vp, _u32, _vp, _vp, _u32, _u32, _u32, ctypes.c_uint64,
+                                    ctypes.c_uint64, ctypes.POINTER(Rollout)]),
 }
 
 _lib = None

@@ -24,6 +24,10 @@ uint32_t mdp_batch_count(const pp2d_mdp_batch* b);                         // md
 // Instance k < count: its goal and its action grid (the snapshot once frozen).
 PlannerView mdp_batch_view(const pp2d_mdp_batch* b, uint32_t k);           // mdp.cu
 
+// The root beliefs of trees 0 .. count-1 of a tree batch, [count][HW] into
+// host memory (pomdp.cu).
+int tree_batch_root_beliefs(pp2d_tree_batch* b, float* out);               // pomdp.cu
+
 struct SimView {
   uint32_t H = 0, W = 0;
   const uint8_t* map_host = nullptr;   // [H][W], 1 = occupied

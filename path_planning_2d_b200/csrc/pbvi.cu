@@ -421,7 +421,7 @@ int expand_belief_set(pp2d_pomdp* h, const float* b0, uint32_t max_size, uint32_
   GlibcRand rng;
   rng.seed(rand_seed ? rand_seed : 1);
   set.clear();
-  PP2D_TRY(pool_reserve(h, (size_t)h->cap - h->free_slots.size() + 10 * (size_t)max_size + 32));
+  PP2D_TRY(pool_reserve(h, (size_t)h->cap - h->free_slots.count() + 10 * (size_t)max_size + 32));
   int s0 = -1;
   PP2D_TRY(alloc_slot(h, &s0));
   set.push_back(s0);
@@ -511,7 +511,7 @@ int expand_belief_set(pp2d_pomdp* h, const float* b0, uint32_t max_size, uint32_
         if (set.size() >= max_size) break;
       }
       for (int c = 0; c < nc; ++c)
-        if (!keep[c]) h->free_slots.push_back(cand[c]);
+        if (!keep[c]) h->free_slots.put(cand[c]);
     }
     return PP2D_OK;
   }();
@@ -619,7 +619,7 @@ int pp2d_pomdp_generate_belief_set(pp2d_pomdp* h, const float* initial_belief, u
     return PP2D_OK;
   }();
   cudaFree(d_rows);
-  for (int s : set) h->free_slots.push_back(s);
+  for (int s : set) h->free_slots.put(s);
   return rc;
 }
 
@@ -692,7 +692,7 @@ int pp2d_pomdp_solve_pbvi(pp2d_pomdp* h, const float* initial_belief, uint32_t n
     return PP2D_OK;
   }();
   cudaFree(d_B); cudaFree(d_al); cudaFree(d_ac);
-  for (int s : set) h->free_slots.push_back(s);
+  for (int s : set) h->free_slots.put(s);
   return rc;
 }
 

@@ -125,7 +125,7 @@ int pool_reserve(pp2d_pomdp* h, size_t slots_wanted) {
     return fail(PP2D_ERR_INVALID, "belief pool of %zu slots is too large", cap);
   float* nb = nullptr;
   size_t old_cap = h->d_bel ? (size_t)h->cap : 0;
-  if (old_cap && h->free_slots.size() == old_cap) {
+  if (old_cap && h->free_slots.count() == old_cap) {
     // No belief is live: release the old pool BEFORE asking for the new one (a
     // batch sizes the pool to half of the memory; old + new need not fit).
     cudaError_t e = cudaDeviceSynchronize();
@@ -138,7 +138,7 @@ int pool_reserve(pp2d_pomdp* h, size_t slots_wanted) {
       return fail(PP2D_ERR_CUDA, "CUDA error releasing the belief pool: %s", cudaGetErrorName(e));
   }
   PP2D_CUDA(cudaMalloc(&nb, cap * (size_t)h->HW * sizeof(float)));
-  if (old_cap && h->free_slots.size() != old_cap) {
+  if (old_cap && h->free_slots.count() != old_cap) {
     cudaError_t e = cudaDeviceSynchronize();     // every stream that touches the pool
     if (e == cudaSuccess)
       e = cudaMemcpyAsync(nb, h->d_bel, old_cap * (size_t)h->HW * sizeof(float),
@@ -152,21 +152,14 @@ int pool_reserve(pp2d_pomdp* h, size_t slots_wanted) {
   if (h->d_bel) cudaFree(h->d_bel);
   h->d_bel = nb;
   h->cap = (int)cap;
-  // new slots go UNDER the still-free old ones so that allocation order of a
-  // fresh pool stays ascending
-  std::vector<int> fresh;
-  fresh.reserve(cap - old_cap + h->free_slots.size());
-  for (size_t i = cap; i-- > old_cap;) fresh.push_back((int)i);
-  fresh.insert(fresh.end(), h->free_slots.begin(), h->free_slots.end());
-  h->free_slots.swap(fresh);
+  h->free_slots.grow(cap);
   return PP2D_OK;
 }
 
 int alloc_slot(pp2d_pomdp* h, int* out) {
   if (h->free_slots.empty())
     PP2D_TRY(pool_reserve(h, std::max<size_t>(4096, 2 * (size_t)h->cap)));
-  *out = h->free_slots.back();
-  h->free_slots.pop_back();
+  *out = h->free_slots.take();
   return PP2D_OK;
 }
 
@@ -465,15 +458,20 @@ int make_roots(pp2d_pomdp* h, std::vector<Tree*>& trees, const float* beliefs,
   return PP2D_OK;
 }
 
-void free_subtree_v(pp2d_pomdp* h, Tree& t, int vi);
-void free_subtree_q(pp2d_pomdp* h, Tree& t, int qi) {
-  for (int c : t.q[qi].children) free_subtree_v(h, t, c);
+// The belief slots of a subtree are appended to `freed` (the caller gives them
+// back to the pool; trees of a batch are re-rooted on several host threads).
+void free_subtree_v(Tree& t, int vi, std::vector<int>& freed);
+void free_subtree_q(Tree& t, int qi, std::vector<int>& freed) {
+  for (int c : t.q[qi].children) free_subtree_v(t, c, freed);
   t.q[qi].children.clear();
 }
-void free_subtree_v(pp2d_pomdp* h, Tree& t, int vi) {
-  for (int c : t.v[vi].children) free_subtree_q(h, t, c);
+void free_subtree_v(Tree& t, int vi, std::vector<int>& freed) {
+  for (int c : t.v[vi].children) free_subtree_q(t, c, freed);
   t.v[vi].children.clear();
-  if (t.v[vi].slot >= 0) { h->free_slots.push_back(t.v[vi].slot); t.v[vi].slot = -1; }
+  if (t.v[vi].slot >= 0) { freed.push_back(t.v[vi].slot); t.v[vi].slot = -1; }
+}
+void give_back(pp2d_pomdp* h, const std::vector<int>& freed) {
+  for (int s : freed) h->free_slots.put(s);
 }
 
 // Page-locked host buffer: source / target of the asynchronous copies of a
@@ -562,17 +560,19 @@ int round_stage1(pp2d_pomdp* h, RoundCtx& c, const std::vector<Tree*>& trees) {
   double t0 = now_s();
   c.jobs.clear();
   c.dense = false;
+  std::vector<int> freed;
   for (Tree* t : trees) {
     if (t->dead) continue;
     c.dense = c.dense || t->dense;
     const int v = t->v[t->root].to_expand;
     if (v < 0) { t->dead = true; continue; }
     if (!t->v[v].children.empty()) {            // re-expansion (leak in the ref)
-      for (int q : t->v[v].children) free_subtree_q(h, *t, q);
+      for (int q : t->v[v].children) free_subtree_q(*t, q, freed);
       t->v[v].children.clear();
     }
     c.jobs.push_back({t, v});
   }
+  give_back(h, freed);
   const int n = c.n = (int)c.jobs.size();
   c.nk = 0;
   if (n == 0) return PP2D_OK;
@@ -807,6 +807,191 @@ void best_action(const Tree& t, uint8_t* a, float* r) {   // tree:510-524
     if (t.q[c].upper > *r) { *r = t.q[c].upper; *a = t.q[c].action; }
 }
 
+/* SearchTree::print (search_tree_cuda.cu:288-309, 452-473, 628-633) */
+int64_t dump_tree(const Tree& t, float* out, uint64_t cap_nodes) {
+  // pass 1: pre-order ids of the V nodes (V and Q nodes share one counter)
+  std::vector<int> vid(t.v.size(), -1);
+  struct Item { int idx; bool is_q; };
+  std::vector<Item> order, stack{{t.root, false}};
+  while (!stack.empty()) {
+    const Item it = stack.back();
+    stack.pop_back();
+    if (!it.is_q) vid[it.idx] = (int)order.size();
+    order.push_back(it);
+    const std::vector<int>& ch = it.is_q ? t.q[it.idx].children : t.v[it.idx].children;
+    for (size_t i = ch.size(); i-- > 0;) stack.push_back({ch[i], !it.is_q});
+  }
+  auto target = [&](int v) { return v >= 0 ? (float)vid[v] : -1.0f; };
+  for (size_t k = 0; out && k < order.size() && k < cap_nodes; ++k) {
+    float* o = out + 9 * k;
+    if (order[k].is_q) {
+      const QNodeH& q = t.q[order[k].idx];
+      o[0] = 1.0f; o[1] = (float)q.action; o[2] = q.reward; o[3] = q.upper; o[4] = q.lower;
+      o[5] = q.heuristic; o[6] = (float)q.depth; o[7] = (float)q.children.size();
+      o[8] = target(q.to_expand);
+    } else {
+      const VNodeH& v = t.v[order[k].idx];
+      o[0] = 0.0f; o[1] = (float)v.obs; o[2] = v.weight; o[3] = v.upper; o[4] = v.lower;
+      o[5] = v.heuristic; o[6] = (float)v.depth; o[7] = (float)v.children.size();
+      o[8] = target(v.to_expand);
+    }
+  }
+  return (int64_t)order.size();
+}
+
+// The nodes SearchTree::update(a, z) keeps (search_tree_cuda.cu:548-555): the
+// root's Q node for a, and its V child for z (-1: none, a new root is needed).
+void kept_nodes(const Tree& t, uint8_t a, uint8_t z, int* root_q, int* root_v) {
+  *root_q = *root_v = -1;
+  for (int c : t.v[t.root].children)
+    if (t.q[c].action == a) *root_q = c;
+  if (*root_q < 0) return;
+  for (int c : t.q[*root_q].children)
+    if (t.v[c].obs == z) *root_v = c;
+}
+
+// The rest of SearchTree::update (search_tree_cuda.cu:556-626) once the new
+// root's belief, if any, is resident: new_slot and its bounds ev when root_v
+// is -1.  The beliefs of the dropped subtrees go to `freed`.
+void reroot(Tree& t, int root_q, int root_v, int new_slot, const float* ev,
+            std::vector<int>& freed) {
+  for (int c : t.v[t.root].children)
+    if (c != root_q) free_subtree_q(t, c, freed);
+  for (int c : t.q[root_q].children)
+    if (c != root_v) free_subtree_v(t, c, freed);
+  VNodeH& old_root = t.v[t.root];
+  if (old_root.slot >= 0) { freed.push_back(old_root.slot); old_root.slot = -1; }
+  // Rebuild the node arrays from the kept subtree: a long-running planner
+  // re-roots once per belief message, and dropped nodes must not accumulate.
+  Tree fresh;
+  fresh.rng = t.rng;
+  fresh.expansions = t.expansions;
+  fresh.dense = t.dense;
+  if (root_v >= 0) {
+    std::vector<int> vmap(t.v.size(), -1), qmap(t.q.size(), -1);
+    struct Item { int idx; bool is_q; };
+    std::vector<Item> stack{{root_v, false}};
+    while (!stack.empty()) {                       // number the kept nodes
+      const Item it = stack.back();
+      stack.pop_back();
+      if (it.is_q) {
+        qmap[it.idx] = (int)fresh.q.size();
+        fresh.q.push_back(t.q[it.idx]);
+        for (int c : t.q[it.idx].children) stack.push_back({c, false});
+      } else {
+        vmap[it.idx] = (int)fresh.v.size();
+        fresh.v.push_back(t.v[it.idx]);
+        for (int c : t.v[it.idx].children) stack.push_back({c, true});
+      }
+    }
+    auto mv = [&](int v) { return v >= 0 ? vmap[v] : -1; };
+    for (VNodeH& v : fresh.v) {
+      v.parent = v.parent >= 0 ? qmap[v.parent] : -1;
+      v.to_expand = mv(v.to_expand);
+      for (int& c : v.children) c = qmap[c];
+    }
+    for (QNodeH& q : fresh.q) {
+      q.parent = vmap[q.parent];
+      q.to_expand = mv(q.to_expand);
+      for (int& c : q.children) c = vmap[c];
+    }
+    fresh.root = vmap[root_v];
+    fresh.v[fresh.root].parent = -1;
+  } else {
+    fresh.v.emplace_back();
+    fresh.root = 0;
+    init_vnode(fresh.v[0], new_slot, 0, 0.0f, -1, ev, 0);
+  }
+  t = std::move(fresh);
+}
+
+// Belief slots a plan may hold: half of what is free once the current pool is
+// counted as free (the pool must not ratchet up from call to call), or
+// PP2D_POMDP_POOL_MB.
+int pool_budget(pp2d_pomdp* h, size_t* max_slots) {
+  size_t free_b = 0, total_b = 0;
+  PP2D_CUDA(cudaMemGetInfo(&free_b, &total_b));
+  size_t budget = (free_b + (size_t)h->cap * h->HW * sizeof(float)) / 2;
+  const char* env = getenv("PP2D_POMDP_POOL_MB");
+  if (env && *env) budget = (size_t)atol(env) << 20;
+  *max_slots = budget / ((size_t)h->HW * sizeof(float));
+  return PP2D_OK;
+}
+
+// Slots reserved up front per tree of a plan, of `worst` it may need.
+// PP2D_POMDP_SLOTS_PER_QUERY: fewer; the pool then grows in place
+// (pool_reserve) when the trees outgrow it.
+size_t slots_per_tree(size_t worst) {
+  const char* spq = getenv("PP2D_POMDP_SLOTS_PER_QUERY");
+  if (spq && atol(spq) > 0) return std::min<size_t>(worst, (size_t)atol(spq));
+  return worst;
+}
+
+// beliefCallback's loop (src/pomdp/path_planning_2d.cu:218-223) on every tree
+// of `trees`: up to max_iter expansion rounds (<= 255) while its root is
+// shallower than max_depth, the trees of a round batched.  `sorted`: `trees`
+// is in the order of the roots' modes (see pp2d_pomdp_plan_batch).  The order
+// and grouping change only how the work is batched: every tree owns its
+// rand() stream, and no result of one tree depends on another.
+int plan_trees(pp2d_pomdp* h, std::vector<Tree*>& trees, uint32_t max_depth, uint32_t max_iter,
+               bool sorted) {
+  const size_t n = trees.size();
+  // Groups of trees a fraction of a round apart: while the device runs the
+  // Bayes / bounds launches of one group, the host absorbs the previous round
+  // of another and prepares its next one (all copies are asynchronous, each
+  // group has its own streams).
+  // (PP2D_POMDP_GROUPS overrides; measured at 1250 queries on a B200: 2 groups
+  // 13.1e3 plans/s, 3 groups 14.4e3, 4 groups 13.1e3 -- more groups overlap
+  // host and device better but launch smaller kernels)
+  int G = n >= 384 ? 3 : (n >= 256 ? 2 : 1);
+  if (const char* ge = getenv("PP2D_POMDP_GROUPS"))
+    if (n >= 256 && atoi(ge) >= 1) G = std::min(atoi(ge), kMaxGroups);
+  RoundCtx* ctx[kMaxGroups];
+  bool more[kMaxGroups];
+  size_t first_tree[kMaxGroups + 1];
+  for (int g = 0; g < G; ++g) {
+    ctx[g] = round_ctx(h, g);
+    ctx[g]->n = 0;
+    more[g] = true;
+    first_tree[g] = n * (size_t)g / (size_t)G;
+  }
+  first_tree[G] = n;
+  if (sorted && G > 1) {
+    // Sorted trees are dealt to the groups in blocks of 16: every group then
+    // spans the whole map (trees far from the goal grow more children than
+    // those next to it; thirds of the sorted order would be unequal rounds)
+    // while the neighbours inside a group stay neighbours.
+    constexpr size_t kDeal = 16;
+    std::vector<Tree*> dealt;
+    dealt.reserve(n);
+    for (int g = 0; g < G; ++g) {
+      first_tree[g] = dealt.size();
+      for (size_t b0 = (size_t)g * kDeal; b0 < n; b0 += (size_t)G * kDeal)
+        for (size_t i = b0; i < std::min(n, b0 + kDeal); ++i) dealt.push_back(trees[i]);
+    }
+    trees.swap(dealt);
+  }
+  std::vector<Tree*> active;
+  auto any_more = [&]() { for (int g = 0; g < G; ++g) if (more[g]) return true; return false; };
+  for (uint32_t it = 0; it < max_iter && any_more(); ++it) {
+    for (int g = 0; g < G; ++g) {
+      if (!more[g]) continue;
+      RoundCtx& c = *ctx[g];
+      PP2D_TRY(round_stage3(h, c));            // previous round of this group
+      active.clear();
+      for (size_t i = first_tree[g]; i < first_tree[g + 1]; ++i) {
+        Tree* t = trees[i];
+        if (!t->dead && t->v[t->root].depth < max_depth) active.push_back(t);
+      }
+      if (active.empty()) { more[g] = false; continue; }
+      PP2D_TRY(round_stage1(h, c, active));
+      PP2D_TRY(round_stage2(h, c));
+    }
+  }
+  for (int g = 0; g < G; ++g) PP2D_TRY(round_stage3(h, *ctx[g]));
+  return PP2D_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -879,7 +1064,7 @@ void pp2d_pomdp_destroy(pp2d_pomdp* h) {
   if (h->pin_rows) cudaFreeHost(h->pin_rows);
   h->d_slots.release(); h->d_items.release(); h->d_prefix.release();
   h->d_draws.release(); h->d_vals.release(); h->d_rows.release();
-  h->d_sums.release(); h->d_obs.release(); h->d_out.release();
+  h->d_sums.release(); h->d_obs.release(); h->d_out.release(); h->d_keys.release();
   for (void*& c : h->round_ctx) { delete static_cast<RoundCtx*>(c); c = nullptr; }
   delete h;
 }
@@ -904,10 +1089,10 @@ int pp2d_pomdp_set_model_tables(pp2d_pomdp* h, const float* trans_prob,
   // Trees keep beliefs that were propagated with the current tables (and were
   // classified against the current live-cell mask): like the reference, which
   // loads its tables once in initialize(), the tables are fixed before any tree.
-  if (h->d_bel && h->free_slots.size() != (size_t)h->cap)
+  if (h->d_bel && h->free_slots.count() != (size_t)h->cap)
     return fail(PP2D_ERR_STATE, "pp2d_pomdp_set_model_tables: destroy the search trees of this "
                                 "handle first (%zu beliefs are resident)",
-                (size_t)h->cap - h->free_slots.size());
+                (size_t)h->cap - h->free_slots.count());
   // every stream that reads the tables (rounds of a batch in flight)
   PP2D_CUDA(cudaDeviceSynchronize());
   if (trans_prob)
@@ -1055,7 +1240,7 @@ int pp2d_pomdp_bayes_update(pp2d_pomdp* h, const float* beliefs_in, uint32_t n,
     if (actions[i] >= kActions || observations[i] >= 16)
       return fail(PP2D_ERR_INVALID, "item %u: action %u / observation %u out of range (9 / 16)",
                   i, actions[i], observations[i]);
-  PP2D_TRY(pool_reserve(h, (size_t)h->cap - h->free_slots.size() + 2 * (size_t)n));
+  PP2D_TRY(pool_reserve(h, (size_t)h->cap - h->free_slots.count() + 2 * (size_t)n));
   const int HW = h->HW;
   std::vector<int> in(n), outs(n);
   std::vector<BayesItem> items(n);
@@ -1100,8 +1285,8 @@ int pp2d_pomdp_bayes_update(pp2d_pomdp* h, const float* beliefs_in, uint32_t n,
     return PP2D_OK;
   }();
   for (uint32_t i = 0; i < n; ++i) {
-    h->free_slots.push_back(in[i]);
-    h->free_slots.push_back(outs[i]);
+    h->free_slots.put(in[i]);
+    h->free_slots.put(outs[i]);
   }
   return rc;
 }
@@ -1112,7 +1297,7 @@ int pp2d_pomdp_evaluate(pp2d_pomdp* h, const float* beliefs, uint32_t n,
   if (!h || !beliefs) return fail(PP2D_ERR_INVALID, "NULL argument");
   if (!h->have_alphas) return fail(PP2D_ERR_STATE, "pp2d_pomdp_set_alphas not called");
   if (n == 0) return PP2D_OK;
-  PP2D_TRY(pool_reserve(h, (size_t)h->cap - h->free_slots.size() + n));
+  PP2D_TRY(pool_reserve(h, (size_t)h->cap - h->free_slots.count() + n));
   const int HW = h->HW;
   std::vector<int> slots(n);
   for (uint32_t i = 0; i < n; ++i) PP2D_TRY(alloc_slot(h, &slots[i]));
@@ -1158,7 +1343,7 @@ int pp2d_pomdp_evaluate(pp2d_pomdp* h, const float* beliefs, uint32_t n,
     }
     return PP2D_OK;
   }();
-  for (uint32_t i = 0; i < n; ++i) h->free_slots.push_back(slots[i]);
+  for (uint32_t i = 0; i < n; ++i) h->free_slots.put(slots[i]);
   return rc;
 }
 
@@ -1170,19 +1355,9 @@ int pp2d_pomdp_plan_batch(pp2d_pomdp* h, const float* beliefs, uint32_t n,
   if (n == 0) return PP2D_OK;
   if (max_iter > 255) max_iter = 255;           // uint8_t counter, pomdp:218-223
   // Worst case per query: root + max_iter * 9 * 16 children.
-  size_t per_query = 1 + (size_t)max_iter * kActions * 16;
-  // PP2D_POMDP_SLOTS_PER_QUERY: reserve fewer slots per query up front; the
-  // pool then grows in place (pool_reserve) when the trees outgrow it.
-  const char* spq = getenv("PP2D_POMDP_SLOTS_PER_QUERY");
-  if (spq && atol(spq) > 0) per_query = std::min<size_t>(per_query, (size_t)atol(spq));
-  size_t free_b = 0, total_b = 0;
-  PP2D_CUDA(cudaMemGetInfo(&free_b, &total_b));
-  // half of what is free once the current pool is counted as free (the pool
-  // must not ratchet up from call to call)
-  size_t budget = (free_b + (size_t)h->cap * h->HW * sizeof(float)) / 2;
-  const char* env = getenv("PP2D_POMDP_POOL_MB");
-  if (env && *env) budget = (size_t)atol(env) << 20;
-  size_t max_slots = budget / ((size_t)h->HW * sizeof(float));
+  const size_t per_query = slots_per_tree(1 + (size_t)max_iter * kActions * 16);
+  size_t max_slots = 0;
+  PP2D_TRY(pool_budget(h, &max_slots));
   if (max_slots < per_query)
     return fail(PP2D_ERR_STATE, "belief pool budget too small for one query");
   size_t group = std::min<size_t>(n, max_slots / per_query);
@@ -1210,59 +1385,7 @@ int pp2d_pomdp_plan_batch(pp2d_pomdp* h, const float* beliefs, uint32_t n,
       for (size_t i = 0; i < gn; ++i) trees[i] = &store[order[i]];
     }
     h->t_phase[5] += now_s() - tr;               // roots: upload + bounds
-    // Groups of trees a fraction of a round apart: while the device runs the
-    // Bayes / bounds launches of one group, the host absorbs the previous round
-    // of another and prepares its next one (all copies are asynchronous, each
-    // group has its own streams).
-    // (PP2D_POMDP_GROUPS overrides; measured at 1250 queries on a B200: 2 groups
-    // 13.1e3 plans/s, 3 groups 14.4e3, 4 groups 13.1e3 -- more groups overlap
-    // host and device better but launch smaller kernels)
-    int G = gn >= 384 ? 3 : (gn >= 256 ? 2 : 1);
-    if (const char* ge = getenv("PP2D_POMDP_GROUPS"))
-      if (gn >= 256 && atoi(ge) >= 1) G = std::min(atoi(ge), kMaxGroups);
-    RoundCtx* ctx[kMaxGroups];
-    bool more[kMaxGroups];
-    size_t first_tree[kMaxGroups + 1];
-    for (int g = 0; g < G; ++g) {
-      ctx[g] = round_ctx(h, g);
-      ctx[g]->n = 0;
-      more[g] = true;
-      first_tree[g] = gn * (size_t)g / (size_t)G;
-    }
-    first_tree[G] = gn;
-    if (sorted && G > 1) {
-      // Sorted trees are dealt to the groups in blocks of 16: every group then
-      // spans the whole map (trees far from the goal grow more children than
-      // those next to it; thirds of the sorted order would be unequal rounds)
-      // while the neighbours inside a group stay neighbours.
-      constexpr size_t kDeal = 16;
-      std::vector<Tree*> dealt;
-      dealt.reserve(gn);
-      for (int g = 0; g < G; ++g) {
-        first_tree[g] = dealt.size();
-        for (size_t b0 = (size_t)g * kDeal; b0 < gn; b0 += (size_t)G * kDeal)
-          for (size_t i = b0; i < std::min(gn, b0 + kDeal); ++i) dealt.push_back(trees[i]);
-      }
-      trees.swap(dealt);
-    }
-    std::vector<Tree*> active;
-    auto any_more = [&]() { for (int g = 0; g < G; ++g) if (more[g]) return true; return false; };
-    for (uint32_t it = 0; it < max_iter && any_more(); ++it) {
-      for (int g = 0; g < G; ++g) {
-        if (!more[g]) continue;
-        RoundCtx& c = *ctx[g];
-        PP2D_TRY(round_stage3(h, c));            // previous round of this group
-        active.clear();
-        for (size_t i = first_tree[g]; i < first_tree[g + 1]; ++i) {
-          Tree* t = trees[i];
-          if (!t->dead && t->v[t->root].depth < max_depth) active.push_back(t);
-        }
-        if (active.empty()) { more[g] = false; continue; }
-        PP2D_TRY(round_stage1(h, c, active));
-        PP2D_TRY(round_stage2(h, c));
-      }
-    }
-    for (int g = 0; g < G; ++g) PP2D_TRY(round_stage3(h, *ctx[g]));
+    PP2D_TRY(plan_trees(h, trees, max_depth, max_iter, sorted));
     tr = now_s();
     const int gni = (int)gn;
 #pragma omp parallel num_threads(host_threads()) if (gni >= 64)
@@ -1283,7 +1406,7 @@ int pp2d_pomdp_plan_batch(pp2d_pomdp* h, const float* beliefs, uint32_t n,
           if (v.slot >= 0) { back.push_back(v.slot); v.slot = -1; }
       }
 #pragma omp critical
-      h->free_slots.insert(h->free_slots.end(), back.begin(), back.end());
+      give_back(h, back);
     }
     h->t_phase[6] += now_s() - tr;               // actions out, slots back
   }
@@ -1317,7 +1440,9 @@ int pp2d_tree_create(pp2d_pomdp* h, const float* belief, pp2d_tree** out) {
 
 void pp2d_tree_destroy(pp2d_tree* t) {
   if (!t) return;
-  if (t->t.root >= 0) free_subtree_v(t->h, t->t, t->t.root);
+  std::vector<int> freed;
+  if (t->t.root >= 0) free_subtree_v(t->t, t->t.root, freed);
+  give_back(t->h, freed);
   delete t;
 }
 
@@ -1346,38 +1471,9 @@ int pp2d_tree_root_bounds(const pp2d_tree* t, float* upper, float* lower) {
   return PP2D_OK;
 }
 
-/* SearchTree::print (search_tree_cuda.cu:288-309, 452-473, 628-633) */
 int64_t pp2d_tree_dump(const pp2d_tree* tt, float* out, uint64_t cap_nodes) {
   if (!tt || tt->t.root < 0) { fail(PP2D_ERR_INVALID, "tree is NULL"); return -1; }
-  const Tree& t = tt->t;
-  // pass 1: pre-order ids of the V nodes (V and Q nodes share one counter)
-  std::vector<int> vid(t.v.size(), -1);
-  struct Item { int idx; bool is_q; };
-  std::vector<Item> order, stack{{t.root, false}};
-  while (!stack.empty()) {
-    const Item it = stack.back();
-    stack.pop_back();
-    if (!it.is_q) vid[it.idx] = (int)order.size();
-    order.push_back(it);
-    const std::vector<int>& ch = it.is_q ? t.q[it.idx].children : t.v[it.idx].children;
-    for (size_t i = ch.size(); i-- > 0;) stack.push_back({ch[i], !it.is_q});
-  }
-  auto target = [&](int v) { return v >= 0 ? (float)vid[v] : -1.0f; };
-  for (size_t k = 0; out && k < order.size() && k < cap_nodes; ++k) {
-    float* o = out + 9 * k;
-    if (order[k].is_q) {
-      const QNodeH& q = t.q[order[k].idx];
-      o[0] = 1.0f; o[1] = (float)q.action; o[2] = q.reward; o[3] = q.upper; o[4] = q.lower;
-      o[5] = q.heuristic; o[6] = (float)q.depth; o[7] = (float)q.children.size();
-      o[8] = target(q.to_expand);
-    } else {
-      const VNodeH& v = t.v[order[k].idx];
-      o[0] = 0.0f; o[1] = (float)v.obs; o[2] = v.weight; o[3] = v.upper; o[4] = v.lower;
-      o[5] = v.heuristic; o[6] = (float)v.depth; o[7] = (float)v.children.size();
-      o[8] = target(v.to_expand);
-    }
-  }
-  return (int64_t)order.size();
+  return dump_tree(tt->t, out, cap_nodes);
 }
 
 /* SearchTree::update(a, z), search_tree_cuda.cu:548-626 */
@@ -1390,13 +1486,9 @@ int pp2d_tree_update(pp2d_tree* tt, uint8_t a, uint8_t z) {
   if (t.v[t.root].children.empty())
     return fail(PP2D_ERR_STATE, "update() on an unexpanded root (nullptr in the reference)");
   // Nothing is freed before the arguments are known to be usable.
-  int root_q = -1;
-  for (int c : t.v[t.root].children)
-    if (t.q[c].action == a) root_q = c;
+  int root_q = -1, root_v = -1;
+  kept_nodes(t, a, z, &root_q, &root_v);
   if (root_q < 0) return fail(PP2D_ERR_INVALID, "no Q node for action %u", a);
-  int root_v = -1;
-  for (int c : t.q[root_q].children)
-    if (t.v[c].obs == z) root_v = c;
   int new_slot = -1;
   float ev[4] = {0, 0, 0, 0};
   if (root_v < 0) {
@@ -1418,58 +1510,12 @@ int pp2d_tree_update(pp2d_tree* tt, uint8_t a, uint8_t z) {
       std::vector<int> s1{new_slot};
       return evaluate_slots(h, s1, ev, t.dense);
     }();
-    if (rc != PP2D_OK) { h->free_slots.push_back(new_slot); return rc; }
-  }
-  // The subtrees that are not kept give their beliefs back (tree:556-584).
-  for (int c : t.v[t.root].children)
-    if (c != root_q) free_subtree_q(h, t, c);
-  for (int c : t.q[root_q].children)
-    if (c != root_v) free_subtree_v(h, t, c);
-  VNodeH& old_root = t.v[t.root];
-  if (old_root.slot >= 0) { h->free_slots.push_back(old_root.slot); old_root.slot = -1; }
-  // Rebuild the node arrays from the kept subtree: a long-running planner
-  // re-roots once per belief message, and dropped nodes must not accumulate.
-  Tree fresh;
-  fresh.rng = t.rng;
-  fresh.expansions = t.expansions;
-  fresh.dense = t.dense;
-  if (root_v >= 0) {
-    std::vector<int> vmap(t.v.size(), -1), qmap(t.q.size(), -1);
-    struct Item { int idx; bool is_q; };
-    std::vector<Item> stack{{root_v, false}};
-    while (!stack.empty()) {                       // number the kept nodes
-      const Item it = stack.back();
-      stack.pop_back();
-      if (it.is_q) {
-        qmap[it.idx] = (int)fresh.q.size();
-        fresh.q.push_back(t.q[it.idx]);
-        for (int c : t.q[it.idx].children) stack.push_back({c, false});
-      } else {
-        vmap[it.idx] = (int)fresh.v.size();
-        fresh.v.push_back(t.v[it.idx]);
-        for (int c : t.v[it.idx].children) stack.push_back({c, true});
-      }
-    }
-    auto mv = [&](int v) { return v >= 0 ? vmap[v] : -1; };
-    for (VNodeH& v : fresh.v) {
-      v.parent = v.parent >= 0 ? qmap[v.parent] : -1;
-      v.to_expand = mv(v.to_expand);
-      for (int& c : v.children) c = qmap[c];
-    }
-    for (QNodeH& q : fresh.q) {
-      q.parent = vmap[q.parent];
-      q.to_expand = mv(q.to_expand);
-      for (int& c : q.children) c = vmap[c];
-    }
-    fresh.root = vmap[root_v];
-    fresh.v[fresh.root].parent = -1;
-  } else {
-    fresh.v.emplace_back();
-    fresh.root = 0;
-    init_vnode(fresh.v[0], new_slot, 0, 0.0f, -1, ev, 0);
+    if (rc != PP2D_OK) { h->free_slots.put(new_slot); return rc; }
     h->n_vnodes++;
   }
-  t = std::move(fresh);
+  std::vector<int> freed;
+  reroot(t, root_q, root_v, new_slot, ev, freed);
+  give_back(h, freed);
   return PP2D_OK;
 }
 
@@ -1485,3 +1531,222 @@ int pp2d_tree_plan(pp2d_tree* t, uint32_t max_depth, uint32_t max_iter,
 }
 
 }  // extern "C"
+
+/* ---- persistent tree batches: many SearchTrees planned together ---------- */
+struct pp2d_tree_batch {
+  pp2d_pomdp* h = nullptr;
+  std::vector<Tree> trees;
+};
+
+namespace {
+
+// A list of tree indices of a call: every entry < count, none twice.
+int check_tree_list(const pp2d_tree_batch* b, const uint32_t* trees, uint32_t n,
+                    const char* fn) {
+  std::vector<uint8_t> seen(b->trees.size(), 0);
+  for (uint32_t i = 0; i < n; ++i) {
+    if (trees[i] >= b->trees.size())
+      return fail(PP2D_ERR_INVALID, "%s: entry %u names tree %u of a batch of %zu", fn, i,
+                  trees[i], b->trees.size());
+    if (seen[trees[i]]++)
+      return fail(PP2D_ERR_INVALID, "%s: tree %u is listed twice", fn, trees[i]);
+  }
+  return PP2D_OK;
+}
+
+// Sort keys of the listed roots (pomdp_root_mode_kernel), read from the pool.
+int root_mode_keys(pp2d_pomdp* h, const std::vector<Tree*>& trees, std::vector<uint32_t>& key) {
+  const int n = (int)trees.size();
+  std::vector<int> slots(n);
+  for (int i = 0; i < n; ++i) slots[i] = trees[i]->v[trees[i]->root].slot;
+  PP2D_TRY(h->d_slots.ensure(n));
+  PP2D_TRY(h->d_keys.ensure(n));
+  PP2D_CUDA(cudaMemcpyAsync(h->d_slots.p, slots.data(), n * sizeof(int), cudaMemcpyHostToDevice,
+                            h->stream));
+  pomdp_root_mode_kernel<<<(n + 3) / 4, 128, 0, h->stream>>>(h->H, h->W, h->d_slots.p, n,
+                                                             h->d_bel, h->d_keys.p);
+  count_launch();
+  PP2D_CUDA(cudaGetLastError());
+  key.resize(n);
+  PP2D_CUDA(cudaMemcpyAsync(key.data(), h->d_keys.p, n * sizeof(uint32_t), cudaMemcpyDeviceToHost,
+                            h->stream));
+  PP2D_CUDA(cudaStreamSynchronize(h->stream));
+  return PP2D_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int pp2d_tree_batch_create(pp2d_pomdp* h, const float* beliefs, uint32_t n,
+                           pp2d_tree_batch** out) {
+  if (!h || !beliefs || !out) return fail(PP2D_ERR_INVALID, "NULL argument");
+  *out = nullptr;
+  if (!h->have_alphas) return fail(PP2D_ERR_STATE, "pp2d_pomdp_set_alphas not called");
+  pp2d_tree_batch* b = new (std::nothrow) pp2d_tree_batch;
+  if (!b) return fail(PP2D_ERR_INVALID, "out of host memory");
+  b->h = h;
+  int rc = [&]() -> int {
+    b->trees.resize(n);
+    std::vector<Tree*> trees(n);
+    for (uint32_t i = 0; i < n; ++i) { b->trees[i].rng.seed(1); trees[i] = &b->trees[i]; }
+    if (n == 0) return PP2D_OK;
+    PP2D_TRY(pool_reserve(h, (size_t)h->cap - h->free_slots.count() + n));
+    return make_roots(h, trees, beliefs);
+  }();
+  if (rc != PP2D_OK) { pp2d_tree_batch_destroy(b); return rc; }
+  *out = b;
+  return PP2D_OK;
+}
+
+void pp2d_tree_batch_destroy(pp2d_tree_batch* b) {
+  if (!b) return;
+  std::vector<int> freed;
+  for (Tree& t : b->trees)
+    if (t.root >= 0) free_subtree_v(t, t.root, freed);
+  give_back(b->h, freed);
+  delete b;
+}
+
+int pp2d_tree_batch_update(pp2d_tree_batch* b, const uint32_t* trees, uint32_t n,
+                           const uint8_t* actions, const uint8_t* observations) {
+  if (!b) return fail(PP2D_ERR_INVALID, "batch is NULL");
+  if (n == 0) return PP2D_OK;
+  if (!trees || !actions || !observations) return fail(PP2D_ERR_INVALID, "NULL argument");
+  PP2D_TRY(check_tree_list(b, trees, n, "pp2d_tree_batch_update"));
+  pp2d_pomdp* h = b->h;
+  std::vector<int> rq(n), rv(n);
+  for (uint32_t i = 0; i < n; ++i) {
+    const uint32_t k = trees[i];
+    if (actions[i] >= kActions || observations[i] >= 16)
+      return fail(PP2D_ERR_INVALID, "tree %u: action %u / observation %u out of range (9 / 16)",
+                  k, actions[i], observations[i]);
+    const Tree& t = b->trees[k];
+    if (t.v[t.root].children.empty())
+      return fail(PP2D_ERR_STATE, "tree %u: update() on an unexpanded root (nullptr in the "
+                                  "reference)", k);
+    kept_nodes(t, actions[i], observations[i], &rq[i], &rv[i]);
+    if (rq[i] < 0) return fail(PP2D_ERR_INVALID, "tree %u: no Q node for action %u", k, actions[i]);
+  }
+  // Misses (an observation without a child): one Bayes update of the old root
+  // each (tree:586-614), all in one set of launches.
+  std::vector<uint32_t> miss;
+  for (uint32_t i = 0; i < n; ++i)
+    if (rv[i] < 0) miss.push_back(i);
+  const size_t nm = miss.size();
+  std::vector<int> slots(nm, -1);
+  std::vector<float> ev(nm * 4, 0.0f);
+  if (nm) {
+    PP2D_TRY(pool_reserve(h, (size_t)h->cap - h->free_slots.count() + nm));
+    std::vector<BayesItem> items(nm);
+    bool dense = false;
+    for (size_t j = 0; j < nm; ++j) {
+      const uint32_t i = miss[j];
+      const Tree& t = b->trees[trees[i]];
+      PP2D_TRY(alloc_slot(h, &slots[j]));            // (reserved: cannot fail)
+      items[j] = BayesItem{t.v[t.root].slot, slots[j], actions[i], observations[i]};
+      dense = dense || t.dense;
+    }
+    int rc = [&]() -> int {
+      PP2D_TRY(launch_bayes(h, items));
+      PP2D_TRY(launch_normalize(h, slots));
+      return evaluate_slots(h, slots, ev.data(), dense);
+    }();
+    if (rc != PP2D_OK) {
+      for (int s : slots) h->free_slots.put(s);
+      return rc;
+    }
+    h->n_vnodes += nm;
+  }
+  std::vector<int> slot_of(n, -1);
+  std::vector<const float*> ev_of(n, nullptr);
+  for (size_t j = 0; j < nm; ++j) { slot_of[miss[j]] = slots[j]; ev_of[miss[j]] = &ev[4 * j]; }
+  const int ni = (int)n;
+#pragma omp parallel num_threads(host_threads()) if (ni >= 64)
+  {
+    std::vector<int> freed;
+#pragma omp for schedule(dynamic, 8) nowait
+    for (int i = 0; i < ni; ++i)
+      reroot(b->trees[trees[i]], rq[i], rv[i], slot_of[i], ev_of[i], freed);
+#pragma omp critical
+    give_back(h, freed);
+  }
+  return PP2D_OK;
+}
+
+int pp2d_tree_batch_plan(pp2d_tree_batch* b, const uint32_t* trees, uint32_t n,
+                         uint32_t max_depth, uint32_t max_iter, uint8_t* actions, float* values,
+                         uint32_t* stats) {
+  if (!b) return fail(PP2D_ERR_INVALID, "batch is NULL");
+  if (n == 0) return PP2D_OK;
+  if (!trees || !actions) return fail(PP2D_ERR_INVALID, "NULL argument");
+  PP2D_TRY(check_tree_list(b, trees, n, "pp2d_tree_batch_plan"));
+  pp2d_pomdp* h = b->h;
+  if (max_iter > 255) max_iter = 255;           // as pp2d_pomdp_plan_batch
+  // live beliefs + the worst case of every listed tree (9 * 16 children per
+  // expansion), within the budget of pp2d_pomdp_plan_batch; past it the pool
+  // grows in place
+  const size_t live = (size_t)h->cap - h->free_slots.count();
+  size_t max_slots = 0;
+  PP2D_TRY(pool_budget(h, &max_slots));
+  const size_t want =
+      std::min(live + (size_t)n * slots_per_tree((size_t)max_iter * kActions * 16),
+               std::max(max_slots, live + n));
+  if ((size_t)h->cap < want) PP2D_TRY(pool_reserve(h, want));
+  std::vector<Tree*> list(n);
+  for (uint32_t i = 0; i < n; ++i) list[i] = &b->trees[trees[i]];
+  // in the order of the roots' modes, as pp2d_pomdp_plan_batch orders its queries
+  const bool sorted = h->sort_queries && n >= 2 * (uint32_t)kEvM;
+  if (sorted) {
+    std::vector<uint32_t> key;
+    PP2D_TRY(root_mode_keys(h, list, key));
+    std::vector<int> order(n);
+    for (uint32_t i = 0; i < n; ++i) order[i] = (int)i;
+    std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return key[x] < key[y]; });
+    for (uint32_t i = 0; i < n; ++i) list[i] = &b->trees[trees[order[i]]];
+  }
+  PP2D_TRY(plan_trees(h, list, max_depth, max_iter, sorted));
+  for (uint32_t i = 0; i < n; ++i) {
+    const Tree& t = b->trees[trees[i]];
+    float r;
+    best_action(t, &actions[i], &r);
+    if (values) values[i] = r;
+    if (stats) {
+      stats[4 * (size_t)i + 0] = (uint32_t)t.v.size();
+      stats[4 * (size_t)i + 1] = (uint32_t)t.q.size();
+      stats[4 * (size_t)i + 2] = t.v[t.root].depth;
+      stats[4 * (size_t)i + 3] = t.expansions;
+    }
+  }
+  return PP2D_OK;
+}
+
+int64_t pp2d_tree_batch_dump(const pp2d_tree_batch* b, uint32_t k, float* out,
+                             uint64_t cap_nodes) {
+  if (!b) { fail(PP2D_ERR_INVALID, "batch is NULL"); return -1; }
+  if (k >= b->trees.size()) {
+    fail(PP2D_ERR_INVALID, "pp2d_tree_batch_dump: tree %u of a batch of %zu", k, b->trees.size());
+    return -1;
+  }
+  return dump_tree(b->trees[k], out, cap_nodes);
+}
+
+}  // extern "C"
+
+namespace pp2d {
+
+int tree_batch_root_beliefs(pp2d_tree_batch* b, float* out) {
+  pp2d_pomdp* h = b->h;
+  const size_t n = b->trees.size();
+  if (n == 0) return PP2D_OK;
+  std::vector<int> slots(n);
+  for (size_t i = 0; i < n; ++i) slots[i] = b->trees[i].v[b->trees[i].root].slot;
+  PP2D_TRY(h->d_rows.ensure(n * h->HW));
+  PP2D_TRY(launch_gather(h, slots, h->d_rows.p));
+  PP2D_CUDA(cudaMemcpyAsync(out, h->d_rows.p, n * h->HW * sizeof(float), cudaMemcpyDeviceToHost,
+                            h->stream));
+  PP2D_CUDA(cudaStreamSynchronize(h->stream));
+  return PP2D_OK;
+}
+
+}  // namespace pp2d

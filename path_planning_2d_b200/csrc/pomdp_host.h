@@ -78,6 +78,43 @@ struct GlibcRand {
   }
 };
 
+// Free slots of the belief pool, handed out lowest first.  The values launches
+// load a tile's columns coalesced only when its beliefs share 32-slot blocks
+// (bel_off): a fresh pool gives a round's children ascending slots, and so
+// does this list after trees have given back scattered slots (re-rooting,
+// finished batches).
+struct FreeSlots {
+  std::vector<uint64_t> bits;     // bit s: slot s is free
+  size_t n = 0;
+  size_t lo = 0;                  // no free slot in words below lo
+  size_t cap = 0;
+  size_t count() const { return n; }
+  bool empty() const { return n == 0; }
+  void clear() { bits.clear(); n = 0; lo = 0; cap = 0; }
+  void grow(size_t new_cap) {     // slots [cap, new_cap) are new and free
+    bits.resize((new_cap + 63) / 64, 0);
+    for (size_t s = cap; s < new_cap;) {
+      if ((s & 63) == 0 && s + 64 <= new_cap) { bits[s >> 6] = ~0ull; s += 64; }
+      else { bits[s >> 6] |= 1ull << (s & 63); ++s; }
+    }
+    n += new_cap - cap;
+    if (cap >> 6 < lo) lo = cap >> 6;
+    cap = new_cap;
+  }
+  void put(int s) {
+    bits[(size_t)s >> 6] |= 1ull << (s & 63);
+    ++n;
+    if ((size_t)s >> 6 < lo) lo = (size_t)s >> 6;
+  }
+  int take() {                    // n > 0
+    while (!bits[lo]) ++lo;
+    const int b = __builtin_ctzll(bits[lo]);
+    bits[lo] &= bits[lo] - 1;
+    --n;
+    return (int)(lo * 64 + (size_t)b);
+  }
+};
+
 template <typename T>
 struct DevBuf {
   T* p = nullptr;
@@ -131,13 +168,14 @@ struct pp2d_pomdp {
   // belief pool [HW][cap]
   float* d_bel = nullptr;
   int cap = 0;
-  std::vector<int> free_slots;
+  pp2d::FreeSlots free_slots;
   // scratch
   pp2d::DevBuf<int> d_slots;
   pp2d::DevBuf<pp2d::BayesItem> d_items;
   pp2d::DevBuf<float> d_prefix, d_draws, d_vals, d_rows, d_sums;
   pp2d::DevBuf<uint8_t> d_obs;
   pp2d::DevBuf<float> d_out;               // 4 floats per evaluated belief
+  pp2d::DevBuf<uint32_t> d_keys;           // mode keys of a tree batch's roots
   float* pin_rows = nullptr;               // page-locked staging of a batch's start beliefs
   size_t pin_rows_cap = 0;
   void* round_ctx[4] = {nullptr, nullptr, nullptr, nullptr};   // RoundCtx of pomdp.cu (lazily created)

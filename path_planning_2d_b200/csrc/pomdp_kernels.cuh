@@ -950,4 +950,29 @@ __global__ void pomdp_gather_kernel(int HW, const int* __restrict__ slots,
   rows[(size_t)i * HW + s] = bel[bel_off(HW, s, slots[i])];
 }
 
+// Mode of each listed belief column as the sort key of the batched planners:
+// column * H + row of the first maximum in cell order.  One warp per column.
+__global__ void __launch_bounds__(128)
+pomdp_root_mode_kernel(int H, int W, const int* __restrict__ slots, int n,
+                       const float* __restrict__ bel, uint32_t* __restrict__ key) {
+  const int i = blockIdx.x * 4 + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (i >= n) return;
+  const int HW = H * W;
+  const float* col = bel + bel_off(HW, 0, slots[i]);
+  float bv = -INFINITY;
+  int bi = INT_MAX;
+  for (int s = lane; s < HW; s += 32) {
+    const float v = col[(size_t)s * kSlotBlock];
+    if (bi == INT_MAX || v > bv) { bv = v; bi = s; }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+    const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+    if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+  }
+  if (lane == 0) key[i] = (uint32_t)(bi % W) * (uint32_t)H + (uint32_t)(bi / W);
+}
+
 }  // namespace pp2d

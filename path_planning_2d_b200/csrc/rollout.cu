@@ -1,10 +1,10 @@
-// rollout.cu -- closed-loop episodes of an MDP planner in the simulator
-// (pp2d_sim_rollout_mdp*, include/pp2d.h; contract in DESIGN.md section 7,
-// "Closed-loop rollouts").
+// rollout.cu -- closed-loop episodes of an MDP planner (pp2d_sim_rollout_mdp*)
+// or of the QV-tree planner (pp2d_sim_rollout_pomdp) in the simulator
+// (include/pp2d.h; contract in DESIGN.md sections 7c and 7d).
 //
-// One CTA runs one episode from its start to its stop, so an episode that has
-// stopped costs nothing more (its CTA has exited and the next one takes the
-// SM slot).  The belief and the prediction plane live in shared memory while
+// MDP rollouts: one CTA runs one episode from its start to its stop, so an
+// episode that has stopped costs nothing more (its CTA has exited and the next
+// one takes the SM slot).  The belief and the prediction plane live in shared memory while
 // both fit (2 * HW floats; 32 KB on the reference's 100x40 map); larger maps
 // run the same code on two planes per episode in global memory.  Each step:
 // belief_mode (the plan kernels' scan) -> action; thread 0 draws the motion
@@ -97,39 +97,12 @@ sim_rollout_kernel(const RolloutParams p) {
     const unsigned long long mode = belief_mode(bel, (size_t)HW);
     if (threadIdx.x == 0) {
       const int u = ep.action[mode];
-      float r[5];
-      pp2d_step_uniforms(p.seed, e, t, r);
-      // move: first slot whose running probability exceeds r[0]
-      int slot = -1, last = 4;
-      float acc = 0.0f;
-      for (int k = 0; k < 9; ++k) {
-        const float pk = naive_prob(u, k);
-        if (pk != 0.0f) last = k;
-        acc = __fadd_rn(acc, pk);
-        if (slot < 0 && r[0] < acc) slot = k;
-      }
-      if (slot < 0) slot = last;
-      int x = (int)(cell % p.W), y = (int)(cell / p.W);
-      if (slot != 4) {
-        const int tx = x + slot % 3 - 1, ty = y + slot / 3 - 1;
-        if (blocked(p, tx, ty)) ++s_coll;
-        else { x = tx; y = ty; }
-      }
-      // sense: up, left, right, down; out of the map reads as occupied
-      const int ox[4] = {0, -1, 1, 0}, oy[4] = {-1, 0, 0, 1};
-      uint32_t m = 0;
-      for (int j = 0; j < 4; ++j) {
-        const int mx = x + ox[j], my = y + oy[j];
-        uint32_t v = (mx < 0 || mx >= p.W || my < 0 || my >= p.H) ? 1u
-                                                                  : (p.map[my * p.W + mx] ? 1u : 0u);
-        if (r[1 + j] < 0.02f) v ^= 1u;
-        m |= v << j;
-      }
-      const uint32_t nc = (uint32_t)(y * p.W + x);
-      s_cell = nc; s_act = (uint32_t)u; s_meas = m;
-      if (p.cells) p.cells[(size_t)i * ((size_t)p.max_steps + 1) + t + 1] = nc;
+      const WorldStep w = world_step(p.H, p.W, p.map, cell, u, p.seed, e, t);
+      if (w.collided) ++s_coll;
+      s_cell = w.cell; s_act = (uint32_t)u; s_meas = w.meas;
+      if (p.cells) p.cells[(size_t)i * ((size_t)p.max_steps + 1) + t + 1] = w.cell;
       if (p.actions) p.actions[(size_t)i * p.max_steps + t] = (uint8_t)u;
-      if (p.meas) p.meas[(size_t)i * p.max_steps + t] = (uint8_t)m;
+      if (p.meas) p.meas[(size_t)i * p.max_steps + t] = (uint8_t)w.meas;
     }
     __syncthreads();
     const int u = (int)s_act;
@@ -355,6 +328,74 @@ int pp2d_sim_rollout_mdp_batch(pp2d_sim* s, pp2d_mdp_batch* planner, const uint3
     views[i] = mdp_batch_view(planner, instances[i]);
   }
   return rollout(s, views, n, starts_xy, beliefs, max_steps, seed, first_episode, out);
+}
+
+/* The loop of the MDP rollouts with the QV-tree as the planner (DESIGN.md
+ * section 7d): one persistent tree per episode, planned and updated through a
+ * tree batch, the world stepped on the host by the function the device
+ * rollouts use. */
+int pp2d_sim_rollout_pomdp(pp2d_sim* s, pp2d_pomdp* planner, uint32_t n, const uint32_t* starts_xy,
+                           const float* beliefs, uint32_t max_steps, uint32_t max_depth,
+                           uint32_t max_iter, uint64_t seed, uint64_t first_episode,
+                           pp2d_rollout* out) {
+  if (!planner) return fail(PP2D_ERR_INVALID, "NULL planner");
+  PlannerView v;
+  v.H = (uint32_t)planner->H; v.W = (uint32_t)planner->W;
+  v.gx = (uint32_t)planner->gx; v.gy = (uint32_t)planner->gy;
+  PP2D_TRY(check_common(s, v, n, starts_xy));
+  // (every step updates the tree that planned it: its root must be expanded)
+  if (max_depth == 0 || max_iter == 0)
+    return fail(PP2D_ERR_INVALID, "pp2d_sim_rollout_pomdp: max_depth and max_iter must be > 0");
+  if (!planner->have_alphas) return fail(PP2D_ERR_STATE, "pp2d_pomdp_set_alphas not called");
+  if (n == 0) return PP2D_OK;
+  const SimView sv = sim_view(s);
+  const size_t hw = (size_t)sv.H * sv.W;
+  const uint32_t goal = v.gy * sv.W + v.gx;
+  std::vector<float> point;
+  if (!beliefs) {
+    point.assign(n * hw, 0.0f);
+    for (uint32_t i = 0; i < n; ++i)
+      point[i * hw + starts_xy[2 * (size_t)i + 1] * sv.W + starts_xy[2 * (size_t)i]] = 1.0f;
+  }
+  pp2d_tree_batch* tb = nullptr;
+  PP2D_TRY(pp2d_tree_batch_create(planner, beliefs ? beliefs : point.data(), n, &tb));
+  struct Guard { pp2d_tree_batch* b; ~Guard() { pp2d_tree_batch_destroy(b); } } guard{tb};
+  std::vector<uint32_t> cell(n), steps(n, 0), coll(n, 0), live(n);
+  std::vector<uint8_t> act(n), meas(n);
+  for (uint32_t i = 0; i < n; ++i) {
+    cell[i] = starts_xy[2 * (size_t)i + 1] * sv.W + starts_xy[2 * (size_t)i];
+    if (out && out->cells) out->cells[i * (max_steps + 1ull)] = cell[i];
+  }
+  for (uint32_t t = 0;; ++t) {
+    uint32_t nl = 0;                             // episodes that take step t
+    for (uint32_t i = 0; i < n; ++i)
+      if (steps[i] == t && cell[i] != goal && t < max_steps) live[nl++] = i;
+    if (nl == 0) break;
+    PP2D_TRY(pp2d_tree_batch_plan(tb, live.data(), nl, max_depth, max_iter, act.data(), nullptr,
+                                  nullptr));
+    for (uint32_t j = 0; j < nl; ++j) {
+      const uint32_t i = live[j];
+      const WorldStep w = world_step((int)sv.H, (int)sv.W, sv.map_host, cell[i], act[j], seed,
+                                     first_episode + i, t);
+      cell[i] = w.cell;
+      coll[i] += w.collided ? 1 : 0;
+      meas[j] = (uint8_t)w.meas;
+      steps[i] = t + 1;
+      if (out && out->cells) out->cells[i * (max_steps + 1ull) + t + 1] = w.cell;
+      if (out && out->actions) out->actions[(size_t)i * max_steps + t] = act[j];
+      if (out && out->measurements) out->measurements[(size_t)i * max_steps + t] = meas[j];
+    }
+    PP2D_TRY(pp2d_tree_batch_update(tb, live.data(), nl, act.data(), meas.data()));
+  }
+  if (!out) return PP2D_OK;
+  if (out->final_belief) PP2D_TRY(tree_batch_root_beliefs(tb, out->final_belief));
+  for (uint32_t i = 0; i < n; ++i) {
+    if (out->steps) out->steps[i] = steps[i];
+    if (out->reached) out->reached[i] = cell[i] == goal ? 1 : 0;
+    if (out->collisions) out->collisions[i] = coll[i];
+    if (out->final_cell) out->final_cell[i] = cell[i];
+  }
+  return PP2D_OK;
 }
 
 }  // extern "C"

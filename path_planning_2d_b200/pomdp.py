@@ -76,6 +76,83 @@ class SearchTree:
         return out
 
 
+class SearchTreeBatch:
+    """Many SearchTrees on the GPU belief pool of one PomdpPathPlanning2d that
+    live across belief callbacks (one per robot of a fleet), updated and
+    planned together (pp2d_tree_batch_* in include/pp2d.h).  Tree k behaves
+    bit for bit like SearchTree(planner, beliefs[k]) fed the same calls."""
+
+    def __init__(self, planner, beliefs):
+        self._lib = planner._lib
+        self._planner = planner
+        hw = planner.map_height * planner.map_width
+        b = np.ascontiguousarray(beliefs, dtype=np.float32)
+        if b.size % hw:
+            raise ValueError("beliefs must be [n][height*width]")
+        b = b.reshape(-1, hw)
+        self.count = b.shape[0]
+        self._b = ctypes.c_void_p()
+        _lib.check(self._lib.pp2d_tree_batch_create(planner._h, b.ctypes.data, self.count,
+                                                    ctypes.byref(self._b)))
+
+    def close(self):
+        if getattr(self, "_b", None) is not None and self._b.value:
+            self._lib.pp2d_tree_batch_destroy(self._b)
+            self._b = ctypes.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def _trees(self, trees):
+        if trees is None:
+            return np.arange(self.count, dtype=np.uint32)
+        return np.ascontiguousarray(trees, dtype=np.uint32).reshape(-1)
+
+    def update(self, trees, actions, observations):
+        """SearchTree.update(actions[i], observations[i]) on tree trees[i]
+        (None: every tree); nothing changes if any entry is refused."""
+        idx = self._trees(trees)
+        n = idx.size
+        a = np.ascontiguousarray(np.broadcast_to(actions, (n,)), dtype=np.uint8)
+        z = np.ascontiguousarray(np.broadcast_to(observations, (n,)), dtype=np.uint8)
+        _lib.check(self._lib.pp2d_tree_batch_update(self._b, idx.ctypes.data, n, a.ctypes.data,
+                                                    z.ctypes.data))
+
+    def plan(self, trees=None, max_depth=None, max_iter=None, with_stats=False):
+        """SearchTree.plan on the listed trees (None: every tree), defaults
+        from the planner (depth 50, 15 iterations).  Returns (actions, values)
+        and with with_stats the [n][4] {V nodes, Q nodes, depth, expansions}."""
+        idx = self._trees(trees)
+        n = idx.size
+        acts = np.zeros(n, np.uint8)
+        vals = np.zeros(n, np.float32)
+        stats = np.zeros((n, 4), np.uint32)
+        _lib.check(self._lib.pp2d_tree_batch_plan(
+            self._b, idx.ctypes.data, n,
+            self._planner.max_search_tree_depth if max_depth is None else max_depth,
+            self._planner.max_online_iteration if max_iter is None else max_iter,
+            acts.ctypes.data, vals.ctypes.data, stats.ctypes.data))
+        return (acts, vals, stats) if with_stats else (acts, vals)
+
+    def dump(self, k):
+        """SearchTree.dump() of tree k."""
+        n = self._lib.pp2d_tree_batch_dump(self._b, k, None, 0)
+        if n < 0:
+            raise _lib.Pp2dError(_lib.PP2D_ERR_INVALID, self._lib.pp2d_last_error().decode())
+        out = np.zeros((n, 9), np.float32)
+        self._lib.pp2d_tree_batch_dump(self._b, k, out.ctypes.data, n)
+        return out
+
+
 class PomdpPathPlanning2d:
     def __init__(self, grid_map, goal, discount_factor, max_search_tree_depth=50,
                  max_online_iteration=15):

@@ -17,6 +17,7 @@ import numpy as np
 
 from . import _lib
 from .mdp import MdpBatchPathPlanning2d, MdpPathPlanning2d
+from .pomdp import PomdpPathPlanning2d
 
 
 class DummySimulator:
@@ -73,10 +74,13 @@ class DummySimulator:
         return b
 
     def rollout(self, planner, starts, max_steps, seed, beliefs=None, instances=None,
-                first_episode=0, record=False):
+                first_episode=0, record=False, max_depth=None, max_iter=None):
         """Closed-loop episodes of `planner` (MdpPathPlanning2d, or
         MdpBatchPathPlanning2d with `instances`: the instance each episode
-        follows) in this simulator's map, from starts [n][2] = (x, y), with
+        follows, or PomdpPathPlanning2d: one search tree per episode, planned
+        with max_depth / max_iter, default the planner's 50 / 15, and updated
+        with each action and measurement; final_belief is then the tree's
+        root belief) in this simulator's map, from starts [n][2] = (x, y), with
         beliefs [n][H*W] (default: a point mass at each start).  Episode i
         draws its noise as episode first_episode + i of `seed`.  Returns a dict
         of steps, reached, collisions and final_cell (y*W+x) per episode; with
@@ -99,7 +103,17 @@ class DummySimulator:
             res["measurements"] = np.zeros((n, max_steps), np.uint8)
         out = _lib.Rollout(**{k: v.ctypes.data for k, v in res.items()})
         bp = b.ctypes.data if b is not None else None
-        if isinstance(planner, MdpBatchPathPlanning2d):
+        if not isinstance(planner, PomdpPathPlanning2d) and (max_depth, max_iter) != (None, None):
+            raise ValueError("max_depth / max_iter are for a PomdpPathPlanning2d")
+        if isinstance(planner, PomdpPathPlanning2d):
+            if instances is not None:
+                raise ValueError("`instances` is for a batch planner")
+            rc = self._lib.pp2d_sim_rollout_pomdp(
+                self._h, planner._h, n, st.ctypes.data, bp, max_steps,
+                planner.max_search_tree_depth if max_depth is None else max_depth,
+                planner.max_online_iteration if max_iter is None else max_iter,
+                seed, first_episode, ctypes.byref(out))
+        elif isinstance(planner, MdpBatchPathPlanning2d):
             if instances is None:
                 raise ValueError("a batch planner needs `instances`, one per episode")
             idx = np.ascontiguousarray(instances, dtype=np.uint32).reshape(-1)
@@ -115,6 +129,7 @@ class DummySimulator:
                                                 max_steps, seed, first_episode,
                                                 ctypes.byref(out))
         else:
-            raise TypeError("planner must be an MdpPathPlanning2d or MdpBatchPathPlanning2d")
+            raise TypeError("planner must be an MdpPathPlanning2d, MdpBatchPathPlanning2d or "
+                            "PomdpPathPlanning2d")
         _lib.check(rc)
         return res
