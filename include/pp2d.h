@@ -615,6 +615,54 @@ int pp2d_tree_batch_plan(pp2d_tree_batch* b, const uint32_t* trees, uint32_t n,
 int64_t pp2d_tree_batch_dump(const pp2d_tree_batch* b, uint32_t k, float* out,
                              uint64_t cap_nodes);
 
+/*
+ * Goal sets (DESIGN.md section 7e): one planner handle for many goals of one
+ * map.  The goal enters the model only through the stage reward (0 instead of
+ * -2 for staying on the goal cell); the transition and likelihood tables, the
+ * live cells and the belief pool are shared.  Goal 0 is the goal the handle
+ * was created with: its reward table is the one pp2d_pomdp_model_tables
+ * returns and pp2d_pomdp_set_model_tables replaces, its bounds the ones
+ * pp2d_pomdp_set_alphas sets, and every entry point without a goal argument
+ * works on goal 0 alone.  A tree with goal g behaves bit for bit like a tree on
+ * a handle created with goal g, with the same tables and goal g's alpha
+ * vectors, fed the same calls.
+ *
+ * set_goals: goals_xy [n][2] = (x, y) replace goals 1..n (n = 0 removes them;
+ * the new goals have no alpha vectors).  stage_rewards NULL: each goal's table
+ * is generated by the model rule from the handle's map (the table
+ * pp2d_pomdp_model_tables returns on a handle created with that goal);
+ * otherwise stage_rewards [n][HW][9] is uploaded as given (tables read back
+ * from text files differ in their bits from generated ones).  A goal outside
+ * the map gives PP2D_ERR_INVALID, an occupied one PP2D_ERR_GOAL_OCCUPIED (the
+ * message names the goal index); while any belief is resident PP2D_ERR_STATE,
+ * as pp2d_pomdp_set_model_tables.  A refused call changes nothing.
+ * goals: count = goals in the set, goal 0 included; goals_xy [count][2] (each
+ * may be NULL).  goal_reward: goal g's stage reward table [HW][9].
+ * set_goal_alphas: pp2d_pomdp_set_alphas for goal g (g = 0: the same call).
+ * All goals of a handle use one PBVI count: a call that would give a goal
+ * another count than a goal already holding alpha vectors is refused with
+ * PP2D_ERR_INVALID (pp2d_pomdp_set_alphas too).  fib_actions / pbvi_actions of
+ * goals >= 1 are not kept: only pp2d_pomdp_evaluate reads actions, on goal 0.
+ * tree_batch_create_goals: pp2d_tree_batch_create, tree k planning to goal
+ * goals[k] (goals NULL: goal 0 for every tree, = pp2d_tree_batch_create).  A
+ * goal index above the set gives PP2D_ERR_INVALID, a goal without alpha
+ * vectors PP2D_ERR_STATE (messages name the tree).  The other pp2d_tree_batch_*
+ * calls work on such batches unchanged.
+ * padding_counters: of the work out[2] of pp2d_pomdp_work_counters, what went
+ * to the padding of goal segments: out[0] = padded entries evaluated, out[1] =
+ * their belief x inner-row products.  Measurement only.
+ */
+int pp2d_pomdp_set_goals(pp2d_pomdp* h, const uint32_t* goals_xy, uint32_t n,
+                         const float* stage_rewards);
+int pp2d_pomdp_goals(pp2d_pomdp* h, uint32_t* count, uint32_t* goals_xy);
+int pp2d_pomdp_goal_reward(pp2d_pomdp* h, uint32_t g, float* stage_reward);
+int pp2d_pomdp_set_goal_alphas(pp2d_pomdp* h, uint32_t g, const float* fib_alphas,
+                               const uint8_t* fib_actions, const float* pbvi_alphas,
+                               const uint8_t* pbvi_actions, uint32_t n_pbvi);
+int pp2d_tree_batch_create_goals(pp2d_pomdp* h, const float* beliefs, const uint32_t* goals,
+                                 uint32_t n, pp2d_tree_batch** out);
+int pp2d_pomdp_padding_counters(pp2d_pomdp* h, uint64_t out[2]);
+
 /* ------------------------------------------------------------------------
  * dummy_simulator's Bayes filter (SURVEY.md section 8f row 4b)
  * ------------------------------------------------------------------------ */
@@ -707,6 +755,17 @@ int pp2d_sim_rollout_pomdp(pp2d_sim* s, pp2d_pomdp* planner, uint32_t n, const u
                            const float* beliefs, uint32_t max_steps, uint32_t max_depth,
                            uint32_t max_iter, uint64_t seed, uint64_t first_episode,
                            pp2d_rollout* out);
+/* pp2d_sim_rollout_pomdp with a goal per episode (DESIGN.md section 7e):
+ * episode i plans to goal goals[i] of the planner's goal set and stops on that
+ * goal's cell.  It is bit for bit episode i (same id) of
+ * pp2d_sim_rollout_pomdp on a handle created with that goal, with the same
+ * tables and that goal's alpha vectors.  Checks as pp2d_sim_rollout_pomdp,
+ * plus NULL goals or an index above the set (PP2D_ERR_INVALID) and a goal
+ * without alpha vectors (PP2D_ERR_STATE), all before any device work. */
+int pp2d_sim_rollout_pomdp_goals(pp2d_sim* s, pp2d_pomdp* planner, const uint32_t* goals,
+                                 uint32_t n, const uint32_t* starts_xy, const float* beliefs,
+                                 uint32_t max_steps, uint32_t max_depth, uint32_t max_iter,
+                                 uint64_t seed, uint64_t first_episode, pp2d_rollout* out);
 
 #ifdef __cplusplus
 }

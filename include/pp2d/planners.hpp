@@ -367,11 +367,17 @@ class SearchTree {                     // search_tree.h:130-165
 // Not in the reference (one tree per process): many SearchTrees on one
 // planner handle that live across belief callbacks, e.g. one per robot of a
 // fleet, updated and planned together (pp2d_tree_batch_*).  Tree k behaves bit
-// for bit like SearchTree(h, beliefs + k * HW) fed the same calls.
+// for bit like SearchTree(h, beliefs + k * HW) fed the same calls.  With
+// `goals`, tree k plans to goal goals[k] of the planner's goal set
+// (PomdpPathPlanning2d::setGoals), bit for bit like a SearchTree on a planner
+// created with that goal.
 class SearchTreeBatch {
  public:
   SearchTreeBatch(pp2d_pomdp* h, const float* beliefs, uint32_t n) {
     PP2D_CHECK(pp2d_tree_batch_create(h, beliefs, n, &b_));
+  }
+  SearchTreeBatch(pp2d_pomdp* h, const float* beliefs, const std::vector<uint32_t>& goals) {
+    PP2D_CHECK(pp2d_tree_batch_create_goals(h, beliefs, goals.data(), (uint32_t)goals.size(), &b_));
   }
   SearchTreeBatch(const SearchTreeBatch&) = delete;
   SearchTreeBatch& operator=(const SearchTreeBatch&) = delete;
@@ -480,6 +486,47 @@ class PomdpPathPlanning2d : public PathPlanning2dBase {
   }
 
   void resetSearchTreeCallback() { delete search_tree; search_tree = nullptr; }
+
+  // Not in the reference (one goal per node): goals 1..n of this planner's
+  // goal set (DESIGN.md section 7e), which trees of a SearchTreeBatch can plan
+  // to; goal 0 is the launch file's goal.  stage_rewards [n][HW][9] as read
+  // from checkpoint files, or nullptr: generated by the model rule.
+  void setGoals(const std::vector<std::array<uint32_t, 2>>& goals,
+                const float* stage_rewards = nullptr) {
+    PP2D_CHECK(pp2d_pomdp_set_goals(pomdp_, goals.empty() ? nullptr : goals[0].data(),
+                                    (uint32_t)goals.size(), stage_rewards));
+  }
+  // setAlphas of goal g (alphas as the solvers or the checkpoint files give them)
+  void setGoalAlphas(uint32_t g, const std::vector<float>& fib, const std::vector<uint8_t>& fib_acts,
+                     const std::vector<float>& pbvi, const std::vector<uint8_t>& pbvi_acts) {
+    PP2D_CHECK(pp2d_pomdp_set_goal_alphas(pomdp_, g, fib.data(), fib_acts.data(), pbvi.data(),
+                                          pbvi_acts.data(), (uint32_t)pbvi_acts.size()));
+  }
+  // Goals 1..n with their checkpoints: dirs[i] holds what the reference's
+  // save_data writes for a planner with goal goals[i] (the text files; only
+  // model_data_stage_reward of the model is read: the transition and
+  // likelihood tables do not depend on the goal).  belief_set_size vectors
+  // per goal, as for goal 0.
+  bool loadGoalsFromFiles(const std::vector<std::array<uint32_t, 2>>& goals,
+                          const std::vector<std::string>& dirs) {
+    if (dirs.size() != goals.size()) return false;
+    const size_t n = (size_t)map_height * map_width;
+    std::vector<float> sr(goals.size() * n * 9), fib(n * 9), pbvi((size_t)belief_set_size * n);
+    std::vector<uint8_t> fa(9), pa(belief_set_size);
+    for (size_t i = 0; i < goals.size(); ++i) {
+      std::vector<float> one(n * 9);
+      if (!readFloats(dirs[i] + "/model_data_stage_reward", one)) return false;
+      std::copy(one.begin(), one.end(), sr.begin() + i * n * 9);
+    }
+    setGoals(goals, sr.data());
+    for (size_t i = 0; i < goals.size(); ++i) {
+      if (!readFloats(dirs[i] + "/fib_alphas", fib) || !readBytes(dirs[i] + "/fib_actions", fa) ||
+          !readFloats(dirs[i] + "/pbvi_alphas", pbvi) || !readBytes(dirs[i] + "/pbvi_actions", pa))
+        return false;
+      setGoalAlphas((uint32_t)i + 1, fib, fa, pbvi, pa);
+    }
+    return true;
+  }
 
   // saveDataCallback's model half (model_generation_cuda.cu:74-115), "%15.8f".
   bool saveModelDataToFile(const std::string& dir) {

@@ -128,6 +128,15 @@ SIGNATURES = {
     "pp2d_tree_batch_dump": (ctypes.c_int64, [_vp, _u32, _vp, ctypes.c_uint64]),
     "pp2d_sim_rollout_pomdp": (_i, [_vp, _vp, _u32, _vp, _vp, _u32, _u32, _u32, ctypes.c_uint64,
                                     ctypes.c_uint64, ctypes.POINTER(Rollout)]),
+    "pp2d_pomdp_set_goals": (_i, [_vp, _vp, _u32, _vp]),
+    "pp2d_pomdp_goals": (_i, [_vp, ctypes.POINTER(_u32), _vp]),
+    "pp2d_pomdp_goal_reward": (_i, [_vp, _u32, _vp]),
+    "pp2d_pomdp_set_goal_alphas": (_i, [_vp, _u32, _vp, _vp, _vp, _vp, _u32]),
+    "pp2d_pomdp_padding_counters": (_i, [_vp, _vp]),
+    "pp2d_tree_batch_create_goals": (_i, [_vp, _vp, _vp, _u32, ctypes.POINTER(_vp)]),
+    "pp2d_sim_rollout_pomdp_goals": (_i, [_vp, _vp, _vp, _u32, _vp, _vp, _u32, _u32, _u32,
+                                          ctypes.c_uint64, ctypes.c_uint64,
+                                          ctypes.POINTER(Rollout)]),
 }
 
 _lib = None

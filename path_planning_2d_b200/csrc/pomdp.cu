@@ -63,6 +63,7 @@ struct Tree {
   bool dead = false;                  // reference would dereference nullptr
   bool dense = false;                 // root belief not +0 on the dead cells: its
                                       // descendants need the dense inner products
+  int goal = 0;                       // index in the handle's goal set
 };
 
 // search_tree_cuda.cu:251-286
@@ -274,11 +275,13 @@ int refresh_live_cells(pp2d_pomdp* h) {
     PP2D_CUDA(cudaMemcpyAsync(h->d_mp_live + (size_t)k * 16, h->d_mp + (size_t)live[k] * 16,
                               16 * sizeof(float), cudaMemcpyDeviceToDevice, h->stream));
   PP2D_CUDA(cudaStreamSynchronize(h->stream));
-  if (h->have_alphas) {
-    std::vector<float> rows((size_t)h->K * h->ld);
-    for (int k = 0; k < h->K; ++k)
-      memcpy(rows.data() + (size_t)k * h->ld, h->alpha_host.data() + (size_t)live[k] * h->ld,
-             (size_t)h->ld * sizeof(float));
+  if (h->ld > 0) {                               // some goal has alpha vectors
+    const size_t goals = (size_t)h->n_goals + 1;
+    std::vector<float> rows(goals * h->K * h->ld);
+    for (size_t g = 0; g < goals; ++g)
+      for (int k = 0; k < h->K; ++k)
+        memcpy(rows.data() + (g * h->K + k) * h->ld,
+               h->alpha_host.data() + (g * HW + live[k]) * h->ld, (size_t)h->ld * sizeof(float));
     if (h->d_alpha_live) cudaFree(h->d_alpha_live);
     h->d_alpha_live = nullptr;
     PP2D_CUDA(cudaMalloc(&h->d_alpha_live, rows.size() * sizeof(float)));
@@ -304,14 +307,53 @@ namespace {
 
 // The inner dimension of the sequential products of one launch: the live
 // cells, or all cells when some belief involved may be non-zero elsewhere.
-// kinv: cell -> inner row (-1: left out); mp: the likelihood rows of the inner rows.
-struct InnerDim { const int* kidx; int K; const float* alpha; const int* kinv; const float* mp; };
+// kinv: cell -> inner row (-1: left out); mp: the likelihood rows of the inner rows;
+// gstride: floats from one goal's bound matrix to the next.
+struct InnerDim {
+  const int* kidx; int K; const float* alpha; const int* kinv; const float* mp; size_t gstride;
+};
 InnerDim inner_dim(const pp2d_pomdp* h, bool dense) {
   // (a non-finite bound makes 0 * alpha a NaN in the reference: nothing is skipped then)
   if (dense || !h->skip_dead || !h->alphas_finite)
-    return {h->d_kidx_all, h->HW, h->d_alpha, h->d_kidx_all, h->d_mp};
-  return {h->d_kidx, h->K, h->d_alpha_live, h->d_kinv, h->d_mp_live};
+    return {h->d_kidx_all, h->HW, h->d_alpha, h->d_kidx_all, h->d_mp, (size_t)h->HW * h->ld};
+  return {h->d_kidx, h->K, h->d_alpha_live, h->d_kinv, h->d_mp_live, (size_t)h->K * h->ld};
 }
+
+// The entry list of the support, values and bounds launches over beliefs that
+// come in runs of one goal (DESIGN.md section 7e).  Every run but the last is
+// padded to whole tiles of kEvM entries by repeating its last slot, so that a
+// tile holds beliefs of one goal; the goals of the tiles follow the entries
+// (one upload).  A repeated belief adds no inner row to its tile and its values
+// are never read.  With one goal the list is the beliefs' slots, unpadded.
+struct GoalTiles {
+  int* out = nullptr;                 // room() ints
+  int n = 0, goal = -1;
+  std::vector<int> tile_goal;
+  std::vector<std::pair<int, int>> pads;   // (tile, repeated entries in it)
+  // entries + tile goals of `beliefs` beliefs in at most `runs` runs
+  static size_t room(size_t beliefs, size_t runs) {
+    const size_t entries = beliefs + runs * (size_t)(kEvM - 1);
+    return entries + entries / kEvM + 1;
+  }
+  void start(int* buf) { out = buf; n = 0; goal = -1; tile_goal.clear(); pads.clear(); }
+  int add(int slot, int g) {          // -> the entry of this belief
+    if (g != goal) {
+      if (n % kEvM) {
+        const int last = out[n - 1], first = n;
+        while (n % kEvM) out[n++] = last;
+        pads.push_back({first / kEvM, n - first});
+      }
+      goal = g;
+    }
+    if (n % kEvM == 0) tile_goal.push_back(g);
+    out[n] = slot;
+    return n++;
+  }
+  int finish() {                      // -> tiles; their goals now follow the entries
+    std::copy(tile_goal.begin(), tile_goal.end(), out + n);
+    return (int)tile_goal.size();
+  }
+};
 
 // Host threads for the per-tree work of a batch: pp2d_set_host_threads, else
 // PP2D_HOST_THREADS, else the CPUs this process may run on divided by the
@@ -342,31 +384,52 @@ double now_s() {
   return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count();
 }
 
-// Evaluate the beliefs in `slots`: per belief 4 floats {upper, lower, packed
-// indices, 0} into host `out` (B4, B5).
-int evaluate_slots(pp2d_pomdp* h, const std::vector<int>& slots, float* out, bool dense) {
+// Evaluate the beliefs in `slots` against the bounds of their goals (`goals`
+// per belief, NULL: goal 0): per belief 4 floats {upper, lower, packed
+// indices, 0} into host `out` (B4, B5).  The beliefs are evaluated goal by
+// goal (GoalTiles); every belief walks all inner rows, so its bits do not
+// depend on which others share its tile.
+int evaluate_slots(pp2d_pomdp* h, const std::vector<int>& slots, const int* goals, float* out,
+                   bool dense) {
   const int n = (int)slots.size();
   if (n == 0) return PP2D_OK;
-  PP2D_TRY(h->d_slots.ensure(n));
-  PP2D_TRY(h->d_vals.ensure((size_t)n * h->ncol));
-  PP2D_TRY(h->d_out.ensure((size_t)n * 4));
-  PP2D_CUDA(cudaMemcpyAsync(h->d_slots.p, slots.data(), n * sizeof(int),
+  std::vector<int> order(n);
+  for (int i = 0; i < n; ++i) order[i] = i;
+  if (goals)
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return goals[a] < goals[b]; });
+  std::vector<int> list(GoalTiles::room(n, (size_t)h->n_goals + 1)), pos(n);
+  GoalTiles gt;
+  gt.start(list.data());
+  for (int j = 0; j < n; ++j) pos[order[j]] = gt.add(slots[order[j]], goals ? goals[order[j]] : 0);
+  const int np = gt.n, ntiles = gt.finish();
+  PP2D_TRY(h->d_slots.ensure(np + ntiles));
+  PP2D_TRY(h->d_vals.ensure((size_t)np * h->ncol));
+  PP2D_TRY(h->d_out.ensure((size_t)np * 4));
+  PP2D_CUDA(cudaMemcpyAsync(h->d_slots.p, list.data(), (np + ntiles) * sizeof(int),
                             cudaMemcpyHostToDevice, h->stream));
-  dim3 grid((n + kEvM - 1) / kEvM, (h->ncol + kEvN - 1) / kEvN);
+  dim3 grid(ntiles, (h->ncol + kEvN - 1) / kEvN);
   const InnerDim in = inner_dim(h, dense);
   pomdp_values_kernel<false><<<grid, 256, 0, h->stream>>>(
-      in.K, in.kidx, h->HW, h->ld, h->ncol, h->d_slots.p, n, h->d_bel, in.alpha,
-      h->d_vals.p, nullptr, nullptr, nullptr, 0);
-  h->work_rows += (uint64_t)in.K * (uint64_t)n;
+      in.K, in.kidx, h->HW, h->ld, h->ncol, h->d_slots.p, np, h->d_bel, in.alpha,
+      h->d_vals.p, nullptr, nullptr, nullptr, 0, h->d_slots.p + np, in.gstride);
+  h->work_rows += (uint64_t)in.K * (uint64_t)np;
+  h->pad_entries += (uint64_t)(np - n);
+  h->pad_rows += (uint64_t)in.K * (uint64_t)(np - n);
   count_launch();
   PP2D_CUDA(cudaGetLastError());
-  pomdp_bounds_kernel<<<(n + 3) / 4, 128, 0, h->stream>>>(
-      n, h->ncol, h->n_pbvi, h->d_vals.p, h->d_out.p);
+  pomdp_bounds_kernel<<<(np + 3) / 4, 128, 0, h->stream>>>(
+      np, h->ncol, h->n_pbvi, h->d_vals.p, h->d_out.p);
   count_launch();
   PP2D_CUDA(cudaGetLastError());
-  PP2D_CUDA(cudaMemcpyAsync(out, h->d_out.p, (size_t)n * 4 * sizeof(float),
+  bool in_place = np == n;                       // entry i is belief i
+  for (int i = 0; i < n && in_place; ++i) in_place = pos[i] == i;
+  std::vector<float> res(in_place ? 0 : (size_t)np * 4);
+  float* dst = in_place ? out : res.data();
+  PP2D_CUDA(cudaMemcpyAsync(dst, h->d_out.p, (size_t)np * 4 * sizeof(float),
                             cudaMemcpyDeviceToHost, h->stream));
   PP2D_CUDA(cudaStreamSynchronize(h->stream));
+  if (!in_place)
+    for (int i = 0; i < n; ++i) memcpy(out + (size_t)i * 4, dst + (size_t)pos[i] * 4, 4 * sizeof(float));
   return PP2D_OK;
 }
 
@@ -447,7 +510,9 @@ int make_roots(pp2d_pomdp* h, std::vector<Tree*>& trees, const float* beliefs,
   count_launch();
   PP2D_CUDA(cudaGetLastError());
   std::vector<float> ev((size_t)n * 4);
-  PP2D_TRY(evaluate_slots(h, slots, ev.data(), any_dense));
+  std::vector<int> goals(n);
+  for (int i = 0; i < n; ++i) goals[i] = trees[i]->goal;
+  PP2D_TRY(evaluate_slots(h, slots, goals.data(), ev.data(), any_dense));
   for (int i = 0; i < n; ++i) {
     Tree& t = *trees[i];
     t.v.emplace_back();
@@ -504,12 +569,17 @@ struct RoundCtx {
   int n = 0, nk = 0;
   bool dense = false;                // some tree of this round needs the dense products
   PinnedBuf<int> slots, kslots, kgroup;
+  PinnedBuf<int> vlist;              // entries of the values launches (GoalTiles), tile goals
+  std::vector<int> vpos;             // child k -> its entry
+  GoalTiles tiles;
+  PinnedBuf<int> tcount;             // rows per tile, read back when a tile has padding
   PinnedBuf<float> draws, rewards, ev;
   PinnedBuf<BayesItem> items;
   PinnedBuf<uint8_t> obs;
   std::vector<int> first;
   std::vector<Child> kids;
-  DevBuf<int> d_jobslots, d_kslots, d_kgroup;
+  bool tiled_pads = false;           // c.tcount holds this round's rows per tile
+  DevBuf<int> d_jobslots, d_vlist, d_kgroup;
   DevBuf<float> d_pred;              // [HW][ngp] predictions of the Q nodes of a round
   DevBuf<float> d_prefix, d_draws, d_rew, d_sums, d_vals, d_out;
   DevBuf<uint8_t> d_obs;
@@ -525,9 +595,10 @@ struct RoundCtx {
                                      // values launch and the host can move on
   ~RoundCtx() {
     slots.release(); kslots.release(); kgroup.release(); draws.release();
+    vlist.release(); tcount.release();
     rewards.release(); d_kgroup.release(); d_pred.release();
     ev.release(); items.release(); obs.release();
-    d_jobslots.release(); d_kslots.release(); d_prefix.release();
+    d_jobslots.release(); d_vlist.release(); d_prefix.release();
     d_draws.release(); d_rew.release(); d_sums.release(); d_vals.release(); d_out.release();
     d_obs.release(); d_items.release(); d_tlist.release(); d_tcount.release(); d_torder.release(); d_tmask.release();
     if (e1) cudaEventDestroy(e1);
@@ -578,23 +649,24 @@ int round_stage1(pp2d_pomdp* h, RoundCtx& c, const std::vector<Tree*>& trees) {
   if (n == 0) return PP2D_OK;
   const int HW = h->HW;
   const size_t nd = (size_t)n * kActions * kSamples;
-  PP2D_TRY(c.slots.ensure(n));
+  PP2D_TRY(c.slots.ensure(2 * (size_t)n));     // slots, then goals
   PP2D_TRY(c.draws.ensure(nd));
   PP2D_TRY(c.obs.ensure(nd));
   PP2D_TRY(c.rewards.ensure((size_t)n * kActions));
 #pragma omp parallel for schedule(static) num_threads(host_threads()) if (n >= 64)
   for (int i = 0; i < n; ++i) {
     c.slots.p[i] = c.jobs[i].t->v[c.jobs[i].v].slot;
+    c.slots.p[n + i] = c.jobs[i].t->goal;
     float* d = c.draws.p + (size_t)i * kActions * kSamples;
     for (int k = 0; k < kActions * kSamples; ++k)
       d[k] = (float)c.jobs[i].t->rng.next() / ((float)2147483647 + 1.0f);
   }
-  PP2D_TRY(c.d_jobslots.ensure(n));
+  PP2D_TRY(c.d_jobslots.ensure(2 * (size_t)n));
   PP2D_TRY(c.d_prefix.ensure((size_t)n * HW));
   PP2D_TRY(c.d_draws.ensure(nd));
   PP2D_TRY(c.d_obs.ensure(nd));
   PP2D_TRY(c.d_rew.ensure((size_t)n * kActions));
-  PP2D_CUDA(cudaMemcpyAsync(c.d_jobslots.p, c.slots.p, n * sizeof(int),
+  PP2D_CUDA(cudaMemcpyAsync(c.d_jobslots.p, c.slots.p, 2 * (size_t)n * sizeof(int),
                             cudaMemcpyHostToDevice, c.stream_hi));
   PP2D_CUDA(cudaMemcpyAsync(c.d_draws.p, c.draws.p, nd * sizeof(float),
                             cudaMemcpyHostToDevice, c.stream_hi));
@@ -602,7 +674,8 @@ int round_stage1(pp2d_pomdp* h, RoundCtx& c, const std::vector<Tree*>& trees) {
   // sampling (which needs the prefix sums)
   const InnerDim in = inner_dim(h, c.dense);
   pomdp_expand_kernel<<<(n + 3) / 4 + (n * 3 + 3) / 4, 128, 0, c.stream_hi>>>(
-      HW, in.K, in.kidx, c.d_jobslots.p, n, h->d_bel, h->d_sr, c.d_prefix.p, c.d_rew.p);
+      HW, in.K, in.kidx, c.d_jobslots.p, c.d_jobslots.p + n, n, h->d_bel, h->d_sr, c.d_prefix.p,
+      c.d_rew.p);
   count_launch();
   const int nt = (int)nd;
   pomdp_sample_kernel<<<(nt + 127) / 128, 128, 0, c.stream_hi>>>(
@@ -645,7 +718,6 @@ int round_stage2(pp2d_pomdp* h, RoundCtx& c) {
   PP2D_TRY(c.kslots.ensure(nk));
   PP2D_TRY(c.items.ensure(nk));
   PP2D_TRY(c.kgroup.ensure(nk));
-  PP2D_TRY(c.ev.ensure((size_t)nk * 4));
   for (int k = 0; k < nk; ++k) PP2D_TRY(alloc_slot(h, &c.kslots.p[k]));
   c.kids.resize(nk);
 #pragma omp parallel for schedule(static) num_threads(host_threads()) if (n >= 64)
@@ -664,16 +736,29 @@ int round_stage2(pp2d_pomdp* h, RoundCtx& c) {
       }
     }
   }
+  // the children in runs of one goal (the jobs are in goal order, see
+  // plan_trees), padded to whole tiles per goal
+  size_t runs = n ? 1 : 0;
+  for (int i = 1; i < n; ++i) runs += c.jobs[i].t->goal != c.jobs[i - 1].t->goal;
+  PP2D_TRY(c.vlist.ensure(GoalTiles::room(nk, runs)));
+  c.vpos.resize(nk);
+  c.tiles.start(c.vlist.p);
+  for (int i = 0; i < n; ++i)
+    for (int k = c.first[i]; k < c.first[i + 1]; ++k)
+      c.vpos[k] = c.tiles.add(c.kslots.p[k], c.jobs[i].t->goal);
+  const int np = c.tiles.n, ntiles = c.tiles.finish();
+  PP2D_TRY(c.ev.ensure((size_t)np * 4));
   const int ng = n * kActions;
   PP2D_TRY(c.d_items.ensure(nk));
-  PP2D_TRY(c.d_kslots.ensure(nk));
+  PP2D_TRY(c.d_vlist.ensure((size_t)np + ntiles));
   PP2D_TRY(c.d_sums.ensure(nk));
-  PP2D_TRY(c.d_vals.ensure((size_t)nk * h->ncol));
-  PP2D_TRY(c.d_out.ensure((size_t)nk * 4));
+  PP2D_TRY(c.d_vals.ensure((size_t)np * h->ncol));
+  PP2D_TRY(c.d_out.ensure((size_t)np * 4));
   PP2D_CUDA(cudaMemcpyAsync(c.d_items.p, c.items.p, nk * sizeof(BayesItem),
                             cudaMemcpyHostToDevice, c.stream));
-  PP2D_CUDA(cudaMemcpyAsync(c.d_kslots.p, c.kslots.p, nk * sizeof(int),
+  PP2D_CUDA(cudaMemcpyAsync(c.d_vlist.p, c.vlist.p, ((size_t)np + ntiles) * sizeof(int),
                             cudaMemcpyHostToDevice, c.stream));
+  const int* d_tgoal = c.d_vlist.p + np;
   const int ngp = (ng + 31) / 32 * 32;
   PP2D_TRY(c.d_kgroup.ensure(nk));
   PP2D_TRY(c.d_pred.ensure((size_t)HW * ngp));
@@ -695,8 +780,9 @@ int round_stage2(pp2d_pomdp* h, RoundCtx& c) {
                                                          c.d_items.p, c.d_kgroup.p, nk,
                                                          c.d_pred.p, c.d_sums.p, h->d_bel);
   count_launch();
-  dim3 vgrid((nk + kEvM - 1) / kEvM, (h->ncol + kEvN - 1) / kEvN);
-  if (h->tile_support && h->alphas_finite) {
+  dim3 vgrid(ntiles, (h->ncol + kEvN - 1) / kEvN);
+  const bool tiled = h->tile_support && h->alphas_finite;
+  if (tiled) {
     // the inner rows each tile of kEvM children really needs (exact, see
     // pomdp_values_kernel<TILED>)
     const int mstride = (in.K + 31) / 32;
@@ -705,10 +791,10 @@ int round_stage2(pp2d_pomdp* h, RoundCtx& c) {
     PP2D_TRY(c.d_tmask.ensure((size_t)vgrid.x * mstride));
     dim3 fgrid(vgrid.x, (in.K + 255) / 256);
     pomdp_support_flags_kernel<<<fgrid, 256, 0, c.stream>>>(
-        HW, in.K, in.kidx, c.d_kslots.p, nk, h->d_bel, c.d_tmask.p, mstride);
+        HW, in.K, in.kidx, c.d_vlist.p, np, h->d_bel, c.d_tmask.p, mstride);
     count_launch();
     pomdp_support_list_kernel<<<vgrid.x, 256, 0, c.stream>>>(in.K, in.kidx, c.d_tmask.p, mstride,
-                                                             c.d_tlist.p, c.d_tcount.p, nk,
+                                                             c.d_tlist.p, c.d_tcount.p, np,
                                                              h->d_work);
     count_launch();
     PP2D_TRY(c.d_torder.ensure(vgrid.x));
@@ -716,21 +802,34 @@ int round_stage2(pp2d_pomdp* h, RoundCtx& c) {
         (int)vgrid.x, c.d_tcount.p, c.d_torder.p);
     count_launch();
     pomdp_values_kernel<true><<<dim3(vgrid.y, vgrid.x), 256, 0, c.stream>>>(
-        in.K, in.kidx, h->HW, h->ld, h->ncol, c.d_kslots.p, nk, h->d_bel, in.alpha, c.d_vals.p,
-        c.d_tlist.p, c.d_tcount.p, c.d_torder.p, in.K);
+        in.K, in.kidx, h->HW, h->ld, h->ncol, c.d_vlist.p, np, h->d_bel, in.alpha, c.d_vals.p,
+        c.d_tlist.p, c.d_tcount.p, c.d_torder.p, in.K, d_tgoal, in.gstride);
   } else {
     pomdp_values_kernel<false><<<vgrid, 256, 0, c.stream>>>(
-        in.K, in.kidx, h->HW, h->ld, h->ncol, c.d_kslots.p, nk, h->d_bel, in.alpha, c.d_vals.p,
-        nullptr, nullptr, nullptr, 0);
-    h->work_rows += (uint64_t)in.K * (uint64_t)nk;
+        in.K, in.kidx, h->HW, h->ld, h->ncol, c.d_vlist.p, np, h->d_bel, in.alpha, c.d_vals.p,
+        nullptr, nullptr, nullptr, 0, d_tgoal, in.gstride);
+    h->work_rows += (uint64_t)in.K * (uint64_t)np;
   }
   count_launch();
-  pomdp_bounds_kernel<<<(nk + 3) / 4, 128, 0, c.stream>>>(nk, h->ncol, h->n_pbvi,
+  pomdp_bounds_kernel<<<(np + 3) / 4, 128, 0, c.stream>>>(np, h->ncol, h->n_pbvi,
                                                                c.d_vals.p, c.d_out.p);
   count_launch();
   PP2D_CUDA(cudaGetLastError());
-  PP2D_CUDA(cudaMemcpyAsync(c.ev.p, c.d_out.p, (size_t)nk * 4 * sizeof(float),
+  PP2D_CUDA(cudaMemcpyAsync(c.ev.p, c.d_out.p, (size_t)np * 4 * sizeof(float),
                             cudaMemcpyDeviceToHost, c.stream));
+  // the work spent on padding (pp2d_pomdp_padding_counters): rows of the
+  // padded tiles, read back with the bounds
+  h->pad_entries += (uint64_t)(np - nk);
+  if (np != nk) {
+    if (tiled) {
+      PP2D_TRY(c.tcount.ensure(ntiles));
+      PP2D_CUDA(cudaMemcpyAsync(c.tcount.p, c.d_tcount.p, ntiles * sizeof(int),
+                                cudaMemcpyDeviceToHost, c.stream));
+    } else {
+      h->pad_rows += (uint64_t)in.K * (uint64_t)(np - nk);
+    }
+  }
+  c.tiled_pads = tiled && np != nk;
   PP2D_CUDA(cudaEventRecord(c.e2, c.stream));
   h->t_phase[2] += now_s() - t0;                 // host: children lists, enqueue
   return PP2D_OK;
@@ -768,7 +867,7 @@ int round_stage3(pp2d_pomdp* h, RoundCtx& c) {
         t.v.emplace_back();
         const int ci = (int)t.v.size() - 1;
         init_vnode(t.v[ci], c.kslots.p[kpos], c.kids[kpos].z, c.kids[kpos].w, qi,
-                   c.ev.p + (size_t)kpos * 4, ci);
+                   c.ev.p + (size_t)c.vpos[kpos] * 4, ci);
         t.q[qi].children.push_back(ci);
         ++kpos;
       }
@@ -786,6 +885,9 @@ int round_stage3(pp2d_pomdp* h, RoundCtx& c) {
     t.expansions++;
   }
   h->n_vnodes += (uint64_t)c.nk;
+  if (c.tiled_pads)
+    for (const auto& p : c.tiles.pads) h->pad_rows += (uint64_t)c.tcount.p[p.first] * p.second;
+  c.tiled_pads = false;
   c.n = 0;                                       // this round is absorbed
   h->t_phase[4] += now_s() - t0;                 // host: tree bookkeeping
   return PP2D_OK;
@@ -864,6 +966,7 @@ void reroot(Tree& t, int root_q, int root_v, int new_slot, const float* ev,
   // Rebuild the node arrays from the kept subtree: a long-running planner
   // re-roots once per belief message, and dropped nodes must not accumulate.
   Tree fresh;
+  fresh.goal = t.goal;
   fresh.rng = t.rng;
   fresh.expansions = t.expansions;
   fresh.dense = t.dense;
@@ -1024,6 +1127,10 @@ int pp2d_pomdp_create(uint32_t height, uint32_t width, const uint8_t* map,
   if (!h) return fail(PP2D_ERR_INVALID, "out of host memory");
   h->H = (int)height; h->W = (int)width; h->HW = h->H * h->W;
   h->gx = (int)goal_x; h->gy = (int)goal_y; h->gamma = gamma;
+  h->map_host.assign(map, map + (size_t)h->HW);
+  h->goal_xy = {goal_x, goal_y};
+  h->goal_alphas = {0};
+  h->goal_finite = {1};
   int rc = [&]() -> int {
     const size_t n = (size_t)h->HW;
     PP2D_CUDA(cudaMalloc(&h->d_map, n));
@@ -1115,36 +1222,155 @@ int pp2d_pomdp_sampling_uniforms(pp2d_pomdp* h, float* out100) {
 int pp2d_pomdp_set_alphas(pp2d_pomdp* h, const float* fib_alphas,
                           const uint8_t* fib_actions, const float* pbvi_alphas,
                           const uint8_t* pbvi_actions, uint32_t n_pbvi) {
+  return pp2d_pomdp_set_goal_alphas(h, 0, fib_alphas, fib_actions, pbvi_alphas, pbvi_actions,
+                                    n_pbvi);
+}
+
+int pp2d_pomdp_set_goal_alphas(pp2d_pomdp* h, uint32_t g, const float* fib_alphas,
+                               const uint8_t* fib_actions, const float* pbvi_alphas,
+                               const uint8_t* pbvi_actions, uint32_t n_pbvi) {
   if (!h || !fib_alphas) return fail(PP2D_ERR_INVALID, "NULL argument");
   if (n_pbvi > 0 && !pbvi_alphas) return fail(PP2D_ERR_INVALID, "pbvi_alphas is NULL");
+  if (g > (uint32_t)h->n_goals)
+    return fail(PP2D_ERR_INVALID, "pp2d_pomdp_set_goal_alphas: goal %u of a set of %d", g,
+                h->n_goals + 1);
+  // All goals use one PBVI count (the bound matrices share ld and ncol).
+  bool others = false;
+  for (int j = 0; j <= h->n_goals; ++j) {
+    if (j == (int)g || !h->goal_alphas[j]) continue;
+    others = true;
+    if ((uint32_t)h->n_pbvi != n_pbvi)
+      return fail(PP2D_ERR_INVALID,
+                  "goal %u: %u PBVI vectors, but goal %d holds %d (the goals of a handle share "
+                  "one count)", g, n_pbvi, j, h->n_pbvi);
+  }
   const int ncol = kColPbvi + (int)n_pbvi;
   const int ld = (ncol + kEvN - 1) / kEvN * kEvN;   // zero-padded to whole column tiles
-  const size_t HW = (size_t)h->HW;
-  std::vector<float> mat(HW * ld, 0.0f);
+  const size_t HW = (size_t)h->HW, goals = (size_t)h->n_goals + 1;
+  // (a new ld only while no other goal holds bounds: their matrices are zero)
+  if (!others && ld != h->ld) h->alpha_host.assign(goals * HW * ld, 0.0f);
+  float* mat = h->alpha_host.data() + (size_t)g * HW * ld;
   bool finite = true;
   for (size_t s = 0; s < HW; ++s) {
-    float* row = mat.data() + s * ld;
+    float* row = mat + s * ld;
+    std::fill(row, row + ld, 0.0f);
     memcpy(row + kColFib, fib_alphas + s * 9, 9 * sizeof(float));
     for (uint32_t i = 0; i < n_pbvi; ++i) row[kColPbvi + i] = pbvi_alphas[(size_t)i * HW + s];
     for (int j = 0; j < ncol; ++j) finite = finite && std::isfinite(row[j]);
   }
+  h->goal_alphas[g] = 1;
+  h->goal_finite[g] = finite;
   // The exact skipping of zero belief entries (dead cells, per-tile inner rows)
-  // needs 0 * alpha == 0.
-  h->alphas_finite = finite;
+  // needs 0 * alpha == 0, for every goal of a launch.
+  h->alphas_finite = true;
+  for (uint8_t f : h->goal_finite) h->alphas_finite = h->alphas_finite && f;
   if (h->d_alpha) cudaFree(h->d_alpha);
   h->d_alpha = nullptr;
-  PP2D_CUDA(cudaMalloc(&h->d_alpha, mat.size() * sizeof(float)));
-  PP2D_CUDA(cudaMemcpy(h->d_alpha, mat.data(), mat.size() * sizeof(float),
+  PP2D_CUDA(cudaMalloc(&h->d_alpha, h->alpha_host.size() * sizeof(float)));
+  PP2D_CUDA(cudaMemcpy(h->d_alpha, h->alpha_host.data(), h->alpha_host.size() * sizeof(float),
                        cudaMemcpyHostToDevice));
   h->ld = ld; h->ncol = ncol; h->n_pbvi = (int)n_pbvi;
-  h->alpha_host.swap(mat);
-  h->have_alphas = true;
   PP2D_TRY(refresh_live_cells(h));
-  h->fib_actions.assign(9, 0);
-  for (int a = 0; a < 9; ++a) h->fib_actions[a] = fib_actions ? fib_actions[a] : (uint8_t)a;
-  h->pbvi_actions.assign(n_pbvi, 0);
-  if (pbvi_actions) memcpy(h->pbvi_actions.data(), pbvi_actions, n_pbvi);
-  h->have_alphas = true;
+  if (g == 0) {
+    h->fib_actions.assign(9, 0);
+    for (int a = 0; a < 9; ++a) h->fib_actions[a] = fib_actions ? fib_actions[a] : (uint8_t)a;
+    h->pbvi_actions.assign(n_pbvi, 0);
+    if (pbvi_actions) memcpy(h->pbvi_actions.data(), pbvi_actions, n_pbvi);
+    h->have_alphas = true;
+  }
+  return PP2D_OK;
+}
+
+int pp2d_pomdp_set_goals(pp2d_pomdp* h, const uint32_t* goals_xy, uint32_t n,
+                         const float* stage_rewards) {
+  if (!h) return fail(PP2D_ERR_INVALID, "handle is NULL");
+  if (n > 0 && !goals_xy) return fail(PP2D_ERR_INVALID, "goals_xy is NULL");
+  if (n > (1u << 20)) return fail(PP2D_ERR_INVALID, "pp2d_pomdp_set_goals: %u goals", n);
+  for (uint32_t i = 0; i < n; ++i) {
+    const uint32_t x = goals_xy[2 * (size_t)i], y = goals_xy[2 * (size_t)i + 1];
+    if (x >= (uint32_t)h->W || y >= (uint32_t)h->H)
+      return fail(PP2D_ERR_INVALID, "pp2d_pomdp_set_goals: goal %u (%u %u) outside the %dx%d map",
+                  i + 1, x, y, h->W, h->H);
+    if (h->map_host[(size_t)y * h->W + x] > 0)
+      return fail(PP2D_ERR_GOAL_OCCUPIED,
+                  "pp2d_pomdp_set_goals: goal %u (%u %u) is at an occupied cell", i + 1, x, y);
+  }
+  // as pp2d_pomdp_set_model_tables: trees hold rewards and bounds of their goals
+  if (h->d_bel && h->free_slots.count() != (size_t)h->cap)
+    return fail(PP2D_ERR_STATE, "pp2d_pomdp_set_goals: destroy the search trees of this "
+                                "handle first (%zu beliefs are resident)",
+                (size_t)h->cap - h->free_slots.count());
+  PP2D_CUDA(cudaDeviceSynchronize());
+  const size_t HW = (size_t)h->HW, tab = HW * 9;
+  float* sr = nullptr;
+  PP2D_CUDA(cudaMalloc(&sr, (n + 1) * tab * sizeof(float)));
+  int rc = [&]() -> int {
+    PP2D_CUDA(cudaMemcpy(sr, h->d_sr, tab * sizeof(float), cudaMemcpyDeviceToDevice));
+    if (stage_rewards) {
+      PP2D_CUDA(cudaMemcpy(sr + tab, stage_rewards, n * tab * sizeof(float),
+                           cudaMemcpyHostToDevice));
+      return PP2D_OK;
+    }
+    if (n == 0) return PP2D_OK;
+    // the model rule of pp2d_pomdp_create per goal; its transition and
+    // likelihood tables go to scratch (the handle's may have been replaced)
+    float *tp = nullptr, *mp = nullptr;
+    int r = [&]() -> int {
+      PP2D_CUDA(cudaMalloc(&tp, HW * 81 * sizeof(float)));
+      PP2D_CUDA(cudaMalloc(&mp, HW * 16 * sizeof(float)));
+      dim3 grid((h->W + 63) / 64, h->H);
+      for (uint32_t i = 0; i < n; ++i) {
+        pomdp_model_kernel<<<grid, 64>>>(h->H, h->W, (int)goals_xy[2 * (size_t)i],
+                                         (int)goals_xy[2 * (size_t)i + 1], h->d_map, tp, mp,
+                                         sr + (i + 1) * tab);
+        count_launch();
+      }
+      PP2D_CUDA(cudaGetLastError());
+      PP2D_CUDA(cudaDeviceSynchronize());
+      return PP2D_OK;
+    }();
+    cudaFree(tp);
+    cudaFree(mp);
+    return r;
+  }();
+  if (rc != PP2D_OK) { cudaFree(sr); return rc; }
+  cudaFree(h->d_sr);
+  h->d_sr = sr;
+  h->n_goals = (int)n;
+  h->goal_xy.assign({(uint32_t)h->gx, (uint32_t)h->gy});
+  if (n) h->goal_xy.insert(h->goal_xy.end(), goals_xy, goals_xy + 2 * (size_t)n);
+  h->goal_alphas.resize(n + 1);
+  h->goal_finite.resize(n + 1);
+  std::fill(h->goal_alphas.begin() + 1, h->goal_alphas.end(), 0);
+  std::fill(h->goal_finite.begin() + 1, h->goal_finite.end(), 1);
+  h->alphas_finite = h->goal_finite[0];
+  if (h->ld == 0) return PP2D_OK;                  // no goal has alpha vectors
+  // goal 0's bounds stay, the new goals have none (zero matrices)
+  h->alpha_host.resize((n + 1) * HW * h->ld);
+  std::fill(h->alpha_host.begin() + HW * h->ld, h->alpha_host.end(), 0.0f);
+  if (h->d_alpha) cudaFree(h->d_alpha);
+  h->d_alpha = nullptr;
+  PP2D_CUDA(cudaMalloc(&h->d_alpha, h->alpha_host.size() * sizeof(float)));
+  PP2D_CUDA(cudaMemcpy(h->d_alpha, h->alpha_host.data(), h->alpha_host.size() * sizeof(float),
+                       cudaMemcpyHostToDevice));
+  return refresh_live_cells(h);
+}
+
+int pp2d_pomdp_goals(pp2d_pomdp* h, uint32_t* count, uint32_t* goals_xy) {
+  if (!h) return fail(PP2D_ERR_INVALID, "handle is NULL");
+  if (count) *count = (uint32_t)h->n_goals + 1;
+  if (goals_xy) memcpy(goals_xy, h->goal_xy.data(), h->goal_xy.size() * sizeof(uint32_t));
+  return PP2D_OK;
+}
+
+int pp2d_pomdp_goal_reward(pp2d_pomdp* h, uint32_t g, float* stage_reward) {
+  if (!h || !stage_reward) return fail(PP2D_ERR_INVALID, "NULL argument");
+  if (g > (uint32_t)h->n_goals)
+    return fail(PP2D_ERR_INVALID, "pp2d_pomdp_goal_reward: goal %u of a set of %d", g,
+                h->n_goals + 1);
+  const size_t tab = (size_t)h->HW * 9;
+  PP2D_CUDA(cudaMemcpy(stage_reward, h->d_sr + g * tab, tab * sizeof(float),
+                       cudaMemcpyDeviceToHost));
   return PP2D_OK;
 }
 
@@ -1220,6 +1446,13 @@ int pp2d_pomdp_work_counters(pp2d_pomdp* h, uint64_t out[3]) {
   out[0] = h->n_vnodes;
   out[1] = h->n_bayes;
   out[2] = h->work_rows + (uint64_t)dev;
+  return PP2D_OK;
+}
+
+int pp2d_pomdp_padding_counters(pp2d_pomdp* h, uint64_t out[2]) {
+  if (!h || !out) return fail(PP2D_ERR_INVALID, "NULL argument");
+  out[0] = h->pad_entries;
+  out[1] = h->pad_rows;
   return PP2D_OK;
 }
 
@@ -1322,7 +1555,7 @@ int pp2d_pomdp_evaluate(pp2d_pomdp* h, const float* beliefs, uint32_t n,
     pomdp_values_kernel<false><<<vgrid, 256, 0, h->stream>>>(in.K, in.kidx, h->HW, h->ld,
                                                              h->ncol, h->d_slots.p, n, h->d_bel,
                                                              in.alpha, h->d_vals.p, nullptr,
-                                                             nullptr, nullptr, 0);
+                                                             nullptr, nullptr, 0, nullptr, 0);
     h->work_rows += (uint64_t)in.K * (uint64_t)n;
     count_launch();
     pomdp_bounds_kernel<<<(n + 3) / 4, 128, 0, h->stream>>>(n, h->ncol, h->n_pbvi,
@@ -1508,7 +1741,7 @@ int pp2d_tree_update(pp2d_tree* tt, uint8_t a, uint8_t z) {
                                 h->stream));
       PP2D_TRY(normalize_slots(h, 1, nullptr));
       std::vector<int> s1{new_slot};
-      return evaluate_slots(h, s1, ev, t.dense);
+      return evaluate_slots(h, s1, nullptr, ev, t.dense);
     }();
     if (rc != PP2D_OK) { h->free_slots.put(new_slot); return rc; }
     h->n_vnodes++;
@@ -1580,16 +1813,33 @@ extern "C" {
 
 int pp2d_tree_batch_create(pp2d_pomdp* h, const float* beliefs, uint32_t n,
                            pp2d_tree_batch** out) {
+  return pp2d_tree_batch_create_goals(h, beliefs, nullptr, n, out);
+}
+
+int pp2d_tree_batch_create_goals(pp2d_pomdp* h, const float* beliefs, const uint32_t* goals,
+                                 uint32_t n, pp2d_tree_batch** out) {
   if (!h || !beliefs || !out) return fail(PP2D_ERR_INVALID, "NULL argument");
   *out = nullptr;
-  if (!h->have_alphas) return fail(PP2D_ERR_STATE, "pp2d_pomdp_set_alphas not called");
+  if (!goals && !h->have_alphas) return fail(PP2D_ERR_STATE, "pp2d_pomdp_set_alphas not called");
+  for (uint32_t k = 0; goals && k < n; ++k)
+    if (goals[k] > (uint32_t)h->n_goals)
+      return fail(PP2D_ERR_INVALID, "pp2d_tree_batch_create_goals: tree %u names goal %u of a "
+                                    "set of %d", k, goals[k], h->n_goals + 1);
+  for (uint32_t k = 0; goals && k < n; ++k)
+    if (!h->goal_alphas[goals[k]])
+      return fail(PP2D_ERR_STATE, "pp2d_tree_batch_create_goals: tree %u: goal %u has no alpha "
+                                  "vectors", k, goals[k]);
   pp2d_tree_batch* b = new (std::nothrow) pp2d_tree_batch;
   if (!b) return fail(PP2D_ERR_INVALID, "out of host memory");
   b->h = h;
   int rc = [&]() -> int {
     b->trees.resize(n);
     std::vector<Tree*> trees(n);
-    for (uint32_t i = 0; i < n; ++i) { b->trees[i].rng.seed(1); trees[i] = &b->trees[i]; }
+    for (uint32_t i = 0; i < n; ++i) {
+      b->trees[i].rng.seed(1);
+      b->trees[i].goal = goals ? (int)goals[i] : 0;
+      trees[i] = &b->trees[i];
+    }
     if (n == 0) return PP2D_OK;
     PP2D_TRY(pool_reserve(h, (size_t)h->cap - h->free_slots.count() + n));
     return make_roots(h, trees, beliefs);
@@ -1639,18 +1889,20 @@ int pp2d_tree_batch_update(pp2d_tree_batch* b, const uint32_t* trees, uint32_t n
   if (nm) {
     PP2D_TRY(pool_reserve(h, (size_t)h->cap - h->free_slots.count() + nm));
     std::vector<BayesItem> items(nm);
+    std::vector<int> goals(nm);
     bool dense = false;
     for (size_t j = 0; j < nm; ++j) {
       const uint32_t i = miss[j];
       const Tree& t = b->trees[trees[i]];
       PP2D_TRY(alloc_slot(h, &slots[j]));            // (reserved: cannot fail)
       items[j] = BayesItem{t.v[t.root].slot, slots[j], actions[i], observations[i]};
+      goals[j] = t.goal;
       dense = dense || t.dense;
     }
     int rc = [&]() -> int {
       PP2D_TRY(launch_bayes(h, items));
       PP2D_TRY(launch_normalize(h, slots));
-      return evaluate_slots(h, slots, ev.data(), dense);
+      return evaluate_slots(h, slots, goals.data(), ev.data(), dense);
     }();
     if (rc != PP2D_OK) {
       for (int s : slots) h->free_slots.put(s);
@@ -1695,16 +1947,19 @@ int pp2d_tree_batch_plan(pp2d_tree_batch* b, const uint32_t* trees, uint32_t n,
   if ((size_t)h->cap < want) PP2D_TRY(pool_reserve(h, want));
   std::vector<Tree*> list(n);
   for (uint32_t i = 0; i < n; ++i) list[i] = &b->trees[trees[i]];
-  // in the order of the roots' modes, as pp2d_pomdp_plan_batch orders its queries
+  // goal by goal (a values tile holds children of one goal, DESIGN.md section
+  // 7e), within a goal in the order of the roots' modes, as
+  // pp2d_pomdp_plan_batch orders its queries, or else as listed
   const bool sorted = h->sort_queries && n >= 2 * (uint32_t)kEvM;
-  if (sorted) {
-    std::vector<uint32_t> key;
-    PP2D_TRY(root_mode_keys(h, list, key));
-    std::vector<int> order(n);
-    for (uint32_t i = 0; i < n; ++i) order[i] = (int)i;
-    std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return key[x] < key[y]; });
-    for (uint32_t i = 0; i < n; ++i) list[i] = &b->trees[trees[order[i]]];
-  }
+  std::vector<uint32_t> key;
+  if (sorted) PP2D_TRY(root_mode_keys(h, list, key));
+  std::vector<int> order(n);
+  for (uint32_t i = 0; i < n; ++i) order[i] = (int)i;
+  std::stable_sort(order.begin(), order.end(), [&](int x, int y) {
+    if (list[x]->goal != list[y]->goal) return list[x]->goal < list[y]->goal;
+    return sorted && key[x] < key[y];
+  });
+  for (uint32_t i = 0; i < n; ++i) list[i] = &b->trees[trees[order[i]]];
   PP2D_TRY(plan_trees(h, list, max_depth, max_iter, sorted));
   for (uint32_t i = 0; i < n; ++i) {
     const Tree& t = b->trees[trees[i]];

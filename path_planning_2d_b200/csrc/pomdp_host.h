@@ -138,8 +138,17 @@ struct pp2d_pomdp {
   int H = 0, W = 0, HW = 0, gx = 0, gy = 0;
   float gamma = 0.f;
   uint8_t* d_map = nullptr;
+  std::vector<uint8_t> map_host;           // [H][W] as given to pp2d_pomdp_create
+  // Goal set (DESIGN.md section 7e): goal 0 is (gx, gy), goals 1..n_goals come
+  // from pp2d_pomdp_set_goals.  Per-goal data is stored goal-major, goal 0
+  // first: d_sr [n_goals+1][HW][9], the bound matrices below.
+  int n_goals = 0;
+  std::vector<uint32_t> goal_xy;           // [n_goals+1][2]
+  std::vector<uint8_t> goal_alphas;        // [n_goals+1]: alpha vectors set
+  std::vector<uint8_t> goal_finite;        // [n_goals+1]: every bound finite
   float *d_tp = nullptr, *d_mp = nullptr, *d_sr = nullptr, *d_uniforms = nullptr;
-  // bound matrix [HW][ld]: FIB | PBVI (zero padded to whole column tiles)
+  // bound matrices [n_goals+1][HW][ld]: FIB | PBVI (zero padded to whole
+  // column tiles; zero for a goal without alpha vectors)
   float* d_alpha = nullptr;
   int ld = 0, ncol = 9, n_pbvi = 0;
   // Live cells (pomdp_dead_cells_kernel): the cells probability mass can enter.
@@ -149,22 +158,22 @@ struct pp2d_pomdp {
   // when every belief of the launch is +0 elsewhere (roots are checked on
   // upload, see Tree::dense in pomdp.cu).
   std::vector<uint8_t> dead;               // host copy of the mask
-  std::vector<float> alpha_host;           // dense bound matrix [HW][ld] as uploaded
+  std::vector<float> alpha_host;           // dense bound matrices [n_goals+1][HW][ld] as uploaded
   int* d_kidx = nullptr;
   int* d_kidx_all = nullptr;
   uint8_t* d_dead = nullptr;               // device copy of the mask
   int* d_kinv = nullptr;                   // cell -> its position in d_kidx, -1 for a dead cell
   float* d_mp_live = nullptr;              // rows d_kidx[0..K) of the likelihood table [K][16]
-  float* d_alpha_live = nullptr;
+  float* d_alpha_live = nullptr;           // [n_goals+1][K][ld]
   int K = 0;
   bool skip_dead = true;                   // PP2D_POMDP_DENSE=1 turns the skipping off
-  bool alphas_finite = true;               // every bound finite (else nothing is skipped)
+  bool alphas_finite = true;               // every bound of every goal finite (else nothing is skipped)
   // batched planner: per-tile inner rows of the values launches
   // (PP2D_POMDP_TILE_SUPPORT=0 off) and queries planned in the order of their
   // start beliefs' modes (PP2D_POMDP_SORT=0 off)
   bool tile_support = true, sort_queries = true;
-  std::vector<uint8_t> fib_actions, pbvi_actions;
-  bool have_alphas = false;
+  std::vector<uint8_t> fib_actions, pbvi_actions;   // goal 0's (pp2d_pomdp_evaluate)
+  bool have_alphas = false;                // goal 0's alpha vectors are set
   // belief pool [HW][cap]
   float* d_bel = nullptr;
   int cap = 0;
@@ -186,6 +195,9 @@ struct pp2d_pomdp {
   // per-tile lists
   uint64_t work_rows = 0;
   unsigned long long* d_work = nullptr;
+  // of which spent on the padding of goal segments (pp2d_pomdp_padding_counters):
+  // padded entries and their belief x inner-row products
+  uint64_t pad_entries = 0, pad_rows = 0;
   double t_phase[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // PP2D_POMDP_PROFILE=1: seconds per phase
 };
 

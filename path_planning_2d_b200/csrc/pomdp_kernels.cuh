@@ -624,6 +624,9 @@ pomdp_tile_order_kernel(int ntiles, const int* __restrict__ tcount, int* __restr
 
 // Grid: untiled (ceil(n / kEvM), column tiles); TILED (column tiles, ceil(n /
 // kEvM)) with the belief tile = torder[blockIdx.y].
+// Goals (DESIGN.md section 7e): every tile holds beliefs of one goal, and
+// alpha is the goal-major stack [goals][rows][ld] with gstride floats per goal;
+// the tile reads goal tile_goal[tile]'s matrix (tile_goal NULL: goal 0).
 template <bool TILED>
 __global__ void __launch_bounds__(256, 2)
 pomdp_values_kernel(int HW, const int* __restrict__ kidx, int cells, int ld, int ncol,
@@ -631,9 +634,11 @@ pomdp_values_kernel(int HW, const int* __restrict__ kidx, int cells, int ld, int
                     const float* __restrict__ bel,
                     const float* __restrict__ alpha, float* __restrict__ out,
                     const int2* __restrict__ tlist, const int* __restrict__ tcount,
-                    const int* __restrict__ torder, int tstride) {
+                    const int* __restrict__ torder, int tstride,
+                    const int* __restrict__ tile_goal, size_t gstride) {
   const int mtile = TILED ? torder[blockIdx.y] : (int)blockIdx.x;
   const int ntile = TILED ? (int)blockIdx.x : (int)blockIdx.y;
+  if (tile_goal) alpha += (size_t)tile_goal[mtile] * gstride;
   if constexpr (TILED) {
     // (HW is a by-value parameter: from here on it is this tile's row count)
     tlist += (size_t)mtile * tstride;
@@ -795,10 +800,12 @@ __device__ __forceinline__ void rewards_body(int K, const int* __restrict__ kidx
 
 // Stage 1 of an expansion round in ONE launch: the prefix sums of the expanded
 // nodes (blocks [0, ceil(n/4))) and their 9 reward dots (the blocks after
-// them) do not depend on each other.
+// them) do not depend on each other.  stage_reward is the goal-major stack
+// [goals][HW][9]; node i reads goal goals[i]'s table.
 __global__ void __launch_bounds__(128)
 pomdp_expand_kernel(int HW, int K, const int* __restrict__ kidx,
-                    const int* __restrict__ slots, int n, const float* __restrict__ bel,
+                    const int* __restrict__ slots, const int* __restrict__ goals, int n,
+                    const float* __restrict__ bel,
                     const float* __restrict__ stage_reward, float* __restrict__ prefix,
                     float* __restrict__ rewards) {
   __shared__ __align__(16) float sw[4][96];
@@ -812,8 +819,9 @@ pomdp_expand_kernel(int HW, int K, const int* __restrict__ kidx,
     const int w = (blockIdx.x - nbp) * 4 + warp;
     if (w >= n * 3) return;
     const int i = w / 3, a0 = (w % 3) * 3;
-    rewards_body(K, kidx, lane, bel + bel_off(HW, 0, slots[i]), stage_reward + a0,
-                 rewards + (size_t)i * 9 + a0, sw[warp]);
+    rewards_body(K, kidx, lane, bel + bel_off(HW, 0, slots[i]),
+                 stage_reward + (size_t)goals[i] * HW * 9 + a0, rewards + (size_t)i * 9 + a0,
+                 sw[warp]);
   }
 }
 

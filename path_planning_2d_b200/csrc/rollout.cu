@@ -330,14 +330,18 @@ int pp2d_sim_rollout_mdp_batch(pp2d_sim* s, pp2d_mdp_batch* planner, const uint3
   return rollout(s, views, n, starts_xy, beliefs, max_steps, seed, first_episode, out);
 }
 
+}  // extern "C"
+
+namespace {
 /* The loop of the MDP rollouts with the QV-tree as the planner (DESIGN.md
- * section 7d): one persistent tree per episode, planned and updated through a
- * tree batch, the world stepped on the host by the function the device
- * rollouts use. */
-int pp2d_sim_rollout_pomdp(pp2d_sim* s, pp2d_pomdp* planner, uint32_t n, const uint32_t* starts_xy,
-                           const float* beliefs, uint32_t max_steps, uint32_t max_depth,
-                           uint32_t max_iter, uint64_t seed, uint64_t first_episode,
-                           pp2d_rollout* out) {
+ * sections 7d, 7e): one persistent tree per episode, planned and updated
+ * through a tree batch, the world stepped on the host by the function the
+ * device rollouts use.  Episode i plans to goal goals[i] of the planner's goal
+ * set (NULL: goal 0) and stops on that goal's cell. */
+int rollout_pomdp(pp2d_sim* s, pp2d_pomdp* planner, const uint32_t* goals, uint32_t n,
+                  const uint32_t* starts_xy, const float* beliefs, uint32_t max_steps,
+                  uint32_t max_depth, uint32_t max_iter, uint64_t seed, uint64_t first_episode,
+                  pp2d_rollout* out, const char* fn) {
   if (!planner) return fail(PP2D_ERR_INVALID, "NULL planner");
   PlannerView v;
   v.H = (uint32_t)planner->H; v.W = (uint32_t)planner->W;
@@ -345,12 +349,25 @@ int pp2d_sim_rollout_pomdp(pp2d_sim* s, pp2d_pomdp* planner, uint32_t n, const u
   PP2D_TRY(check_common(s, v, n, starts_xy));
   // (every step updates the tree that planned it: its root must be expanded)
   if (max_depth == 0 || max_iter == 0)
-    return fail(PP2D_ERR_INVALID, "pp2d_sim_rollout_pomdp: max_depth and max_iter must be > 0");
-  if (!planner->have_alphas) return fail(PP2D_ERR_STATE, "pp2d_pomdp_set_alphas not called");
+    return fail(PP2D_ERR_INVALID, "%s: max_depth and max_iter must be > 0", fn);
+  if (!goals && !planner->have_alphas)
+    return fail(PP2D_ERR_STATE, "pp2d_pomdp_set_alphas not called");
+  for (uint32_t i = 0; goals && i < n; ++i) {
+    if (goals[i] > (uint32_t)planner->n_goals)
+      return fail(PP2D_ERR_INVALID, "%s: episode %u names goal %u of a set of %d", fn, i,
+                  goals[i], planner->n_goals + 1);
+    if (!planner->goal_alphas[goals[i]])
+      return fail(PP2D_ERR_STATE, "%s: episode %u: goal %u has no alpha vectors", fn, i, goals[i]);
+  }
   if (n == 0) return PP2D_OK;
   const SimView sv = sim_view(s);
   const size_t hw = (size_t)sv.H * sv.W;
-  const uint32_t goal = v.gy * sv.W + v.gx;
+  // the goal cell of every episode, from the host copy of the goal set
+  std::vector<uint32_t> goal(n);
+  for (uint32_t i = 0; i < n; ++i) {
+    const uint32_t g = goals ? goals[i] : 0;
+    goal[i] = planner->goal_xy[2 * (size_t)g + 1] * sv.W + planner->goal_xy[2 * (size_t)g];
+  }
   std::vector<float> point;
   if (!beliefs) {
     point.assign(n * hw, 0.0f);
@@ -358,7 +375,7 @@ int pp2d_sim_rollout_pomdp(pp2d_sim* s, pp2d_pomdp* planner, uint32_t n, const u
       point[i * hw + starts_xy[2 * (size_t)i + 1] * sv.W + starts_xy[2 * (size_t)i]] = 1.0f;
   }
   pp2d_tree_batch* tb = nullptr;
-  PP2D_TRY(pp2d_tree_batch_create(planner, beliefs ? beliefs : point.data(), n, &tb));
+  PP2D_TRY(pp2d_tree_batch_create_goals(planner, beliefs ? beliefs : point.data(), goals, n, &tb));
   struct Guard { pp2d_tree_batch* b; ~Guard() { pp2d_tree_batch_destroy(b); } } guard{tb};
   std::vector<uint32_t> cell(n), steps(n, 0), coll(n, 0), live(n);
   std::vector<uint8_t> act(n), meas(n);
@@ -369,7 +386,7 @@ int pp2d_sim_rollout_pomdp(pp2d_sim* s, pp2d_pomdp* planner, uint32_t n, const u
   for (uint32_t t = 0;; ++t) {
     uint32_t nl = 0;                             // episodes that take step t
     for (uint32_t i = 0; i < n; ++i)
-      if (steps[i] == t && cell[i] != goal && t < max_steps) live[nl++] = i;
+      if (steps[i] == t && cell[i] != goal[i] && t < max_steps) live[nl++] = i;
     if (nl == 0) break;
     PP2D_TRY(pp2d_tree_batch_plan(tb, live.data(), nl, max_depth, max_iter, act.data(), nullptr,
                                   nullptr));
@@ -391,11 +408,31 @@ int pp2d_sim_rollout_pomdp(pp2d_sim* s, pp2d_pomdp* planner, uint32_t n, const u
   if (out->final_belief) PP2D_TRY(tree_batch_root_beliefs(tb, out->final_belief));
   for (uint32_t i = 0; i < n; ++i) {
     if (out->steps) out->steps[i] = steps[i];
-    if (out->reached) out->reached[i] = cell[i] == goal ? 1 : 0;
+    if (out->reached) out->reached[i] = cell[i] == goal[i] ? 1 : 0;
     if (out->collisions) out->collisions[i] = coll[i];
     if (out->final_cell) out->final_cell[i] = cell[i];
   }
   return PP2D_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int pp2d_sim_rollout_pomdp(pp2d_sim* s, pp2d_pomdp* planner, uint32_t n, const uint32_t* starts_xy,
+                           const float* beliefs, uint32_t max_steps, uint32_t max_depth,
+                           uint32_t max_iter, uint64_t seed, uint64_t first_episode,
+                           pp2d_rollout* out) {
+  return rollout_pomdp(s, planner, nullptr, n, starts_xy, beliefs, max_steps, max_depth, max_iter,
+                       seed, first_episode, out, "pp2d_sim_rollout_pomdp");
+}
+
+int pp2d_sim_rollout_pomdp_goals(pp2d_sim* s, pp2d_pomdp* planner, const uint32_t* goals,
+                                 uint32_t n, const uint32_t* starts_xy, const float* beliefs,
+                                 uint32_t max_steps, uint32_t max_depth, uint32_t max_iter,
+                                 uint64_t seed, uint64_t first_episode, pp2d_rollout* out) {
+  if (n > 0 && !goals) return fail(PP2D_ERR_INVALID, "NULL goals");
+  return rollout_pomdp(s, planner, goals, n, starts_xy, beliefs, max_steps, max_depth, max_iter,
+                       seed, first_episode, out, "pp2d_sim_rollout_pomdp_goals");
 }
 
 }  // extern "C"

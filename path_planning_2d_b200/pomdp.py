@@ -76,13 +76,27 @@ class SearchTree:
         return out
 
 
+def _goal_indices(goals, n, what):
+    """Goal indices as uint32 [n]; negative or non-integer entries are refused
+    here (the library checks the upper end)."""
+    g = np.asarray(goals)
+    if g.ndim != 1 or g.size != n:
+        raise ValueError(f"one goal index per {what} ({n}), got shape {g.shape}")
+    if g.size and (not np.issubdtype(g.dtype, np.integer) or g.min() < 0):
+        raise ValueError("goal indices must be integers >= 0")
+    return np.ascontiguousarray(g, dtype=np.uint32)
+
+
 class SearchTreeBatch:
     """Many SearchTrees on the GPU belief pool of one PomdpPathPlanning2d that
     live across belief callbacks (one per robot of a fleet), updated and
     planned together (pp2d_tree_batch_* in include/pp2d.h).  Tree k behaves
-    bit for bit like SearchTree(planner, beliefs[k]) fed the same calls."""
+    bit for bit like SearchTree(planner, beliefs[k]) fed the same calls.
+    goals (optional, one per tree): tree k plans to goal goals[k] of the
+    planner's goal set (set_goals), bit for bit like a SearchTree on a planner
+    created with that goal."""
 
-    def __init__(self, planner, beliefs):
+    def __init__(self, planner, beliefs, goals=None):
         self._lib = planner._lib
         self._planner = planner
         hw = planner.map_height * planner.map_width
@@ -92,8 +106,13 @@ class SearchTreeBatch:
         b = b.reshape(-1, hw)
         self.count = b.shape[0]
         self._b = ctypes.c_void_p()
-        _lib.check(self._lib.pp2d_tree_batch_create(planner._h, b.ctypes.data, self.count,
-                                                    ctypes.byref(self._b)))
+        if goals is None:
+            _lib.check(self._lib.pp2d_tree_batch_create(planner._h, b.ctypes.data, self.count,
+                                                        ctypes.byref(self._b)))
+            return
+        g = _goal_indices(goals, self.count, "tree")
+        _lib.check(self._lib.pp2d_tree_batch_create_goals(planner._h, b.ctypes.data, g.ctypes.data,
+                                                          self.count, ctypes.byref(self._b)))
 
     def close(self):
         if getattr(self, "_b", None) is not None and self._b.value:
@@ -300,6 +319,66 @@ class PomdpPathPlanning2d:
         _lib.check(self._lib.pp2d_pomdp_set_alphas(
             self._h, fa.ctypes.data, fac.ctypes.data if fac is not None else None,
             pa.ctypes.data, pac.ctypes.data if pac is not None else None, pa.shape[0]))
+
+    # -- goal sets (include/pp2d.h, DESIGN.md section 7e) -----------------------
+    def set_goals(self, goals, stage_rewards=None):
+        """Goals 1..n of this handle's goal set = goals [n][2] (x, y); goal 0
+        stays the goal it was created with.  stage_rewards [n][HW][9]: the
+        goals' reward tables as given (e.g. read back from checkpoint files);
+        None: generated by the model rule."""
+        n = self.map_height * self.map_width
+        g = np.asarray(goals)
+        if g.size == 0:
+            g = np.zeros((0, 2), np.int64)
+        if g.ndim != 2 or g.shape[1] != 2:
+            raise ValueError("goals must be [n][2] = (x, y)")
+        if not np.issubdtype(g.dtype, np.integer) or (g.size and g.min() < 0):
+            raise ValueError("goal coordinates must be integers >= 0")
+        g = np.ascontiguousarray(g, dtype=np.uint32)
+        sr = None
+        if stage_rewards is not None:
+            sr = np.ascontiguousarray(stage_rewards, dtype=np.float32)
+            if sr.size != g.shape[0] * n * 9:
+                raise ValueError(f"stage_rewards must be [{g.shape[0]}][{n}][9]")
+        _lib.check(self._lib.pp2d_pomdp_set_goals(self._h, g.ctypes.data if g.size else None,
+                                                  g.shape[0],
+                                                  sr.ctypes.data if sr is not None else None))
+
+    def goals(self):
+        """The goal set as [count][2] (x, y), goal 0 first."""
+        c = ctypes.c_uint32()
+        _lib.check(self._lib.pp2d_pomdp_goals(self._h, ctypes.byref(c), None))
+        out = np.zeros((c.value, 2), np.uint32)
+        _lib.check(self._lib.pp2d_pomdp_goals(self._h, ctypes.byref(c), out.ctypes.data))
+        return out
+
+    def goal_reward(self, g):
+        """Goal g's stage reward table [HW][9]."""
+        out = np.empty((self.map_height * self.map_width, 9), np.float32)
+        _lib.check(self._lib.pp2d_pomdp_goal_reward(self._h, g, out.ctypes.data))
+        return out
+
+    def set_goal_alphas(self, g, fib_alphas, pbvi_alphas, fib_actions=None, pbvi_actions=None):
+        """set_alphas for goal g of the goal set (g = 0: set_alphas)."""
+        if not isinstance(g, (int, np.integer)) or g < 0:
+            raise ValueError("goal index must be an integer >= 0")
+        fa = np.ascontiguousarray(fib_alphas, dtype=np.float32)
+        pa = np.ascontiguousarray(pbvi_alphas, dtype=np.float32)
+        n = self.map_height * self.map_width
+        if fa.shape != (n, 9) or pa.ndim != 2 or pa.shape[1] != n:
+            raise ValueError("fib_alphas must be [HW][9], pbvi_alphas [N][HW]")
+        fac = np.ascontiguousarray(fib_actions, np.uint8) if fib_actions is not None else None
+        pac = np.ascontiguousarray(pbvi_actions, np.uint8) if pbvi_actions is not None else None
+        _lib.check(self._lib.pp2d_pomdp_set_goal_alphas(
+            self._h, int(g), fa.ctypes.data, fac.ctypes.data if fac is not None else None,
+            pa.ctypes.data, pac.ctypes.data if pac is not None else None, pa.shape[0]))
+
+    def padding_counters(self):
+        """(padded entries, their belief x inner-row products): the part of
+        work_counters()[2] spent on padding goal segments to whole tiles."""
+        out = np.zeros(2, np.uint64)
+        _lib.check(self._lib.pp2d_pomdp_padding_counters(self._h, out.ctypes.data))
+        return int(out[0]), int(out[1])
 
     # -- batched primitives ---------------------------------------------------
     def bayes_update(self, beliefs, actions, observations, normalize=False):

@@ -17,7 +17,7 @@ import numpy as np
 
 from . import _lib
 from .mdp import MdpBatchPathPlanning2d, MdpPathPlanning2d
-from .pomdp import PomdpPathPlanning2d
+from .pomdp import PomdpPathPlanning2d, _goal_indices
 
 
 class DummySimulator:
@@ -74,13 +74,14 @@ class DummySimulator:
         return b
 
     def rollout(self, planner, starts, max_steps, seed, beliefs=None, instances=None,
-                first_episode=0, record=False, max_depth=None, max_iter=None):
+                first_episode=0, record=False, max_depth=None, max_iter=None, goals=None):
         """Closed-loop episodes of `planner` (MdpPathPlanning2d, or
         MdpBatchPathPlanning2d with `instances`: the instance each episode
         follows, or PomdpPathPlanning2d: one search tree per episode, planned
         with max_depth / max_iter, default the planner's 50 / 15, and updated
         with each action and measurement; final_belief is then the tree's
-        root belief) in this simulator's map, from starts [n][2] = (x, y), with
+        root belief; with `goals`, episode i plans to goal goals[i] of the
+        planner's goal set and stops on that goal's cell) in this simulator's map, from starts [n][2] = (x, y), with
         beliefs [n][H*W] (default: a point mass at each start).  Episode i
         draws its noise as episode first_episode + i of `seed`.  Returns a dict
         of steps, reached, collisions and final_cell (y*W+x) per episode; with
@@ -105,14 +106,22 @@ class DummySimulator:
         bp = b.ctypes.data if b is not None else None
         if not isinstance(planner, PomdpPathPlanning2d) and (max_depth, max_iter) != (None, None):
             raise ValueError("max_depth / max_iter are for a PomdpPathPlanning2d")
+        if not isinstance(planner, PomdpPathPlanning2d) and goals is not None:
+            raise ValueError("`goals` is for a PomdpPathPlanning2d")
         if isinstance(planner, PomdpPathPlanning2d):
             if instances is not None:
                 raise ValueError("`instances` is for a batch planner")
-            rc = self._lib.pp2d_sim_rollout_pomdp(
-                self._h, planner._h, n, st.ctypes.data, bp, max_steps,
-                planner.max_search_tree_depth if max_depth is None else max_depth,
-                planner.max_online_iteration if max_iter is None else max_iter,
-                seed, first_episode, ctypes.byref(out))
+            depth = planner.max_search_tree_depth if max_depth is None else max_depth
+            it = planner.max_online_iteration if max_iter is None else max_iter
+            if goals is None:
+                rc = self._lib.pp2d_sim_rollout_pomdp(self._h, planner._h, n, st.ctypes.data, bp,
+                                                      max_steps, depth, it, seed, first_episode,
+                                                      ctypes.byref(out))
+            else:
+                g = _goal_indices(goals, n, "episode")
+                rc = self._lib.pp2d_sim_rollout_pomdp_goals(
+                    self._h, planner._h, g.ctypes.data, n, st.ctypes.data, bp, max_steps, depth,
+                    it, seed, first_episode, ctypes.byref(out))
         elif isinstance(planner, MdpBatchPathPlanning2d):
             if instances is None:
                 raise ValueError("a batch planner needs `instances`, one per episode")
